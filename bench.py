@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the batched whole-body QP control step (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (dynamics + ID-QP: the reduce kernel and the solve kernel, stream ordered; a 4096-65536
 instance batch goes through as 2-4 chunks of that pair on as many streams, forked from and joined to the launch stream, so
@@ -17,6 +17,8 @@ D2H inside the timed region); roofline / cpu_baseline as the contract asks; late
 robot through the LeafSystem mirror (the reference's operating point: one step per 5 ms, simulate.py:20-22).
 `--impl reference` times the CPU restatement of the reference path (oracle/, C port) on the host cores instead - pydrake /
 OSQP themselves are not installable (DESIGN.md 5); `import pydrake` is probed at start and reported either way.
+`--dump-outputs DIR` writes the outputs of the last timed step as DIR/<name>.npy; with N > 1 these are rank 0's shard only,
+so two builds are compared on that shard.
 """
 from __future__ import annotations
 
@@ -66,6 +68,29 @@ def flop_model():
     of this kernel build (tools/ncu_flops.py -> profiles/r2_flop_model.json); the file names the captures and the commit."""
     p = ROOT / "profiles" / "r2_flop_model.json"
     return json.loads(p.read_text()) if p.exists() else None
+
+
+DUMP_MAX_ROWS = 1 << 18             # 5 float64 files of 22 columns in all: 176 B a row, 46 MB at this cap
+
+
+def dump_rows(n):
+    """Instances written by --dump-outputs: the whole batch, or above DUMP_MAX_ROWS a fixed seeded sample (sorted)."""
+    if n <= DUMP_MAX_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(SEED).choice(n, DUMP_MAX_ROWS, replace=False))
+
+
+def dump_outputs(out_dir, n, outputs):
+    """Writes the device outputs of the last timed step as out_dir/<name>.npy (float64; status codes and the row indices
+    in rows.npy are exact in float64), so that two builds run with the same arguments can be compared output for output."""
+    import torch
+    rows = dump_rows(n)
+    idx = torch.from_numpy(rows).to(next(iter(outputs.values())).device)
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "rows.npy", rows.astype(np.float64))
+    for name, t in outputs.items():
+        np.save(d / f"{name}.npy", t.index_select(0, idx).cpu().numpy().astype(np.float64))
 
 
 class ClockSampler:
@@ -346,6 +371,8 @@ def run_gpu(args):
         e1.record(stream)
     torch.cuda.synchronize()
     sampler.timed = False
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, {"tau": tau, "metrics": met, "status": st, "qp_info": qi})
     if world > 1:
         dist.barrier()
     gpu_launches = ctl.launches - launches0
@@ -549,13 +576,20 @@ def main():
     ap.add_argument("--torque-limits", action="store_true", help="experiments only: |tau| <= effort rows (BASELINE configs[2])")
     ap.add_argument("--workload", default="step", choices=["step", "wire", "traj", "rollout"],
                     help="step = the BASELINE metric (default); wire / traj / rollout = the rows next to it (tools/bench_aux.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write what the last one computed (tau, metrics, "
+                    "status, qp_info of rank 0's batch, or a fixed seeded sample of at most %d instances, listed in rows.npy) "
+                    "as DIR/<name>.npy, e.g. DIR = bench_outputs/" % DUMP_MAX_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "step"):
+        ap.error("--dump-outputs writes the outputs of the GPU control step (--impl ours --workload step)")
     if args.workload != "step":
         import __graft_entry__ as g
         g.build()
         sys.path.insert(0, str(ROOT / "tools"))
         import bench_aux
-        bench_aux.run(args.workload, steps=min(args.steps, 50), warmup=args.warmup)
+        bench_aux.run(args.workload, steps=args.steps, warmup=args.warmup)
         return
     if args.impl == "reference":
         run_reference(args)

@@ -142,6 +142,24 @@ def test_anymal_frozen_table():
     assert sum(l["mass"] for l in d["links"]) == pytest.approx(30.4214, abs=5e-5)
 
 
+def test_frozen_actuation_order_frames_and_mirroring():
+    """SURVEY A.5: actuator order = <transmission> order, legs LF/fl, RF/fr, LH/hl, RH/hr x (abduction, hip, knee);
+    SURVEY 7: every joint rpy is zero in both URDFs; Appendix B: anymal products of inertia are mirrored per leg."""
+    mc = json.loads((ROBOTS / "mini_cheetah.json").read_text())
+    by_child = {j["child"]: j["name"] for j in mc["joints"]}
+    assert mc["actuated_joints"] == [by_child[f"{part}_{leg}"] for leg in MC_LEGS for part in ("abduct", "thigh", "shank")]
+    an = json.loads((ROBOTS / "anymal_b.json").read_text())
+    assert an["actuated_joints"] == [f"{leg}_{j}" for leg in ("LF", "RF", "LH", "RH") for j in ("HAA", "HFE", "KFE")]
+    for d in (mc, an):
+        assert all(j["rpy"] == [0.0, 0.0, 0.0] for j in d["joints"])
+    L = {l["name"]: l for l in an["links"]}
+    for leg, (sx, sy) in {"LF": (1, 1), "RF": (1, -1), "LH": (-1, 1), "RH": (-1, -1)}.items():
+        for part in ("HIP", "THIGH", "SHANK"):
+            # S I S with S = diag(sx, sy, 1): diagonal kept, Ixy x sx sy, Ixz x sx, Iyz x sy
+            lf = np.array(L[f"LF_{part}"]["inertia_com"])
+            assert np.array_equal(L[f"{leg}_{part}"]["inertia_com"], lf * np.array([1, 1, 1, sx * sy, sx, sy]))
+
+
 @pytest.mark.parametrize("robot,total", [("mini_cheetah", 8.252), ("anymal_b", 30.4214)])
 def test_flattened_model_conserves_mass_moments(robot, total):
     """Welding (anymal: base_inertia into base, adapter into shank) conserves mass, first and second moments: the
