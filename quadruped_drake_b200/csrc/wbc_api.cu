@@ -4,6 +4,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <string>
 
 // named barrier `id` over `threads` threads of the CTA (a multiple of 32; skipped when at most one warp takes part)
@@ -370,9 +371,6 @@ struct wbc_handle {
   int* ro_counter = nullptr;
   // hand-over records of the split step (reduce -> solve), one slot per internal stream lane
   cudaEvent_t prof_ev[3] = {nullptr, nullptr, nullptr};   // wbc_profile_step: before reduce / between / after solve
-  bool prof_on = false;
-  bool side_by_side = false;                              // set while a step is issued as several concurrent chains
-  bool host_mapped = false;                               // set around the zero-copy launches of wbc_step_host
   // per-slot ordering of the scratch users: the stream of the last step that used the slot and an event to chain a new one
   cudaStream_t last_stream[WBC_NSLOT] = {};
   bool slot_used[WBC_NSLOT] = {};
@@ -380,7 +378,7 @@ struct wbc_handle {
   double* d_rec[WBC_NSLOT] = {};
   double* d_vdmap[WBC_NSLOT] = {};
   int64_t rec_cap[WBC_NSLOT] = {}, vdmap_cap[WBC_NSLOT] = {};
-  cudaStream_t xstream[WBC_NSLOT] = {};                  // lanes 2.. of a step issued as more than two chunks (created on demand)
+  cudaStream_t xstream[WBC_NSLOT] = {};                  // lanes 2.. of a step issued as more than two chunks
 };
 
 #define WBC_CUDA(h, call)                                                                       \
@@ -536,8 +534,7 @@ extern "C" int wbc_coriolis(wbc_handle* h, int64_t n, const double* q, const dou
 namespace {
 // Scratch device buffers of the host-buffer debug / codec entries: freed when the scope ends (early error returns included).
 struct DevScratch {
-  void* p[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // at most 8 buffers per scratch
-  int used = 0;
+  std::vector<void*> p;
   cudaError_t err = cudaSuccess;
   template <typename T> T* in(const T* host, size_t count, cudaStream_t st) {      // NULL stays NULL
     if (!host || err != cudaSuccess) return nullptr;
@@ -550,13 +547,13 @@ struct DevScratch {
     void* d = nullptr;
     err = cudaMalloc(&d, count * sizeof(T) > 0 ? count * sizeof(T) : 1);
     if (err != cudaSuccess) return nullptr;
-    p[used++] = d;
+    p.push_back(d);
     return static_cast<T*>(d);
   }
   template <typename T> void back(T* host, const T* dev, size_t count, cudaStream_t st) {
     if (host && dev && err == cudaSuccess) err = cudaMemcpyAsync(host, dev, count * sizeof(T), cudaMemcpyDeviceToHost, st);
   }
-  ~DevScratch() { for (int i = 0; i < used; ++i) cudaFree(p[i]); }
+  ~DevScratch() { for (void* d : p) cudaFree(d); }
 };
 }  // namespace
 
@@ -616,37 +613,132 @@ static int ensure_split_scratch(wbc_handle* h, int slot, int64_t n, bool with_vd
   return WBC_OK;
 }
 
-static wbc::StepArgs offset_args(const wbc_io* io, int64_t o, int64_t m, int kind) {
-  return wbc::StepArgs{io->q + o * WBC_NQ, io->v + o * WBC_NV, io->traj + o * WBC_NTRAJ, io->contact + o * 4, io->tau + o * WBC_NU,
-                       io->metrics + o * WBC_NMETRIC, io->status + o, io->vd ? io->vd + o * WBC_NV : nullptr,
-                       io->f ? io->f + o * 12 : nullptr, io->qp_info ? io->qp_info + o * 4 : nullptr,
-                       io->lam ? io->lam + o * WBC_NLAM : nullptr, (long long)m, kind};
+// ------------------------------------------------------------------------------ launch schedule
+// Which kernels a step entry point issues, by batch size. The thresholds were measured on B200 (profiles/README.md); an
+// experiment with them is a local edit built as a variant (tools/sweep_variants.sh).
+
+// Programmatic dependent launch of the solve kernel (its CTAs become resident while the last reduce CTAs run): +1.5 % at 4096
+// instances, neutral above; never inside a stream capture, and not for chains below 4096 instances that run beside other
+// chains of the same step (chunked issue): there the early-resident solve CTAs take the slots the other chunk's reduce CTAs
+// need (-22 % at 2 x 2048). A lone chain gains at every size (+3-4 % at 64 - 1024).
+static bool use_pdl(int64_t m, bool beside_others) { return !beside_others || m >= 4096; }
+
+// wbc_step: small batches go through as chunks of about 2048 instances, independent reduce -> solve chains on as many streams
+// (the caller's and internal ones, joined by events): the solve kernel of one chunk overlaps the reduce kernel and the
+// ramp-down of the others. Measured against one chain: +5.5 % at 4096 instances (2 chunks; 3: +4.5 %, 4: +2.5 %), +7.7 % at
+// 8192 (4 chunks; 2: +4.1 %), +2.6 % at 16384, +1 % at 65536, -2 % at 2048. Never inside a stream capture.
+constexpr int64_t CHUNKED_STEP_MIN = 4096, CHUNKED_STEP_MAX = 65536;
+constexpr int device_step_chunks(int64_t n) { return n >= 7168 ? 4 : n >= 5120 ? 3 : 2; }
+static_assert(device_step_chunks(CHUNKED_STEP_MAX) <= WBC_NSLOT, "every chunk needs its own stream and hand-over slot");
+
+// wbc_step_host on page-locked buffers: reading the inputs over the host link from the SMs (zero-copy, ~32 GB/s) wins up to
+// ~48 k instances per call (no staging copies, no extra API calls); above that the inputs go through the copy engine
+// (~55 GB/s) in a chunked two-stream pipeline. Page-locked outputs are written straight to host memory in both modes.
+//  * below 24576 instances the reduce kernel reads its inputs over the host link (zero-copy), two halves from 4096 on:
+//    the solve kernel of one half overlaps the link-bound reduce kernel of the other (e2e +4.6 % at 4096, +3.8 % at
+//    16384; three or more chunks lose);
+//  * above, the inputs go through the copy engine into device staging and the single-warp reduce CTAs read resident
+//    inputs: e2e +5 % at 32768, +16 % at 65536, +10 % at 2^17 - 2^20.
+// PC / MPTC are compute bound at a third of the rate: the zero-copy reads hide under the reduce kernel up to 131072
+// instances (e2e 22.3 M steps/s against 20.0 M staged at 65536)
+static bool stage_pinned_inputs(int kind, int64_t n) { return n >= (kind == WBC_CTRL_PC || kind == WBC_CTRL_MPTC ? 131072 : 24576); }
+// staged: four chunks below 98304 instances, then chunks of n / 8 clamped to [16384, 32768] instances
+static int pinned_chunks(int64_t n, bool staged) {
+  if (!staged) return n >= 4096 ? 2 : 1;
+  if (n < 98304) return 4;
+  const int64_t per = std::clamp<int64_t>(n / 8, 16384, 32768);
+  return (int)((n + per - 1) / per);
 }
 
-static int pdl_mode() {   // WBC_PDL=0: ordinary launch of the solve kernel (A/B comparisons)
-  static int mode = -1;
-  if (mode < 0) { const char* e = getenv("WBC_PDL"); mode = e ? atoi(e) : 1; }
-  return mode;
+// wbc_step_host on pageable buffers: chunked two-stream pipeline, the upload of chunk c + 1 overlaps the kernel of chunk c,
+// the download of chunk c the kernel of chunk c + 1 (separate copy engines); small batches go through in one piece.
+// chunk = n / 8 clamped to [8192, 65536] instances: short pipeline fill, copies long enough for the copy engines
+static int pageable_chunks(int64_t n) {
+  if (n < 32768) return n >= 2048 ? 2 : 1;
+  const int64_t per = std::clamp<int64_t>(n / 8, 8192, 65536);
+  return (int)std::min<int64_t>((n + per - 1) / per, 64);
 }
+
+// wbc_sample_trajectory, instances per warp: 32 (lane = instance) is the throughput shape; small batches are latency bound on
+// the 14 dependent binary searches per instance, so they spread them over 4 or 16 lanes per instance (rollout of 4096 robots:
+// 45.2 / 48.7 / 49.7 M robot-steps/s with 32 / 8 / 2)
+static int sample_ipw(int64_t n) { return n >= 32768 ? 32 : n >= 8192 ? 8 : 2; }
+
+// ------------------------------------------------------------------------------ step issue
+// How the chains of one step are issued; the entry point decides, launch_split follows.
+struct Issue {
+  bool host_mapped = false;     // the reduce kernel reads page-locked host memory: 4-warp CTAs, every array staged per CTA
+  bool beside_others = false;   // the chain runs beside other chains of the same step (chunked issue)
+  bool profile = false;         // wbc_profile_step: events before the reduce kernel, between the kernels, after the solve kernel
+};
+
+// The instances from `o` on of every array of `io`; optional (null) arrays stay null.
+static wbc_io io_at(const wbc_io& io, int64_t o) {
+  auto at = [o](auto* p, int width) { return p ? p + o * width : nullptr; };
+  return wbc_io{at(io.q, WBC_NQ), at(io.v, WBC_NV), at(io.traj, WBC_NTRAJ), at(io.contact, 4), at(io.tau, WBC_NU),
+                at(io.metrics, WBC_NMETRIC), at(io.status, 1), at(io.vd, WBC_NV), at(io.f, 12), at(io.qp_info, 4), at(io.lam, WBC_NLAM)};
+}
+static wbc::StepArgs step_args(const wbc_io& io, int64_t m, int kind) {
+  return wbc::StepArgs{io.q, io.v, io.traj, io.contact, io.tau, io.metrics, io.status, io.vd, io.f, io.qp_info, io.lam, (long long)m, kind};
+}
+
+// Splits [0, n) into k chunks of a multiple of 4 instances, the last one shorter, and calls f(c, offset, count) for each
+// non-empty one; stops at the first error f returns. The rounding keeps the CTA-level bulk copies of 4-warp reduce CTAs
+// on 16-byte boundaries.
+template <typename F>
+static int for_each_chunk(int64_t n, int k, F f) {
+  const int64_t per = ((n + k - 1) / k + 3) & ~(int64_t)3;
+  for (int c = 0; c < k && c * per < n; ++c) {
+    const int rc = f(c, c * per, std::min(per, n - c * per));
+    if (rc) return rc;
+  }
+  return WBC_OK;
+}
+
+// Device aliases of page-locked host buffers (wbc_host_alloc / cudaHostRegister): when every non-null pointer is page-locked,
+// replaces each by the address the kernels read and write it through and returns true; otherwise changes nothing and
+// returns false.
+template <typename... T>
+static bool to_device_aliases(T*&... p) {
+  const void* host[] = {p...};
+  void* dev[sizeof...(T)] = {};
+  for (size_t i = 0; i < sizeof...(T); ++i) {
+    if (!host[i]) continue;
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, host[i]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) {
+      cudaGetLastError();
+      return false;
+    }
+    dev[i] = at.devicePointer;
+  }
+  size_t i = 0;
+  ((p = static_cast<T*>(dev[i++])), ...);
+  return true;
+}
+
+// Streams to[0 .. k) wait for everything submitted to `from` so far: the fork of chunk streams from the caller's stream and
+// the join of a chunk stream back into it, through an event of the handle (created with it, so never inside a capture).
+static int streams_wait(wbc_handle* h, cudaEvent_t ev, cudaStream_t from, const cudaStream_t* to, int k) {
+  WBC_CUDA(h, cudaEventRecord(ev, from));
+  for (int i = 0; i < k; ++i) WBC_CUDA(h, cudaStreamWaitEvent(to[i], ev, 0));
+  return WBC_OK;
+}
+
+static bool capturing(cudaStream_t st) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  cudaStreamIsCapturing(st, &cap);
+  return cap != cudaStreamCaptureStatusNone;
+}
+
 static bool aligned16p(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-static int bulk_in_mode() {   // WBC_BULK_IN=0: per-lane input loads everywhere (A/B comparisons)
-  static int mode = -1;
-  if (mode < 0) { const char* e = getenv("WBC_BULK_IN"); mode = e ? atoi(e) : 1; }
-  return mode;
-}
 
 // The hand-over scratch of a slot belongs to one step at a time. A step on another stream than the slot's previous user is
 // ordered behind everything submitted to that stream so far (event dependency; never inside a stream capture, where the
 // caller owns the ordering).
 static int order_slot(wbc_handle* h, int slot, cudaStream_t st) {
-  if (h->slot_used[slot] && h->last_stream[slot] != st) {
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    cudaStreamIsCapturing(st, &cap);
-    if (cap == cudaStreamCaptureStatusNone) {
-      if (!h->order_ev) WBC_CUDA(h, cudaEventCreateWithFlags(&h->order_ev, cudaEventDisableTiming));
-      if (cudaEventRecord(h->order_ev, h->last_stream[slot]) == cudaSuccess) WBC_CUDA(h, cudaStreamWaitEvent(st, h->order_ev, 0));
-      else cudaGetLastError();      // the previous stream no longer exists: its work has completed
-    }
+  if (h->slot_used[slot] && h->last_stream[slot] != st && !capturing(st)) {
+    if (cudaEventRecord(h->order_ev, h->last_stream[slot]) == cudaSuccess) WBC_CUDA(h, cudaStreamWaitEvent(st, h->order_ev, 0));
+    else cudaGetLastError();      // the previous stream no longer exists: its work has completed
   }
   h->slot_used[slot] = true;
   h->last_stream[slot] = st;
@@ -654,54 +746,47 @@ static int order_slot(wbc_handle* h, int slot, cudaStream_t st) {
 }
 
 template <int KIND>
-static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cudaStream_t st, int slot) {
-  int rc = ensure_split_scratch(h, slot, n, io->vd != nullptr);
+static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is) {
+  int rc = ensure_split_scratch(h, slot, n, io.vd != nullptr);
   if (rc) return rc;
   rc = order_slot(h, slot, st);
   if (rc) return rc;
-  double* vdmap = io->vd ? h->d_vdmap[slot] : nullptr;
+  double* vdmap = io.vd ? h->d_vdmap[slot] : nullptr;
   for (int64_t o = 0; o < n; o += SPLIT_CHUNK) {
     const int64_t m = (n - o) < SPLIT_CHUNK ? (n - o) : SPLIT_CHUNK;
-    const wbc::StepArgs a = offset_args(io, o, m, kind);
+    const wbc::StepArgs a = step_args(io_at(io, o), m, kind);
     // bulk input staging needs 16-byte aligned rows at the CTA boundaries (chunk offsets are multiples of 4)
     const bool al_vt = aligned16p(a.v) && aligned16p(a.traj), al_qc = aligned16p(a.q) && aligned16p(a.contact);
-    if (h->prof_on) cudaEventRecord(h->prof_ev[0], st);
-    if (h->host_mapped || KIND == WBC_CTRL_PC) {   // zero-copy call of wbc_step_host: 4-warp CTAs, every array staged per CTA
+    if (is.profile) cudaEventRecord(h->prof_ev[0], st);
+    if (is.host_mapped || KIND == WBC_CTRL_PC) {   // zero-copy call of wbc_step_host: 4-warp CTAs, every array staged per CTA
                                                    // (PC / MPTC too: 20.0 vs 19.7 M steps/s with single-warp CTAs)
       constexpr int W = (KIND == WBC_CTRL_PC) ? WARPS_PC : WARPS_HOST;
       const unsigned grid = (unsigned)((m + W - 1) / W);
-      const int bulk_ok = bulk_in_mode() && al_vt && al_qc;
+      const int bulk_ok = al_vt && al_qc;
       if constexpr (KIND == WBC_CTRL_PC) wbc_reduce_pc_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
       else wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
     } else {
       constexpr int W = WARPS;
       const unsigned grid = (unsigned)((m + W - 1) / W);
-      const int bulk_ok = bulk_in_mode() && al_vt;
+      const int bulk_ok = al_vt;
       if constexpr (KIND != WBC_CTRL_PC) wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
     }
-    if (h->prof_on) cudaEventRecord(h->prof_ev[1], st);
+    if (is.profile) cudaEventRecord(h->prof_ev[1], st);
     const unsigned sgrid = (unsigned)((m + SOLVE_WARPS - 1) / SOLVE_WARPS);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    // programmatic dependent launch of the solve kernel (its CTAs become resident while the last reduce CTAs run): +1.5 % at 4096
-    // instances, neutral above; never inside a stream capture ...
-    static const long long pdl_min = getenv("WBC_PDL_MIN") ? atoll(getenv("WBC_PDL_MIN")) : 4096;
-    // ... and chains that run beside other chains of the same step (chunked issue): there the early-resident solve CTAs take the
-    // slots the other chunk's reduce CTAs need (-22 % at 2 x 2048). A lone chain gains at every size (+3-4 % at 64 - 1024).
-    const bool pdl = pdl_mode() && (m >= pdl_min || !h->side_by_side);
-    if (pdl) cudaStreamIsCapturing(st, &cap);
-    const bool with_vd = io->vd != nullptr;
+    const bool pdl = use_pdl(m, is.beside_others) && !capturing(st);
+    const bool with_vd = io.vd != nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(sgrid); cfg.blockDim = dim3(SOLVE_WARPS * 32); cfg.stream = st;
     cfg.dynamicSmemBytes = with_vd ? sizeof(SmemLayoutSolveT<true>) : sizeof(SmemLayoutSolveT<false>);
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = (pdl && cap == cudaStreamCaptureStatusNone) ? 1 : 0;
+    cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
     const double* crec = h->d_rec[slot];
     const double* cvd = vdmap;
     if (with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, true>, (const DevConst*)h->d_const, a, crec, cvd));
     else WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, false>, (const DevConst*)h->d_const, a, crec, cvd));
-    if (h->prof_on) cudaEventRecord(h->prof_ev[2], st);
+    if (is.profile) cudaEventRecord(h->prof_ev[2], st);
     h->launches += 2;
   }
   return WBC_OK;
@@ -709,13 +794,13 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cu
 
 // One control step = reduce kernel (per controller kind) + solve kernel, stream ordered; `slot` selects the hand-over scratch
 // (the host pipelines run two streams side by side).
-static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cudaStream_t st, int slot) {
+static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is) {
   int rc = WBC_OK;
   switch (kind) {
-    case WBC_CTRL_ID: rc = launch_split<WBC_CTRL_ID>(h, kind, n, io, st, slot); break;
-    case WBC_CTRL_CLF: rc = launch_split<WBC_CTRL_CLF>(h, kind, n, io, st, slot); break;
+    case WBC_CTRL_ID: rc = launch_split<WBC_CTRL_ID>(h, kind, n, io, st, slot, is); break;
+    case WBC_CTRL_CLF: rc = launch_split<WBC_CTRL_CLF>(h, kind, n, io, st, slot, is); break;
     case WBC_CTRL_PC:
-    case WBC_CTRL_MPTC: rc = launch_split<WBC_CTRL_PC>(h, kind, n, io, st, slot); break;   // MPTC: a.kind drops the passivity row
+    case WBC_CTRL_MPTC: rc = launch_split<WBC_CTRL_PC>(h, kind, n, io, st, slot, is); break;   // MPTC: a.kind drops the passivity row
     default: return fail_arg(h, "wbc_step: unknown controller kind");
   }
   if (rc) return rc;
@@ -723,64 +808,31 @@ static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cud
   return WBC_OK;
 }
 
-static int two_stream_mode() {   // WBC_TWO_STREAMS=0: one reduce -> solve chain per step (A/B comparisons); k >= 2: k chunks;
-  static int mode = -1;          // unset (1): chunks of about 2048 instances, 2 to 4 of them
-  if (mode < 0) { const char* e = getenv("WBC_TWO_STREAMS"); mode = e ? atoi(e) : 1; }
-  return mode;
-}
-static int64_t two_stream_max() {
-  static int64_t v = -1;
-  if (v < 0) { const char* e = getenv("WBC_TWO_STREAMS_MAX"); v = e ? atoll(e) : 65536; }
-  return v;
-}
-
-extern "C" int wbc_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, void* stream) {
+// wbc_step on device buffers; `profile` (wbc_profile_step) issues one chain with events around its two kernels.
+static int device_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cudaStream_t st, bool profile) {
   if (!h) return WBC_ERR_ARG;
   if (!io || n < 0) return fail_arg(h, "wbc_step: bad arguments");
   if (n == 0) return WBC_OK;
-  if (kind == WBC_CTRL_PD) return wbc_step_pd(h, n, io->q, io->v, io->tau, stream);
+  if (kind == WBC_CTRL_PD) return wbc_step_pd(h, n, io->q, io->v, io->tau, st);
   if (!io->q || !io->v || !io->traj || !io->contact || !io->tau || !io->metrics || !io->status)
     return fail_arg(h, "wbc_step: q, v, traj, contact, tau, metrics and status are required");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  if (two_stream_mode() && !h->prof_on && n >= 4096 && n <= two_stream_max()) {
-    // Small batches go through as chunks of about 2048 instances, independent reduce -> solve chains on as many streams (the
-    // caller's and internal ones, joined by events): the solve kernel of one chunk overlaps the reduce kernel and the ramp-down
-    // of the others. Measured against one chain: +5.5 % at 4096 instances (2 chunks; 3: +4.5 %, 4: +2.5 %), +7.7 % at 8192
-    // (4 chunks; 2: +4.1 %), +2.6 % at 16384, +1 % at 65536, -2 % at 2048 (profiles/README.md). Never inside a stream capture.
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    cudaStreamIsCapturing(st, &cap);
-    if (cap == cudaStreamCaptureStatusNone) {
-      if (!h->order_ev) WBC_CUDA(h, cudaEventCreateWithFlags(&h->order_ev, cudaEventDisableTiming));
-      if (!h->join_ev) WBC_CUDA(h, cudaEventCreateWithFlags(&h->join_ev, cudaEventDisableTiming));
-      int chunks = two_stream_mode() < 2 ? (n >= 7168 ? 4 : n >= 5120 ? 3 : 2) : two_stream_mode();
-      if (chunks > WBC_NSLOT) chunks = WBC_NSLOT;
-      const int64_t per = (((n + chunks - 1) / chunks) + 3) & ~(int64_t)3;
-      WBC_CUDA(h, cudaEventRecord(h->order_ev, st));
-      for (int c = 1; c < chunks; ++c) {
-        if (c >= 2 && !h->xstream[c]) WBC_CUDA(h, cudaStreamCreateWithFlags(&h->xstream[c], cudaStreamNonBlocking));
-        WBC_CUDA(h, cudaStreamWaitEvent(c == 1 ? h->stream2 : h->xstream[c], h->order_ev, 0));
-      }
-      for (int c = 0; c < chunks; ++c) {
-        const int64_t o = c * per, m = (o + per <= n) ? per : n - o;
-        if (m <= 0) break;
-        const wbc_io cio{io->q + o * WBC_NQ, io->v + o * WBC_NV, io->traj + o * WBC_NTRAJ, io->contact + o * 4, io->tau + o * WBC_NU,
-                         io->metrics + o * WBC_NMETRIC, io->status + o, io->vd ? io->vd + o * WBC_NV : nullptr,
-                         io->f ? io->f + o * 12 : nullptr, io->qp_info ? io->qp_info + o * 4 : nullptr, io->lam ? io->lam + o * WBC_NLAM : nullptr};
-        cudaStream_t cs = c == 0 ? st : c == 1 ? h->stream2 : h->xstream[c];
-        h->side_by_side = true;
-        const int rc = step_launch(h, kind, m, &cio, cs, c);
-        h->side_by_side = false;
-        if (rc) return rc;
-        if (c) {
-          WBC_CUDA(h, cudaEventRecord(h->join_ev, cs));
-          WBC_CUDA(h, cudaStreamWaitEvent(st, h->join_ev, 0));
-        }
-      }
-      return WBC_OK;
-    }
-  }
-  return step_launch(h, kind, n, io, st, 0);
+  if (profile || n < CHUNKED_STEP_MIN || n > CHUNKED_STEP_MAX || capturing(st))
+    return step_launch(h, kind, n, *io, st, 0, Issue{false, false, profile});
+  const int k = device_step_chunks(n);
+  cudaStream_t lanes[WBC_NSLOT] = {st, h->stream2};
+  for (int c = 2; c < k; ++c) lanes[c] = h->xstream[c];
+  const int rc = streams_wait(h, h->order_ev, st, lanes + 1, k - 1);
+  if (rc) return rc;
+  return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
+    int r = step_launch(h, kind, m, io_at(*io, o), lanes[c], c, Issue{false, true});
+    if (!r && c) r = streams_wait(h, h->join_ev, lanes[c], &st, 1);
+    return r;
+  });
+}
+
+extern "C" int wbc_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, void* stream) {
+  return device_step(h, kind, n, io, (cudaStream_t)stream, false);
 }
 
 #define WBC_STEP_WRAPPER(name, kind)                                                                               \
@@ -830,132 +882,62 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
   if (!io->q || !io->v || !io->tau || (!pd && (!io->traj || !io->contact || !io->metrics || !io->status)))
     return fail_arg(h, "wbc_step_host: q, v, traj, contact, tau, metrics and status are required");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  int rc = WBC_OK;
+  const cudaStream_t lanes[2] = {h->stream, h->stream2};
   // Zero-copy path: when every buffer is page-locked host memory (wbc_host_alloc / cudaHostRegister) the kernel reads
   // its 732 B of inputs and writes its 132 B of outputs per instance straight over the host link - one launch, no
   // staging copies, the transfers of one warp overlap the arithmetic of the others.
-  {
-    int mode = -1;   // auto; WBC_HOST_ZEROCOPY=0 / 1 forces the staged / zero-copy path (experiments)
-    if (const char* env = getenv("WBC_HOST_ZEROCOPY")) mode = atoi(env);
-    const void* ptrs[11] = {io->q, io->v, io->traj, io->contact, io->tau, io->metrics, io->status, io->vd, io->f, io->qp_info, io->lam};
-    void* dev[11] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    // Measured on B200 (profiles/README.md): reading the inputs over the host link from the SMs (zero-copy, ~32 GB/s) wins up
-    // to ~48 k instances per call (no staging copies, no extra API calls); above that the inputs go through the copy engine
-    // (~55 GB/s) in a chunked two-stream pipeline. Page-locked outputs are written straight to host memory in both modes.
-    if (mode < 0) mode = 1;
-    bool pinned = mode != 0;
-    for (int i = 0; i < 11 && pinned; ++i) {
-      if (!ptrs[i]) continue;
-      cudaPointerAttributes at;
-      if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) { pinned = false; cudaGetLastError(); }
-      else dev[i] = at.devicePointer;
+  wbc_io hio = *io;
+  if (to_device_aliases(hio.q, hio.v, hio.traj, hio.contact, hio.tau, hio.metrics, hio.status, hio.vd, hio.f, hio.qp_info, hio.lam)) {
+    // The batch goes through in chunks alternating between the two internal streams (each with its own hand-over scratch); the
+    // outputs are written straight to host memory by the solve kernel in every mode. PD takes the chunk count of the staged
+    // mode but reads its inputs over the link at every size.
+    const bool stage_in = stage_pinned_inputs(kind, n), staged = stage_in && !pd;
+    const int k = pinned_chunks(n, stage_in);
+    if (staged) {
+      const int rc = ensure_staging(h, n);
+      if (rc) return rc;
+      hio.q = h->d_q; hio.v = h->d_v; hio.traj = h->d_traj; hio.contact = h->d_contact;
     }
-    if (pinned) {
-      const wbc_io hio{(const double*)dev[0], (const double*)dev[1], (const double*)dev[2], (const uint8_t*)dev[3], (double*)dev[4],
-                       (double*)dev[5], (int32_t*)dev[6], (double*)dev[7], (double*)dev[8], (double*)dev[9], (double*)dev[10]};
-      // The batch goes through in chunks alternating between the two internal streams (each with its own hand-over scratch); the
-      // outputs are written straight to host memory by the solve kernel in every mode.
-      //  * below 24576 instances the reduce kernel reads its inputs over the host link (zero-copy), two halves from 4096 on:
-      //    the solve kernel of one half overlaps the link-bound reduce kernel of the other (e2e +4.6 % at 4096, +3.8 % at
-      //    16384; three or more chunks lose);
-      //  * above, the inputs go through the copy engine into device staging (WBC_ZC_STAGE bit 0: traj, bit 1: q, v, contact) and
-      //    the single-warp reduce CTAs read resident inputs: e2e +5 % at 32768, +16 % at 65536, +10 % at 2^17 - 2^20.
-      static const long long stage_min = getenv("WBC_ZC_MAX") ? atoll(getenv("WBC_ZC_MAX")) : 24576;
-      static const int stage_env = getenv("WBC_ZC_STAGE") ? atoi(getenv("WBC_ZC_STAGE")) : -1;
-      // PC / MPTC are compute bound at a third of the rate: the zero-copy reads hide under the reduce kernel up to 131072
-      // instances (e2e 22.3 M steps/s against 20.0 M staged at 65536)
-      const bool pc_kind = kind == WBC_CTRL_PC || kind == WBC_CTRL_MPTC;
-      const int stage_in = stage_env >= 0 ? stage_env : (n >= (pc_kind ? 131072 : stage_min) ? 3 : 0);
-      int zc = n >= 4096 ? 2 : 1;
-      if (stage_in) {   // four chunks up to 65536 instances, then chunks of n / 8 clamped to [16384, 32768] instances
-        int64_t per_c = n / 8; per_c = per_c < 16384 ? 16384 : (per_c > 32768 ? 32768 : per_c);
-        if (n < 98304) per_c = ((n + 3) / 4 + 3) & ~(int64_t)3;
-        zc = (int)((n + per_c - 1) / per_c);
+    return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
+      const cudaStream_t st = lanes[c & 1];
+      const wbc_io s = io_at(*io, o), d = io_at(hio, o);
+      if (staged) {
+        WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
+        WBC_CUDA(h, cudaMemcpyAsync((void*)d.v, s.v, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
+        WBC_CUDA(h, cudaMemcpyAsync((void*)d.traj, s.traj, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, st));
+        WBC_CUDA(h, cudaMemcpyAsync((void*)d.contact, s.contact, m * 4, cudaMemcpyHostToDevice, st));
       }
-      if (const char* env = getenv("WBC_ZC_CHUNKS")) { const int v = atoi(env); if (v >= 1 && v <= 64) zc = v; }
-      if ((int64_t)zc > n) zc = (int)n;
-      const int64_t per = ((n + zc - 1) / zc + 3) & ~(int64_t)3;
-      cudaStream_t lanes[2] = {h->stream, h->stream2};
-      int used = 0;
-      if (stage_in && !pd) { rc = ensure_staging(h, n); if (rc) return rc; }
-      for (int c = 0; c < zc; ++c) {
-        const int64_t o = c * per, m = (o + per <= n) ? per : n - o;
-        if (m <= 0) break;
-        const bool staged = stage_in && !pd;
-        wbc_io dio = hio;
-        if (staged) {
-          cudaStream_t cs = lanes[c & 1];
-          if (stage_in & 2) {
-            WBC_CUDA(h, cudaMemcpyAsync(h->d_q + o * WBC_NQ, io->q + o * WBC_NQ, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, cs));
-            WBC_CUDA(h, cudaMemcpyAsync(h->d_v + o * WBC_NV, io->v + o * WBC_NV, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, cs));
-            WBC_CUDA(h, cudaMemcpyAsync(h->d_contact + o * 4, io->contact + o * 4, m * 4, cudaMemcpyHostToDevice, cs));
-            dio.q = h->d_q; dio.v = h->d_v; dio.contact = h->d_contact;
-          }
-          if (stage_in & 1) {
-            WBC_CUDA(h, cudaMemcpyAsync(h->d_traj + o * WBC_NTRAJ, io->traj + o * WBC_NTRAJ, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, cs));
-            dio.traj = h->d_traj;
-          }
-        }
-        const wbc_io cio{dio.q + o * WBC_NQ, dio.v + o * WBC_NV, dio.traj ? dio.traj + o * WBC_NTRAJ : nullptr,
-                         dio.contact ? dio.contact + o * 4 : nullptr, dio.tau + o * WBC_NU,
-                         dio.metrics ? dio.metrics + o * WBC_NMETRIC : nullptr, dio.status ? dio.status + o : nullptr,
-                         dio.vd ? dio.vd + o * WBC_NV : nullptr, dio.f ? dio.f + o * 12 : nullptr, dio.qp_info ? dio.qp_info + o * 4 : nullptr,
-                         dio.lam ? dio.lam + o * WBC_NLAM : nullptr};
-        h->host_mapped = !staged || (stage_in & 3) != 3;   // the reduce kernel reads host memory (4-warp CTAs, everything staged per CTA)
-        h->side_by_side = zc > 1;
-        rc = pd ? wbc_step_pd(h, m, cio.q, cio.v, cio.tau, lanes[c & 1]) : step_launch(h, kind, m, &cio, lanes[c & 1], c & 1);
-        h->host_mapped = false; h->side_by_side = false;
-        if (rc) return rc;
-        used |= 1 << (c & 1);
-      }
-      (void)used;
-      return WBC_OK;
-    }
+      return pd ? wbc_step_pd(h, m, d.q, d.v, d.tau, st) : step_launch(h, kind, m, d, st, c & 1, Issue{!staged, k > 1});
+    });
   }
-  rc = ensure_staging(h, n);
+  const int rc = ensure_staging(h, n);
   if (rc) return rc;
-  // Chunked two-stream pipeline: the upload of chunk c + 1 overlaps the kernel of chunk c, the download of chunk c the
-  // kernel of chunk c + 1 (separate copy engines); small batches go through in one piece.
-  // chunk = n / 8 clamped to [8192, 65536] instances: short pipeline fill, copies long enough for the copy engines
-  int n_chunks = n >= 2048 ? 2 : 1;
-  if (n >= 32768) {
-    int64_t per_c = n / 8; per_c = per_c < 8192 ? 8192 : (per_c > 65536 ? 65536 : per_c);
-    const int64_t c = (n + per_c - 1) / per_c;
-    n_chunks = (int)(c > 64 ? 64 : c);
-  }
-  if (const char* env = getenv("WBC_HOST_CHUNKS")) { const int v = atoi(env); if (v >= 1 && v <= 64) n_chunks = v; }
-  if ((int64_t)n_chunks > n) n_chunks = (int)n;
-  const int64_t per = (n + n_chunks - 1) / n_chunks;
-  cudaStream_t lanes[2] = {h->stream, h->stream2};
-  for (int c = 0; c < n_chunks; ++c) {
-    const int64_t o = c * per, m = (o + per <= n) ? per : n - o;
-    if (m <= 0) break;
-    cudaStream_t st = lanes[c & 1];
-    WBC_CUDA(h, cudaMemcpyAsync(h->d_q + o * WBC_NQ, io->q + o * WBC_NQ, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
-    WBC_CUDA(h, cudaMemcpyAsync(h->d_v + o * WBC_NV, io->v + o * WBC_NV, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
+  // pageable buffers: the device staging rows, with the optional outputs the caller asked for
+  const wbc_io dev{h->d_q, h->d_v, h->d_traj, h->d_contact, h->d_tau, h->d_metrics, h->d_status, io->vd ? h->d_vd : nullptr,
+                   io->f ? h->d_f : nullptr, io->qp_info ? h->d_info : nullptr, io->lam ? h->d_lam : nullptr};
+  const int k = pageable_chunks(n);
+  return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
+    const cudaStream_t st = lanes[c & 1];
+    const wbc_io s = io_at(*io, o), d = io_at(dev, o);
+    WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
+    WBC_CUDA(h, cudaMemcpyAsync((void*)d.v, s.v, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
     if (!pd) {
-      WBC_CUDA(h, cudaMemcpyAsync(h->d_traj + o * WBC_NTRAJ, io->traj + o * WBC_NTRAJ, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, st));
-      WBC_CUDA(h, cudaMemcpyAsync(h->d_contact + o * 4, io->contact + o * 4, m * 4, cudaMemcpyHostToDevice, st));
+      WBC_CUDA(h, cudaMemcpyAsync((void*)d.traj, s.traj, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, st));
+      WBC_CUDA(h, cudaMemcpyAsync((void*)d.contact, s.contact, m * 4, cudaMemcpyHostToDevice, st));
     }
-    wbc_io dio{h->d_q + o * WBC_NQ, h->d_v + o * WBC_NV, h->d_traj + o * WBC_NTRAJ, h->d_contact + o * 4, h->d_tau + o * WBC_NU,
-               h->d_metrics + o * WBC_NMETRIC, h->d_status + o,
-               io->vd ? h->d_vd + o * WBC_NV : nullptr, io->f ? h->d_f + o * 12 : nullptr, io->qp_info ? h->d_info + o * 4 : nullptr,
-               io->lam ? h->d_lam + o * WBC_NLAM : nullptr};
-    h->side_by_side = n_chunks > 1;
-    rc = pd ? wbc_step_pd(h, m, dio.q, dio.v, dio.tau, st) : step_launch(h, kind, m, &dio, st, c & 1);
-    h->side_by_side = false;
-    if (rc) return rc;
-    WBC_CUDA(h, cudaMemcpyAsync(io->tau + o * WBC_NU, h->d_tau + o * WBC_NU, m * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
+    const int r = pd ? wbc_step_pd(h, m, d.q, d.v, d.tau, st) : step_launch(h, kind, m, d, st, c & 1, Issue{false, k > 1});
+    if (r) return r;
+    WBC_CUDA(h, cudaMemcpyAsync(s.tau, d.tau, m * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (!pd) {
-      WBC_CUDA(h, cudaMemcpyAsync(io->metrics + o * WBC_NMETRIC, h->d_metrics + o * WBC_NMETRIC, m * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
-      WBC_CUDA(h, cudaMemcpyAsync(io->status + o, h->d_status + o, m * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-      if (io->vd) WBC_CUDA(h, cudaMemcpyAsync(io->vd + o * WBC_NV, h->d_vd + o * WBC_NV, m * WBC_NV * sizeof(double), cudaMemcpyDeviceToHost, st));
-      if (io->f) WBC_CUDA(h, cudaMemcpyAsync(io->f + o * 12, h->d_f + o * 12, m * 12 * sizeof(double), cudaMemcpyDeviceToHost, st));
-      if (io->qp_info) WBC_CUDA(h, cudaMemcpyAsync(io->qp_info + o * 4, h->d_info + o * 4, m * 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
-      if (io->lam) WBC_CUDA(h, cudaMemcpyAsync(io->lam + o * WBC_NLAM, h->d_lam + o * WBC_NLAM, m * WBC_NLAM * sizeof(double), cudaMemcpyDeviceToHost, st));
+      WBC_CUDA(h, cudaMemcpyAsync(s.metrics, d.metrics, m * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
+      WBC_CUDA(h, cudaMemcpyAsync(s.status, d.status, m * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+      if (s.vd) WBC_CUDA(h, cudaMemcpyAsync(s.vd, d.vd, m * WBC_NV * sizeof(double), cudaMemcpyDeviceToHost, st));
+      if (s.f) WBC_CUDA(h, cudaMemcpyAsync(s.f, d.f, m * 12 * sizeof(double), cudaMemcpyDeviceToHost, st));
+      if (s.qp_info) WBC_CUDA(h, cudaMemcpyAsync(s.qp_info, d.qp_info, m * 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
+      if (s.lam) WBC_CUDA(h, cudaMemcpyAsync(s.lam, d.lam, m * WBC_NLAM * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
-  }
-  return WBC_OK;
+    return WBC_OK;
+  });
 }
 
 extern "C" int wbc_step_host(wbc_handle* h, int kind, int64_t n, const wbc_io* io) {
@@ -1020,11 +1002,7 @@ extern "C" int wbc_multi_step_host(wbc_multi* m, int kind, int64_t n, const wbc_
     int64_t lo, hi;
     shard_of(n, r, w, &lo, &hi);
     if (hi <= lo) { ++enq; continue; }
-    const wbc_io sio{io->q + lo * WBC_NQ, io->v + lo * WBC_NV, io->traj ? io->traj + lo * WBC_NTRAJ : nullptr,
-                     io->contact ? io->contact + lo * 4 : nullptr, io->tau + lo * WBC_NU,
-                     io->metrics ? io->metrics + lo * WBC_NMETRIC : nullptr, io->status ? io->status + lo : nullptr,
-                     io->vd ? io->vd + lo * WBC_NV : nullptr, io->f ? io->f + lo * 12 : nullptr,
-                     io->qp_info ? io->qp_info + lo * 4 : nullptr, io->lam ? io->lam + lo * WBC_NLAM : nullptr};
+    const wbc_io sio = io_at(*io, lo);
     rc = step_host_enqueue(m->h[r], kind, hi - lo, &sio);
     if (rc) m->err = m->h[r]->err;
     ++enq;
@@ -1091,9 +1069,7 @@ extern "C" int wbc_profile_step(wbc_handle* h, int kind, int64_t n, const wbc_io
   for (int i = 0; i < 3; ++i) if (!h->prof_ev[i]) WBC_CUDA(h, cudaEventCreate(&h->prof_ev[i]));
   double r = 0.0, s = 0.0;
   for (int k = 0; k < reps; ++k) {
-    h->prof_on = true;
-    const int rc = wbc_step(h, kind, n, io, stream);
-    h->prof_on = false;
+    const int rc = device_step(h, kind, n, io, (cudaStream_t)stream, true);
     if (rc) return rc;
     WBC_CUDA(h, cudaEventSynchronize(h->prof_ev[2]));
     float a = 0.f, b = 0.f;
@@ -1368,10 +1344,7 @@ extern "C" int wbc_sample_trajectory(wbc_handle* h, const wbc_plan* plan, int64_
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
   if (reinterpret_cast<uintptr_t>(contact) & 3u) return fail_arg(h, "wbc_sample_trajectory: contact must be 4-byte aligned");
-  // instances per warp: 32 (lane = instance) is the throughput shape; small batches are latency bound on the 14 dependent binary
-  // searches per instance, so they spread them over 4 or 16 lanes per instance
-  static const int ipw_env = getenv("WBC_SAMPLE_IPW") ? atoi(getenv("WBC_SAMPLE_IPW")) : 0;
-  const int ipw = ipw_env ? ipw_env : (n >= 32768 ? 32 : n >= 8192 ? 8 : 2);   // rollout of 4096 robots: 45.2 / 48.7 / 49.7 M robot-steps/s with 32 / 8 / 2
+  const int ipw = sample_ipw(n);
   const long long chunks = (n + ipw - 1) / ipw, blocks = (chunks + wbctraj::SAMPLE_WARPS - 1) / wbctraj::SAMPLE_WARPS, cap = (long long)h->sm_count * 16;
   const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
   cudaStream_t sst = (cudaStream_t)stream;
@@ -1420,39 +1393,23 @@ extern "C" int wbc_step_plan_host(wbc_handle* h, int kind, const wbc_plan* plan,
   int rc = ensure_rollout_scratch(h, n);
   if (rc) return rc;
   cudaStream_t st = h->stream;
-  const void* ptrs[7] = {q, v, t, plan_index, tau, metrics, status};
-  void* dev[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  bool pinned = true;
-  for (int i = 0; i < 7 && pinned; ++i) {
-    if (!ptrs[i]) continue;
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, ptrs[i]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) { pinned = false; cudaGetLastError(); }
-    else dev[i] = at.devicePointer;
-  }
-  if (pinned) {
-    rc = wbc_sample_trajectory(h, plan, n, (const int32_t*)dev[3], (const double*)dev[2], h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
+  if (to_device_aliases(q, v, t, plan_index, tau, metrics, status)) {   // from here on the kernels' aliases of the host arrays
+    rc = wbc_sample_trajectory(h, plan, n, plan_index, t, h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
     if (rc) return rc;
     // the step itself as in the zero-copy mode of wbc_step_host: two halves on the two internal streams. q and v are 304 B per
     // instance, which the reduce CTAs pull over the link without slowing down at any batch size (57.3 M steps/s at 65536,
     // 60.8 M at 2^20; copy-engine staging of q and v: 51.5 / 60.6 M)
-    const int zc = n >= 4096 ? 2 : 1;
-    const int64_t per = ((n + zc - 1) / zc + 3) & ~(int64_t)3;
-    cudaStream_t lanes[2] = {st, h->stream2};
-    if (zc > 1) {
-      if (!h->order_ev) WBC_CUDA(h, cudaEventCreateWithFlags(&h->order_ev, cudaEventDisableTiming));
-      WBC_CUDA(h, cudaEventRecord(h->order_ev, st));                 // the sampled rows
-      WBC_CUDA(h, cudaStreamWaitEvent(h->stream2, h->order_ev, 0));
-    }
-    for (int c = 0; c < zc; ++c) {
-      const int64_t o = c * per, m = (o + per <= n) ? per : n - o;
-      if (m <= 0) break;
-      const wbc_io io{(const double*)dev[0] + o * WBC_NQ, (const double*)dev[1] + o * WBC_NV, h->ro_traj + o * WBC_NTRAJ, h->ro_contact + o * 4,
-                      (double*)dev[4] + o * WBC_NU, (double*)dev[5] + o * WBC_NMETRIC, (int32_t*)dev[6] + o};
-      h->host_mapped = true; h->side_by_side = zc > 1;
-      rc = step_launch(h, kind, m, &io, lanes[c & 1], c & 1);
-      h->host_mapped = false; h->side_by_side = false;
+    const int k = pinned_chunks(n, false);
+    const cudaStream_t lanes[2] = {st, h->stream2};
+    if (k > 1) {
+      rc = streams_wait(h, h->order_ev, st, lanes + 1, 1);   // the sampled rows
       if (rc) return rc;
     }
+    const wbc_io zio{q, v, h->ro_traj, h->ro_contact, tau, metrics, status};
+    rc = for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
+      return step_launch(h, kind, m, io_at(zio, o), lanes[c & 1], c & 1, Issue{true, k > 1});
+    });
+    if (rc) return rc;
     return step_host_wait(h);
   }
   rc = ensure_staging(h, n);
@@ -1466,7 +1423,7 @@ extern "C" int wbc_step_plan_host(wbc_handle* h, int kind, const wbc_plan* plan,
   rc = wbc_sample_trajectory(h, plan, n, dpi, h->ro_t, h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
   if (rc) return rc;
   const wbc_io io{h->d_q, h->d_v, h->ro_traj, h->ro_contact, h->d_tau, h->d_metrics, h->d_status};
-  rc = step_launch(h, kind, n, &io, st, 0);
+  rc = step_launch(h, kind, n, io, st, 0, Issue{});
   if (rc) return rc;
   WBC_CUDA(h, cudaMemcpyAsync(tau, h->d_tau, n * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
   WBC_CUDA(h, cudaMemcpyAsync(metrics, h->d_metrics, n * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1652,23 +1609,22 @@ extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan
   wbc_rollout_io d{};
   d.q = s.in(io->q, N * WBC_NQ, st); d.v = s.in(io->v, N * WBC_NV, st); d.t = s.in(io->t, N, st);
   d.plan_index = s.in(io->plan_index, N, st);
-  DevScratch s2;     // DevScratch holds 8 buffers
-  d.tau = s2.out(io->tau, N * WBC_NU); d.metrics = s2.out(io->metrics, N * WBC_NMETRIC);
-  d.status_or = s2.out(io->status_or, N); d.err_max = s2.out(io->err_max, N);
-  d.metrics_log = s2.out(io->metrics_log, N * WBC_NMETRIC * (size_t)n_steps);
+  d.tau = s.out(io->tau, N * WBC_NU); d.metrics = s.out(io->metrics, N * WBC_NMETRIC);
+  d.status_or = s.out(io->status_or, N); d.err_max = s.out(io->err_max, N);
+  d.metrics_log = s.out(io->metrics_log, N * WBC_NMETRIC * (size_t)n_steps);
   wbc_rollout_opts o{};
   if (opts) o = *opts; else { o.use_graph = 1; wbc_default_plant_opts(&o.plant_opts); }
   double* host_f = o.f_contact;
-  o.f_contact = s2.out(host_f, N * 12);
-  WBC_SCRATCH_CHECK(h, s); WBC_SCRATCH_CHECK(h, s2);
+  o.f_contact = s.out(host_f, N * 12);
+  WBC_SCRATCH_CHECK(h, s);
   int rc = wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, st);
   if (rc) return rc;
   s.back(io->q, d.q, N * WBC_NQ, st); s.back(io->v, d.v, N * WBC_NV, st); s.back(io->t, d.t, N, st);
-  s2.back(io->tau, d.tau, N * WBC_NU, st); s2.back(io->metrics, d.metrics, N * WBC_NMETRIC, st);
-  s2.back(io->status_or, d.status_or, N, st); s2.back(io->err_max, d.err_max, N, st);
-  s2.back(io->metrics_log, d.metrics_log, N * WBC_NMETRIC * (size_t)n_steps, st);
-  s2.back(host_f, o.f_contact, N * 12, st);
-  WBC_SCRATCH_CHECK(h, s); WBC_SCRATCH_CHECK(h, s2);
+  s.back(io->tau, d.tau, N * WBC_NU, st); s.back(io->metrics, d.metrics, N * WBC_NMETRIC, st);
+  s.back(io->status_or, d.status_or, N, st); s.back(io->err_max, d.err_max, N, st);
+  s.back(io->metrics_log, d.metrics_log, N * WBC_NMETRIC * (size_t)n_steps, st);
+  s.back(host_f, o.f_contact, N * 12, st);
+  WBC_SCRATCH_CHECK(h, s);
   WBC_CUDA(h, cudaStreamSynchronize(st));
   return WBC_OK;
 }

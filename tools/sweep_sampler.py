@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Device time of wbc_sample_trajectory by batch size and instances per warp (WBC_SAMPLE_IPW = 32 / 8 / 2; set before the
-library is loaded): python tools/sweep_sampler.py  -> one line per size."""
-import os, sys
+"""Device time of wbc_sample_trajectory by batch size; the sizes cover all three instances-per-warp shapes of the sampler
+kernel (2 / 8 / 32): python tools/sweep_sampler.py  -> one line per size."""
+import sys
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 import numpy as np
@@ -26,4 +26,4 @@ for n in (1, 256, 4096, 16384, 65536, 262144, 1 << 20):
         s.sample(t, pi)
     e1.record(); torch.cuda.synchronize()
     us = e0.elapsed_time(e1) * 1e3 / reps
-    print("ipw %s  n %8d  %9.2f us per call  %8.1f M samples/s" % (os.environ.get("WBC_SAMPLE_IPW", "auto"), n, us, n / us))
+    print("n %8d  %9.2f us per call  %8.1f M samples/s" % (n, us, n / us))
