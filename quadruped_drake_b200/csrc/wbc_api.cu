@@ -5,6 +5,8 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <deque>
+#include <memory>
 #include <string>
 
 // named barrier `id` over `threads` threads of the CTA (a multiple of 32; skipped when at most one warp takes part)
@@ -344,41 +346,125 @@ __global__ void fp64_peak_kernel(double* out, int iters) {
   out[blockIdx.x * blockDim.x + threadIdx.x] = a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7;
 }
 
+// ------------------------------------------------------------------------------ resource owners
+// Every device resource of the library is held by one of these and released in its destructor, on whatever device is
+// current then (the owners of a handle or a plan select theirs first).
+
+// Device array that only grows: reserve(n) reallocates, without keeping the contents, when n exceeds the capacity.
+template <typename T>
+struct DevArray {
+  T* p = nullptr;
+  size_t cap = 0;
+  DevArray() = default;
+  DevArray(const DevArray&) = delete;
+  DevArray& operator=(const DevArray&) = delete;
+  ~DevArray() { if (p) cudaFree(p); }
+  cudaError_t reserve(size_t n) {
+    if (n <= cap) return cudaSuccess;
+    if (p) cudaFree(p);
+    p = nullptr; cap = 0;
+    const cudaError_t e = cudaMalloc(&p, n * sizeof(T));
+    if (e == cudaSuccess) cap = n;
+    return e;
+  }
+};
+
+// A stream, event, graph or graph exec; created through &v.
+template <typename R, cudaError_t (*Destroy)(R)>
+struct Owned {
+  R v = nullptr;
+  Owned() = default;
+  Owned(const Owned&) = delete;
+  Owned& operator=(const Owned&) = delete;
+  ~Owned() { if (v) Destroy(v); }
+  operator R() const { return v; }
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+using Graph = Owned<cudaGraph_t, cudaGraphDestroy>;
+using GraphExec = Owned<cudaGraphExec_t, cudaGraphExecDestroy>;
+
+// Instances per reduce / solve launch pair of the split path: bounds the hand-over scratch (4224 B per instance) at 1.1 GB
+// while each kernel still runs for milliseconds, so the drain at the kernel boundaries stays below ~1 % of the step.
+constexpr int64_t SPLIT_CHUNK = 262144;
+
+// Hand-over scratch of the split step (reduce -> solve) for one stream lane, and the ordering of its users: the stream of
+// the last step that used it.
+struct Slot {
+  DevArray<double> rec, vdmap;
+  cudaStream_t last_stream = nullptr;
+  bool used = false;
+  // Records (and the accelerations of the vd outputs) for min(n, SPLIT_CHUNK) instances. Never grows inside a stream
+  // capture: callers that capture reserve first.
+  cudaError_t reserve(int64_t n, bool with_vd) {
+    const int64_t m = std::min(n, SPLIT_CHUNK);
+    cudaError_t e = rec.reserve(m * wbc::REC_DOUBLES);
+    if (e == cudaSuccess && with_vd) e = vdmap.reserve(m * wbc::VDMAP_DOUBLES);
+    return e;
+  }
+};
+
+// Device rows of wbc_step_host and wbc_step_plan_host, for n instances.
+struct Staging {
+  DevArray<double> q, v, traj, tau, metrics, vd, f, info, lam;
+  DevArray<uint8_t> contact;
+  DevArray<int32_t> status;
+  cudaError_t reserve(int64_t n) {
+    cudaError_t e = q.reserve(n * WBC_NQ);
+    if (e == cudaSuccess) e = v.reserve(n * WBC_NV);
+    if (e == cudaSuccess) e = traj.reserve(n * WBC_NTRAJ);
+    if (e == cudaSuccess) e = contact.reserve(n * 4);
+    if (e == cudaSuccess) e = tau.reserve(n * WBC_NU);
+    if (e == cudaSuccess) e = metrics.reserve(n * WBC_NMETRIC);
+    if (e == cudaSuccess) e = status.reserve(n);
+    if (e == cudaSuccess) e = vd.reserve(n * WBC_NV);
+    if (e == cudaSuccess) e = f.reserve(n * 12);
+    if (e == cudaSuccess) e = info.reserve(n * 4);
+    if (e == cudaSuccess) e = lam.reserve(n * WBC_NLAM);
+    return e;
+  }
+};
+
+// Scratch of wbc_rollout and wbc_step_plan_host, for n instances: the sampled targets, the outputs the caller does not
+// keep, and the step counter of the metrics log.
+struct RolloutScratch {
+  DevArray<double> traj, vd, metrics, tau, t;
+  DevArray<uint8_t> contact;
+  DevArray<int32_t> status;
+  DevArray<int> counter;
+  cudaError_t reserve(int64_t n) {
+    cudaError_t e = counter.reserve(1);
+    if (e == cudaSuccess) e = traj.reserve(n * WBC_NTRAJ);
+    if (e == cudaSuccess) e = vd.reserve(n * WBC_NV);
+    if (e == cudaSuccess) e = metrics.reserve(n * WBC_NMETRIC);
+    if (e == cudaSuccess) e = tau.reserve(n * WBC_NU);
+    if (e == cudaSuccess) e = t.reserve(n);
+    if (e == cudaSuccess) e = contact.reserve(n * 4);
+    if (e == cudaSuccess) e = status.reserve(n);
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
 struct wbc_handle {
   int device = 0;
-  DevConst* d_const = nullptr;
+  DevArray<DevConst> d_const;
   wbc_params params;
   std::string err;
   int64_t launches = 0;
   int sm_count = 148;
-  int* d_tau_map = nullptr;            // message slot (velocity order) -> actuator index, for wbc_lcm_encode_robot_state
-  cudaStream_t stream = nullptr;       // used by the host entry points
-  cudaStream_t stream2 = nullptr;      // second lane of the chunked wbc_step_host pipeline
-  // device staging for wbc_step_host
-  int64_t cap = 0;
-  double *d_q = nullptr, *d_v = nullptr, *d_traj = nullptr, *d_tau = nullptr, *d_metrics = nullptr, *d_vd = nullptr,
-         *d_f = nullptr, *d_info = nullptr, *d_lam = nullptr;
-  uint8_t* d_contact = nullptr;
-  int32_t* d_status = nullptr;
-  // scratch of wbc_rollout (sized for ro_cap instances)
-  int64_t ro_cap = 0;
-  double *ro_traj = nullptr, *ro_vd = nullptr, *ro_metrics = nullptr, *ro_tau = nullptr, *ro_t = nullptr;
-  uint8_t* ro_contact = nullptr;
-  int32_t* ro_status = nullptr;
-  int* ro_counter = nullptr;
-  // hand-over records of the split step (reduce -> solve), one slot per internal stream lane
-  cudaEvent_t prof_ev[3] = {nullptr, nullptr, nullptr};   // wbc_profile_step: before reduce / between / after solve
-  // per-slot ordering of the scratch users: the stream of the last step that used the slot and an event to chain a new one
-  cudaStream_t last_stream[WBC_NSLOT] = {};
-  bool slot_used[WBC_NSLOT] = {};
-  cudaEvent_t order_ev = nullptr, join_ev = nullptr;
-  double* d_rec[WBC_NSLOT] = {};
-  double* d_vdmap[WBC_NSLOT] = {};
-  int64_t rec_cap[WBC_NSLOT] = {}, vdmap_cap[WBC_NSLOT] = {};
-  cudaStream_t xstream[WBC_NSLOT] = {};                  // lanes 2.. of a step issued as more than two chunks
+  DevArray<int> d_tau_map;             // message slot (velocity order) -> actuator index, for wbc_lcm_encode_robot_state
+  // internal streams: lane 0 serves the host entries, lanes 0-1 the host pipelines, lanes 1.. chunks 1.. of a device step
+  // (its chunk 0 runs on the caller's stream); slot[i] is the hand-over scratch of the chain on lane i
+  Stream lane[WBC_NSLOT];
+  Slot slot[WBC_NSLOT];
+  Event order_ev, join_ev;
+  Event prof_ev[3];                    // wbc_profile_step: before reduce / between / after solve
+  Staging stage;
+  RolloutScratch ro;
+  ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
 #define WBC_CUDA(h, call)                                                                       \
@@ -432,72 +518,39 @@ static int set_smem_attr(wbc_handle* h) {
 
 extern "C" int wbc_create(const wbc_model* model, const wbc_params* params, int device, wbc_handle** out) {
   if (!model || !out) return WBC_ERR_ARG;
-  *out = nullptr;
   wbc_handle* h = new (std::nothrow) wbc_handle();
+  *out = h;                            // handed back even when creation fails part-way, so that wbc_last_error works
   if (!h) return WBC_ERR_NOMEM;
   h->device = device;
   if (params) h->params = *params; else wbc_default_params(&h->params);
-  int rc = WBC_OK;
-  auto bail = [&](int code) { *out = h; return code; };  // hand the handle back so wbc_last_error works
-  if (h->params.reg_vd != 0.0) { h->err = "reg_vd is not supported yet (must be 0)"; return bail(WBC_ERR_ARG); }
-  if (!(h->params.reg_f > 0.0)) { h->err = "reg_f must be > 0 (tie-break that makes the QP strictly convex)"; return bail(WBC_ERR_ARG); }
+  if (h->params.reg_vd != 0.0) return fail_arg(h, "reg_vd is not supported yet (must be 0)");
+  if (!(h->params.reg_f > 0.0)) return fail_arg(h, "reg_f must be > 0 (tie-break that makes the QP strictly convex)");
   for (int k = 0; k < WBC_NU; ++k) {
-    if (model->v_index[k] < 6 || model->v_index[k] >= WBC_NV || model->act_index[k] < 0 || model->act_index[k] >= WBC_NU) {
-      h->err = "wbc_model: v_index/act_index out of range"; return bail(WBC_ERR_ARG);
-    }
+    if (model->v_index[k] < 6 || model->v_index[k] >= WBC_NV || model->act_index[k] < 0 || model->act_index[k] >= WBC_NU)
+      return fail_arg(h, "wbc_model: v_index/act_index out of range");
   }
-  cudaError_t e = cudaSetDevice(device);
-  if (e != cudaSuccess) { h->err = std::string("cudaSetDevice: ") + cudaGetErrorString(e); return bail(WBC_ERR_CUDA); }
+  WBC_CUDA(h, cudaSetDevice(device));
   DevConst hc;
   hc.md = *model; hc.pr = h->params;
   wbc::derive_constants(h->params, hc.dv);
-  e = cudaMalloc(&h->d_const, sizeof(DevConst));
-  if (e != cudaSuccess) { h->err = std::string("cudaMalloc: ") + cudaGetErrorString(e); return bail(WBC_ERR_CUDA); }
-  e = cudaMemcpy(h->d_const, &hc, sizeof(DevConst), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) { h->err = std::string("cudaMemcpy: ") + cudaGetErrorString(e); return bail(WBC_ERR_CUDA); }
-  e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
-  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking);
-  // lanes 2.. of a chunked step and the fork / join events: created here, not on first use, so that a step never calls a
-  // resource-creating API while some other stream of the process is being captured
-  for (int l = 2; l < WBC_NSLOT && e == cudaSuccess; ++l) e = cudaStreamCreateWithFlags(&h->xstream[l], cudaStreamNonBlocking);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->order_ev, cudaEventDisableTiming);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->join_ev, cudaEventDisableTiming);
-  if (e != cudaSuccess) { h->err = std::string("cudaStreamCreate: ") + cudaGetErrorString(e); return bail(WBC_ERR_CUDA); }
-  {
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) h->sm_count = prop.multiProcessorCount;
-    int tmap[WBC_NU];
-    for (int k = 0; k < WBC_NU; ++k) tmap[model->v_index[k] - 6] = model->act_index[k];
-    e = cudaMalloc(&h->d_tau_map, sizeof(tmap));
-    if (e == cudaSuccess) e = cudaMemcpy(h->d_tau_map, tmap, sizeof(tmap), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { h->err = std::string("tau map upload: ") + cudaGetErrorString(e); return bail(WBC_ERR_CUDA); }
-  }
-  rc = set_smem_attr(h);
-  *out = h;
-  return rc;
-}
-
-static void free_staging(wbc_handle* h) {
-  cudaFree(h->d_q); cudaFree(h->d_v); cudaFree(h->d_traj); cudaFree(h->d_tau); cudaFree(h->d_metrics);
-  cudaFree(h->d_vd); cudaFree(h->d_f); cudaFree(h->d_info); cudaFree(h->d_lam); cudaFree(h->d_contact); cudaFree(h->d_status);
-  h->d_q = h->d_v = h->d_traj = h->d_tau = h->d_metrics = h->d_vd = h->d_f = h->d_info = h->d_lam = nullptr;
-  h->d_contact = nullptr; h->d_status = nullptr; h->cap = 0;
+  WBC_CUDA(h, h->d_const.reserve(1));
+  WBC_CUDA(h, cudaMemcpy(h->d_const.p, &hc, sizeof(DevConst), cudaMemcpyHostToDevice));
+  // the streams and events: created here, not on first use, so that a step never calls a resource-creating API while some
+  // other stream of the process is being captured
+  for (Stream& s : h->lane) WBC_CUDA(h, cudaStreamCreateWithFlags(&s.v, cudaStreamNonBlocking));
+  WBC_CUDA(h, cudaEventCreateWithFlags(&h->order_ev.v, cudaEventDisableTiming));
+  WBC_CUDA(h, cudaEventCreateWithFlags(&h->join_ev.v, cudaEventDisableTiming));
+  for (Event& e : h->prof_ev) WBC_CUDA(h, cudaEventCreate(&e.v));
+  cudaDeviceProp prop;
+  if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) h->sm_count = prop.multiProcessorCount;
+  int tmap[WBC_NU];
+  for (int k = 0; k < WBC_NU; ++k) tmap[model->v_index[k] - 6] = model->act_index[k];
+  WBC_CUDA(h, h->d_tau_map.reserve(WBC_NU));
+  WBC_CUDA(h, cudaMemcpy(h->d_tau_map.p, tmap, sizeof(tmap), cudaMemcpyHostToDevice));
+  return set_smem_attr(h);
 }
 
 extern "C" int wbc_destroy(wbc_handle* h) {
-  if (!h) return WBC_OK;
-  cudaSetDevice(h->device);
-  free_staging(h);
-  if (h->d_const) cudaFree(h->d_const);
-  if (h->d_tau_map) cudaFree(h->d_tau_map);
-  cudaFree(h->ro_traj); cudaFree(h->ro_vd); cudaFree(h->ro_metrics); cudaFree(h->ro_tau); cudaFree(h->ro_t);
-  cudaFree(h->ro_contact); cudaFree(h->ro_status); cudaFree(h->ro_counter);
-  for (int i = 0; i < WBC_NSLOT; ++i) { cudaFree(h->d_rec[i]); cudaFree(h->d_vdmap[i]); if (h->xstream[i]) cudaStreamDestroy(h->xstream[i]); }
-  for (int i = 0; i < 3; ++i) if (h->prof_ev[i]) cudaEventDestroy(h->prof_ev[i]);
-  if (h->order_ev) cudaEventDestroy(h->order_ev);
-  if (h->join_ev) cudaEventDestroy(h->join_ev);
-  if (h->stream) cudaStreamDestroy(h->stream);
-  if (h->stream2) cudaStreamDestroy(h->stream2);
   delete h;
   return WBC_OK;
 }
@@ -513,7 +566,7 @@ extern "C" int wbc_dynamics(wbc_handle* h, int64_t n, const double* q, const dou
   WBC_CUDA(h, cudaSetDevice(h->device));
   wbc::DynOut o{M, Cv, taug, Jfeet, Jdv, pfeet};
   const unsigned grid = (unsigned)((n + WARPS - 1) / WARPS);
-  wbc_dynamics_kernel<<<grid, WARPS * 32, sizeof(SmemLayout), (cudaStream_t)stream>>>(h->d_const, q, v, o, n);
+  wbc_dynamics_kernel<<<grid, WARPS * 32, sizeof(SmemLayout), (cudaStream_t)stream>>>(h->d_const.p, q, v, o, n);
   h->launches++;
   WBC_CUDA(h, cudaGetLastError());
   return WBC_OK;
@@ -525,60 +578,62 @@ extern "C" int wbc_coriolis(wbc_handle* h, int64_t n, const double* q, const dou
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
   const unsigned grid = (unsigned)((n + WARPS - 1) / WARPS);
-  wbc_coriolis_kernel<<<grid, WARPS * 32, sizeof(SmemLayoutPC), (cudaStream_t)stream>>>(h->d_const, q, v, Cm, Jd, n);
+  wbc_coriolis_kernel<<<grid, WARPS * 32, sizeof(SmemLayoutPC), (cudaStream_t)stream>>>(h->d_const.p, q, v, Cm, Jd, n);
   h->launches++;
   WBC_CUDA(h, cudaGetLastError());
   return WBC_OK;
 }
-
-namespace {
-// Scratch device buffers of the host-buffer debug / codec entries: freed when the scope ends (early error returns included).
-struct DevScratch {
-  std::vector<void*> p;
-  cudaError_t err = cudaSuccess;
-  template <typename T> T* in(const T* host, size_t count, cudaStream_t st) {      // NULL stays NULL
-    if (!host || err != cudaSuccess) return nullptr;
-    T* d = out<T>(host, count);
-    if (d) err = cudaMemcpyAsync(d, host, count * sizeof(T), cudaMemcpyHostToDevice, st);
-    return d;
-  }
-  template <typename T> T* out(const T* host, size_t count) {
-    if (!host || err != cudaSuccess) return nullptr;
-    void* d = nullptr;
-    err = cudaMalloc(&d, count * sizeof(T) > 0 ? count * sizeof(T) : 1);
-    if (err != cudaSuccess) return nullptr;
-    p.push_back(d);
-    return static_cast<T*>(d);
-  }
-  template <typename T> void back(T* host, const T* dev, size_t count, cudaStream_t st) {
-    if (host && dev && err == cudaSuccess) err = cudaMemcpyAsync(host, dev, count * sizeof(T), cudaMemcpyDeviceToHost, st);
-  }
-  ~DevScratch() { for (void* d : p) cudaFree(d); }
-};
-}  // namespace
 
 #define WBC_SCRATCH_CHECK(h, s)                                                                  \
   do {                                                                                           \
     if ((s).err != cudaSuccess) { (h)->err = std::string("host-buffer entry: ") + cudaGetErrorString((s).err); return WBC_ERR_CUDA; } \
   } while (0)
 
+namespace {
+// Device copies of the host arrays of one host-buffer entry, on the stream `st`. Each array is recorded once, with its
+// element count: in() uploads it, out() downloads it in finish(), inout() does both. A null host array stays null. The
+// device memory is freed when the scope ends (early error returns included).
+struct DevScratch {
+  struct Copy { DevArray<unsigned char> dev; void* back = nullptr; size_t bytes = 0; };
+  cudaStream_t st;
+  std::deque<Copy> copies;             // (a deque never moves its elements)
+  cudaError_t err = cudaSuccess;
+  explicit DevScratch(cudaStream_t s) : st(s) {}
+  template <typename T> T* in(const T* host, size_t count) { return add(host, (T*)nullptr, count); }
+  template <typename T> T* out(T* host, size_t count) { return add((const T*)nullptr, host, count); }
+  template <typename T> T* inout(T* host, size_t count) { return add((const T*)host, host, count); }
+  // After the launch: downloads every out / inout array, waits for the stream and reports the first error.
+  int finish(wbc_handle* h) {
+    for (const Copy& c : copies)
+      if (c.back && err == cudaSuccess) err = cudaMemcpyAsync(c.back, c.dev.p, c.bytes, cudaMemcpyDeviceToHost, st);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(st);
+    WBC_SCRATCH_CHECK(h, *this);
+    return WBC_OK;
+  }
+
+ private:
+  template <typename T> T* add(const T* up, T* back, size_t count) {
+    if ((!up && !back) || err != cudaSuccess) return nullptr;
+    Copy& c = copies.emplace_back();
+    c.back = back; c.bytes = count * sizeof(T);
+    err = c.dev.reserve(c.bytes > 0 ? c.bytes : 1);
+    if (err == cudaSuccess && up) err = cudaMemcpyAsync(c.dev.p, up, c.bytes, cudaMemcpyHostToDevice, st);
+    return err == cudaSuccess ? reinterpret_cast<T*>(c.dev.p) : nullptr;
+  }
+};
+}  // namespace
+
 extern "C" int wbc_coriolis_host(wbc_handle* h, int64_t n, const double* q, const double* v, double* Cm, double* Jd) {
   if (!h) return WBC_ERR_ARG;
   if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_coriolis_host: n < 0");
-  if (!q || !v) return fail_arg(h, "wbc_coriolis_host: null input");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  const double* dq = s.in(q, N * WBC_NQ, st); const double* dv = s.in(v, N * WBC_NV, st);
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV);
   double* dC = s.out(Cm, N * 324); double* dJ = s.out(Jd, N * 216);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_coriolis(h, n, dq, dv, dC, dJ, st);
-  if (rc) return rc;
-  s.back(Cm, dC, N * 324, st); s.back(Jd, dJ, N * 216, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_coriolis(h, n, dq, dv, dC, dJ, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_step_pd(wbc_handle* h, int64_t n, const double* q, const double* v, double* tau, void* stream) {
@@ -587,29 +642,9 @@ extern "C" int wbc_step_pd(wbc_handle* h, int64_t n, const double* q, const doub
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
   const long long total = (long long)n * WBC_NU;
-  wbc_pd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_const, q, v, tau, n);
+  wbc_pd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_const.p, q, v, tau, n);
   h->launches++;
   WBC_CUDA(h, cudaGetLastError());
-  return WBC_OK;
-}
-
-// Instances per reduce / solve launch pair of the split path: bounds the hand-over scratch (4224 B per instance) at 1.1 GB
-// while each kernel still runs for milliseconds, so the drain at the kernel boundaries stays below ~1 % of the step.
-constexpr int64_t SPLIT_CHUNK = 262144;
-
-// Grows the hand-over scratch of `slot` to `n` instances (never inside a stream capture: callers that capture call this first).
-static int ensure_split_scratch(wbc_handle* h, int slot, int64_t n, bool with_vd) {
-  const int64_t m = n < SPLIT_CHUNK ? n : SPLIT_CHUNK;
-  if (m > h->rec_cap[slot]) {
-    cudaFree(h->d_rec[slot]); h->d_rec[slot] = nullptr; h->rec_cap[slot] = 0;
-    WBC_CUDA(h, cudaMalloc(&h->d_rec[slot], m * wbc::REC_DOUBLES * sizeof(double)));
-    h->rec_cap[slot] = m;
-  }
-  if (with_vd && m > h->vdmap_cap[slot]) {
-    cudaFree(h->d_vdmap[slot]); h->d_vdmap[slot] = nullptr; h->vdmap_cap[slot] = 0;
-    WBC_CUDA(h, cudaMalloc(&h->d_vdmap[slot], m * wbc::VDMAP_DOUBLES * sizeof(double)));
-    h->vdmap_cap[slot] = m;
-  }
   return WBC_OK;
 }
 
@@ -730,46 +765,48 @@ static bool capturing(cudaStream_t st) {
   return cap != cudaStreamCaptureStatusNone;
 }
 
-static bool aligned16p(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // The hand-over scratch of a slot belongs to one step at a time. A step on another stream than the slot's previous user is
 // ordered behind everything submitted to that stream so far (event dependency; never inside a stream capture, where the
 // caller owns the ordering).
-static int order_slot(wbc_handle* h, int slot, cudaStream_t st) {
-  if (h->slot_used[slot] && h->last_stream[slot] != st && !capturing(st)) {
-    if (cudaEventRecord(h->order_ev, h->last_stream[slot]) == cudaSuccess) WBC_CUDA(h, cudaStreamWaitEvent(st, h->order_ev, 0));
+static int order_slot(wbc_handle* h, Slot& s, cudaStream_t st) {
+  if (s.used && s.last_stream != st && !capturing(st)) {
+    if (cudaEventRecord(h->order_ev, s.last_stream) == cudaSuccess) WBC_CUDA(h, cudaStreamWaitEvent(st, h->order_ev, 0));
     else cudaGetLastError();      // the previous stream no longer exists: its work has completed
   }
-  h->slot_used[slot] = true;
-  h->last_stream[slot] = st;
+  s.used = true;
+  s.last_stream = st;
   return WBC_OK;
 }
 
 template <int KIND>
 static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is) {
-  int rc = ensure_split_scratch(h, slot, n, io.vd != nullptr);
+  Slot& sl = h->slot[slot];
+  WBC_CUDA(h, sl.reserve(n, io.vd != nullptr));
+  const int rc = order_slot(h, sl, st);
   if (rc) return rc;
-  rc = order_slot(h, slot, st);
-  if (rc) return rc;
-  double* vdmap = io.vd ? h->d_vdmap[slot] : nullptr;
+  const DevConst* dc = h->d_const.p;
+  double* rec = sl.rec.p;
+  double* vdmap = io.vd ? sl.vdmap.p : nullptr;
   for (int64_t o = 0; o < n; o += SPLIT_CHUNK) {
     const int64_t m = (n - o) < SPLIT_CHUNK ? (n - o) : SPLIT_CHUNK;
     const wbc::StepArgs a = step_args(io_at(io, o), m, kind);
     // bulk input staging needs 16-byte aligned rows at the CTA boundaries (chunk offsets are multiples of 4)
-    const bool al_vt = aligned16p(a.v) && aligned16p(a.traj), al_qc = aligned16p(a.q) && aligned16p(a.contact);
+    const bool al_vt = aligned16(a.v) && aligned16(a.traj), al_qc = aligned16(a.q) && aligned16(a.contact);
     if (is.profile) cudaEventRecord(h->prof_ev[0], st);
     if (is.host_mapped || KIND == WBC_CTRL_PC) {   // zero-copy call of wbc_step_host: 4-warp CTAs, every array staged per CTA
                                                    // (PC / MPTC too: 20.0 vs 19.7 M steps/s with single-warp CTAs)
       constexpr int W = (KIND == WBC_CTRL_PC) ? WARPS_PC : WARPS_HOST;
       const unsigned grid = (unsigned)((m + W - 1) / W);
       const int bulk_ok = al_vt && al_qc;
-      if constexpr (KIND == WBC_CTRL_PC) wbc_reduce_pc_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
-      else wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
+      if constexpr (KIND == WBC_CTRL_PC) wbc_reduce_pc_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      else wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
     } else {
       constexpr int W = WARPS;
       const unsigned grid = (unsigned)((m + W - 1) / W);
       const int bulk_ok = al_vt;
-      if constexpr (KIND != WBC_CTRL_PC) wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(h->d_const, a, h->d_rec[slot], vdmap, bulk_ok);
+      if constexpr (KIND != WBC_CTRL_PC) wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
     }
     if (is.profile) cudaEventRecord(h->prof_ev[1], st);
     const unsigned sgrid = (unsigned)((m + SOLVE_WARPS - 1) / SOLVE_WARPS);
@@ -782,10 +819,10 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cu
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-    const double* crec = h->d_rec[slot];
+    const double* crec = rec;
     const double* cvd = vdmap;
-    if (with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, true>, (const DevConst*)h->d_const, a, crec, cvd));
-    else WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, false>, (const DevConst*)h->d_const, a, crec, cvd));
+    if (with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, true>, dc, a, crec, cvd));
+    else WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, false>, dc, a, crec, cvd));
     if (is.profile) cudaEventRecord(h->prof_ev[2], st);
     h->launches += 2;
   }
@@ -820,8 +857,8 @@ static int device_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cud
   if (profile || n < CHUNKED_STEP_MIN || n > CHUNKED_STEP_MAX || capturing(st))
     return step_launch(h, kind, n, *io, st, 0, Issue{false, false, profile});
   const int k = device_step_chunks(n);
-  cudaStream_t lanes[WBC_NSLOT] = {st, h->stream2};
-  for (int c = 2; c < k; ++c) lanes[c] = h->xstream[c];
+  cudaStream_t lanes[WBC_NSLOT] = {st};
+  for (int c = 1; c < k; ++c) lanes[c] = h->lane[c];
   const int rc = streams_wait(h, h->order_ev, st, lanes + 1, k - 1);
   if (rc) return rc;
   return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
@@ -846,31 +883,13 @@ WBC_STEP_WRAPPER(wbc_step_clf, WBC_CTRL_CLF)
 WBC_STEP_WRAPPER(wbc_step_pc, WBC_CTRL_PC)
 WBC_STEP_WRAPPER(wbc_step_mptc, WBC_CTRL_MPTC)
 
-static int ensure_staging(wbc_handle* h, int64_t n) {
-  if (n <= h->cap) return WBC_OK;
-  free_staging(h);
-  WBC_CUDA(h, cudaMalloc(&h->d_q, n * WBC_NQ * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_v, n * WBC_NV * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_traj, n * WBC_NTRAJ * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_contact, n * 4));
-  WBC_CUDA(h, cudaMalloc(&h->d_tau, n * WBC_NU * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_metrics, n * WBC_NMETRIC * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_status, n * sizeof(int32_t)));
-  WBC_CUDA(h, cudaMalloc(&h->d_vd, n * WBC_NV * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_f, n * 12 * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_info, n * 4 * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->d_lam, n * WBC_NLAM * sizeof(double)));
-  h->cap = n;
-  return WBC_OK;
-}
-
 // Enqueues one host-buffer step on the handle's two internal streams without waiting for it; `wait` must follow before the
 // outputs are read or the next step is enqueued on this handle (wbc_step_host = enqueue + wait; wbc_multi_step_host enqueues on
 // every device first and waits afterwards, so the devices run side by side from one host thread).
 static int step_host_wait(wbc_handle* h) {
   WBC_CUDA(h, cudaSetDevice(h->device));
-  WBC_CUDA(h, cudaStreamSynchronize(h->stream));
-  WBC_CUDA(h, cudaStreamSynchronize(h->stream2));
+  WBC_CUDA(h, cudaStreamSynchronize(h->lane[0]));
+  WBC_CUDA(h, cudaStreamSynchronize(h->lane[1]));
   return WBC_OK;
 }
 
@@ -882,7 +901,7 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
   if (!io->q || !io->v || !io->tau || (!pd && (!io->traj || !io->contact || !io->metrics || !io->status)))
     return fail_arg(h, "wbc_step_host: q, v, traj, contact, tau, metrics and status are required");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  const cudaStream_t lanes[2] = {h->stream, h->stream2};
+  const Staging& sg = h->stage;
   // Zero-copy path: when every buffer is page-locked host memory (wbc_host_alloc / cudaHostRegister) the kernel reads
   // its 732 B of inputs and writes its 132 B of outputs per instance straight over the host link - one launch, no
   // staging copies, the transfers of one warp overlap the arithmetic of the others.
@@ -894,12 +913,11 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
     const bool stage_in = stage_pinned_inputs(kind, n), staged = stage_in && !pd;
     const int k = pinned_chunks(n, stage_in);
     if (staged) {
-      const int rc = ensure_staging(h, n);
-      if (rc) return rc;
-      hio.q = h->d_q; hio.v = h->d_v; hio.traj = h->d_traj; hio.contact = h->d_contact;
+      WBC_CUDA(h, h->stage.reserve(n));
+      hio.q = sg.q.p; hio.v = sg.v.p; hio.traj = sg.traj.p; hio.contact = sg.contact.p;
     }
     return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
-      const cudaStream_t st = lanes[c & 1];
+      const cudaStream_t st = h->lane[c & 1];
       const wbc_io s = io_at(*io, o), d = io_at(hio, o);
       if (staged) {
         WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -910,14 +928,13 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
       return pd ? wbc_step_pd(h, m, d.q, d.v, d.tau, st) : step_launch(h, kind, m, d, st, c & 1, Issue{!staged, k > 1});
     });
   }
-  const int rc = ensure_staging(h, n);
-  if (rc) return rc;
+  WBC_CUDA(h, h->stage.reserve(n));
   // pageable buffers: the device staging rows, with the optional outputs the caller asked for
-  const wbc_io dev{h->d_q, h->d_v, h->d_traj, h->d_contact, h->d_tau, h->d_metrics, h->d_status, io->vd ? h->d_vd : nullptr,
-                   io->f ? h->d_f : nullptr, io->qp_info ? h->d_info : nullptr, io->lam ? h->d_lam : nullptr};
+  const wbc_io dev{sg.q.p, sg.v.p, sg.traj.p, sg.contact.p, sg.tau.p, sg.metrics.p, sg.status.p, io->vd ? sg.vd.p : nullptr,
+                   io->f ? sg.f.p : nullptr, io->qp_info ? sg.info.p : nullptr, io->lam ? sg.lam.p : nullptr};
   const int k = pageable_chunks(n);
   return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
-    const cudaStream_t st = lanes[c & 1];
+    const cudaStream_t st = h->lane[c & 1];
     const wbc_io s = io_at(*io, o), d = io_at(dev, o);
     WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
     WBC_CUDA(h, cudaMemcpyAsync((void*)d.v, s.v, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -951,13 +968,11 @@ extern "C" int wbc_step_host(wbc_handle* h, int kind, int64_t n, const wbc_io* i
 // handle per device; a call splits [0, n) into contiguous equal shards (SURVEY 8e), enqueues each shard on its device and
 // waits for all of them: the outputs land in the caller's (page-locked or pageable) host arrays, which IS the host gather.
 struct wbc_multi {
-  std::vector<wbc_handle*> h;
+  std::vector<std::unique_ptr<wbc_handle>> h;
   std::string err;
 };
 
 extern "C" int wbc_multi_destroy(wbc_multi* m) {
-  if (!m) return WBC_OK;
-  for (wbc_handle* h : m->h) wbc_destroy(h);
   delete m;
   return WBC_OK;
 }
@@ -970,7 +985,7 @@ extern "C" int wbc_multi_create(const wbc_model* model, const wbc_params* params
   for (int i = 0; i < n_devices; ++i) {
     wbc_handle* h = nullptr;
     const int rc = wbc_create(model, params, devices ? devices[i] : i, &h);
-    if (h) m->h.push_back(h);
+    if (h) m->h.emplace_back(h);
     if (rc) { m->err = h ? h->err : "wbc_create failed"; *out = m; return rc; }
   }
   *out = m;
@@ -981,7 +996,7 @@ extern "C" const char* wbc_multi_last_error(const wbc_multi* m) { return m ? m->
 extern "C" int wbc_multi_device_count(const wbc_multi* m) { return m ? (int)m->h.size() : 0; }
 extern "C" int64_t wbc_multi_launch_count(const wbc_multi* m) {
   int64_t s = 0;
-  if (m) for (const wbc_handle* h : m->h) s += h->launches;
+  if (m) for (const auto& h : m->h) s += h->launches;
   return s;
 }
 
@@ -1003,12 +1018,12 @@ extern "C" int wbc_multi_step_host(wbc_multi* m, int kind, int64_t n, const wbc_
     shard_of(n, r, w, &lo, &hi);
     if (hi <= lo) { ++enq; continue; }
     const wbc_io sio = io_at(*io, lo);
-    rc = step_host_enqueue(m->h[r], kind, hi - lo, &sio);
+    rc = step_host_enqueue(m->h[r].get(), kind, hi - lo, &sio);
     if (rc) m->err = m->h[r]->err;
     ++enq;
   }
   for (int r = 0; r < enq && r < w; ++r) {                 // always drain what was enqueued, even after an error
-    const int rw = step_host_wait(m->h[r]);
+    const int rw = step_host_wait(m->h[r].get());
     if (rw && rc == WBC_OK) { rc = rw; m->err = m->h[r]->err; }
   }
   return rc;
@@ -1018,22 +1033,15 @@ extern "C" int wbc_dynamics_host(wbc_handle* h, int64_t n, const double* q, cons
                                  double* taug, double* Jfeet, double* Jdv, double* pfeet) {
   if (!h) return WBC_ERR_ARG;
   if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_dynamics_host: n < 0");
-  if (!q || !v) return fail_arg(h, "wbc_dynamics_host: null input");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  const double* dq = s.in(q, N * WBC_NQ, st); const double* dv = s.in(v, N * WBC_NV, st);
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV);
   double* dM = s.out(M, N * 324); double* dCv = s.out(Cv, N * 18); double* dtg = s.out(taug, N * 18);
   double* dJ = s.out(Jfeet, N * 216); double* dJdv = s.out(Jdv, N * 12); double* dp = s.out(pfeet, N * 12);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_dynamics(h, n, dq, dv, dM, dCv, dtg, dJ, dJdv, dp, st);
-  if (rc) return rc;
-  s.back(M, dM, N * 324, st); s.back(Cv, dCv, N * 18, st); s.back(taug, dtg, N * 18, st);
-  s.back(Jfeet, dJ, N * 216, st); s.back(Jdv, dJdv, N * 12, st); s.back(pfeet, dp, N * 12, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_dynamics(h, n, dq, dv, dM, dCv, dtg, dJ, dJdv, dp, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_time_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, int reps, void* stream,
@@ -1042,19 +1050,18 @@ extern "C" int wbc_time_step(wbc_handle* h, int kind, int64_t n, const wbc_io* i
   if (!ms_per_launch || reps <= 0) return fail_arg(h, "wbc_time_step: bad arguments");
   WBC_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
-  cudaEvent_t e0, e1;
-  WBC_CUDA(h, cudaEventCreate(&e0));
-  WBC_CUDA(h, cudaEventCreate(&e1));
+  Event e0, e1;
+  WBC_CUDA(h, cudaEventCreate(&e0.v));
+  WBC_CUDA(h, cudaEventCreate(&e1.v));
   WBC_CUDA(h, cudaEventRecord(e0, st));
   for (int r = 0; r < reps; ++r) {
-    int rc = wbc_step(h, kind, n, io, stream);
-    if (rc) { cudaEventDestroy(e0); cudaEventDestroy(e1); return rc; }
+    const int rc = wbc_step(h, kind, n, io, stream);
+    if (rc) return rc;
   }
   WBC_CUDA(h, cudaEventRecord(e1, st));
   WBC_CUDA(h, cudaEventSynchronize(e1));
   float ms = 0.f;
   WBC_CUDA(h, cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
   *ms_per_launch = (double)ms / reps;
   return WBC_OK;
 }
@@ -1066,7 +1073,6 @@ extern "C" int wbc_profile_step(wbc_handle* h, int kind, int64_t n, const wbc_io
   if (!h) return WBC_ERR_ARG;
   if (!ms_reduce || !ms_solve || reps <= 0 || n <= 0 || n > SPLIT_CHUNK || kind == WBC_CTRL_PD) return fail_arg(h, "wbc_profile_step: bad arguments");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  for (int i = 0; i < 3; ++i) if (!h->prof_ev[i]) WBC_CUDA(h, cudaEventCreate(&h->prof_ev[i]));
   double r = 0.0, s = 0.0;
   for (int k = 0; k < reps; ++k) {
     const int rc = device_step(h, kind, n, io, (cudaStream_t)stream, true);
@@ -1086,7 +1092,6 @@ static unsigned wire_grid(const wbc_handle* h, int64_t n, int tile) {
   const int64_t tiles = (n + tile - 1) / tile, cap = (int64_t)h->sm_count * 8;     // grid-stride over tiles
   return (unsigned)(tiles < cap ? tiles : cap);
 }
-static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 extern "C" int wbc_lcm_decode_trunk_state(wbc_handle* h, int64_t n, const uint8_t* msgs, double* timestamp, uint8_t* finished,
                                           double* traj, uint8_t* contact, double* f_plan, int32_t* status, void* stream) {
@@ -1138,7 +1143,7 @@ extern "C" int wbc_lcm_encode_robot_state(wbc_handle* h, int64_t n, const double
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
   wbcwire::encode_robot_kernel<<<wire_grid(h, n, wbcwire::RTILE), wbcwire::THREADS, 0, (cudaStream_t)stream>>>(
-      msgs, n, q, v, tau, tau_in_actuator_order ? h->d_tau_map : nullptr, status);
+      msgs, n, q, v, tau, tau_in_actuator_order ? h->d_tau_map.p : nullptr, status);
   h->launches++;
   WBC_CUDA(h, cudaGetLastError());
   return WBC_OK;
@@ -1147,100 +1152,74 @@ extern "C" int wbc_lcm_encode_robot_state(wbc_handle* h, int64_t n, const double
 extern "C" int wbc_lcm_decode_trunk_state_host(wbc_handle* h, int64_t n, const uint8_t* msgs, double* timestamp, uint8_t* finished,
                                                double* traj, uint8_t* contact, double* f_plan, int32_t* status) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || (n > 0 && (!msgs || !traj || !contact))) return fail_arg(h, "wbc_lcm_decode_trunk_state_host: msgs, traj and contact are required");
-  if (n == 0) return WBC_OK;
+  if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_lcm_decode_trunk_state_host: n < 0");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  uint8_t* dm = s.in(msgs, N * WBC_LCM_TRUNK_STATE_BYTES, st);
+  uint8_t* dm = s.in(msgs, N * WBC_LCM_TRUNK_STATE_BYTES);
   double* dts = s.out(timestamp, N); uint8_t* dfin = s.out(finished, N);
   double* dtr = s.out(traj, N * WBC_NTRAJ); uint8_t* dc = s.out(contact, N * 4);
   double* dfp = s.out(f_plan, N * 12); int32_t* dst = s.out(status, N);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_lcm_decode_trunk_state(h, n, dm, dts, dfin, dtr, dc, dfp, dst, st);
-  if (rc) return rc;
-  s.back(timestamp, dts, N, st); s.back(finished, dfin, N, st); s.back(traj, dtr, N * WBC_NTRAJ, st);
-  s.back(contact, dc, N * 4, st); s.back(f_plan, dfp, N * 12, st); s.back(status, dst, N, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_lcm_decode_trunk_state(h, n, dm, dts, dfin, dtr, dc, dfp, dst, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_lcm_encode_trunk_state_host(wbc_handle* h, int64_t n, const double* timestamp, const uint8_t* finished,
                                                const double* traj, const uint8_t* contact, const double* f_plan, uint8_t* msgs) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || (n > 0 && (!msgs || !traj || !contact))) return fail_arg(h, "wbc_lcm_encode_trunk_state_host: msgs, traj and contact are required");
-  if (n == 0) return WBC_OK;
+  if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_lcm_encode_trunk_state_host: n < 0");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  const double* dts = s.in(timestamp, N, st); const uint8_t* dfin = s.in(finished, N, st);
-  const double* dtr = s.in(traj, N * WBC_NTRAJ, st); const uint8_t* dc = s.in(contact, N * 4, st);
-  const double* dfp = s.in(f_plan, N * 12, st);
+  const double* dts = s.in(timestamp, N); const uint8_t* dfin = s.in(finished, N);
+  const double* dtr = s.in(traj, N * WBC_NTRAJ); const uint8_t* dc = s.in(contact, N * 4);
+  const double* dfp = s.in(f_plan, N * 12);
   uint8_t* dm = s.out(msgs, N * WBC_LCM_TRUNK_STATE_BYTES);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_lcm_encode_trunk_state(h, n, dts, dfin, dtr, dc, dfp, dm, st);
-  if (rc) return rc;
-  s.back(msgs, dm, N * WBC_LCM_TRUNK_STATE_BYTES, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_lcm_encode_trunk_state(h, n, dts, dfin, dtr, dc, dfp, dm, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_lcm_decode_robot_state_host(wbc_handle* h, int64_t n, const uint8_t* msgs, double* q, double* v, double* tau,
                                                int32_t* status) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || (n > 0 && (!msgs || !q || !v))) return fail_arg(h, "wbc_lcm_decode_robot_state_host: msgs, q and v are required");
-  if (n == 0) return WBC_OK;
+  if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_lcm_decode_robot_state_host: n < 0");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  uint8_t* dm = s.in(msgs, N * WBC_LCM_ROBOT_STATE_BYTES, st);
+  uint8_t* dm = s.in(msgs, N * WBC_LCM_ROBOT_STATE_BYTES);
   double* dq = s.out(q, N * WBC_NQ); double* dv = s.out(v, N * WBC_NV); double* dt = s.out(tau, N * WBC_NU);
   int32_t* dst = s.out(status, N);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_lcm_decode_robot_state(h, n, dm, dq, dv, dt, dst, st);
-  if (rc) return rc;
-  s.back(q, dq, N * WBC_NQ, st); s.back(v, dv, N * WBC_NV, st); s.back(tau, dt, N * WBC_NU, st); s.back(status, dst, N, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_lcm_decode_robot_state(h, n, dm, dq, dv, dt, dst, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_lcm_encode_robot_state_host(wbc_handle* h, int64_t n, const double* q, const double* v, const double* tau,
                                                int tau_in_actuator_order, uint8_t* msgs, int32_t* status) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || (n > 0 && (!msgs || !tau))) return fail_arg(h, "wbc_lcm_encode_robot_state_host: msgs and tau are required");
-  if (n == 0) return WBC_OK;
+  if (n <= 0) return n == 0 ? WBC_OK : fail_arg(h, "wbc_lcm_encode_robot_state_host: n < 0");
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  const double* dq = s.in(q, N * WBC_NQ, st); const double* dv = s.in(v, N * WBC_NV, st); const double* dt = s.in(tau, N * WBC_NU, st);
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV); const double* dt = s.in(tau, N * WBC_NU);
   uint8_t* dm = s.out(msgs, N * WBC_LCM_ROBOT_STATE_BYTES); int32_t* dst = s.out(status, N);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_lcm_encode_robot_state(h, n, dq, dv, dt, tau_in_actuator_order, dm, dst, st);
-  if (rc) return rc;
-  s.back(msgs, dm, N * WBC_LCM_ROBOT_STATE_BYTES, st); s.back(status, dst, N, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_lcm_encode_robot_state(h, n, dq, dv, dt, tau_in_actuator_order, dm, dst, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 // ------------------------------------------------------------------------------ trajectory sampler (wbc_traj.cuh)
+// A plan keeps the number of the device its tables live on, not its handle: it may be destroyed after the handle.
 struct wbc_plan {
-  wbc_handle* h = nullptr;
+  int device = 0;
   wbctraj::PlanTables t{};
-  std::vector<void*> bufs;
+  std::deque<DevArray<unsigned char>> bufs;
+  ~wbc_plan() { cudaSetDevice(device); }   // the tables are freed after this, on the plan's device
 };
 
 extern "C" int wbc_plan_destroy(wbc_plan* p) {
-  if (!p) return WBC_OK;
-  if (p->h) cudaSetDevice(p->h->device);
-  for (void* b : p->bufs) cudaFree(b);
   delete p;
   return WBC_OK;
 }
@@ -1293,18 +1272,16 @@ extern "C" int wbc_plan_create(wbc_handle* h, int32_t n_plans, const wbc_plan_de
   }
   if (grid_ts.empty()) grid_ts.push_back(0.0);
   WBC_CUDA(h, cudaSetDevice(h->device));
-  wbc_plan* pl = new (std::nothrow) wbc_plan();
+  std::unique_ptr<wbc_plan> pl(new (std::nothrow) wbc_plan());
   if (!pl) return WBC_ERR_NOMEM;
-  pl->h = h;
+  pl->device = h->device;
   cudaError_t err = cudaSuccess;
   auto up = [&](const void* src, size_t bytes) -> void* {
-    void* dptr = nullptr;
     if (err != cudaSuccess) return nullptr;
-    err = cudaMalloc(&dptr, bytes ? bytes : 1);
-    if (err != cudaSuccess) return nullptr;
-    pl->bufs.push_back(dptr);
-    if (src) err = cudaMemcpy(dptr, src, bytes, cudaMemcpyHostToDevice);
-    return dptr;
+    DevArray<unsigned char>& d = pl->bufs.emplace_back();
+    err = d.reserve(bytes ? bytes : 1);
+    if (err == cudaSuccess && src) err = cudaMemcpy(d.p, src, bytes, cudaMemcpyHostToDevice);
+    return err == cudaSuccess ? d.p : nullptr;
   };
   const int n_poly_total = (int)tend.size();
   pl->t.n_plans = n_plans;
@@ -1323,17 +1300,16 @@ extern "C" int wbc_plan_create(wbc_handle* h, int32_t n_plans, const wbc_plan_de
   const double* d_nodes = (const double*)up(nodes.data(), nodes.size() * sizeof(double));
   const double* d_dur = (const double*)up(dur.data(), dur.size() * sizeof(double));
   if (err == cudaSuccess) {
-    wbctraj::hermite_coeff_kernel<<<(n_poly_total * 3 + 255) / 256, 256, 0, h->stream>>>(n_poly_total, d_node_of, d_nodes, d_dur, d_coef);
+    wbctraj::hermite_coeff_kernel<<<(n_poly_total * 3 + 255) / 256, 256, 0, h->lane[0]>>>(n_poly_total, d_node_of, d_nodes, d_dur, d_coef);
     h->launches++;
     err = cudaGetLastError();
-    if (err == cudaSuccess) err = cudaStreamSynchronize(h->stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(h->lane[0]);
   }
   if (err != cudaSuccess) {
     h->err = std::string("wbc_plan_create: ") + cudaGetErrorString(err);
-    wbc_plan_destroy(pl);
     return WBC_ERR_CUDA;
   }
-  *out = pl;
+  *out = pl.release();
   return WBC_OK;
 }
 
@@ -1359,30 +1335,23 @@ extern "C" int wbc_sample_trajectory(wbc_handle* h, const wbc_plan* plan, int64_
 extern "C" int wbc_sample_trajectory_host(wbc_handle* h, const wbc_plan* plan, int64_t n, const int32_t* plan_index, const double* t,
                                           double* traj, uint8_t* contact, double* f_plan, double* t_eval, int32_t* status) {
   if (!h) return WBC_ERR_ARG;
-  if (!plan || n < 0 || (n > 0 && (!t || !traj || !contact))) return fail_arg(h, "wbc_sample_trajectory_host: plan, t, traj and contact are required");
+  if (!plan || n < 0) return fail_arg(h, "wbc_sample_trajectory_host: plan and n >= 0 are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  const int32_t* dpi = s.in(plan_index, N, st); const double* dt = s.in(t, N, st);
+  const int32_t* dpi = s.in(plan_index, N); const double* dt = s.in(t, N);
   double* dtr = s.out(traj, N * WBC_NTRAJ); uint8_t* dc = s.out(contact, N * 4); double* dfp = s.out(f_plan, N * 12);
   double* dte = s.out(t_eval, N); int32_t* dst = s.out(status, N);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_sample_trajectory(h, plan, n, dpi, dt, dtr, dc, dfp, dte, dst, st);
-  if (rc) return rc;
-  s.back(traj, dtr, N * WBC_NTRAJ, st); s.back(contact, dc, N * 4, st); s.back(f_plan, dfp, N * 12, st);
-  s.back(t_eval, dte, N, st); s.back(status, dst, N, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_sample_trajectory(h, plan, n, dpi, dt, dtr, dc, dfp, dte, dst, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 // Control step whose trunk targets come from a device-resident plan: the host sends q, v and the plan time only (300 B + 8 B
 // per instance instead of 732 B - the 54-double trajectory row is 59 % of the step's input bytes), wbc_sample_trajectory fills
 // traj / contact in device scratch and the step kernels read them from there. Page-locked buffers are read / written by the
 // kernels directly (zero-copy), pageable ones are staged.
-static int ensure_rollout_scratch(wbc_handle* h, int64_t n);
 extern "C" int wbc_step_plan_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, const double* q, const double* v,
                                   const double* t, const int32_t* plan_index, double* tau, double* metrics, int32_t* status) {
   if (!h) return WBC_ERR_ARG;
@@ -1390,44 +1359,45 @@ extern "C" int wbc_step_plan_host(wbc_handle* h, int kind, const wbc_plan* plan,
   if (n > 0 && (!q || !v || !t || !tau || !metrics || !status)) return fail_arg(h, "wbc_step_plan_host: q, v, t, tau, metrics and status are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  int rc = ensure_rollout_scratch(h, n);
-  if (rc) return rc;
-  cudaStream_t st = h->stream;
+  WBC_CUDA(h, h->ro.reserve(n));
+  const RolloutScratch& ro = h->ro;
+  const Staging& sg = h->stage;
+  const cudaStream_t st = h->lane[0];
+  int rc;
   if (to_device_aliases(q, v, t, plan_index, tau, metrics, status)) {   // from here on the kernels' aliases of the host arrays
-    rc = wbc_sample_trajectory(h, plan, n, plan_index, t, h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
+    rc = wbc_sample_trajectory(h, plan, n, plan_index, t, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
     if (rc) return rc;
     // the step itself as in the zero-copy mode of wbc_step_host: two halves on the two internal streams. q and v are 304 B per
     // instance, which the reduce CTAs pull over the link without slowing down at any batch size (57.3 M steps/s at 65536,
     // 60.8 M at 2^20; copy-engine staging of q and v: 51.5 / 60.6 M)
     const int k = pinned_chunks(n, false);
-    const cudaStream_t lanes[2] = {st, h->stream2};
+    const cudaStream_t lanes[2] = {st, h->lane[1]};
     if (k > 1) {
       rc = streams_wait(h, h->order_ev, st, lanes + 1, 1);   // the sampled rows
       if (rc) return rc;
     }
-    const wbc_io zio{q, v, h->ro_traj, h->ro_contact, tau, metrics, status};
+    const wbc_io zio{q, v, ro.traj.p, ro.contact.p, tau, metrics, status};
     rc = for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
       return step_launch(h, kind, m, io_at(zio, o), lanes[c & 1], c & 1, Issue{true, k > 1});
     });
     if (rc) return rc;
     return step_host_wait(h);
   }
-  rc = ensure_staging(h, n);
-  if (rc) return rc;
-  DevScratch s;
-  const int32_t* dpi = s.in(plan_index, (size_t)n, st);
+  WBC_CUDA(h, h->stage.reserve(n));
+  DevScratch s(st);
+  const int32_t* dpi = s.in(plan_index, (size_t)n);
   WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaMemcpyAsync(h->d_q, q, n * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
-  WBC_CUDA(h, cudaMemcpyAsync(h->d_v, v, n * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
-  WBC_CUDA(h, cudaMemcpyAsync(h->ro_t, t, n * sizeof(double), cudaMemcpyHostToDevice, st));
-  rc = wbc_sample_trajectory(h, plan, n, dpi, h->ro_t, h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
+  WBC_CUDA(h, cudaMemcpyAsync(sg.q.p, q, n * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
+  WBC_CUDA(h, cudaMemcpyAsync(sg.v.p, v, n * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
+  WBC_CUDA(h, cudaMemcpyAsync(ro.t.p, t, n * sizeof(double), cudaMemcpyHostToDevice, st));
+  rc = wbc_sample_trajectory(h, plan, n, dpi, ro.t.p, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
   if (rc) return rc;
-  const wbc_io io{h->d_q, h->d_v, h->ro_traj, h->ro_contact, h->d_tau, h->d_metrics, h->d_status};
+  const wbc_io io{sg.q.p, sg.v.p, ro.traj.p, ro.contact.p, sg.tau.p, sg.metrics.p, sg.status.p};
   rc = step_launch(h, kind, n, io, st, 0, Issue{});
   if (rc) return rc;
-  WBC_CUDA(h, cudaMemcpyAsync(tau, h->d_tau, n * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
-  WBC_CUDA(h, cudaMemcpyAsync(metrics, h->d_metrics, n * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
-  WBC_CUDA(h, cudaMemcpyAsync(status, h->d_status, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  WBC_CUDA(h, cudaMemcpyAsync(tau, sg.tau.p, n * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
+  WBC_CUDA(h, cudaMemcpyAsync(metrics, sg.metrics.p, n * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
+  WBC_CUDA(h, cudaMemcpyAsync(status, sg.status.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   WBC_CUDA(h, cudaStreamSynchronize(st));
   return WBC_OK;
 }
@@ -1445,23 +1415,6 @@ extern "C" int wbc_integrate(wbc_handle* h, int64_t n, double dt, double* q, dou
   return WBC_OK;
 }
 
-static int ensure_rollout_scratch(wbc_handle* h, int64_t n) {
-  if (!h->ro_counter) WBC_CUDA(h, cudaMalloc(&h->ro_counter, sizeof(int)));
-  if (n <= h->ro_cap) return WBC_OK;
-  cudaFree(h->ro_traj); cudaFree(h->ro_vd); cudaFree(h->ro_metrics); cudaFree(h->ro_tau); cudaFree(h->ro_t);
-  cudaFree(h->ro_contact); cudaFree(h->ro_status);
-  h->ro_traj = h->ro_vd = h->ro_metrics = h->ro_tau = h->ro_t = nullptr; h->ro_contact = nullptr; h->ro_status = nullptr; h->ro_cap = 0;
-  WBC_CUDA(h, cudaMalloc(&h->ro_traj, n * WBC_NTRAJ * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->ro_vd, n * WBC_NV * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->ro_metrics, n * WBC_NMETRIC * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->ro_tau, n * WBC_NU * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->ro_t, n * sizeof(double)));
-  WBC_CUDA(h, cudaMalloc(&h->ro_contact, n * 4));
-  WBC_CUDA(h, cudaMalloc(&h->ro_status, n * sizeof(int32_t)));
-  h->ro_cap = n;
-  return WBC_OK;
-}
-
 extern "C" int wbc_default_plant_opts(wbc_plant_opts* o) {
   if (!o) return WBC_ERR_ARG;
   o->mu = 1.0; o->erp = 0.2; o->iters = 30; o->reserved = 0;      // simulate.py:44-46: static = dynamic friction 1.0
@@ -1476,7 +1429,7 @@ static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opt
   if (!(o.mu >= 0.0) || !(o.erp >= 0.0 && o.erp <= 1.0) || o.iters < 1 || o.iters > 1000) return fail_arg(h, "wbc_plant_step: bad options");
   const wbcplant::PlantArgs a{q, v, tau, t, ctrl_status, status_or, f_contact, metrics, err_max, metrics_log, counter, (long long)n, dt,
                               o.mu, o.erp, o.iters};
-  wbc_plant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlant), st>>>(h->d_const, a);
+  wbc_plant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlant), st>>>(h->d_const.p, a);
   h->launches++;
   return WBC_OK;
 }
@@ -1496,23 +1449,17 @@ extern "C" int wbc_plant_step(wbc_handle* h, int64_t n, double dt, const wbc_pla
 extern "C" int wbc_plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, double* q, double* v, const double* tau,
                                    double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || !(dt > 0.0) || (n > 0 && (!q || !v || !tau))) return fail_arg(h, "wbc_plant_step_host: q, v, tau and dt > 0 are required");
+  if (n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_plant_step_host: n >= 0 and dt > 0 are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
-  double* dq = s.in(q, N * WBC_NQ, st); double* dv = s.in(v, N * WBC_NV, st); const double* dtau = s.in(tau, N * WBC_NU, st);
-  double* dt_ = s.in(t, N, st); const int32_t* dcs = s.in(ctrl_status, N, st); int32_t* dso = s.in(status_or, N, st);
+  double* dq = s.inout(q, N * WBC_NQ); double* dv = s.inout(v, N * WBC_NV); const double* dtau = s.in(tau, N * WBC_NU);
+  double* dt_ = s.inout(t, N); const int32_t* dcs = s.in(ctrl_status, N); int32_t* dso = s.inout(status_or, N);
   double* df = s.out(f_contact, N * 12);
   WBC_SCRATCH_CHECK(h, s);
-  const int rc = wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, st);
-  if (rc) return rc;
-  s.back(q, dq, N * WBC_NQ, st); s.back(v, dv, N * WBC_NV, st); s.back(t, dt_, N, st); s.back(status_or, dso, N, st);
-  s.back(f_contact, df, N * 12, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
@@ -1525,62 +1472,59 @@ extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int
   if (n > 0 && (!io->q || !io->v || !io->t)) return fail_arg(h, "wbc_rollout: q, v and t are required");
   if (n == 0 || n_steps == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  int rc = ensure_rollout_scratch(h, n);
-  if (rc) return rc;
-  rc = ensure_split_scratch(h, 0, n, !plant);
-  if (rc) return rc;
+  WBC_CUDA(h, h->ro.reserve(n));
+  WBC_CUDA(h, h->slot[0].reserve(n, !plant));   // before the capture below: a step grows no scratch while being captured
+  const RolloutScratch& ro = h->ro;
   cudaStream_t st = (cudaStream_t)stream;
-  double* tau = io->tau ? io->tau : h->ro_tau;
-  double* metrics = io->metrics ? io->metrics : h->ro_metrics;
-  WBC_CUDA(h, cudaMemsetAsync(h->ro_counter, 0, sizeof(int), st));
+  double* tau = io->tau ? io->tau : ro.tau.p;
+  double* metrics = io->metrics ? io->metrics : ro.metrics.p;
+  WBC_CUDA(h, cudaMemsetAsync(ro.counter.p, 0, sizeof(int), st));
   if (io->status_or) WBC_CUDA(h, cudaMemsetAsync(io->status_or, 0, n * sizeof(int32_t), st));
   if (io->err_max) WBC_CUDA(h, cudaMemsetAsync(io->err_max, 0, n * sizeof(double), st));
   if (kind == WBC_CTRL_PD) {                       // the PD law has no QP: no status / metrics of its own
-    WBC_CUDA(h, cudaMemsetAsync(h->ro_status, 0, n * sizeof(int32_t), st));
+    WBC_CUDA(h, cudaMemsetAsync(ro.status.p, 0, n * sizeof(int32_t), st));
     WBC_CUDA(h, cudaMemsetAsync(metrics, 0, n * WBC_NMETRIC * sizeof(double), st));
   }
   // with the ground plant the controller's accelerations are not needed: the step runs without the vd outputs
-  wbc_io sio{io->q, io->v, h->ro_traj, h->ro_contact, tau, metrics, h->ro_status, plant ? nullptr : h->ro_vd, nullptr, nullptr};
+  wbc_io sio{io->q, io->v, ro.traj.p, ro.contact.p, tau, metrics, ro.status.p, plant ? nullptr : ro.vd.p, nullptr, nullptr};
   auto one_step = [&]() -> int {
-    int r = wbc_sample_trajectory(h, plan, n, io->plan_index, io->t, h->ro_traj, h->ro_contact, nullptr, nullptr, nullptr, st);
+    int r = wbc_sample_trajectory(h, plan, n, io->plan_index, io->t, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
     if (r) return r;
     r = wbc_step(h, kind, n, &sio, st);
     if (r) return r;
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, io->q, io->v, tau, io->t, h->ro_status, io->status_or, opts->f_contact, metrics,
-                       io->err_max, io->metrics_log, h->ro_counter, st);
+      r = plant_launch(h, n, dt, &opts->plant_opts, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
+                       io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
     } else {
-      wbcroll::integrate_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, dt, io->q, io->v, h->ro_vd, io->t, h->ro_status, io->status_or,
-                                                                           metrics, io->err_max, io->metrics_log, h->ro_counter);
+      wbcroll::integrate_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, dt, io->q, io->v, ro.vd.p, io->t, ro.status.p, io->status_or,
+                                                                           metrics, io->err_max, io->metrics_log, ro.counter.p);
       h->launches++;
     }
-    if (io->metrics_log) { wbcroll::bump_counter_kernel<<<1, 1, 0, st>>>(h->ro_counter); h->launches++; }
+    if (io->metrics_log) { wbcroll::bump_counter_kernel<<<1, 1, 0, st>>>(ro.counter.p); h->launches++; }
     return WBC_OK;
   };
   if (use_graph && n_steps > 1 && st != nullptr && st != cudaStreamLegacy) {   // the legacy default stream cannot be captured
     // capture one control step (3-4 kernels) once, replay it n_steps times: one graph launch per step instead of 3-4 kernel launches
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
+    Graph graph;
+    GraphExec exec;
     const int64_t launches0 = h->launches;
     WBC_CUDA(h, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    rc = one_step();
-    cudaError_t e = cudaStreamEndCapture(st, &graph);
+    const int rc = one_step();
+    cudaError_t e = cudaStreamEndCapture(st, &graph.v);
     const int64_t per_step = h->launches - launches0;
-    if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
+    if (rc) return rc;
     if (e != cudaSuccess) { h->err = std::string("wbc_rollout: graph capture: ") + cudaGetErrorString(e); return WBC_ERR_CUDA; }
-    e = cudaGraphInstantiate(&exec, graph, 0);
-    if (e != cudaSuccess) { cudaGraphDestroy(graph); h->err = std::string("wbc_rollout: graph instantiate: ") + cudaGetErrorString(e); return WBC_ERR_CUDA; }
+    e = cudaGraphInstantiate(&exec.v, graph, 0);
+    if (e != cudaSuccess) { h->err = std::string("wbc_rollout: graph instantiate: ") + cudaGetErrorString(e); return WBC_ERR_CUDA; }
     h->launches = launches0;
     for (int k = 0; k < n_steps && e == cudaSuccess; ++k) { e = cudaGraphLaunch(exec, st); h->launches += per_step; }
-    // the exec graph must outlive its launches: wait for the stream before destroying it
+    // the exec graph must outlive its launches: wait for the stream before it is destroyed
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaGraphExecDestroy(exec);
-    cudaGraphDestroy(graph);
     if (e != cudaSuccess) { h->err = std::string("wbc_rollout: graph launch: ") + cudaGetErrorString(e); return WBC_ERR_CUDA; }
   } else {
     for (int k = 0; k < n_steps; ++k) {
-      rc = one_step();
+      const int rc = one_step();
       if (rc) return rc;
     }
   }
@@ -1600,33 +1544,22 @@ extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan
                                    const wbc_rollout_io* io, const wbc_rollout_opts* opts) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
-  if (n > 0 && (!io->q || !io->v || !io->t)) return fail_arg(h, "wbc_rollout_host: q, v and t are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  cudaStream_t st = h->stream;
-  DevScratch s;
+  DevScratch s(h->lane[0]);
   const size_t N = (size_t)n;
   wbc_rollout_io d{};
-  d.q = s.in(io->q, N * WBC_NQ, st); d.v = s.in(io->v, N * WBC_NV, st); d.t = s.in(io->t, N, st);
-  d.plan_index = s.in(io->plan_index, N, st);
+  d.q = s.inout(io->q, N * WBC_NQ); d.v = s.inout(io->v, N * WBC_NV); d.t = s.inout(io->t, N);
+  d.plan_index = s.in(io->plan_index, N);
   d.tau = s.out(io->tau, N * WBC_NU); d.metrics = s.out(io->metrics, N * WBC_NMETRIC);
   d.status_or = s.out(io->status_or, N); d.err_max = s.out(io->err_max, N);
   d.metrics_log = s.out(io->metrics_log, N * WBC_NMETRIC * (size_t)n_steps);
   wbc_rollout_opts o{};
   if (opts) o = *opts; else { o.use_graph = 1; wbc_default_plant_opts(&o.plant_opts); }
-  double* host_f = o.f_contact;
-  o.f_contact = s.out(host_f, N * 12);
+  o.f_contact = s.out(o.f_contact, N * 12);
   WBC_SCRATCH_CHECK(h, s);
-  int rc = wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, st);
-  if (rc) return rc;
-  s.back(io->q, d.q, N * WBC_NQ, st); s.back(io->v, d.v, N * WBC_NV, st); s.back(io->t, d.t, N, st);
-  s.back(io->tau, d.tau, N * WBC_NU, st); s.back(io->metrics, d.metrics, N * WBC_NMETRIC, st);
-  s.back(io->status_or, d.status_or, N, st); s.back(io->err_max, d.err_max, N, st);
-  s.back(io->metrics_log, d.metrics_log, N * WBC_NMETRIC * (size_t)n_steps, st);
-  s.back(host_f, o.f_contact, N * 12, st);
-  WBC_SCRATCH_CHECK(h, s);
-  WBC_CUDA(h, cudaStreamSynchronize(st));
-  return WBC_OK;
+  const int rc = wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
+  return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
@@ -1650,25 +1583,23 @@ extern "C" int wbc_measure_fp64_peak(int device, double* tflops) {
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return WBC_ERR_CUDA;
   const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 15;
-  double* out = nullptr;
-  if (cudaMalloc(&out, (size_t)blocks * threads * sizeof(double)) != cudaSuccess) return WBC_ERR_CUDA;
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
-  fp64_peak_kernel<<<blocks, threads>>>(out, 1024);  // warm-up
+  DevArray<double> out;
+  if (out.reserve((size_t)blocks * threads) != cudaSuccess) return WBC_ERR_CUDA;
+  Event e0, e1;
+  cudaEventCreate(&e0.v); cudaEventCreate(&e1.v);
+  fp64_peak_kernel<<<blocks, threads>>>(out.p, 1024);  // warm-up
   double best = 0.0;
   for (int rep = 0; rep < 5; ++rep) {
     cudaEventRecord(e0);
-    fp64_peak_kernel<<<blocks, threads>>>(out, iters);
+    fp64_peak_kernel<<<blocks, threads>>>(out.p, iters);
     cudaEventRecord(e1);
-    if (cudaEventSynchronize(e1) != cudaSuccess) { cudaFree(out); return WBC_ERR_CUDA; }
+    if (cudaEventSynchronize(e1) != cudaSuccess) return WBC_ERR_CUDA;
     float ms = 0.f;
     cudaEventElapsedTime(&ms, e0, e1);
     const double fl = 2.0 * 8.0 * (double)iters * blocks * threads;
     const double tf = fl / (ms * 1e-3) / 1e12;
     if (tf > best) best = tf;
   }
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(out);
   *tflops = best;
   return WBC_OK;
 }
