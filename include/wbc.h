@@ -23,7 +23,8 @@
  *   - per-instance failures go to status[i] (bit mask below), never abort the batch
  *     (the reference asserts instead: inverse_dynamics_controller.py:224). An instance with ANY status bit set
  *     returns tau = 0 (and f = vd = lam = 0 where requested): an unfinished active-set iterate, a substituted
- *     orientation (bad quaternion, gimbal lock) or a rank-deficient problem never leaves the library as torques.
+ *     orientation (bad quaternion, gimbal lock), a rank-deficient problem or a NaN / inf input never leaves the library as
+ *     torques (WBC_CTRL_PD excepted: it has no status, and a NaN input gives a NaN torque, as np.clip does in the reference).
  *     metrics[1] (err) is still the tracking error of the state; callers must mask on status;
  *   - "device" entry points take device pointers and a cudaStream_t passed as void*;
  *     "_host" entry points take host pointers and do the copies themselves.
@@ -58,12 +59,15 @@ extern "C" {
 #define WBC_ST_OK 0
 #define WBC_ST_MAXITER 1       /* active-set iteration cap reached                       */
 #define WBC_ST_INFEASIBLE 2    /* QP constraints inconsistent                            */
-#define WBC_ST_RANKDEF 4       /* equality constraints rank deficient (e.g. singular leg) */
+#define WBC_ST_RANKDEF 4       /* equality constraints rank deficient (e.g. singular leg)  */
+                               /* a stance leg counts as singular when |det L_k| <= 2e-3 |c0||c1||c2|, L_k its 3x3 foot
+                                * Jacobian block with columns c_j: a test on the sine-volume, independent of the leg's size */
 #define WBC_ST_GIMBAL 8        /* |cos(pitch)| < 1e-6: rpy rates undefined (SURVEY A.7)   */
 #define WBC_ST_NOTPD 16        /* reduced Hessian not positive definite                   */
 #define WBC_ST_BADQUAT 32      /* zero / non-finite quaternion                            */
 #define WBC_ST_UNSUPPORTED 64  /* PC controller with no stance foot (the reference raises too) */
 #define WBC_ST_DIVERGED 128    /* rollout only: non-finite / runaway velocity, instance frozen   */
+#define WBC_ST_NONFINITE 256   /* a NaN / inf among the q, v, traj values of the instance, or a non-finite solution */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -266,7 +270,9 @@ int wbc_lcm_encode_robot_state_host(wbc_handle* h, int64_t n, const double* q, c
 /* ---- Trunk-trajectory sampler (SURVEY 8 f1): TOWR spline solution -> controller input on the device.
  * A plan is what towr's SplineHolder holds after the solve (towr/trunk_mpc.cpp:151-156): cubic Hermite node splines for
  * base position, base Euler angles (rpy), 4 foot positions, 4 foot forces, and the per-foot phase durations. */
-#define WBC_TRAJ_CLAMPED 1   /* t outside [0, total]: evaluated at the nearest end (the reference asserts / runs off) */
+#define WBC_TRAJ_CLAMPED 1   /* t outside [0, total]: evaluated at the nearest end (the reference asserts / runs off);
+                              * a NaN t is flagged and taken as t = 0, with and without a grid (n_grid > 0: standing
+                              * while 0 < wait_time, else the stored sample nearest to 0)                              */
 #define WBC_TRAJ_BADPLAN 2   /* plan index out of range: plan 0 used                                                  */
 
 typedef struct wbc_spline_desc {

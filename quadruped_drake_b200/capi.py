@@ -20,9 +20,11 @@ LIB_PATH = Path(os.environ.get("WBC_LIB") or (Path(__file__).resolve().parent / 
 WBC_CTRL_ID, WBC_CTRL_CLF, WBC_CTRL_PC, WBC_CTRL_MPTC, WBC_CTRL_PD = 0, 1, 2, 3, 4
 KINDS = {"id": WBC_CTRL_ID, "clf": WBC_CTRL_CLF, "pc": WBC_CTRL_PC, "mptc": WBC_CTRL_MPTC, "pd": WBC_CTRL_PD}
 ST_MAXITER, ST_INFEASIBLE, ST_RANKDEF, ST_GIMBAL, ST_NOTPD, ST_BADQUAT, ST_UNSUPPORTED, ST_DIVERGED = 1, 2, 4, 8, 16, 32, 64, 128
+ST_NONFINITE = 256
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
-             ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED"}
+             ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
+             ST_NONFINITE: "NONFINITE"}
 
 
 def status_names(status: int) -> str:

@@ -35,6 +35,12 @@ constexpr int YS = 15;      // row stride of Y: 13 coefficients + constant + 1 p
 constexpr int YROWS = 32;   // 0-5 a_b | 6-17 leg rows (f of a stance leg / task accel of a swing leg) | 18-29 tau | 30,31 extra
 constexpr int AR = 6;       // rows of the reduced base system (the stance-leg rows are eliminated analytically)
 constexpr int AC = 32;      // columns of [A|b]: lane c owns column c, lane 31 the right-hand side
+// A stance leg is RANKDEF when |det L_k| <= RANKDEF_SINVOL * |c0| |c1| |c2| (c_j the columns of its 3x3 foot Jacobian block).
+// The contact rows are solved through L_k^-1, so the error of the leg's joint accelerations grows like 1 / det. Against the
+// oracle (stretched-knee sweep of tests/test_edge_states.py) the vd error of PC reaches 1.6e-7 at a sine-volume of 1.5e-3 on
+// mini_cheetah; from 2e-3 up every unflagged instance of both robots is 10x inside the 1e-5 (tau) / 1e-6 (vd) parity bars.
+// That flags knees within about 4e-3 rad (mini_cheetah) / 5e-3 rad (anymal_b) of the stretched pose.
+constexpr double RANKDEF_SINVOL = 2e-3;
 
 // Host-precomputed constants (wbc_create): per-channel CARE solution of the double integrator and the
 // decay rate gamma of clf_controller.py:170-188 (closed form, SURVEY Appendix C.2).
@@ -523,8 +529,11 @@ WBC_DEV void build_base_system(WarpSmem& s, int lane, unsigned cmask, double kd,
       const V3 c2 = mk(s.L[k][0][i2], s.L[k][1][i2], s.L[k][2][i2]);
       const V3 cx = cross(c1, c2);
       const double det = dot(ci, cx);
-      bad = !(fabs(det) > 1e-12);                              // singular stance leg (stretched knee)
-      const V3 li = frcp(fabs(det) > 1e-12 ? det : 1.0) * cx;  // row i of L_k^-1
+      // singular stance leg (stretched knee): |det| against the product of the column norms, i.e. the sine-volume of the
+      // leg's columns, so that the test does not depend on the leg's size; compared squared (no square root)
+      const double vol2 = dot(ci, ci) * dot(c1, c1) * dot(c2, c2);
+      bad = !(det * det > RANKDEF_SINVOL * RANKDEF_SINVOL * vol2);
+      const V3 li = frcp(bad ? 1.0 : det) * cx;                // row i of L_k^-1
       const V3 rh = ld3(s.rho[k]);
       // Li Jb = [-Li skew(rho) | Li];  li' skew(rho) = (li x rho)'  ->  row of -Li skew(rho) = rho x li
       const V3 lxr = cross(rh, li);
@@ -1402,6 +1411,14 @@ WBC_DEV void reduce_instance(WarpSmem& s, const wbc_model& md, const wbc_params&
   } else dynamics_phase<DYN_STEP>(s, md, lane, status, nullptr);
   async_wait_all();
   __syncwarp();
+  {
+    // every input value this instance reads (q 19, v 18, traj 54) is in the warp's block now: one vote flags a NaN / inf.
+    // The instance runs on as before and its outputs are zeroed in phase 7 like any other failure.
+    bool nonfin = lane < WBC_NQ && !isfinite(s.q[lane]);
+    nonfin |= lane < WBC_NV && !isfinite(s.v[lane]);
+    nonfin |= !isfinite(s.traj[lane]) || (lane < WBC_NTRAJ - 32 && !isfinite(s.traj[32 + lane]));
+    if (__any_sync(WBC_FULL, nonfin)) status |= WBC_ST_NONFINITE;
+  }
   BodyTask bt;
   body_task(s, lane, status, bt);
   // ---- PC: operational-space quantities (uses the A region as scratch, so it runs before the equalities are built)
@@ -1557,20 +1574,25 @@ WBC_DEV void solve_instance(SM& s, const wbc_model& md, const wbc_params& pr, co
     }
     // ---- phase 7: y = Y x + y0 is current in s.y. Any status bit (unfinished active-set iterate, substituted orientation,
     //      rank-deficient problem) zeroes the torques: nothing that is not the optimum of the reference QP leaves as tau
-    //      (the reference asserts there, inverse_dynamics_controller.py:224); status is warp uniform.
+    //      (the reference asserts there, inverse_dynamics_controller.py:224); status is warp uniform. A non-finite tau, f or vd
+    //      (a finite state whose dynamics overflow) is flagged here, so it cannot leave either.
+    const bool want_vd = SM::kVd && a.vd && lane < 18;
+    double vdv = 0.0;
+    if (want_vd) {
+      // accelerations as affine maps of w (rows stored by the reduce half: a_b, then the joints in internal order)
+      const double* mrow = vdmap + lane * YS;
+      vdv = mrow[NF];
+      for (int w = 0; w < nf; ++w) vdv = fma(mrow[w], s.x[w], vdv);
+    }
+    const bool nonfin = (lane < 12 && !(isfinite(s.y[18 + lane]) && isfinite(s.y[6 + lane]))) || !isfinite(vdv);
+    if (__any_sync(WBC_FULL, nonfin)) status |= WBC_ST_NONFINITE;
     const bool failed = status != 0;
     const double res = minslack < 0.0 ? -minslack : 0.0;
     if (lane < 12) {
       a.tau[inst * WBC_NU + md.act_index[lane]] = failed ? 0.0 : s.y[18 + lane];
       if (a.f) a.f[inst * 12 + lane] = (!failed && ((cmask >> (lane / 3)) & 1)) ? s.y[6 + lane] : 0.0;
     }
-    if (SM::kVd && a.vd && lane < 18) {
-      // accelerations as affine maps of w (rows stored by the reduce half: a_b, then the joints in internal order)
-      const double* mrow = vdmap + lane * YS;
-      double val = mrow[NF];
-      for (int w = 0; w < nf; ++w) val = fma(mrow[w], s.x[w], val);
-      a.vd[inst * WBC_NV + (lane < 6 ? lane : md.v_index[lane - 6])] = failed ? 0.0 : val;
-    }
+    if (want_vd) a.vd[inst * WBC_NV + (lane < 6 ? lane : md.v_index[lane - 6])] = failed ? 0.0 : vdv;
     if (a.lam) {
       // multipliers of the active rows in the fixed layout of wbc.h (R is dead after the solve: scratch for the row)
       double* lrow = &s.Rp[0];
@@ -1718,7 +1740,7 @@ WBC_DEV void pd_element(const wbc_model& md, const wbc_params& pr, const double*
   const int vi = md.v_index[k];
   const double e = q[inst * WBC_NQ + vi + 1] - pr.pd_q_nom[vi - 6];
   double u = -pr.pd_kp * e - pr.pd_kd * v[inst * WBC_NV + vi];
-  u = fmin(fmax(u, -pr.pd_clip), pr.pd_clip);
+  u = u < -pr.pd_clip ? -pr.pd_clip : (u > pr.pd_clip ? pr.pd_clip : u);   // comparisons keep a NaN (np.clip does; fmin / fmax drop it)
   tau[inst * WBC_NU + md.act_index[k]] = u;
 }
 

@@ -43,7 +43,7 @@ struct PlantArgs {
 
 // Freeze mask: a robot whose controller reported any failure keeps its state (the reference asserts there) and stays flagged.
 constexpr int PLANT_FREEZE = WBC_ST_MAXITER | WBC_ST_INFEASIBLE | WBC_ST_RANKDEF | WBC_ST_GIMBAL | WBC_ST_NOTPD | WBC_ST_BADQUAT |
-                             WBC_ST_UNSUPPORTED | WBC_ST_DIVERGED;
+                             WBC_ST_UNSUPPORTED | WBC_ST_DIVERGED | WBC_ST_NONFINITE;
 
 WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md, const PlantArgs& a, long long inst, int lane) {
   int status = a.ctrl_status ? a.ctrl_status[inst] : 0;

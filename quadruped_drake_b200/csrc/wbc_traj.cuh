@@ -110,6 +110,7 @@ __global__ void __launch_bounds__(SAMPLE_WARPS * 32) sample_kernel(PlanTables pt
       int st = 0;
       if (pl < 0 || pl >= pt.n_plans) { pl = 0; st |= WBC_TRAJ_BADPLAN; }
       double t = tin[inst];
+      if (isnan(t)) { t = 0.0; st |= WBC_TRAJ_CLAMPED; }              // a NaN would fail every comparison below (wbc.h)
       // planner semantics (planners/towr.py:96-110): stand while t < wait_time, then the nearest stored sample
       const int g0 = __ldg(pt.grid_off + pl), gn = __ldg(pt.grid_off + pl + 1) - g0;
       bool standing = false;
