@@ -68,6 +68,7 @@ extern "C" {
 #define WBC_ST_UNSUPPORTED 64  /* PC controller with no stance foot (the reference raises too) */
 #define WBC_ST_DIVERGED 128    /* rollout only: non-finite / runaway velocity, instance frozen   */
 #define WBC_ST_NONFINITE 256   /* a NaN / inf among the q, v, traj values of the instance, or a non-finite solution */
+#define WBC_ST_BADVARIANT 512  /* perturbed plant only: variant index out of range; the robot is frozen, zero ground forces */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -372,6 +373,43 @@ int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int
                    const wbc_rollout_io* io, const wbc_rollout_opts* opts, void* stream);
 int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                         const wbc_rollout_io* host_io, const wbc_rollout_opts* opts);
+
+/* ---- Perturbed robots for the ground plant: the plant simulates a different robot than the controller believes in, on its
+ * own ground friction, and may push it. The controller keeps the handle's model and its own friction pyramid (params.mu).
+ *
+ * wbc_plant_set_create uploads n_variants robots to the handle's device: models[k] is what the plant simulates for variant k
+ * (a payload merged into the base, scaled link masses, another inertia ...); mu[k] >= 0 is that variant's ground friction
+ * (mu == NULL: the call's wbc_plant_opts.mu for every variant). Every model must have the handle's v_index and act_index (q, v
+ * and tau layouts are shared with the controller), masses > 0, positive definite inertia_com and finite values. Like a
+ * plan, a set keeps its device number, not its handle: it may be destroyed after the handle. */
+typedef struct wbc_plant_set wbc_plant_set;
+int wbc_plant_set_create(wbc_handle* h, int32_t n_variants, const wbc_model* models, const double* mu, wbc_plant_set** out);
+int wbc_plant_set_destroy(wbc_plant_set* s);
+
+/* Per-robot perturbation of a plant step or rollout (device pointers for the device entries, host pointers for _host). */
+typedef struct wbc_plant_perturb {
+  const wbc_plant_set* set;  /* NULL: every robot is the handle's model with opts.mu (one variant, index 0)              */
+  const int32_t* variant;    /* [N] variant of each robot, NULL = variant 0. An index < 0 or >= n_variants sets
+                              * WBC_ST_BADVARIANT in status_or: that robot keeps its state and gets zero f_contact      */
+  const double* push;        /* [N][8] or NULL: force (world, N) [0:3], point of application in base coordinates relative
+                              * to the base origin [3:6], t_on [6], t_off [7]; applied during every step whose start time t
+                              * satisfies t_on <= t < t_off (t is then required)                                         */
+} wbc_plant_perturb;
+
+/* wbc_plant_step for perturbed robots: the step of robot i simulates its variant's model with its variant's friction and adds
+ * its push, if active, to the applied forces. perturb == NULL is the nominal model with opts.mu and no push. */
+int wbc_plant_step_perturbed(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                             double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status,
+                             int32_t* status_or, double* f_contact, void* stream);
+int wbc_plant_step_perturbed_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                  double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status,
+                                  int32_t* status_or, double* f_contact);
+/* wbc_rollout_ex with the ground plant (opts->plant must be 1) stepping perturbed robots: the same launches per step, the same
+ * graph capture and bookkeeping; only the plant kernel differs. */
+int wbc_rollout_perturbed(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                          const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb, void* stream);
+int wbc_rollout_perturbed_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                               const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

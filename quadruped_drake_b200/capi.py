@@ -21,10 +21,11 @@ WBC_CTRL_ID, WBC_CTRL_CLF, WBC_CTRL_PC, WBC_CTRL_MPTC, WBC_CTRL_PD = 0, 1, 2, 3,
 KINDS = {"id": WBC_CTRL_ID, "clf": WBC_CTRL_CLF, "pc": WBC_CTRL_PC, "mptc": WBC_CTRL_MPTC, "pd": WBC_CTRL_PD}
 ST_MAXITER, ST_INFEASIBLE, ST_RANKDEF, ST_GIMBAL, ST_NOTPD, ST_BADQUAT, ST_UNSUPPORTED, ST_DIVERGED = 1, 2, 4, 8, 16, 32, 64, 128
 ST_NONFINITE = 256
+ST_BADVARIANT = 512
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
-             ST_NONFINITE: "NONFINITE"}
+             ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT"}
 
 
 def status_names(status: int) -> str:
@@ -94,6 +95,11 @@ class WbcPlantOpts(C.Structure):
 class WbcRolloutOpts(C.Structure):
     """ctypes mirror of `wbc_rollout_opts`."""
     _fields_ = [("use_graph", C.c_int32), ("plant", C.c_int32), ("plant_opts", WbcPlantOpts), ("f_contact", C.c_void_p)]
+
+
+class WbcPlantPerturb(C.Structure):
+    """ctypes mirror of `wbc_plant_perturb` (variant set, per-robot variant index, per-robot push rows)."""
+    _fields_ = [("set", C.c_void_p), ("variant", C.c_void_p), ("push", C.c_void_p)]
 
 
 def np_ptr(a: np.ndarray):
@@ -167,6 +173,16 @@ def load_library() -> C.CDLL:
     lib.wbc_rollout_ex_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts)]
     lib.wbc_default_plant_opts.restype = lib.wbc_plant_step.restype = lib.wbc_plant_step_host.restype = C.c_int
     lib.wbc_rollout_ex.restype = lib.wbc_rollout_ex_host.restype = C.c_int
+    lib.wbc_plant_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcModelStruct), dp, C.POINTER(H)]
+    lib.wbc_plant_set_destroy.argtypes = [dp]
+    lib.wbc_plant_step_perturbed.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantOpts), C.POINTER(WbcPlantPerturb)] + [dp] * 8
+    lib.wbc_plant_step_perturbed_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantOpts), C.POINTER(WbcPlantPerturb)] + [dp] * 7
+    lib.wbc_rollout_perturbed.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                          C.POINTER(WbcPlantPerturb), dp]
+    lib.wbc_rollout_perturbed_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                               C.POINTER(WbcPlantPerturb)]
+    for name in PERTURB_SYMBOLS:
+        getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     lib.wbc_multi_create.argtypes = [C.POINTER(WbcModelStruct), C.POINTER(WbcParams), i32, C.POINTER(C.c_int), C.POINTER(H)]
@@ -192,7 +208,9 @@ WIRE_SYMBOLS = ["wbc_lcm_decode_trunk_state", "wbc_lcm_encode_trunk_state", "wbc
                 "wbc_lcm_encode_robot_state_host"]
 ROLLOUT_SYMBOLS = ["wbc_integrate", "wbc_rollout", "wbc_rollout_host", "wbc_rollout_ex", "wbc_rollout_ex_host", "wbc_plant_step",
                    "wbc_plant_step_host", "wbc_default_plant_opts"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+PERTURB_SYMBOLS = ["wbc_plant_set_create", "wbc_plant_set_destroy", "wbc_plant_step_perturbed", "wbc_plant_step_perturbed_host",
+                   "wbc_rollout_perturbed", "wbc_rollout_perturbed_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

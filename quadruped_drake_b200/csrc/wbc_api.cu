@@ -5,6 +5,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <cmath>
 #include <deque>
 #include <memory>
 #include <string>
@@ -82,17 +83,20 @@ struct SmemLayoutPCT {     // PC controller / Coriolis entry: extra operational-
 using SmemLayout = SmemLayoutT<WARPS>;
 using SmemLayoutPC = SmemLayoutPCT<WARPS>;
 
-template <typename L>
-__device__ __forceinline__ const DevConst& stage_consts(L* sm, const DevConst* g) {
-  // model + gains into shared memory once per CTA (lane-divergent table lookups stay on chip), 16 bytes per thread and trip
-  static_assert(sizeof(DevConst) % 16 == 0, "DevConst is staged with 16-byte vectors");
-  const int nvec = sizeof(DevConst) / 16;
+// A constant table into shared memory once per CTA (lane-divergent table lookups stay on chip), 16 bytes per thread and trip
+template <typename T>
+__device__ __forceinline__ const T& stage16(T* sm_dst, const T* g) {
+  static_assert(sizeof(T) % 16 == 0, "staged with 16-byte vectors");
+  const int nvec = sizeof(T) / 16;
   const uint4* src = reinterpret_cast<const uint4*>(g);
-  uint4* dst = reinterpret_cast<uint4*>(&sm->dc);
+  uint4* dst = reinterpret_cast<uint4*>(sm_dst);
   for (int i = threadIdx.x; i < nvec; i += blockDim.x) dst[i] = src[i];
   __syncthreads();
-  return sm->dc;
+  return *sm_dst;
 }
+// model + gains
+template <typename L>
+__device__ __forceinline__ const DevConst& stage_consts(L* sm, const DevConst* g) { return stage16(&sm->dc, g); }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Split path (ID / CLF): the step is launched as two kernels with their own register / occupancy budgets.
@@ -330,6 +334,20 @@ __global__ void __launch_bounds__(32, WBC_PLANT_CTAS) wbc_plant_kernel(const Dev
   if (inst < a.n) wbcplant::plant_step_instance(sm->w, sm->p, dc.md, a, inst, lane);
 }
 
+// The same step for perturbed robots (wbc_plant_step_perturbed): the CTA stages its robot's variant record (1936 B) instead of
+// the handle's constants, and the step adds the variant's friction and the robot's push.
+struct SmemLayoutPlantVariant { wbcplant::PlantVariant pv; wbc::WarpSmem w; wbcplant::PlantSmem p; };
+__global__ void __launch_bounds__(32, WBC_PLANT_CTAS) wbc_plant_variant_kernel(wbcplant::PerturbArgs pa, wbcplant::PlantArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  SmemLayoutPlantVariant* sm = reinterpret_cast<SmemLayoutPlantVariant*>(smem_raw);
+  const long long inst = blockIdx.x;
+  const int k = inst < a.n ? wbcplant::plant_variant(pa, inst) : 0;
+  const wbcplant::PlantVariant& pv = stage16(&sm->pv, pa.set + (k < 0 ? 0 : k));   // a bad index is frozen: any record will do
+  const int lane = lane_index();
+  if (inst < a.n)
+    wbcplant::plant_step_instance<true>(sm->w, sm->p, pv.md, a, inst, lane, wbcplant::plant_perturb(pa, a, inst, k, pv.mu));
+}
+
 __global__ void wbc_pd_kernel(const DevConst* __restrict__ gdc, const double* q, const double* v, double* tau, long long n) {
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t < n * WBC_NU) wbc::pd_element(gdc->md, gdc->pr, q, v, tau, t / WBC_NU, (int)(t % WBC_NU));
@@ -451,7 +469,9 @@ constexpr int WBC_NSLOT = 4;
 struct wbc_handle {
   int device = 0;
   DevArray<DevConst> d_const;
+  wbc_model model;
   wbc_params params;
+  DevArray<wbcplant::PlantVariant> d_nominal;   // the handle's model as the one variant of a perturbed step without a set
   std::string err;
   int64_t launches = 0;
   int sm_count = 148;
@@ -513,6 +533,7 @@ static int set_smem_attr(wbc_handle* h) {
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_coriolis_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPC)));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_dynamics_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlant)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_variant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlantVariant)));
   return WBC_OK;
 }
 
@@ -535,6 +556,10 @@ extern "C" int wbc_create(const wbc_model* model, const wbc_params* params, int 
   wbc::derive_constants(h->params, hc.dv);
   WBC_CUDA(h, h->d_const.reserve(1));
   WBC_CUDA(h, cudaMemcpy(h->d_const.p, &hc, sizeof(DevConst), cudaMemcpyHostToDevice));
+  h->model = *model;
+  wbcplant::PlantVariant nominal{*model, 0.0};
+  WBC_CUDA(h, h->d_nominal.reserve(1));
+  WBC_CUDA(h, cudaMemcpy(h->d_nominal.p, &nominal, sizeof(nominal), cudaMemcpyHostToDevice));
   // the streams and events: created here, not on first use, so that a step never calls a resource-creating API while some
   // other stream of the process is being captured
   for (Stream& s : h->lane) WBC_CUDA(h, cudaStreamCreateWithFlags(&s.v, cudaStreamNonBlocking));
@@ -1421,16 +1446,84 @@ extern "C" int wbc_default_plant_opts(wbc_plant_opts* o) {
   return WBC_OK;
 }
 
-static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, double* q, double* v, const double* tau,
-                        double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact, const double* metrics,
-                        double* err_max, double* metrics_log, const int* counter, cudaStream_t st) {
+// pa == nullptr: the unperturbed plant kernel; otherwise the variant kernel with these perturbations.
+static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbcplant::PerturbArgs* pa, double* q,
+                        double* v, const double* tau, double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact,
+                        const double* metrics, double* err_max, double* metrics_log, const int* counter, cudaStream_t st) {
   wbc_plant_opts o;
   if (opts) o = *opts; else wbc_default_plant_opts(&o);
   if (!(o.mu >= 0.0) || !(o.erp >= 0.0 && o.erp <= 1.0) || o.iters < 1 || o.iters > 1000) return fail_arg(h, "wbc_plant_step: bad options");
   const wbcplant::PlantArgs a{q, v, tau, t, ctrl_status, status_or, f_contact, metrics, err_max, metrics_log, counter, (long long)n, dt,
                               o.mu, o.erp, o.iters};
-  wbc_plant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlant), st>>>(h->d_const.p, a);
+  if (pa) wbc_plant_variant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlantVariant), st>>>(*pa, a);
+  else wbc_plant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlant), st>>>(h->d_const.p, a);
   h->launches++;
+  return WBC_OK;
+}
+
+// ------------------------------------------------------------------------------ perturbed robots (wbc_plant.cuh)
+// A set keeps the number of the device its table lives on, not its handle: it may be destroyed after the handle.
+struct wbc_plant_set {
+  int device = 0;
+  int32_t n_variants = 0;
+  bool own_mu = false;
+  DevArray<wbcplant::PlantVariant> table;
+  ~wbc_plant_set() { cudaSetDevice(device); }   // the table is freed after this, on the set's device
+};
+
+extern "C" int wbc_plant_set_destroy(wbc_plant_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+static bool finite_all(const double* x, size_t n) {
+  for (size_t i = 0; i < n; ++i)
+    if (!std::isfinite(x[i])) return false;
+  return true;
+}
+
+extern "C" int wbc_plant_set_create(wbc_handle* h, int32_t n_variants, const wbc_model* models, const double* mu, wbc_plant_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !models || n_variants <= 0) return fail_arg(h, "wbc_plant_set_create: models and n_variants > 0 are required");
+  *out = nullptr;
+  std::vector<wbcplant::PlantVariant> rec((size_t)n_variants);
+  for (int32_t k = 0; k < n_variants; ++k) {
+    const wbc_model& m = models[k];
+    if (memcmp(m.v_index, h->model.v_index, sizeof(m.v_index)) || memcmp(m.act_index, h->model.act_index, sizeof(m.act_index)))
+      return fail_arg(h, "wbc_plant_set_create: every model must have the handle's v_index and act_index");
+    static_assert(offsetof(wbc_model, mass) == 0 && offsetof(wbc_model, v_index) % sizeof(double) == 0, "the doubles of wbc_model come first");
+    if (!finite_all(reinterpret_cast<const double*>(&m), offsetof(wbc_model, v_index) / sizeof(double)))
+      return fail_arg(h, "wbc_plant_set_create: non-finite model value");
+    for (int b = 0; b < WBC_NBODY; ++b) {
+      const double* I = m.inertia_com[b];      // xx yy zz xy xz yz
+      const double m2 = I[0] * I[1] - I[3] * I[3];
+      const double det = I[0] * (I[1] * I[2] - I[5] * I[5]) - I[3] * (I[3] * I[2] - I[5] * I[4]) + I[4] * (I[3] * I[5] - I[1] * I[4]);
+      if (!(m.mass[b] > 0.0)) return fail_arg(h, "wbc_plant_set_create: every body mass must be > 0");
+      if (!(I[0] > 0.0 && m2 > 0.0 && det > 0.0)) return fail_arg(h, "wbc_plant_set_create: every inertia_com must be positive definite");
+    }
+    if (mu && !(std::isfinite(mu[k]) && mu[k] >= 0.0)) return fail_arg(h, "wbc_plant_set_create: every mu must be finite and >= 0");
+    rec[k].md = m;
+    rec[k].mu = mu ? mu[k] : 0.0;
+  }
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_plant_set> ps(new (std::nothrow) wbc_plant_set());
+  if (!ps) return WBC_ERR_NOMEM;
+  ps->device = h->device;
+  ps->n_variants = n_variants;
+  ps->own_mu = mu != nullptr;
+  WBC_CUDA(h, ps->table.reserve(rec.size()));
+  WBC_CUDA(h, cudaMemcpy(ps->table.p, rec.data(), rec.size() * sizeof(rec[0]), cudaMemcpyHostToDevice));
+  *out = ps.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of a perturbation whose variant / push arrays are already on the device.
+static int perturb_args(wbc_handle* h, const wbc_plant_perturb* p, const int32_t* variant, const double* push, bool has_t,
+                        wbcplant::PerturbArgs* pa) {
+  const wbc_plant_set* set = p ? p->set : nullptr;
+  if (set && set->device != h->device) return fail_arg(h, "wbc_plant_perturb: the set lives on another device than the handle");
+  if (push && !has_t) return fail_arg(h, "wbc_plant_perturb: pushes need the robots' times t");
+  *pa = wbcplant::PerturbArgs{set ? set->table.p : h->d_nominal.p, variant, push, set ? set->n_variants : 1, set && set->own_mu ? 1 : 0};
   return WBC_OK;
 }
 
@@ -1440,16 +1533,34 @@ extern "C" int wbc_plant_step(wbc_handle* h, int64_t n, double dt, const wbc_pla
   if (n < 0 || !(dt > 0.0) || (n > 0 && (!q || !v || !tau))) return fail_arg(h, "wbc_plant_step: q, v, tau and dt > 0 are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  const int rc = plant_launch(h, n, dt, opts, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+  const int rc = plant_launch(h, n, dt, opts, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr,
+                              (cudaStream_t)stream);
   if (rc) return rc;
   WBC_CUDA(h, cudaGetLastError());
   return WBC_OK;
 }
 
-extern "C" int wbc_plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, double* q, double* v, const double* tau,
-                                   double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact) {
+extern "C" int wbc_plant_step_perturbed(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                        double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status, int32_t* status_or,
+                                        double* f_contact, void* stream) {
   if (!h) return WBC_ERR_ARG;
-  if (n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_plant_step_host: n >= 0 and dt > 0 are required");
+  if (n < 0 || !(dt > 0.0) || (n > 0 && (!q || !v || !tau))) return fail_arg(h, "wbc_plant_step_perturbed: q, v, tau and dt > 0 are required");
+  wbcplant::PerturbArgs pa;
+  int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, t != nullptr, &pa);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  rc = plant_launch(h, n, dt, opts, &pa, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+  if (rc) return rc;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Host buffers of both plant steps; perturbed = false is wbc_plant_step_host.
+static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, bool perturbed, const wbc_plant_perturb* perturb,
+                           double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status, int32_t* status_or,
+                           double* f_contact, const char* what) {
+  if (!h) return WBC_ERR_ARG;
+  if (n < 0 || !(dt > 0.0)) return fail_arg(h, what);
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
   DevScratch s(h->lane[0]);
@@ -1457,15 +1568,30 @@ extern "C" int wbc_plant_step_host(wbc_handle* h, int64_t n, double dt, const wb
   double* dq = s.inout(q, N * WBC_NQ); double* dv = s.inout(v, N * WBC_NV); const double* dtau = s.in(tau, N * WBC_NU);
   double* dt_ = s.inout(t, N); const int32_t* dcs = s.in(ctrl_status, N); int32_t* dso = s.inout(status_or, N);
   double* df = s.out(f_contact, N * 12);
+  wbc_plant_perturb dp{};
+  if (perturb) dp = wbc_plant_perturb{perturb->set, s.in(perturb->variant, N), s.in(perturb->push, N * 8)};
   WBC_SCRATCH_CHECK(h, s);
-  const int rc = wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, s.st);
+  const int rc = perturbed ? wbc_plant_step_perturbed(h, n, dt, opts, perturb ? &dp : nullptr, dq, dv, dtau, dt_, dcs, dso, df, s.st)
+                           : wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, s.st);
   return rc ? rc : s.finish(h);
 }
 
-extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
-                              const wbc_rollout_io* io, const wbc_rollout_opts* opts, void* stream) {
-  if (!h) return WBC_ERR_ARG;
-  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout: bad arguments");
+extern "C" int wbc_plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, double* q, double* v, const double* tau,
+                                   double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact) {
+  return plant_step_host(h, n, dt, opts, false, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact,
+                         "wbc_plant_step_host: n >= 0 and dt > 0 are required");
+}
+
+extern "C" int wbc_plant_step_perturbed_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                             double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status,
+                                             int32_t* status_or, double* f_contact) {
+  return plant_step_host(h, n, dt, opts, true, perturb, q, v, tau, t, ctrl_status, status_or, f_contact,
+                         "wbc_plant_step_perturbed_host: n >= 0 and dt > 0 are required");
+}
+
+// The rollout loop of wbc_rollout_ex and wbc_rollout_perturbed; pa != nullptr: the plant step runs the variant kernel.
+static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
+                       const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, cudaStream_t st) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -1475,7 +1601,6 @@ extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int
   WBC_CUDA(h, h->ro.reserve(n));
   WBC_CUDA(h, h->slot[0].reserve(n, !plant));   // before the capture below: a step grows no scratch while being captured
   const RolloutScratch& ro = h->ro;
-  cudaStream_t st = (cudaStream_t)stream;
   double* tau = io->tau ? io->tau : ro.tau.p;
   double* metrics = io->metrics ? io->metrics : ro.metrics.p;
   WBC_CUDA(h, cudaMemsetAsync(ro.counter.p, 0, sizeof(int), st));
@@ -1493,7 +1618,7 @@ extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int
     r = wbc_step(h, kind, n, &sio, st);
     if (r) return r;
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
+      r = plant_launch(h, n, dt, &opts->plant_opts, pa, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
     } else {
@@ -1532,6 +1657,23 @@ extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int
   return WBC_OK;
 }
 
+extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                              const wbc_rollout_io* io, const wbc_rollout_opts* opts, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout: bad arguments");
+  return rollout_run(h, kind, plan, n, n_steps, dt, io, opts, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int wbc_rollout_perturbed(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                     const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || !opts || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_perturbed: bad arguments");
+  if (opts->plant == 0) return fail_arg(h, "wbc_rollout_perturbed: perturbations act on the ground plant (opts->plant = 1)");
+  wbcplant::PerturbArgs pa;
+  const int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, &pa, (cudaStream_t)stream);
+}
+
 extern "C" int wbc_rollout(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                            const wbc_rollout_io* io, int use_graph, void* stream) {
   wbc_rollout_opts o{};
@@ -1540,8 +1682,9 @@ extern "C" int wbc_rollout(wbc_handle* h, int kind, const wbc_plan* plan, int64_
   return wbc_rollout_ex(h, kind, plan, n, n_steps, dt, io, &o, stream);
 }
 
-extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
-                                   const wbc_rollout_io* io, const wbc_rollout_opts* opts) {
+// Host buffers of both rollouts; perturbed = false is wbc_rollout_ex_host.
+static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
+                        const wbc_rollout_opts* opts, bool perturbed, const wbc_plant_perturb* perturb) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -1557,9 +1700,22 @@ extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan
   wbc_rollout_opts o{};
   if (opts) o = *opts; else { o.use_graph = 1; wbc_default_plant_opts(&o.plant_opts); }
   o.f_contact = s.out(o.f_contact, N * 12);
+  wbc_plant_perturb dp{};
+  if (perturb) dp = wbc_plant_perturb{perturb->set, s.in(perturb->variant, N), s.in(perturb->push, N * 8)};
   WBC_SCRATCH_CHECK(h, s);
-  const int rc = wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
+  const int rc = perturbed ? wbc_rollout_perturbed(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, s.st)
+                           : wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
   return rc ? rc : s.finish(h);
+}
+
+extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                   const wbc_rollout_io* io, const wbc_rollout_opts* opts) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, false, nullptr);
+}
+
+extern "C" int wbc_rollout_perturbed_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                          const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, true, perturb);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

@@ -45,8 +45,47 @@ struct PlantArgs {
 constexpr int PLANT_FREEZE = WBC_ST_MAXITER | WBC_ST_INFEASIBLE | WBC_ST_RANKDEF | WBC_ST_GIMBAL | WBC_ST_NOTPD | WBC_ST_BADQUAT |
                              WBC_ST_UNSUPPORTED | WBC_ST_DIVERGED | WBC_ST_NONFINITE;
 
-WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md, const PlantArgs& a, long long inst, int lane) {
+// ---- perturbed robots (wbc_plant_step_perturbed): the plant simulates a variant of the robot, the controller keeps its model.
+// One entry of a variant table: 1936 B = 121 x 16 B, so a CTA stages it with the 16-byte vector loop of the model constants.
+struct alignas(16) PlantVariant {
+  wbc_model md;   // what the plant simulates for this variant
+  double mu;      // its ground friction
+};
+static_assert(sizeof(PlantVariant) == 1936, "variant record: wbc_model + mu, a multiple of 16 bytes");
+
+// Device inputs of the variant kernel. variant [N] (NULL: variant 0); push [N][8]: force F (world) [0:3], point r in base
+// coordinates relative to the base origin [3:6], t_on [6], t_off [7] (NULL: no pushes). own_mu == 0: every variant uses the
+// call's mu instead of its own.
+struct PerturbArgs {
+  const PlantVariant* set; const int32_t* variant; const double* push; int n_variants; int own_mu;
+};
+
+// What the step of one robot sees: its friction, its push row while t_on <= t < t_off holds for the step's start time t (NULL
+// otherwise), and whether its variant index was out of range (the robot is then frozen and flagged WBC_ST_BADVARIANT).
+struct Perturb {
+  double mu; const double* push; bool bad_variant;
+};
+
+// Variant of robot `inst`, or -1 when its index is out of range.
+WBC_DEV int plant_variant(const PerturbArgs& pa, long long inst) {
+  const int k = pa.variant ? pa.variant[inst] : 0;
+  return (k >= 0 && k < pa.n_variants) ? k : -1;
+}
+
+WBC_DEV Perturb plant_perturb(const PerturbArgs& pa, const PlantArgs& a, long long inst, int k, double variant_mu) {
+  const double* row = pa.push ? pa.push + inst * 8 : nullptr;
+  const double t = row ? a.t[inst] : 0.0;
+  return Perturb{pa.own_mu ? variant_mu : a.mu, (row && row[6] <= t && t < row[7]) ? row : nullptr, k < 0};
+}
+
+// PERTURB = false: the unperturbed step (md = the handle's model, a.mu). PERTURB = true: md is the robot's variant and `pt`
+// adds its friction, its push and the freeze of a bad variant index; nothing else differs.
+template <bool PERTURB = false>
+WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md, const PlantArgs& a, long long inst, int lane,
+                                 const Perturb& pt = Perturb{}) {
+  constexpr int FREEZE = PERTURB ? (PLANT_FREEZE | WBC_ST_BADVARIANT) : PLANT_FREEZE;
   int status = a.ctrl_status ? a.ctrl_status[inst] : 0;
+  if (PERTURB && pt.bad_variant) status |= WBC_ST_BADVARIANT;
   for (int i = lane; i < WBC_NQ; i += 32) s.q[i] = a.q[inst * WBC_NQ + i];
   for (int i = lane; i < WBC_NV; i += 32) s.v[i] = a.v[inst * WBC_NV + i];
   if (lane < 12) ps.tauk[lane] = a.tau[inst * WBC_NU + md.act_index[lane]];
@@ -98,6 +137,13 @@ WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md
     } else {
 #pragma unroll
       for (int c = 0; c < 6; ++c) rb[c] = -s.hb[c];
+      if (PERTURB && pt.push) {                     // generalized force J_p' F of the push: [(R0 r) x F ; F], none on the joints
+        const V3 F = ld3(pt.push), r = ld3(pt.push + 3);
+        const V3 rw = r.x * ld3(&s.task[7]) + r.y * ld3(&s.task[10]) + r.z * ld3(&s.task[13]);
+        const V3 m = cross(rw, F);
+        rb[0] += m.x; rb[1] += m.y; rb[2] += m.z;
+        rb[3] += F.x; rb[4] += F.y; rb[5] += F.z;
+      }
 #pragma unroll
       for (int kk = 0; kk < 4; ++kk)
 #pragma unroll
@@ -190,7 +236,7 @@ WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
         const int r = 3 * k + i;
-        const double lim = a.mu * pn;
+        const double lim = (PERTURB ? pt.mu : a.mu) * pn;
         const double pnew = fmin(fmax(p - u * ainv, -lim), lim);
         const double dl = shfl(pnew - p, r);
         if (lane == r) p = pnew;
@@ -218,9 +264,9 @@ WBC_DEV void plant_step_instance(WarpSmem& s, PlantSmem& ps, const wbc_model& md
     if (a.metrics_log && lane < WBC_NMETRIC)
       a.metrics_log[((long long)(*a.step_counter) * a.n + inst) * WBC_NMETRIC + lane] = a.metrics[inst * WBC_NMETRIC + lane];
   }
-  if (a.f_contact && lane < 12) a.f_contact[inst * 12 + lane] = (status & PLANT_FREEZE) ? 0.0 : p / a.dt;
+  if (a.f_contact && lane < 12) a.f_contact[inst * 12 + lane] = (status & FREEZE) ? 0.0 : p / a.dt;
   if (lane == 0 && a.t) a.t[inst] += a.dt;
-  if (status & PLANT_FREEZE) return;
+  if (status & FREEZE) return;
   const double wx = shfl(vn, 0), wy = shfl(vn, 1), wz = shfl(vn, 2);
   if (lane < 18) a.v[inst * WBC_NV + vi] = vn;
   if (lane == 0) {

@@ -13,6 +13,7 @@ thighs, then all knees. An explicit list of joint names is accepted too.
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 from dataclasses import dataclass, field
 from pathlib import Path
@@ -216,6 +217,20 @@ def flatten(desc: dict, dof_order="depth_first") -> RobotModel:
     return RobotModel(name=desc["name"], mass=mass, com=com, inertia_com=inertia, joint_xyz=joint_xyz,
                       joint_axis=joint_axis, foot_xyz=foot_xyz, effort=effort, v_index=v_index,
                       act_index=act_index, joint_names=joint_names, base_link=base)
+
+
+def with_payload(desc: dict, mass, com, inertia=None, name="payload") -> dict:
+    """Copy of a robot description with one more link welded to the base link: `mass` (kg) with its CoM at `com` (base
+    coordinates, m) and `inertia` about that CoM (xx yy zz xy xz yz; None: a point mass). `flatten` merges it into body 0;
+    oracle.dynamics.Plant keeps it as a separate welded body."""
+    d = copy.deepcopy(desc)
+    if any(l["name"] == name for l in d["links"]):
+        raise ValueError(f"the description already has a link named {name!r}")
+    d["links"].append({"name": name, "mass": float(mass), "com": [0.0, 0.0, 0.0],
+                       "inertia_com": [float(x) for x in (inertia if inertia is not None else np.zeros(6))]})
+    d["joints"].append({"name": f"{d['base_link']}_to_{name}", "type": "fixed", "parent": d["base_link"], "child": name,
+                        "xyz": [float(x) for x in com], "rpy": [0.0, 0.0, 0.0], "axis": [1, 0, 0], "effort": float("inf")})
+    return d
 
 
 def load_robot(name_or_path="mini_cheetah", dof_order="depth_first", base_link=None, foot_frames=None) -> RobotModel:

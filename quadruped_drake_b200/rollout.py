@@ -6,6 +6,11 @@ Two plants: `plant=False` advances the state with the QP's own contact-consisten
 csrc/wbc_rollout.cuh); `plant=True` applies the controller's TORQUES to the simulated robot on flat ground (forward dynamics +
 velocity-level contact with Coulomb friction, csrc/wbc_plant.cuh), so that a controller can fail physically. Everything runs
 through `wbc_rollout_ex` in the C ABI. There is no CPU fallback.
+
+Perturbed robots (`plant_set`, `variant`, `push`; ground plant only): the plant simulates a variant of the robot - a payload
+(model.with_payload), other link masses or inertias - on the variant's own ground friction, and a push acts on the base during
+a time window, while the controller keeps the handle's nominal model. They run through `wbc_rollout_perturbed` /
+`wbc_plant_step_perturbed`.
 """
 from __future__ import annotations
 
@@ -13,14 +18,52 @@ import ctypes as C
 
 import numpy as np
 
-from .capi import KINDS, WbcPlantOpts, WbcRolloutIO, WbcRolloutOpts, np_ptr
-from .model import NQ, NU, NV
+from .capi import KINDS, WbcPlantOpts, WbcPlantPerturb, WbcRolloutIO, WbcRolloutOpts, np_ptr
+from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
 Q0_MINI_CHEETAH = np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.3] + [0.0, -0.8, 1.6] * 4)     # simulate.py:171-176
 
 
 def _is_torch(x):
     return type(x).__module__.startswith("torch")
+
+
+class PlantSet:
+    """Device-resident table of K robots for the ground plant (wbc_plant_set_create): models[k] (RobotModel or WbcModelStruct,
+    with the controller's DOF and actuator order) is what the plant simulates for variant k, mu[k] its ground friction
+    (None: the call's `mu` for every variant)."""
+
+    def __init__(self, ctl, models, mu=None):
+        self.ctl, self.lib = ctl, ctl.lib
+        structs = [m.as_struct() if isinstance(m, RobotModel) else m for m in models]
+        self.n_variants = len(structs)
+        arr = (WbcModelStruct * self.n_variants)(*structs)
+        self._mu = None if mu is None else np.ascontiguousarray(np.broadcast_to(np.asarray(mu, np.float64), (self.n_variants,)))
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_plant_set_create(ctl._h, self.n_variants, arr, None if self._mu is None else np_ptr(self._mu),
+                                                      C.byref(self._p)), "wbc_plant_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_plant_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _perturb(plant_set, variant, push, ptr):
+    return WbcPlantPerturb(None if plant_set is None else plant_set._p, ptr(variant), ptr(push))
+
+
+def _perturb_arrays(n, variant, push):
+    """Host copies in the layouts of the C ABI: variant [N] int32, push [N][8] float64 (None stays None)."""
+    vi = None if variant is None else np.ascontiguousarray(np.broadcast_to(np.asarray(variant, np.int32), (n,)))
+    pu = None if push is None else np.ascontiguousarray(np.broadcast_to(np.asarray(push, np.float64), (n, 8)))
+    return vi, pu
 
 
 class RolloutResult:
@@ -36,11 +79,15 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
-            mu=1.0, erp=0.2, iters=30) -> RolloutResult:
+            mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
-    carries the last step's ground forces `f_contact[N,4,3]`."""
+    carries the last step's ground forces `f_contact[N,4,3]`.
+    Perturbed robots (plant=True only): plant_set (PlantSet or None: the nominal model), variant [N] int32 (None: variant 0),
+    push [N,8] = force (world) | point (base frame) | t_on | t_off (None: no pushes); torch tensors on the device with torch
+    inputs, arrays otherwise. A robot with an out-of-range variant index is frozen and flagged ST_BADVARIANT."""
+    perturbed = plant_set is not None or variant is not None or push is not None
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
     if _is_torch(q):
         import torch
@@ -52,7 +99,12 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        ctl._check(ctl.lib.wbc_rollout_ex(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), stream), "wbc_rollout_ex")
+        if perturbed:
+            pt = _perturb(plant_set, variant, push, p)
+            ctl._check(ctl.lib.wbc_rollout_perturbed(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
+                                                     stream), "wbc_rollout_perturbed")
+        else:
+            ctl._check(ctl.lib.wbc_rollout_ex(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), stream), "wbc_rollout_ex")
         return r
     q = np.array(q, dtype=np.float64).reshape(-1, NQ)
     n = len(q)
@@ -65,22 +117,49 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    ctl._check(ctl.lib.wbc_rollout_ex_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o)), "wbc_rollout_ex_host")
+    if perturbed:
+        pt = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt)
+        ctl._check(ctl.lib.wbc_rollout_perturbed_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt)),
+                   "wbc_rollout_perturbed_host")
+    else:
+        ctl._check(ctl.lib.wbc_rollout_ex_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o)), "wbc_rollout_ex_host")
     return r
 
 
-def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=None):
-    """One time step of N simulated robots on flat ground (wbc_plant_step_host) for host arrays:
-    -> q+[N,19], v+[N,18], f_contact[N,4,3] (ground forces LF RF LH RH, world axes), status[N]."""
+def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=None, plant_set=None, variant=None, push=None, t=None):
+    """One time step of N simulated robots on flat ground -> q+[N,19], v+[N,18], f_contact[N,4,3] (ground forces LF RF LH RH,
+    world axes), status[N]. Host arrays go through wbc_plant_step_host (q, v copied); torch CUDA tensors are updated IN PLACE
+    on torch's current stream (wbc_plant_step). plant_set / variant / push as in `rollout` (wbc_plant_step_perturbed); t [N] is
+    each robot's time at the start of the step, required with pushes (a torch tensor is advanced by dt in place)."""
+    perturbed = plant_set is not None or variant is not None or push is not None
+    o = WbcPlantOpts(float(mu), float(erp), int(iters), 0)
+    if _is_torch(q):
+        import torch
+        n, dev = q.shape[0], q.device
+        f, st = torch.zeros((n, 4, 3), dtype=torch.float64, device=dev), torch.zeros(n, dtype=torch.int32, device=dev)
+        p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        args = (p(q), p(v), p(tau), p(t), p(ctrl_status), p(st), p(f), stream)
+        if perturbed:
+            pt = _perturb(plant_set, variant, push, p)
+            ctl._check(ctl.lib.wbc_plant_step_perturbed(ctl._h, n, float(dt), C.byref(o), C.byref(pt), *args), "wbc_plant_step_perturbed")
+        else:
+            ctl._check(ctl.lib.wbc_plant_step(ctl._h, n, float(dt), C.byref(o), *args), "wbc_plant_step")
+        return q, v, f, st
     q = np.array(q, dtype=np.float64).reshape(-1, NQ)
     n = len(q)
     v = np.array(v, dtype=np.float64).reshape(n, NV)
     tau = np.ascontiguousarray(tau, dtype=np.float64).reshape(n, NU)
     f, st = np.zeros((n, 4, 3)), np.zeros(n, np.int32)
     cs = None if ctrl_status is None else np.ascontiguousarray(ctrl_status, dtype=np.int32).reshape(n)
-    o = WbcPlantOpts(float(mu), float(erp), int(iters), 0)
-    ctl._check(ctl.lib.wbc_plant_step_host(ctl._h, n, float(dt), C.byref(o), np_ptr(q), np_ptr(v), np_ptr(tau), None,
-                                           None if cs is None else np_ptr(cs), np_ptr(st), np_ptr(f)), "wbc_plant_step_host")
+    opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
+    ta = None if t is None else np.array(np.broadcast_to(np.asarray(t, dtype=np.float64), (n,)))
+    args = (np_ptr(q), np_ptr(v), np_ptr(tau), opt(ta), opt(cs), np_ptr(st), np_ptr(f))
+    if perturbed:
+        pt = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt)
+        ctl._check(ctl.lib.wbc_plant_step_perturbed_host(ctl._h, n, float(dt), C.byref(o), C.byref(pt), *args), "wbc_plant_step_perturbed_host")
+    else:
+        ctl._check(ctl.lib.wbc_plant_step_host(ctl._h, n, float(dt), C.byref(o), *args), "wbc_plant_step_host")
     return q, v, f, st
 
 
