@@ -69,6 +69,7 @@ extern "C" {
 #define WBC_ST_DIVERGED 128    /* rollout only: non-finite / runaway velocity, instance frozen   */
 #define WBC_ST_NONFINITE 256   /* a NaN / inf among the q, v, traj values of the instance, or a non-finite solution */
 #define WBC_ST_BADVARIANT 512  /* perturbed plant only: variant index out of range; the robot is frozen, zero ground forces */
+#define WBC_ST_BADTERRAIN 1024 /* terrain plant only: terrain index out of range; the robot is frozen, zero ground forces */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -410,6 +411,55 @@ int wbc_rollout_perturbed(wbc_handle* h, int kind, const wbc_plan* plan, int64_t
                           const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb, void* stream);
 int wbc_rollout_perturbed_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                                const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb);
+
+/* ---- Uneven ground for the ground plant: each robot stands on its own terrain. The controller is unchanged and sees none of
+ * it (its friction pyramid stays about world z, its feet come from the flat-ground plan).
+ *
+ * A terrain is a plane plus an optional height field,  h(x, y) = z0 + sx x + sy y + H(x, y),  where H is the bilinear
+ * interpolant of the row-major grid heights[ny][nx] with origin (x0, y0) and spacing (dx, dy); nx = ny = 0 is no grid (H = 0).
+ * Outside the grid the grid coordinates are clamped to its edge (the clamped direction has zero gradient); the cell of a point
+ * on the far edge is the last one. H is continuous, so a vertical step in the heights is a ramp one cell wide. Each foot
+ * contacts the terrain at its position at the start of the step, along the local normal n = (-h_x, -h_y, 1) / |.|, with the
+ * friction pyramid in the frame t1 = normalize(e_x - n_x n), t2 = n x t1, n; its gap is (p_z - h(p_x, p_y)) n_z. f_contact
+ * stays in world axes. Only the four foot points touch the ground. On flat terrain (all zero, no grid) the step gives the
+ * bits of wbc_plant_step_perturbed.
+ *
+ * wbc_terrain_set_create uploads n_terrains terrains to the handle's device (heights are copied). Every value must be finite;
+ * nx and ny are both 0 or both >= 2; with a grid, dx, dy > 0 and heights != NULL. Like a plan, a set keeps its device number,
+ * not its handle: it may be destroyed after the handle. */
+typedef struct wbc_terrain_desc {
+  double z0, sx, sy;       /* plane z0 + sx x + sy y                                    */
+  int32_t nx, ny;          /* grid size, 0 x 0: no grid                                 */
+  double x0, y0, dx, dy;   /* world position of heights[0][0], spacing along x and y    */
+  const double* heights;   /* [ny][nx] row-major (host), NULL without a grid            */
+} wbc_terrain_desc;
+typedef struct wbc_terrain_set wbc_terrain_set;
+int wbc_terrain_set_create(wbc_handle* h, int32_t n_terrains, const wbc_terrain_desc* terrains, wbc_terrain_set** out);
+int wbc_terrain_set_destroy(wbc_terrain_set* s);
+
+/* Per-robot terrain of a plant step or rollout (device pointer for the device entries, host pointer for _host). */
+typedef struct wbc_plant_terrain {
+  const wbc_terrain_set* set;  /* NULL: flat ground z = 0 for every robot (one terrain, index 0)                        */
+  const int32_t* index;        /* [N] terrain of each robot, NULL = terrain 0. An index < 0 or >= n_terrains sets
+                                * WBC_ST_BADTERRAIN in status_or: that robot keeps its state and gets zero f_contact  */
+} wbc_plant_terrain;
+
+/* wbc_plant_step_perturbed on each robot's terrain. perturb == NULL is the nominal model with opts.mu and no push;
+ * terrain == NULL is flat ground. */
+int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                           const wbc_plant_terrain* terrain, double* q, double* v, const double* tau, double* t,
+                           const int32_t* ctrl_status, int32_t* status_or, double* f_contact, void* stream);
+int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                const wbc_plant_terrain* terrain, double* q, double* v, const double* tau, double* t,
+                                const int32_t* ctrl_status, int32_t* status_or, double* f_contact);
+/* wbc_rollout_perturbed on each robot's terrain (opts->plant must be 1): the same launches per step, the same graph capture and
+ * bookkeeping; only the plant kernel differs. */
+int wbc_rollout_terrain(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                        const wbc_plant_terrain* terrain, void* stream);
+int wbc_rollout_terrain_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                             const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                             const wbc_plant_terrain* terrain);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

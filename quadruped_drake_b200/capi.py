@@ -22,10 +22,11 @@ KINDS = {"id": WBC_CTRL_ID, "clf": WBC_CTRL_CLF, "pc": WBC_CTRL_PC, "mptc": WBC_
 ST_MAXITER, ST_INFEASIBLE, ST_RANKDEF, ST_GIMBAL, ST_NOTPD, ST_BADQUAT, ST_UNSUPPORTED, ST_DIVERGED = 1, 2, 4, 8, 16, 32, 64, 128
 ST_NONFINITE = 256
 ST_BADVARIANT = 512
+ST_BADTERRAIN = 1024
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
-             ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT"}
+             ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN"}
 
 
 def status_names(status: int) -> str:
@@ -100,6 +101,17 @@ class WbcRolloutOpts(C.Structure):
 class WbcPlantPerturb(C.Structure):
     """ctypes mirror of `wbc_plant_perturb` (variant set, per-robot variant index, per-robot push rows)."""
     _fields_ = [("set", C.c_void_p), ("variant", C.c_void_p), ("push", C.c_void_p)]
+
+
+class WbcTerrainDesc(C.Structure):
+    """ctypes mirror of `wbc_terrain_desc` (plane z0 + sx x + sy y, optional height grid [ny][nx] at (x0, y0), spacing dx, dy)."""
+    _fields_ = [("z0", C.c_double), ("sx", C.c_double), ("sy", C.c_double), ("nx", C.c_int32), ("ny", C.c_int32),
+                ("x0", C.c_double), ("y0", C.c_double), ("dx", C.c_double), ("dy", C.c_double), ("heights", C.c_void_p)]
+
+
+class WbcPlantTerrain(C.Structure):
+    """ctypes mirror of `wbc_plant_terrain` (terrain set, per-robot terrain index)."""
+    _fields_ = [("set", C.c_void_p), ("index", C.c_void_p)]
 
 
 def np_ptr(a: np.ndarray):
@@ -181,7 +193,17 @@ def load_library() -> C.CDLL:
                                           C.POINTER(WbcPlantPerturb), dp]
     lib.wbc_rollout_perturbed_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
                                                C.POINTER(WbcPlantPerturb)]
-    for name in PERTURB_SYMBOLS:
+    lib.wbc_terrain_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcTerrainDesc), C.POINTER(H)]
+    lib.wbc_terrain_set_destroy.argtypes = [dp]
+    lib.wbc_plant_step_terrain.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantOpts), C.POINTER(WbcPlantPerturb),
+                                           C.POINTER(WbcPlantTerrain)] + [dp] * 8
+    lib.wbc_plant_step_terrain_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantOpts), C.POINTER(WbcPlantPerturb),
+                                                C.POINTER(WbcPlantTerrain)] + [dp] * 7
+    lib.wbc_rollout_terrain.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                        C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), dp]
+    lib.wbc_rollout_terrain_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                             C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain)]
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -210,7 +232,9 @@ ROLLOUT_SYMBOLS = ["wbc_integrate", "wbc_rollout", "wbc_rollout_host", "wbc_roll
                    "wbc_plant_step_host", "wbc_default_plant_opts"]
 PERTURB_SYMBOLS = ["wbc_plant_set_create", "wbc_plant_set_destroy", "wbc_plant_step_perturbed", "wbc_plant_step_perturbed_host",
                    "wbc_rollout_perturbed", "wbc_rollout_perturbed_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+TERRAIN_SYMBOLS = ["wbc_terrain_set_create", "wbc_terrain_set_destroy", "wbc_plant_step_terrain", "wbc_plant_step_terrain_host",
+                   "wbc_rollout_terrain", "wbc_rollout_terrain_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

@@ -348,6 +348,21 @@ __global__ void __launch_bounds__(32, WBC_PLANT_CTAS) wbc_plant_variant_kernel(w
     wbcplant::plant_step_instance<true>(sm->w, sm->p, pv.md, a, inst, lane, wbcplant::plant_perturb(pa, a, inst, k, pv.mu));
 }
 
+// The perturbed step on each robot's terrain (wbc_plant_step_terrain): staged like the variant kernel; lanes 0-3 read their
+// foot's terrain record and grid corners from global memory into the small terrain block of this layout.
+struct SmemLayoutPlantTerrain { wbcplant::PlantVariant pv; wbc::WarpSmem w; wbcplant::PlantSmem p; wbcplant::TerrainSmem t; };
+__global__ void __launch_bounds__(32, WBC_PLANT_CTAS) wbc_plant_terrain_kernel(wbcplant::PerturbArgs pa, wbcplant::TerrainArgs ta,
+                                                                                wbcplant::PlantArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  SmemLayoutPlantTerrain* sm = reinterpret_cast<SmemLayoutPlantTerrain*>(smem_raw);
+  const long long inst = blockIdx.x;
+  const int k = inst < a.n ? wbcplant::plant_variant(pa, inst) : 0;
+  const wbcplant::PlantVariant& pv = stage16(&sm->pv, pa.set + (k < 0 ? 0 : k));
+  const int lane = lane_index();
+  if (inst < a.n)
+    wbcplant::plant_step_instance<true, true>(sm->w, sm->p, pv.md, a, inst, lane, wbcplant::plant_perturb(pa, a, inst, k, pv.mu), &sm->t, ta);
+}
+
 __global__ void wbc_pd_kernel(const DevConst* __restrict__ gdc, const double* q, const double* v, double* tau, long long n) {
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t < n * WBC_NU) wbc::pd_element(gdc->md, gdc->pr, q, v, tau, t / WBC_NU, (int)(t % WBC_NU));
@@ -534,6 +549,7 @@ static int set_smem_attr(wbc_handle* h) {
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_dynamics_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlant)));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_variant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlantVariant)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_terrain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlantTerrain)));
   return WBC_OK;
 }
 
@@ -1446,8 +1462,10 @@ extern "C" int wbc_default_plant_opts(wbc_plant_opts* o) {
   return WBC_OK;
 }
 
-// pa == nullptr: the unperturbed plant kernel; otherwise the variant kernel with these perturbations.
-static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbcplant::PerturbArgs* pa, double* q,
+// pa == nullptr: the unperturbed plant kernel; otherwise the variant kernel with these perturbations, or with ta != nullptr the
+// terrain kernel.
+static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbcplant::PerturbArgs* pa,
+                        const wbcplant::TerrainArgs* ta, double* q,
                         double* v, const double* tau, double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact,
                         const double* metrics, double* err_max, double* metrics_log, const int* counter, cudaStream_t st) {
   wbc_plant_opts o;
@@ -1455,7 +1473,8 @@ static int plant_launch(wbc_handle* h, int64_t n, double dt, const wbc_plant_opt
   if (!(o.mu >= 0.0) || !(o.erp >= 0.0 && o.erp <= 1.0) || o.iters < 1 || o.iters > 1000) return fail_arg(h, "wbc_plant_step: bad options");
   const wbcplant::PlantArgs a{q, v, tau, t, ctrl_status, status_or, f_contact, metrics, err_max, metrics_log, counter, (long long)n, dt,
                               o.mu, o.erp, o.iters};
-  if (pa) wbc_plant_variant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlantVariant), st>>>(*pa, a);
+  if (pa && ta) wbc_plant_terrain_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlantTerrain), st>>>(*pa, *ta, a);
+  else if (pa) wbc_plant_variant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlantVariant), st>>>(*pa, a);
   else wbc_plant_kernel<<<(unsigned)n, 32, sizeof(SmemLayoutPlant), st>>>(h->d_const.p, a);
   h->launches++;
   return WBC_OK;
@@ -1533,7 +1552,7 @@ extern "C" int wbc_plant_step(wbc_handle* h, int64_t n, double dt, const wbc_pla
   if (n < 0 || !(dt > 0.0) || (n > 0 && (!q || !v || !tau))) return fail_arg(h, "wbc_plant_step: q, v, tau and dt > 0 are required");
   if (n == 0) return WBC_OK;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  const int rc = plant_launch(h, n, dt, opts, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr,
+  const int rc = plant_launch(h, n, dt, opts, nullptr, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr,
                               (cudaStream_t)stream);
   if (rc) return rc;
   WBC_CUDA(h, cudaGetLastError());
@@ -1549,16 +1568,93 @@ extern "C" int wbc_plant_step_perturbed(wbc_handle* h, int64_t n, double dt, con
   int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, t != nullptr, &pa);
   if (rc || n == 0) return rc;
   WBC_CUDA(h, cudaSetDevice(h->device));
-  rc = plant_launch(h, n, dt, opts, &pa, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+  rc = plant_launch(h, n, dt, opts, &pa, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
   if (rc) return rc;
   WBC_CUDA(h, cudaGetLastError());
   return WBC_OK;
 }
 
-// Host buffers of both plant steps; perturbed = false is wbc_plant_step_host.
-static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, bool perturbed, const wbc_plant_perturb* perturb,
-                           double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status, int32_t* status_or,
-                           double* f_contact, const char* what) {
+// ------------------------------------------------------------------------------ uneven ground (wbc_plant.cuh)
+// A set keeps the number of the device its records live on, not its handle: it may be destroyed after the handle.
+struct wbc_terrain_set {
+  int device = 0;
+  int32_t n_terrains = 0;
+  DevArray<wbcplant::TerrainRec> table;
+  DevArray<double> heights;       // every grid, concatenated (TerrainRec::off)
+  ~wbc_terrain_set() { cudaSetDevice(device); }   // the arrays are freed after this, on the set's device
+};
+
+extern "C" int wbc_terrain_set_destroy(wbc_terrain_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+extern "C" int wbc_terrain_set_create(wbc_handle* h, int32_t n_terrains, const wbc_terrain_desc* terrains, wbc_terrain_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !terrains || n_terrains <= 0) return fail_arg(h, "wbc_terrain_set_create: terrains and n_terrains > 0 are required");
+  *out = nullptr;
+  std::vector<wbcplant::TerrainRec> rec((size_t)n_terrains);
+  std::vector<double> heights;
+  for (int32_t k = 0; k < n_terrains; ++k) {
+    const wbc_terrain_desc& d = terrains[k];
+    const double vals[] = {d.z0, d.sx, d.sy, d.x0, d.y0, d.dx, d.dy};
+    if (!finite_all(vals, 7)) return fail_arg(h, "wbc_terrain_set_create: non-finite terrain value");
+    const bool grid = d.nx != 0 || d.ny != 0;
+    if (grid && !(d.nx >= 2 && d.ny >= 2)) return fail_arg(h, "wbc_terrain_set_create: nx and ny must both be 0 or both >= 2");
+    if (grid && !(d.dx > 0.0 && d.dy > 0.0)) return fail_arg(h, "wbc_terrain_set_create: a grid needs dx > 0 and dy > 0");
+    if (grid && !d.heights) return fail_arg(h, "wbc_terrain_set_create: a grid needs heights");
+    const size_t cells = grid ? (size_t)d.nx * (size_t)d.ny : 0;
+    if (grid && !finite_all(d.heights, cells)) return fail_arg(h, "wbc_terrain_set_create: non-finite height");
+    rec[k] = wbcplant::terrain_record(d, (long long)heights.size());
+    if (grid) heights.insert(heights.end(), d.heights, d.heights + cells);
+  }
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_terrain_set> ts(new (std::nothrow) wbc_terrain_set());
+  if (!ts) return WBC_ERR_NOMEM;
+  ts->device = h->device;
+  ts->n_terrains = n_terrains;
+  WBC_CUDA(h, ts->table.reserve(rec.size()));
+  WBC_CUDA(h, cudaMemcpy(ts->table.p, rec.data(), rec.size() * sizeof(rec[0]), cudaMemcpyHostToDevice));
+  if (!heights.empty()) {
+    WBC_CUDA(h, ts->heights.reserve(heights.size()));
+    WBC_CUDA(h, cudaMemcpy(ts->heights.p, heights.data(), heights.size() * sizeof(double), cudaMemcpyHostToDevice));
+  }
+  *out = ts.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of a terrain whose index array is already on the device.
+static int terrain_args(wbc_handle* h, const wbc_plant_terrain* p, wbcplant::TerrainArgs* ta) {
+  const wbc_terrain_set* set = p ? p->set : nullptr;
+  if (set && set->device != h->device) return fail_arg(h, "wbc_plant_terrain: the set lives on another device than the handle");
+  *ta = wbcplant::TerrainArgs{set ? set->table.p : nullptr, set ? set->heights.p : nullptr, p ? p->index : nullptr, set ? set->n_terrains : 1};
+  return WBC_OK;
+}
+
+extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                      const wbc_plant_terrain* terrain, double* q, double* v, const double* tau, double* t,
+                                      const int32_t* ctrl_status, int32_t* status_or, double* f_contact, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (n < 0 || !(dt > 0.0) || (n > 0 && (!q || !v || !tau))) return fail_arg(h, "wbc_plant_step_terrain: q, v, tau and dt > 0 are required");
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, t != nullptr, &pa);
+  if (!rc) rc = terrain_args(h, terrain, &ta);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  rc = plant_launch(h, n, dt, opts, &pa, &ta, q, v, tau, t, ctrl_status, status_or, f_contact, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+  if (rc) return rc;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Which plant a host entry runs.
+enum class PlantEntry { plain, perturbed, terrain };
+
+// Host buffers of the three plant steps.
+static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
+                           const wbc_plant_terrain* terrain, double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status,
+                           int32_t* status_or, double* f_contact, const char* what) {
   if (!h) return WBC_ERR_ARG;
   if (n < 0 || !(dt > 0.0)) return fail_arg(h, what);
   if (n == 0) return WBC_OK;
@@ -1570,28 +1666,41 @@ static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_
   double* df = s.out(f_contact, N * 12);
   wbc_plant_perturb dp{};
   if (perturb) dp = wbc_plant_perturb{perturb->set, s.in(perturb->variant, N), s.in(perturb->push, N * 8)};
+  wbc_plant_terrain dtr{};
+  if (terrain) dtr = wbc_plant_terrain{terrain->set, s.in(terrain->index, N)};
   WBC_SCRATCH_CHECK(h, s);
-  const int rc = perturbed ? wbc_plant_step_perturbed(h, n, dt, opts, perturb ? &dp : nullptr, dq, dv, dtau, dt_, dcs, dso, df, s.st)
-                           : wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, s.st);
+  const int rc =
+      entry == PlantEntry::terrain ? wbc_plant_step_terrain(h, n, dt, opts, perturb ? &dp : nullptr, terrain ? &dtr : nullptr, dq, dv, dtau,
+                                                            dt_, dcs, dso, df, s.st)
+      : entry == PlantEntry::perturbed ? wbc_plant_step_perturbed(h, n, dt, opts, perturb ? &dp : nullptr, dq, dv, dtau, dt_, dcs, dso, df, s.st)
+                                       : wbc_plant_step(h, n, dt, opts, dq, dv, dtau, dt_, dcs, dso, df, s.st);
   return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, double* q, double* v, const double* tau,
                                    double* t, const int32_t* ctrl_status, int32_t* status_or, double* f_contact) {
-  return plant_step_host(h, n, dt, opts, false, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact,
+  return plant_step_host(h, n, dt, opts, PlantEntry::plain, nullptr, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact,
                          "wbc_plant_step_host: n >= 0 and dt > 0 are required");
 }
 
 extern "C" int wbc_plant_step_perturbed_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
                                              double* q, double* v, const double* tau, double* t, const int32_t* ctrl_status,
                                              int32_t* status_or, double* f_contact) {
-  return plant_step_host(h, n, dt, opts, true, perturb, q, v, tau, t, ctrl_status, status_or, f_contact,
+  return plant_step_host(h, n, dt, opts, PlantEntry::perturbed, perturb, nullptr, q, v, tau, t, ctrl_status, status_or, f_contact,
                          "wbc_plant_step_perturbed_host: n >= 0 and dt > 0 are required");
 }
 
-// The rollout loop of wbc_rollout_ex and wbc_rollout_perturbed; pa != nullptr: the plant step runs the variant kernel.
+extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, const wbc_plant_perturb* perturb,
+                                           const wbc_plant_terrain* terrain, double* q, double* v, const double* tau, double* t,
+                                           const int32_t* ctrl_status, int32_t* status_or, double* f_contact) {
+  return plant_step_host(h, n, dt, opts, PlantEntry::terrain, perturb, terrain, q, v, tau, t, ctrl_status, status_or, f_contact,
+                         "wbc_plant_step_terrain_host: n >= 0 and dt > 0 are required");
+}
+
+// The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed and wbc_rollout_terrain; pa != nullptr: the plant step runs the
+// variant kernel, or with ta != nullptr the terrain kernel.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
-                       const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, cudaStream_t st) {
+                       const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -1618,7 +1727,7 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
     r = wbc_step(h, kind, n, &sio, st);
     if (r) return r;
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, pa, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
+      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
     } else {
@@ -1661,7 +1770,7 @@ extern "C" int wbc_rollout_ex(wbc_handle* h, int kind, const wbc_plan* plan, int
                               const wbc_rollout_io* io, const wbc_rollout_opts* opts, void* stream) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout: bad arguments");
-  return rollout_run(h, kind, plan, n, n_steps, dt, io, opts, nullptr, (cudaStream_t)stream);
+  return rollout_run(h, kind, plan, n, n_steps, dt, io, opts, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int wbc_rollout_perturbed(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
@@ -1671,7 +1780,20 @@ extern "C" int wbc_rollout_perturbed(wbc_handle* h, int kind, const wbc_plan* pl
   if (opts->plant == 0) return fail_arg(h, "wbc_rollout_perturbed: perturbations act on the ground plant (opts->plant = 1)");
   wbcplant::PerturbArgs pa;
   const int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
-  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, &pa, (cudaStream_t)stream);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, &pa, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int wbc_rollout_terrain(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                   const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                   const wbc_plant_terrain* terrain, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || !opts || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_terrain: bad arguments");
+  if (opts->plant == 0) return fail_arg(h, "wbc_rollout_terrain: terrain is ground for the ground plant (opts->plant = 1)");
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  int rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, &pa, &ta, (cudaStream_t)stream);
 }
 
 extern "C" int wbc_rollout(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
@@ -1682,9 +1804,9 @@ extern "C" int wbc_rollout(wbc_handle* h, int kind, const wbc_plan* plan, int64_
   return wbc_rollout_ex(h, kind, plan, n, n_steps, dt, io, &o, stream);
 }
 
-// Host buffers of both rollouts; perturbed = false is wbc_rollout_ex_host.
+// Host buffers of the three rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
-                        const wbc_rollout_opts* opts, bool perturbed, const wbc_plant_perturb* perturb) {
+                        const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -1702,20 +1824,31 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   o.f_contact = s.out(o.f_contact, N * 12);
   wbc_plant_perturb dp{};
   if (perturb) dp = wbc_plant_perturb{perturb->set, s.in(perturb->variant, N), s.in(perturb->push, N * 8)};
+  wbc_plant_terrain dtr{};
+  if (terrain) dtr = wbc_plant_terrain{terrain->set, s.in(terrain->index, N)};
   WBC_SCRATCH_CHECK(h, s);
-  const int rc = perturbed ? wbc_rollout_perturbed(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, s.st)
-                           : wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
+  const int rc =
+      entry == PlantEntry::terrain ? wbc_rollout_terrain(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+                                                         terrain ? &dtr : nullptr, s.st)
+      : entry == PlantEntry::perturbed ? wbc_rollout_perturbed(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, s.st)
+                                       : wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
   return rc ? rc : s.finish(h);
 }
 
 extern "C" int wbc_rollout_ex_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                                    const wbc_rollout_io* io, const wbc_rollout_opts* opts) {
-  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, false, nullptr);
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::plain, nullptr, nullptr);
 }
 
 extern "C" int wbc_rollout_perturbed_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                                           const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb) {
-  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, true, perturb);
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::perturbed, perturb, nullptr);
+}
+
+extern "C" int wbc_rollout_terrain_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                        const wbc_plant_terrain* terrain) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::terrain, perturb, terrain);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

@@ -11,14 +11,20 @@ Perturbed robots (`plant_set`, `variant`, `push`; ground plant only): the plant 
 (model.with_payload), other link masses or inertias - on the variant's own ground friction, and a push acts on the base during
 a time window, while the controller keeps the handle's nominal model. They run through `wbc_rollout_perturbed` /
 `wbc_plant_step_perturbed`.
+
+Uneven ground (`terrain_set`, `terrain`; ground plant only): each robot stands on its own terrain - a plane plus an optional
+height field (`Terrain`, defined in include/wbc.h) - while the controller keeps assuming flat ground. It runs through
+`wbc_rollout_terrain` / `wbc_plant_step_terrain`, together with any variants and pushes.
 """
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 
 import numpy as np
 
-from .capi import KINDS, WbcPlantOpts, WbcPlantPerturb, WbcRolloutIO, WbcRolloutOpts, np_ptr
+from .capi import (KINDS, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc,
+                   np_ptr)
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
 Q0_MINI_CHEETAH = np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.3] + [0.0, -0.8, 1.6] * 4)     # simulate.py:171-176
@@ -55,6 +61,53 @@ class PlantSet:
             pass
 
 
+@dataclass
+class Terrain:
+    """h(x, y) = z0 + slope[0] x + slope[1] y + H(x, y); H bilinear in heights[ny, nx] (None: no grid) with heights[0, 0] at
+    `origin` and spacing (dx, dy). Outside the grid its edge values continue flat."""
+    z0: float = 0.0
+    slope: tuple = (0.0, 0.0)
+    origin: tuple = (0.0, 0.0)
+    spacing: tuple = (1.0, 1.0)
+    heights: np.ndarray | None = None
+
+
+class TerrainSet:
+    """Device-resident table of T terrains for the ground plant (wbc_terrain_set_create); robot i stands on terrains[index[i]]."""
+
+    def __init__(self, ctl, terrains):
+        self.ctl, self.lib = ctl, ctl.lib
+        self.n_terrains = len(terrains)
+        grids = [None if t.heights is None else np.ascontiguousarray(t.heights, np.float64) for t in terrains]
+        descs = []
+        for t, g in zip(terrains, grids):
+            ny, nx = (0, 0) if g is None else g.shape
+            descs.append(WbcTerrainDesc(float(t.z0), float(t.slope[0]), float(t.slope[1]), nx, ny, float(t.origin[0]), float(t.origin[1]),
+                                        float(t.spacing[0]), float(t.spacing[1]), None if g is None else g.ctypes.data))
+        arr = (WbcTerrainDesc * self.n_terrains)(*descs)
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_terrain_set_create(ctl._h, self.n_terrains, arr, C.byref(self._p)), "wbc_terrain_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_terrain_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _terrain(terrain_set, index, ptr):
+    return WbcPlantTerrain(None if terrain_set is None else terrain_set._p, ptr(index))
+
+
+def _terrain_index(n, index):
+    return None if index is None else np.ascontiguousarray(np.broadcast_to(np.asarray(index, np.int32), (n,)))
+
+
 def _perturb(plant_set, variant, push, ptr):
     return WbcPlantPerturb(None if plant_set is None else plant_set._p, ptr(variant), ptr(push))
 
@@ -79,14 +132,17 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
-            mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None) -> RolloutResult:
+            mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
     carries the last step's ground forces `f_contact[N,4,3]`.
     Perturbed robots (plant=True only): plant_set (PlantSet or None: the nominal model), variant [N] int32 (None: variant 0),
     push [N,8] = force (world) | point (base frame) | t_on | t_off (None: no pushes); torch tensors on the device with torch
-    inputs, arrays otherwise. A robot with an out-of-range variant index is frozen and flagged ST_BADVARIANT."""
+    inputs, arrays otherwise. A robot with an out-of-range variant index is frozen and flagged ST_BADVARIANT.
+    Uneven ground (plant=True only): terrain_set (TerrainSet or None: flat ground), terrain [N] int32 (None: terrain 0); an
+    out-of-range terrain index freezes that robot, flagged ST_BADTERRAIN."""
+    on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
     if _is_torch(q):
@@ -99,7 +155,11 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if perturbed:
+        if on_terrain:
+            pt, tr = _perturb(plant_set, variant, push, p), _terrain(terrain_set, terrain, p)
+            ctl._check(ctl.lib.wbc_rollout_terrain(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
+                                                   C.byref(tr), stream), "wbc_rollout_terrain")
+        elif perturbed:
             pt = _perturb(plant_set, variant, push, p)
             ctl._check(ctl.lib.wbc_rollout_perturbed(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
                                                      stream), "wbc_rollout_perturbed")
@@ -117,7 +177,11 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if perturbed:
+    if on_terrain:
+        pt, tr = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt), _terrain(terrain_set, _terrain_index(n, terrain), opt)
+        ctl._check(ctl.lib.wbc_rollout_terrain_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
+                                                    C.byref(tr)), "wbc_rollout_terrain_host")
+    elif perturbed:
         pt = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt)
         ctl._check(ctl.lib.wbc_rollout_perturbed_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt)),
                    "wbc_rollout_perturbed_host")
@@ -126,11 +190,14 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     return r
 
 
-def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=None, plant_set=None, variant=None, push=None, t=None):
+def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=None, plant_set=None, variant=None, push=None, t=None,
+               terrain_set=None, terrain=None):
     """One time step of N simulated robots on flat ground -> q+[N,19], v+[N,18], f_contact[N,4,3] (ground forces LF RF LH RH,
     world axes), status[N]. Host arrays go through wbc_plant_step_host (q, v copied); torch CUDA tensors are updated IN PLACE
     on torch's current stream (wbc_plant_step). plant_set / variant / push as in `rollout` (wbc_plant_step_perturbed); t [N] is
-    each robot's time at the start of the step, required with pushes (a torch tensor is advanced by dt in place)."""
+    each robot's time at the start of the step, required with pushes (a torch tensor is advanced by dt in place). terrain_set /
+    terrain as in `rollout` (wbc_plant_step_terrain)."""
+    on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     o = WbcPlantOpts(float(mu), float(erp), int(iters), 0)
     if _is_torch(q):
@@ -140,7 +207,10 @@ def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=N
         p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         args = (p(q), p(v), p(tau), p(t), p(ctrl_status), p(st), p(f), stream)
-        if perturbed:
+        if on_terrain:
+            pt, tr = _perturb(plant_set, variant, push, p), _terrain(terrain_set, terrain, p)
+            ctl._check(ctl.lib.wbc_plant_step_terrain(ctl._h, n, float(dt), C.byref(o), C.byref(pt), C.byref(tr), *args), "wbc_plant_step_terrain")
+        elif perturbed:
             pt = _perturb(plant_set, variant, push, p)
             ctl._check(ctl.lib.wbc_plant_step_perturbed(ctl._h, n, float(dt), C.byref(o), C.byref(pt), *args), "wbc_plant_step_perturbed")
         else:
@@ -155,7 +225,11 @@ def plant_step(ctl, q, v, tau, dt=5e-3, mu=1.0, erp=0.2, iters=30, ctrl_status=N
     opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
     ta = None if t is None else np.array(np.broadcast_to(np.asarray(t, dtype=np.float64), (n,)))
     args = (np_ptr(q), np_ptr(v), np_ptr(tau), opt(ta), opt(cs), np_ptr(st), np_ptr(f))
-    if perturbed:
+    if on_terrain:
+        pt, tr = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt), _terrain(terrain_set, _terrain_index(n, terrain), opt)
+        ctl._check(ctl.lib.wbc_plant_step_terrain_host(ctl._h, n, float(dt), C.byref(o), C.byref(pt), C.byref(tr), *args),
+                   "wbc_plant_step_terrain_host")
+    elif perturbed:
         pt = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt)
         ctl._check(ctl.lib.wbc_plant_step_perturbed_host(ctl._h, n, float(dt), C.byref(o), C.byref(pt), *args), "wbc_plant_step_perturbed_host")
     else:
