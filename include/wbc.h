@@ -70,6 +70,7 @@ extern "C" {
 #define WBC_ST_NONFINITE 256   /* a NaN / inf among the q, v, traj values of the instance, or a non-finite solution */
 #define WBC_ST_BADVARIANT 512  /* perturbed plant only: variant index out of range; the robot is frozen, zero ground forces */
 #define WBC_ST_BADTERRAIN 1024 /* terrain plant only: terrain index out of range; the robot is frozen, zero ground forces */
+#define WBC_ST_BADPARAMS 2048  /* wbc_step_params only: parameter-set index out of range; zero outputs                  */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -460,6 +461,43 @@ int wbc_rollout_terrain(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
 int wbc_rollout_terrain_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                              const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
                              const wbc_plant_terrain* terrain);
+
+/* ---- Per-robot controller parameters: one batched step or rollout runs many gain and weight sets. The controller keeps the
+ * handle's model; only the wbc_params differ from robot to robot.
+ *
+ * wbc_param_set_create uploads n_sets >= 1 parameter sets to the handle's device, each with the constants derived from it
+ * (the CLF Riccati solution). Each set must pass the checks of wbc_create (reg_vd == 0, reg_f > 0) and have finite values,
+ * max_iter >= 1, torque_limits 0 or 1, mu >= 0, clf_r > 0 and non-negative CLF weights (clf_q_*, clf_w_delta). Like a plan, a
+ * set keeps its device number, not its handle: it may be destroyed after the handle. */
+typedef struct wbc_param_set wbc_param_set;
+int wbc_param_set_create(wbc_handle* h, int32_t n_sets, const wbc_params* params, wbc_param_set** out);
+int wbc_param_set_destroy(wbc_param_set* s);
+
+/* Per-robot parameters of a step or rollout (device pointer for the device entries, host pointer for _host). */
+typedef struct wbc_ctrl_params {
+  const wbc_param_set* set;  /* NULL: the handle's params for every robot (one set, index 0)                            */
+  const int32_t* index;      /* [N] set of each robot, NULL = set 0. An index < 0 or >= n_sets sets WBC_ST_BADPARAMS:
+                              * that robot returns tau = 0 (and f = vd = lam = 0), its neighbours are unaffected        */
+} wbc_ctrl_params;
+
+/* wbc_step / wbc_step_host with robot i controlled by the set index[i]: the same buffer rules, chunking and stream semantics,
+ * the same kernels' arithmetic and the same launch count. With a set whose every record equals the handle's params it gives
+ * the bits of wbc_step. WBC_CTRL_PD reads pd_kp, pd_kd, pd_clip and pd_q_nom per robot; it writes status[i] (WBC_ST_BADPARAMS
+ * or 0) when io->status is non-NULL. p == NULL is the handle's params. */
+int wbc_step_params(wbc_handle* h, int kind, int64_t n, const wbc_io* io, const wbc_ctrl_params* p, void* stream);
+int wbc_step_params_host(wbc_handle* h, int kind, int64_t n, const wbc_io* host_io, const wbc_ctrl_params* p);
+
+/* The rollout loop of wbc_rollout_ex with per-robot controller parameters (ctrl == NULL: the handle's). With the ground plant
+ * (opts->plant = 1) the plant step is the terrain kernel when terrain != NULL, else the variant kernel when perturb != NULL,
+ * else the plain one; perturb or terrain without the ground plant is an argument error. The same launches per step, graph
+ * capture and bookkeeping as wbc_rollout_ex. A robot flagged WBC_ST_BADPARAMS gets zero torques: the integrator plant freezes
+ * it (as any flagged robot); the ground plant lets it go limp, and status_or keeps the flag. */
+int wbc_rollout_params(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                       const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                       const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, void* stream);
+int wbc_rollout_params_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                            const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                            const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

@@ -23,10 +23,12 @@ ST_MAXITER, ST_INFEASIBLE, ST_RANKDEF, ST_GIMBAL, ST_NOTPD, ST_BADQUAT, ST_UNSUP
 ST_NONFINITE = 256
 ST_BADVARIANT = 512
 ST_BADTERRAIN = 1024
+ST_BADPARAMS = 2048
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
-             ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN"}
+             ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN",
+             ST_BADPARAMS: "BADPARAMS"}
 
 
 def status_names(status: int) -> str:
@@ -111,6 +113,11 @@ class WbcTerrainDesc(C.Structure):
 
 class WbcPlantTerrain(C.Structure):
     """ctypes mirror of `wbc_plant_terrain` (terrain set, per-robot terrain index)."""
+    _fields_ = [("set", C.c_void_p), ("index", C.c_void_p)]
+
+
+class WbcCtrlParams(C.Structure):
+    """ctypes mirror of `wbc_ctrl_params` (parameter set, per-robot set index)."""
     _fields_ = [("set", C.c_void_p), ("index", C.c_void_p)]
 
 
@@ -203,7 +210,15 @@ def load_library() -> C.CDLL:
                                         C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), dp]
     lib.wbc_rollout_terrain_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
                                              C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain)]
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS:
+    lib.wbc_param_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcParams), C.POINTER(H)]
+    lib.wbc_param_set_destroy.argtypes = [dp]
+    lib.wbc_step_params.argtypes = [H, i32, i64, C.POINTER(WbcIO), C.POINTER(WbcCtrlParams), dp]
+    lib.wbc_step_params_host.argtypes = [H, i32, i64, C.POINTER(WbcIO), C.POINTER(WbcCtrlParams)]
+    lib.wbc_rollout_params.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                       C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), dp]
+    lib.wbc_rollout_params_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                            C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams)]
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -234,7 +249,9 @@ PERTURB_SYMBOLS = ["wbc_plant_set_create", "wbc_plant_set_destroy", "wbc_plant_s
                    "wbc_rollout_perturbed", "wbc_rollout_perturbed_host"]
 TERRAIN_SYMBOLS = ["wbc_terrain_set_create", "wbc_terrain_set_destroy", "wbc_plant_step_terrain", "wbc_plant_step_terrain_host",
                    "wbc_rollout_terrain", "wbc_rollout_terrain_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+PARAM_SYMBOLS = ["wbc_param_set_create", "wbc_param_set_destroy", "wbc_step_params", "wbc_step_params_host", "wbc_rollout_params",
+                 "wbc_rollout_params_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

@@ -5,7 +5,8 @@
     step(kind, q[N,19], v[N,18], traj[N,54], contact[N,4]) -> tau[N,12], metrics[N,4], status[N]
 
 on NumPy arrays (host buffers; copies happen inside `wbc_step_host`) or torch CUDA tensors
-(device pointers, launched on torch's current stream).
+(device pointers, launched on torch's current stream). `ParamSet` holds K gain / weight sets on the device; with
+`param_set=` / `param_index=` each robot of one step runs with its own set (`wbc_step_params[_host]`).
 
 `IDController`, `CLFController`, `PCController` keep the reference constructor
 `(plant, dt, use_lcm=False)` and port layout (reference controllers/basic_controller.py:21-77,
@@ -23,7 +24,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .capi import KINDS, WbcIO, make_params, np_ptr
+from .capi import KINDS, WbcCtrlParams, WbcIO, WbcParams, make_params, np_ptr
 from .model import NQ, NTRAJ, NU, NV, RobotModel, load_robot
 
 FEET = ["lf", "rf", "lh", "rh"]
@@ -70,6 +71,49 @@ class StepOutput:
         return iter((self.tau, self.metrics, self.status))
 
 
+class ParamSet:
+    """Device-resident table of K controller parameter sets (wbc_param_set_create) on the device of `ctl`: params[k] is a
+    dict of overrides for `make_params` or a `WbcParams` struct. Robot i of a step or rollout given `param_set=` runs with
+    params[param_index[i]]; an index outside [0, K) is flagged ST_BADPARAMS with zero outputs."""
+
+    def __init__(self, ctl, params):
+        self.ctl, self.lib = ctl, ctl.lib
+        structs = [p if isinstance(p, WbcParams) else make_params(**p) for p in params]
+        self.n_sets = len(structs)
+        arr = (WbcParams * self.n_sets)(*structs)
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_param_set_create(ctl._h, self.n_sets, arr, C.byref(self._p)), "wbc_param_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_param_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _ctrl_params(param_set, index_ptr):
+    return WbcCtrlParams(None if param_set is None else param_set._p, index_ptr)
+
+
+def check_device_index(index, n, what="param_index"):
+    """A per-robot index on the device must be a contiguous int32 CUDA tensor of shape (N,): the kernels read it as int32
+    through its device pointer."""
+    import torch
+    if index is not None and not (_is_torch(index) and index.is_cuda and index.is_contiguous() and index.dtype == torch.int32
+                                  and tuple(index.shape) == (n,)):
+        raise ValueError(f"{what} on the device must be a contiguous CUDA tensor int32[{n}]")
+
+
+def _param_index(n, index):
+    """Host copy of a per-robot set index in the layout of the C ABI (int32 [N]); None stays None."""
+    return None if index is None else np.ascontiguousarray(np.broadcast_to(np.asarray(index, np.int32), (n,)))
+
+
 class BatchedController:
     """One handle of libwbc_b200.so on one device."""
 
@@ -108,10 +152,13 @@ class BatchedController:
         return int(self.lib.wbc_launch_count(self._h))
 
     # ------------------------------------------------------------------ batch step
-    def step(self, kind, q, v, traj, contact, debug=False) -> StepOutput:
+    def step(self, kind, q, v, traj, contact, debug=False, param_set=None, param_index=None) -> StepOutput:
+        """param_set (ParamSet or None: the handle's params) / param_index [N] (None: set 0): per-robot controller parameters
+        through wbc_step_params[_host]; a torch index is an int32 CUDA tensor. Left at None, wbc_step[_host] runs."""
         k = KINDS[kind] if isinstance(kind, str) else int(kind)
+        per_robot = param_set is not None or param_index is not None
         if _is_torch(q):
-            return self._step_torch(k, q, v, traj, contact, debug)
+            return self._step_torch(k, q, v, traj, contact, debug, param_set, param_index, per_robot)
         q = np.ascontiguousarray(q, dtype=np.float64).reshape(-1, NQ)
         n = q.shape[0]
         v = np.ascontiguousarray(v, dtype=np.float64).reshape(n, NV)
@@ -125,7 +172,12 @@ class BatchedController:
         io = WbcIO(np_ptr(q), np_ptr(v), np_ptr(traj), np_ptr(contact), np_ptr(tau), np_ptr(met), np_ptr(st),
                    np_ptr(vd) if debug else None, np_ptr(f) if debug else None, np_ptr(qi) if debug else None,
                    np_ptr(lam) if debug else None)
-        self._check(self.lib.wbc_step_host(self._h, k, n, C.byref(io)), "wbc_step_host")
+        if per_robot:
+            pi = _param_index(n, param_index)
+            cp = _ctrl_params(param_set, None if pi is None else np_ptr(pi))
+            self._check(self.lib.wbc_step_params_host(self._h, k, n, C.byref(io), C.byref(cp)), "wbc_step_params_host")
+        else:
+            self._check(self.lib.wbc_step_host(self._h, k, n, C.byref(io)), "wbc_step_host")
         return StepOutput(tau, met, st, vd, f, qi, lam)
 
     def step_plan(self, kind, sampler, q, v, t, plan_index=None, tau=None, metrics=None, status=None) -> StepOutput:
@@ -144,22 +196,48 @@ class BatchedController:
                                                 np_ptr(tau), np_ptr(metrics), np_ptr(status)), "wbc_step_plan_host")
         return StepOutput(tau, metrics, status)
 
-    def step_pd(self, q, v):
-        """BasicController.ControlLaw (basic_controller.py:322-352) for a batch of host states -> tau[N,12]."""
+    def step_pd(self, q, v, param_set=None, param_index=None):
+        """BasicController.ControlLaw (basic_controller.py:322-352) for a batch of host states -> tau[N,12]. With param_set /
+        param_index (as in `step`) each robot uses its set's pd_kp, pd_kd, pd_clip and pd_q_nom, and the call returns
+        (tau, status[N]) with ST_BADPARAMS for an index out of range. Torch CUDA tensors (in place of the arrays, param_index
+        int32) always go through wbc_step_params on torch's current stream and return (tau, status)."""
+        if _is_torch(q):
+            import torch
+            n = q.shape[0]
+            for t, w in ((q, NQ), (v, NV)):
+                if not (_is_torch(t) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float64 and tuple(t.shape) == (n, w)):
+                    raise ValueError("device inputs must be contiguous CUDA tensors: q f64[N,19], v f64[N,18]")
+            check_device_index(param_index, n)
+            tau = torch.empty((n, NU), dtype=torch.float64, device=q.device)
+            st = torch.empty((n,), dtype=torch.int32, device=q.device)
+            p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+            io = WbcIO(p(q), p(v), None, None, p(tau), None, p(st), None, None, None)
+            cp = _ctrl_params(param_set, p(param_index))
+            stream = torch.cuda.current_stream(q.device).cuda_stream
+            self._check(self.lib.wbc_step_params(self._h, capi.WBC_CTRL_PD, n, C.byref(io), C.byref(cp), C.c_void_p(stream)), "wbc_step_params")
+            return tau, st
         q = np.ascontiguousarray(q, dtype=np.float64).reshape(-1, NQ)
         n = q.shape[0]
         v = np.ascontiguousarray(v, dtype=np.float64).reshape(n, NV)
         tau = np.empty((n, NU))
+        if param_set is not None or param_index is not None:
+            st = np.empty(n, dtype=np.int32)
+            pi = _param_index(n, param_index)
+            io = WbcIO(np_ptr(q), np_ptr(v), None, None, np_ptr(tau), None, np_ptr(st), None, None, None)
+            cp = _ctrl_params(param_set, None if pi is None else np_ptr(pi))
+            self._check(self.lib.wbc_step_params_host(self._h, capi.WBC_CTRL_PD, n, C.byref(io), C.byref(cp)), "wbc_step_params_host")
+            return tau, st
         io = WbcIO(np_ptr(q), np_ptr(v), None, None, np_ptr(tau), None, None, None, None, None)
         self._check(self.lib.wbc_step_host(self._h, capi.WBC_CTRL_PD, n, C.byref(io)), "wbc_step_host")
         return tau
 
-    def _step_torch(self, k, q, v, traj, contact, debug):
+    def _step_torch(self, k, q, v, traj, contact, debug, param_set=None, param_index=None, per_robot=False):
         import torch
         n = q.shape[0]
         for t, w, dt in ((q, NQ, torch.float64), (v, NV, torch.float64), (traj, NTRAJ, torch.float64), (contact, 4, torch.uint8)):
             if not (t.is_cuda and t.is_contiguous() and t.dtype == dt and t.shape == (n, w)):
                 raise ValueError("device inputs must be contiguous CUDA tensors: q f64[N,19], v f64[N,18], traj f64[N,54], contact u8[N,4]")
+        check_device_index(param_index, n)
         dev = q.device
         tau = torch.empty((n, NU), dtype=torch.float64, device=dev)
         met = torch.empty((n, 4), dtype=torch.float64, device=dev)
@@ -170,7 +248,11 @@ class BatchedController:
         lam = torch.empty((n, capi.NLAM), dtype=torch.float64, device=dev) if debug else None
         io = self.make_io(q, v, traj, contact, tau, met, st, vd, f, qi, lam)
         stream = torch.cuda.current_stream(dev).cuda_stream
-        self._check(self.lib.wbc_step(self._h, k, n, C.byref(io), C.c_void_p(stream)), "wbc_step")
+        if per_robot:
+            cp = _ctrl_params(param_set, None if param_index is None else C.c_void_p(param_index.data_ptr()))
+            self._check(self.lib.wbc_step_params(self._h, k, n, C.byref(io), C.byref(cp), C.c_void_p(stream)), "wbc_step_params")
+        else:
+            self._check(self.lib.wbc_step(self._h, k, n, C.byref(io), C.c_void_p(stream)), "wbc_step")
         return StepOutput(tau, met, st, vd, f, qi, lam)
 
     @staticmethod

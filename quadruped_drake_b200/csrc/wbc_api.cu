@@ -368,6 +368,147 @@ __global__ void wbc_pd_kernel(const DevConst* __restrict__ gdc, const double* q,
   if (t < n * WBC_NU) wbc::pd_element(gdc->md, gdc->pr, q, v, tau, t / WBC_NU, (int)(t % WBC_NU));
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Per-robot controller parameters (wbc_step_params): twins of the step kernels above that take each robot's wbc_params and
+// derived constants from its record of a parameter set (wbc::ParamRec) instead of the handle's DevConst. The model stays the
+// handle's. They run the same device functions; a reduce CTA stages the model and one record per warp, which at W = 1 is the
+// byte count of DevConst, so shared memory and occupancy match the plain kernels.
+struct alignas(16) ModelConst { wbc_model md; };   // the model at the head of DevConst, rounded up to 16 bytes
+static_assert(offsetof(DevConst, md) == 0 && sizeof(ModelConst) <= sizeof(DevConst) && sizeof(wbc::ParamRec) % 16 == 0,
+              "the model is staged from the head of DevConst; records are staged with 16-byte vectors");
+
+template <int W>
+struct SmemLayoutParamsT {
+  ModelConst mc;
+  wbc::ParamRec prm[W];
+  InStage<W> in;
+  wbc::WarpSmem w[W];
+};
+template <int W>
+struct SmemLayoutPCParamsT {
+  ModelConst mc;
+  wbc::ParamRec prm[W];
+  InStage<W> in;
+  wbc::WarpSmem w[W];
+  wbc::PcSmem pc[W];
+};
+static_assert(sizeof(SmemLayoutParamsT<WARPS>) == sizeof(SmemLayoutT<WARPS>), "single-warp CTAs stage as many bytes as the plain kernel");
+
+// Stages the model and the records of the CTA's W robots (record 0 for a slot past the end) with 16-byte vectors and one CTA
+// barrier at the end; returns the status bits of the calling warp's robot (WBC_ST_BADPARAMS for an index out of range).
+template <int W, typename L>
+__device__ __forceinline__ int stage_params(L* sm, const DevConst* gdc, const wbc::ParamArgs& p, long long n, int warp) {
+  constexpr int NM = (int)(sizeof(ModelConst) / 16), NR = (int)(sizeof(wbc::ParamRec) / 16);
+  const uint4* gm = reinterpret_cast<const uint4*>(gdc);
+  uint4* dm = reinterpret_cast<uint4*>(&sm->mc);
+  for (int i = threadIdx.x; i < NM; i += blockDim.x) dm[i] = gm[i];
+  const long long first = (long long)blockIdx.x * W;
+  int mine = 0;
+#pragma unroll
+  for (int w = 0; w < W; ++w) {
+    int st = 0;
+    const wbc::ParamRec& r = first + w < n ? wbc::param_record(p, first + w, st) : p.set[0];
+    if (w == warp) mine = st;
+    const uint4* src = reinterpret_cast<const uint4*>(&r);
+    uint4* dst = reinterpret_cast<uint4*>(&sm->prm[w]);
+    for (int i = threadIdx.x; i < NR; i += blockDim.x) dst[i] = src[i];
+  }
+  __syncthreads();
+  return mine;
+}
+
+template <int KIND, int W>
+__global__ void __launch_bounds__(W * 32, WBC_MIN_WARPS / W) wbc_reduce_params_kernel(const DevConst* __restrict__ gdc, wbc::ParamArgs p,
+                                                                                   wbc::StepArgs a, double* __restrict__ rec,
+                                                                                   double* __restrict__ vdmap, int bulk_ok) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  SmemLayoutParamsT<W>* sm = reinterpret_cast<SmemLayoutParamsT<W>*>(smem_raw);
+  pdl_launch_dependents();
+  const bool staged = stage_inputs_issue(sm->in, a, bulk_ok != 0);
+  const int warp = W == 1 ? 0 : (int)(threadIdx.x >> 5), lane = lane_index();
+  const int pstatus = stage_params<W>(sm, gdc, p, a.n, warp);
+  const long long inst = (long long)blockIdx.x * W + warp;
+  if (inst >= a.n) return;
+  wbc::WarpSmem& s = sm->w[warp];
+  const wbc::ParamRec& pr = sm->prm[warp];
+  wbc::StepCarry c;
+  const wbc::StagedInputs in = staged_rows(sm->in, warp);
+  if (staged) mbar_wait(&sm->in.mbar, 0);
+  wbc::reduce_instance<KIND>(s, sm->mc.md, pr.pr, pr.dv, a, inst, lane, c, nullptr, vdmap ? vdmap + inst * wbc::VDMAP_DOUBLES : nullptr,
+                             staged ? &in : nullptr);
+  c.status |= pstatus;
+  __syncwarp();
+  if (lane == 0) store_record(rec + inst * wbc::REC_DOUBLES, c, s);
+}
+
+template <int KIND, bool VD>
+__global__ void __launch_bounds__(SOLVE_WARPS * 32, VD ? (24 / SOLVE_WARPS) : WBC_SOLVE_CTAS) wbc_solve_params_kernel(
+    const DevConst* __restrict__ gdc, wbc::ParamArgs p, wbc::StepArgs a, const double* __restrict__ rec, const double* __restrict__ vdmap) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  SmemLayoutSolveT<VD>* sm = reinterpret_cast<SmemLayoutSolveT<VD>*>(smem_raw);
+  const int warp = SOLVE_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5), lane = lane_index();
+  const long long inst = (long long)blockIdx.x * SOLVE_WARPS + warp;
+  if (inst >= a.n) return;
+  wbc::SolveSmemT<VD>& s = sm->w[warp];
+  const double* r = rec + inst * wbc::REC_DOUBLES;
+  const double2* m = reinterpret_cast<const double2*>(r + wbc::REC_Y);
+  int pstatus = 0;                 // (the reduce kernel has set the same bit in the record's status word)
+  const wbc::ParamRec& pr = wbc::param_record(p, inst, pstatus);
+  pdl_wait();
+  const double2 m2 = m[2];
+  const bool ok = m2.x != 0.0;
+  if (ok && lane == 0) bulk_load(&s.Y[0][0], r, REC_Y_BYTES, &s.mbar);
+  const double2 m0 = m[0], m1 = m[1], m3 = m[3], m4 = m[4], m5 = m[5];
+  wbc::StepCarry c;
+  c.status = (int)m0.x | pstatus; c.cmask = (unsigned)m0.y; c.nf = (int)m1.x; c.nextra = (int)m1.y;
+  c.ok = ok; c.pc_ok = m2.y != 0.0; c.extra_bound = m3.x; c.err = m3.y; c.Vl = m4.x; c.PFl = m4.y; c.csum = m5.x; c.Vpc = m5.y;
+  __syncwarp();
+  if (ok) mbar_wait(&s.mbar, 0);
+  wbc::solve_instance<KIND, wbc::SolveSmemT<VD>>(s, gdc->md, pr.pr, a, inst, lane, c, vdmap ? vdmap + inst * wbc::VDMAP_DOUBLES : nullptr, r);
+}
+
+template <int W>
+__global__ void __launch_bounds__(W * 32, WBC_PC_MIN_WARPS / W) wbc_reduce_pc_params_kernel(const DevConst* __restrict__ gdc, wbc::ParamArgs p,
+                                                                                          wbc::StepArgs a, double* __restrict__ rec,
+                                                                                          double* __restrict__ vdmap, int bulk_ok) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  SmemLayoutPCParamsT<W>* sm = reinterpret_cast<SmemLayoutPCParamsT<W>*>(smem_raw);
+  pdl_launch_dependents();
+  const bool staged = stage_inputs_issue(sm->in, a, bulk_ok != 0);
+  const int warp = W == 1 ? 0 : (int)(threadIdx.x >> 5), lane = lane_index();
+  const int pstatus = stage_params<W>(sm, gdc, p, a.n, warp);
+  const long long inst = (long long)blockIdx.x * W + warp;
+  if (inst >= a.n) return;
+  wbc::WarpSmem& s = sm->w[warp];
+  const wbc::ParamRec& pr = sm->prm[warp];
+  wbc::StepCarry c;
+  const wbc::StagedInputs in = staged_rows(sm->in, warp);
+  if (staged) mbar_wait(&sm->in.mbar, 0);
+  {
+    // the meeting points of wbc_reduce_pc_kernel
+    const long long first = (long long)blockIdx.x * W;
+    const int n_act = (int)((a.n - first) < W ? (a.n - first) : W);
+    int n_pc = 0;
+    for (int w = 0; w < n_act; ++w) {
+      const uint8_t* cp = (staged && in.contact) ? sm->in.contact + w * 4 : a.contact + (first + w) * 4;
+      n_pc += (cp[0] | cp[1] | cp[2] | cp[3]) ? 1 : 0;
+    }
+    sm->pc[warp].sync_all = 32 * n_act;
+    sm->pc[warp].sync_pc = 32 * n_pc;
+  }
+  wbc::reduce_instance<WBC_CTRL_PC>(s, sm->mc.md, pr.pr, pr.dv, a, inst, lane, c, &sm->pc[warp], vdmap ? vdmap + inst * wbc::VDMAP_DOUBLES : nullptr,
+                                    staged ? &in : nullptr);
+  c.status |= pstatus;
+  __syncwarp();
+  if (lane == 0) store_record(rec + inst * wbc::REC_DOUBLES, c, s);
+}
+
+__global__ void wbc_pd_params_kernel(const DevConst* __restrict__ gdc, wbc::ParamArgs p, const double* q, const double* v, double* tau,
+                                     int32_t* status, long long n) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n * WBC_NU) wbc::pd_params_element(gdc->md, p, q, v, tau, status, t / WBC_NU, (int)(t % WBC_NU));
+}
+
 // Register-resident DFMA loop: 8 independent chains per thread, 2 flop per FMA.
 __global__ void fp64_peak_kernel(double* out, int iters) {
   double a0 = threadIdx.x * 1e-9, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -442,6 +583,7 @@ struct Staging {
   DevArray<double> q, v, traj, tau, metrics, vd, f, info, lam;
   DevArray<uint8_t> contact;
   DevArray<int32_t> status;
+  DevArray<int32_t> index;             // parameter-set index of wbc_step_params_host (reserved by that entry only)
   cudaError_t reserve(int64_t n) {
     cudaError_t e = q.reserve(n * WBC_NQ);
     if (e == cudaSuccess) e = v.reserve(n * WBC_NV);
@@ -487,6 +629,7 @@ struct wbc_handle {
   wbc_model model;
   wbc_params params;
   DevArray<wbcplant::PlantVariant> d_nominal;   // the handle's model as the one variant of a perturbed step without a set
+  DevArray<wbc::ParamRec> d_params;            // the handle's params as the one record of a parameter step without a set
   std::string err;
   int64_t launches = 0;
   int sm_count = 148;
@@ -550,6 +693,17 @@ static int set_smem_attr(wbc_handle* h) {
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlant)));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_variant_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlantVariant)));
   WBC_CUDA(h, cudaFuncSetAttribute(wbc_plant_terrain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPlantTerrain)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_reduce_params_kernel<WBC_CTRL_ID, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutParamsT<WARPS>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_reduce_params_kernel<WBC_CTRL_CLF, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutParamsT<WARPS>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_reduce_params_kernel<WBC_CTRL_ID, WARPS_HOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutParamsT<WARPS_HOST>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_reduce_params_kernel<WBC_CTRL_CLF, WARPS_HOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutParamsT<WARPS_HOST>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_reduce_pc_params_kernel<WARPS_PC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutPCParamsT<WARPS_PC>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_ID, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<false>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_CLF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<false>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_PC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<false>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_ID, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<true>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_CLF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<true>)));
+  WBC_CUDA(h, cudaFuncSetAttribute(wbc_solve_params_kernel<WBC_CTRL_PC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemLayoutSolveT<true>)));
   return WBC_OK;
 }
 
@@ -576,6 +730,9 @@ extern "C" int wbc_create(const wbc_model* model, const wbc_params* params, int 
   wbcplant::PlantVariant nominal{*model, 0.0};
   WBC_CUDA(h, h->d_nominal.reserve(1));
   WBC_CUDA(h, cudaMemcpy(h->d_nominal.p, &nominal, sizeof(nominal), cudaMemcpyHostToDevice));
+  const wbc::ParamRec own{hc.pr, hc.dv};
+  WBC_CUDA(h, h->d_params.reserve(1));
+  WBC_CUDA(h, cudaMemcpy(h->d_params.p, &own, sizeof(own), cudaMemcpyHostToDevice));
   // the streams and events: created here, not on first use, so that a step never calls a resource-creating API while some
   // other stream of the process is being captured
   for (Stream& s : h->lane) WBC_CUDA(h, cudaStreamCreateWithFlags(&s.v, cudaStreamNonBlocking));
@@ -748,12 +905,17 @@ struct Issue {
   bool profile = false;         // wbc_profile_step: events before the reduce kernel, between the kernels, after the solve kernel
 };
 
-// The instances from `o` on of every array of `io`; optional (null) arrays stay null.
+// The instances from `o` on of a per-instance array with `width` elements per instance; a null array stays null.
+template <typename T>
+static T* rows_at(T* p, int64_t o, int width) { return p ? p + o * width : nullptr; }
+// ... of every array of `io`
 static wbc_io io_at(const wbc_io& io, int64_t o) {
-  auto at = [o](auto* p, int width) { return p ? p + o * width : nullptr; };
+  auto at = [o](auto* p, int width) { return rows_at(p, o, width); };
   return wbc_io{at(io.q, WBC_NQ), at(io.v, WBC_NV), at(io.traj, WBC_NTRAJ), at(io.contact, 4), at(io.tau, WBC_NU),
                 at(io.metrics, WBC_NMETRIC), at(io.status, 1), at(io.vd, WBC_NV), at(io.f, 12), at(io.qp_info, 4), at(io.lam, WBC_NLAM)};
 }
+// ... of the set indices of a parameter step
+static wbc::ParamArgs params_at(const wbc::ParamArgs& p, int64_t o) { return wbc::ParamArgs{p.set, rows_at(p.index, o, 1), p.n_sets}; }
 static wbc::StepArgs step_args(const wbc_io& io, int64_t m, int kind) {
   return wbc::StepArgs{io.q, io.v, io.traj, io.contact, io.tau, io.metrics, io.status, io.vd, io.f, io.qp_info, io.lam, (long long)m, kind};
 }
@@ -821,8 +983,10 @@ static int order_slot(wbc_handle* h, Slot& s, cudaStream_t st) {
   return WBC_OK;
 }
 
+// pa != nullptr: the parameter-aware kernels with these per-robot parameters (the index array is sliced with the chunk).
 template <int KIND>
-static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is) {
+static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is,
+                        const wbc::ParamArgs* pa) {
   Slot& sl = h->slot[slot];
   WBC_CUDA(h, sl.reserve(n, io.vd != nullptr));
   const int rc = order_slot(h, sl, st);
@@ -833,6 +997,7 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cu
   for (int64_t o = 0; o < n; o += SPLIT_CHUNK) {
     const int64_t m = (n - o) < SPLIT_CHUNK ? (n - o) : SPLIT_CHUNK;
     const wbc::StepArgs a = step_args(io_at(io, o), m, kind);
+    const wbc::ParamArgs p = pa ? params_at(*pa, o) : wbc::ParamArgs{};
     // bulk input staging needs 16-byte aligned rows at the CTA boundaries (chunk offsets are multiples of 4)
     const bool al_vt = aligned16(a.v) && aligned16(a.traj), al_qc = aligned16(a.q) && aligned16(a.contact);
     if (is.profile) cudaEventRecord(h->prof_ev[0], st);
@@ -841,13 +1006,22 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cu
       constexpr int W = (KIND == WBC_CTRL_PC) ? WARPS_PC : WARPS_HOST;
       const unsigned grid = (unsigned)((m + W - 1) / W);
       const int bulk_ok = al_vt && al_qc;
-      if constexpr (KIND == WBC_CTRL_PC) wbc_reduce_pc_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
-      else wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      if constexpr (KIND == WBC_CTRL_PC) {
+        if (pa) wbc_reduce_pc_params_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCParamsT<W>), st>>>(dc, p, a, rec, vdmap, bulk_ok);
+        else wbc_reduce_pc_kernel<W><<<grid, W * 32, sizeof(SmemLayoutPCT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      } else if (pa) {
+        wbc_reduce_params_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutParamsT<W>), st>>>(dc, p, a, rec, vdmap, bulk_ok);
+      } else {
+        wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      }
     } else {
       constexpr int W = WARPS;
       const unsigned grid = (unsigned)((m + W - 1) / W);
       const int bulk_ok = al_vt;
-      if constexpr (KIND != WBC_CTRL_PC) wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      if constexpr (KIND != WBC_CTRL_PC) {
+        if (pa) wbc_reduce_params_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutParamsT<W>), st>>>(dc, p, a, rec, vdmap, bulk_ok);
+        else wbc_reduce_kernel<KIND, W><<<grid, W * 32, sizeof(SmemLayoutT<W>), st>>>(dc, a, rec, vdmap, bulk_ok);
+      }
     }
     if (is.profile) cudaEventRecord(h->prof_ev[1], st);
     const unsigned sgrid = (unsigned)((m + SOLVE_WARPS - 1) / SOLVE_WARPS);
@@ -862,7 +1036,9 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cu
     cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
     const double* crec = rec;
     const double* cvd = vdmap;
-    if (with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, true>, dc, a, crec, cvd));
+    if (pa && with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_params_kernel<KIND, true>, dc, p, a, crec, cvd));
+    else if (pa) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_params_kernel<KIND, false>, dc, p, a, crec, cvd));
+    else if (with_vd) WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, true>, dc, a, crec, cvd));
     else WBC_CUDA(h, cudaLaunchKernelEx(&cfg, wbc_solve_kernel<KIND, false>, dc, a, crec, cvd));
     if (is.profile) cudaEventRecord(h->prof_ev[2], st);
     h->launches += 2;
@@ -871,14 +1047,15 @@ static int launch_split(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cu
 }
 
 // One control step = reduce kernel (per controller kind) + solve kernel, stream ordered; `slot` selects the hand-over scratch
-// (the host pipelines run two streams side by side).
-static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is) {
+// (the host pipelines run two streams side by side); pa: per-robot parameters (nullptr: the handle's).
+static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cudaStream_t st, int slot, Issue is,
+                       const wbc::ParamArgs* pa = nullptr) {
   int rc = WBC_OK;
   switch (kind) {
-    case WBC_CTRL_ID: rc = launch_split<WBC_CTRL_ID>(h, kind, n, io, st, slot, is); break;
-    case WBC_CTRL_CLF: rc = launch_split<WBC_CTRL_CLF>(h, kind, n, io, st, slot, is); break;
+    case WBC_CTRL_ID: rc = launch_split<WBC_CTRL_ID>(h, kind, n, io, st, slot, is, pa); break;
+    case WBC_CTRL_CLF: rc = launch_split<WBC_CTRL_CLF>(h, kind, n, io, st, slot, is, pa); break;
     case WBC_CTRL_PC:
-    case WBC_CTRL_MPTC: rc = launch_split<WBC_CTRL_PC>(h, kind, n, io, st, slot, is); break;   // MPTC: a.kind drops the passivity row
+    case WBC_CTRL_MPTC: rc = launch_split<WBC_CTRL_PC>(h, kind, n, io, st, slot, is, pa); break;   // MPTC: a.kind drops the passivity row
     default: return fail_arg(h, "wbc_step: unknown controller kind");
   }
   if (rc) return rc;
@@ -886,24 +1063,40 @@ static int step_launch(wbc_handle* h, int kind, int64_t n, const wbc_io& io, cud
   return WBC_OK;
 }
 
-// wbc_step on device buffers; `profile` (wbc_profile_step) issues one chain with events around its two kernels.
-static int device_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cudaStream_t st, bool profile) {
+// The PD law on device rows; with pa, each robot's gains (and its status word when io.status is given).
+static int pd_launch(wbc_handle* h, int64_t n, const wbc_io& io, const wbc::ParamArgs* pa, cudaStream_t st) {
+  if (!pa) return wbc_step_pd(h, n, io.q, io.v, io.tau, st);
+  if (n < 0 || (n > 0 && (!io.q || !io.v || !io.tau))) return fail_arg(h, "wbc_step_params: q, v and tau are required");
+  if (n == 0) return WBC_OK;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  const long long total = (long long)n * WBC_NU;
+  wbc_pd_params_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(h->d_const.p, *pa, io.q, io.v, io.tau, io.status, n);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// wbc_step on device buffers; `profile` (wbc_profile_step) issues one chain with events around its two kernels; pa:
+// per-robot parameters (wbc_step_params), nullptr for the handle's.
+static int device_step(wbc_handle* h, int kind, int64_t n, const wbc_io* io, cudaStream_t st, bool profile,
+                       const wbc::ParamArgs* pa = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!io || n < 0) return fail_arg(h, "wbc_step: bad arguments");
   if (n == 0) return WBC_OK;
-  if (kind == WBC_CTRL_PD) return wbc_step_pd(h, n, io->q, io->v, io->tau, st);
+  if (kind == WBC_CTRL_PD) return pd_launch(h, n, *io, pa, st);
   if (!io->q || !io->v || !io->traj || !io->contact || !io->tau || !io->metrics || !io->status)
     return fail_arg(h, "wbc_step: q, v, traj, contact, tau, metrics and status are required");
   WBC_CUDA(h, cudaSetDevice(h->device));
   if (profile || n < CHUNKED_STEP_MIN || n > CHUNKED_STEP_MAX || capturing(st))
-    return step_launch(h, kind, n, *io, st, 0, Issue{false, false, profile});
+    return step_launch(h, kind, n, *io, st, 0, Issue{false, false, profile}, pa);
   const int k = device_step_chunks(n);
   cudaStream_t lanes[WBC_NSLOT] = {st};
   for (int c = 1; c < k; ++c) lanes[c] = h->lane[c];
   const int rc = streams_wait(h, h->order_ev, st, lanes + 1, k - 1);
   if (rc) return rc;
   return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
-    int r = step_launch(h, kind, m, io_at(*io, o), lanes[c], c, Issue{false, true});
+    const wbc::ParamArgs p = pa ? params_at(*pa, o) : wbc::ParamArgs{};
+    int r = step_launch(h, kind, m, io_at(*io, o), lanes[c], c, Issue{false, true}, pa ? &p : nullptr);
     if (!r && c) r = streams_wait(h, h->join_ev, lanes[c], &st, 1);
     return r;
   });
@@ -934,7 +1127,9 @@ static int step_host_wait(wbc_handle* h) {
   return WBC_OK;
 }
 
-static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* io) {
+// pa: per-robot parameters whose index array is a host array (wbc_step_params_host), nullptr for the handle's. The index is one
+// more input: read by the kernels with the others (zero-copy) or copied with them.
+static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* io, const wbc::ParamArgs* pa = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!io || n < 0) return fail_arg(h, "wbc_step_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -947,7 +1142,8 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
   // its 732 B of inputs and writes its 132 B of outputs per instance straight over the host link - one launch, no
   // staging copies, the transfers of one warp overlap the arithmetic of the others.
   wbc_io hio = *io;
-  if (to_device_aliases(hio.q, hio.v, hio.traj, hio.contact, hio.tau, hio.metrics, hio.status, hio.vd, hio.f, hio.qp_info, hio.lam)) {
+  const int32_t* hidx = pa ? pa->index : nullptr;    // the index array as the kernels read it
+  if (to_device_aliases(hio.q, hio.v, hio.traj, hio.contact, hio.tau, hio.metrics, hio.status, hio.vd, hio.f, hio.qp_info, hio.lam, hidx)) {
     // The batch goes through in chunks alternating between the two internal streams (each with its own hand-over scratch); the
     // outputs are written straight to host memory by the solve kernel in every mode. PD takes the chunk count of the staged
     // mode but reads its inputs over the link at every size.
@@ -956,17 +1152,24 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
     if (staged) {
       WBC_CUDA(h, h->stage.reserve(n));
       hio.q = sg.q.p; hio.v = sg.v.p; hio.traj = sg.traj.p; hio.contact = sg.contact.p;
+      if (hidx) {
+        WBC_CUDA(h, h->stage.index.reserve(n));
+        hidx = sg.index.p;
+      }
     }
+    const wbc::ParamArgs dpa = pa ? wbc::ParamArgs{pa->set, hidx, pa->n_sets} : wbc::ParamArgs{};
     return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
       const cudaStream_t st = h->lane[c & 1];
       const wbc_io s = io_at(*io, o), d = io_at(hio, o);
+      const wbc::ParamArgs sp = pa ? params_at(*pa, o) : wbc::ParamArgs{}, dp = pa ? params_at(dpa, o) : wbc::ParamArgs{};
       if (staged) {
         WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
         WBC_CUDA(h, cudaMemcpyAsync((void*)d.v, s.v, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
         WBC_CUDA(h, cudaMemcpyAsync((void*)d.traj, s.traj, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, st));
         WBC_CUDA(h, cudaMemcpyAsync((void*)d.contact, s.contact, m * 4, cudaMemcpyHostToDevice, st));
+        if (dp.index) WBC_CUDA(h, cudaMemcpyAsync((void*)dp.index, sp.index, m * sizeof(int32_t), cudaMemcpyHostToDevice, st));
       }
-      return pd ? wbc_step_pd(h, m, d.q, d.v, d.tau, st) : step_launch(h, kind, m, d, st, c & 1, Issue{!staged, k > 1});
+      return pd ? pd_launch(h, m, d, pa ? &dp : nullptr, st) : step_launch(h, kind, m, d, st, c & 1, Issue{!staged, k > 1}, pa ? &dp : nullptr);
     });
   }
   WBC_CUDA(h, h->stage.reserve(n));
@@ -974,17 +1177,24 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
   const wbc_io dev{sg.q.p, sg.v.p, sg.traj.p, sg.contact.p, sg.tau.p, sg.metrics.p, sg.status.p, io->vd ? sg.vd.p : nullptr,
                    io->f ? sg.f.p : nullptr, io->qp_info ? sg.info.p : nullptr, io->lam ? sg.lam.p : nullptr};
   const int k = pageable_chunks(n);
+  if (pa && pa->index) WBC_CUDA(h, h->stage.index.reserve(n));
+  const wbc::ParamArgs dpa = pa ? wbc::ParamArgs{pa->set, pa->index ? sg.index.p : nullptr, pa->n_sets} : wbc::ParamArgs{};
   return for_each_chunk(n, k, [&](int c, int64_t o, int64_t m) {
     const cudaStream_t st = h->lane[c & 1];
     const wbc_io s = io_at(*io, o), d = io_at(dev, o);
+    const wbc::ParamArgs sp = pa ? params_at(*pa, o) : wbc::ParamArgs{}, dp = pa ? params_at(dpa, o) : wbc::ParamArgs{};
     WBC_CUDA(h, cudaMemcpyAsync((void*)d.q, s.q, m * WBC_NQ * sizeof(double), cudaMemcpyHostToDevice, st));
     WBC_CUDA(h, cudaMemcpyAsync((void*)d.v, s.v, m * WBC_NV * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (dp.index) WBC_CUDA(h, cudaMemcpyAsync((void*)dp.index, sp.index, m * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     if (!pd) {
       WBC_CUDA(h, cudaMemcpyAsync((void*)d.traj, s.traj, m * WBC_NTRAJ * sizeof(double), cudaMemcpyHostToDevice, st));
       WBC_CUDA(h, cudaMemcpyAsync((void*)d.contact, s.contact, m * 4, cudaMemcpyHostToDevice, st));
     }
-    const int r = pd ? wbc_step_pd(h, m, d.q, d.v, d.tau, st) : step_launch(h, kind, m, d, st, c & 1, Issue{false, k > 1});
+    // (the PD law with parameters writes status only where the caller asked for it)
+    const wbc_io dpd = pa && !s.status ? wbc_io{d.q, d.v, nullptr, nullptr, d.tau} : d;
+    const int r = pd ? pd_launch(h, m, dpd, pa ? &dp : nullptr, st) : step_launch(h, kind, m, d, st, c & 1, Issue{false, k > 1}, pa ? &dp : nullptr);
     if (r) return r;
+    if (pd && pa && s.status) WBC_CUDA(h, cudaMemcpyAsync(s.status, d.status, m * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     WBC_CUDA(h, cudaMemcpyAsync(s.tau, d.tau, m * WBC_NU * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (!pd) {
       WBC_CUDA(h, cudaMemcpyAsync(s.metrics, d.metrics, m * WBC_NMETRIC * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1001,6 +1211,90 @@ static int step_host_enqueue(wbc_handle* h, int kind, int64_t n, const wbc_io* i
 extern "C" int wbc_step_host(wbc_handle* h, int kind, int64_t n, const wbc_io* io) {
   const int rc = step_host_enqueue(h, kind, n, io);
   if (rc || !h || n <= 0) return rc;
+  return step_host_wait(h);
+}
+
+// ------------------------------------------------------------------------------ per-robot controller parameters
+// A set keeps the number of the device its records live on, not its handle: it may be destroyed after the handle.
+struct wbc_param_set {
+  int device = 0;
+  int32_t n_sets = 0;
+  DevArray<wbc::ParamRec> table;
+  ~wbc_param_set() { cudaSetDevice(device); }   // the table is freed after this, on the set's device
+};
+
+extern "C" int wbc_param_set_destroy(wbc_param_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+static bool finite_all(const double* x, size_t n) {
+  for (size_t i = 0; i < n; ++i)
+    if (!std::isfinite(x[i])) return false;
+  return true;
+}
+
+// Why a parameter set cannot be used, or nullptr: the checks of wbc_create, and what derive_constants and the step assume.
+static const char* params_problem(const wbc_params& p) {
+  static_assert(offsetof(wbc_params, torque_limits) % sizeof(double) == 0 && offsetof(wbc_params, pd_kp) % sizeof(double) == 0,
+                "the doubles of wbc_params surround its two integers");
+  const double* d = reinterpret_cast<const double*>(&p);
+  if (!finite_all(d, offsetof(wbc_params, torque_limits) / sizeof(double)) || !finite_all(&p.pd_kp, 3 + WBC_NU))
+    return "wbc_param_set_create: non-finite parameter";
+  if (p.reg_vd != 0.0) return "wbc_param_set_create: reg_vd is not supported yet (must be 0)";
+  if (!(p.reg_f > 0.0)) return "wbc_param_set_create: reg_f must be > 0 (tie-break that makes the QP strictly convex)";
+  if (p.max_iter < 1) return "wbc_param_set_create: max_iter must be >= 1";
+  if (p.torque_limits != 0 && p.torque_limits != 1) return "wbc_param_set_create: torque_limits must be 0 or 1";
+  if (!(p.mu >= 0.0)) return "wbc_param_set_create: mu must be >= 0";
+  if (!(p.clf_r > 0.0)) return "wbc_param_set_create: clf_r must be > 0";
+  const double clf_w[] = {p.clf_q_body_p, p.clf_q_body_pd, p.clf_q_body_rpy, p.clf_q_body_rpyd, p.clf_q_foot_p, p.clf_q_foot_pd, p.clf_w_delta};
+  for (double w : clf_w)
+    if (!(w >= 0.0)) return "wbc_param_set_create: the CLF weights clf_q_* and clf_w_delta must be >= 0";
+  return nullptr;
+}
+
+extern "C" int wbc_param_set_create(wbc_handle* h, int32_t n_sets, const wbc_params* params, wbc_param_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !params || n_sets < 1) return fail_arg(h, "wbc_param_set_create: params and n_sets >= 1 are required");
+  *out = nullptr;
+  std::vector<wbc::ParamRec> rec((size_t)n_sets);
+  for (int32_t k = 0; k < n_sets; ++k) {
+    if (const char* why = params_problem(params[k])) return fail_arg(h, why);
+    rec[k].pr = params[k];
+    wbc::derive_constants(params[k], rec[k].dv);
+  }
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_param_set> ps(new (std::nothrow) wbc_param_set());
+  if (!ps) return WBC_ERR_NOMEM;
+  ps->device = h->device;
+  ps->n_sets = n_sets;
+  WBC_CUDA(h, ps->table.reserve(rec.size()));
+  WBC_CUDA(h, cudaMemcpy(ps->table.p, rec.data(), rec.size() * sizeof(rec[0]), cudaMemcpyHostToDevice));
+  *out = ps.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of per-robot parameters with the index array `index` (as the kernels read it).
+static int ctrl_args(wbc_handle* h, const wbc_ctrl_params* p, const int32_t* index, wbc::ParamArgs* pa) {
+  const wbc_param_set* set = p ? p->set : nullptr;
+  if (set && set->device != h->device) return fail_arg(h, "wbc_ctrl_params: the set lives on another device than the handle");
+  *pa = wbc::ParamArgs{set ? set->table.p : h->d_params.p, index, set ? set->n_sets : 1};
+  return WBC_OK;
+}
+
+extern "C" int wbc_step_params(wbc_handle* h, int kind, int64_t n, const wbc_io* io, const wbc_ctrl_params* p, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  wbc::ParamArgs pa;
+  const int rc = ctrl_args(h, p, p ? p->index : nullptr, &pa);
+  return rc ? rc : device_step(h, kind, n, io, (cudaStream_t)stream, false, &pa);
+}
+
+extern "C" int wbc_step_params_host(wbc_handle* h, int kind, int64_t n, const wbc_io* io, const wbc_ctrl_params* p) {
+  if (!h) return WBC_ERR_ARG;
+  wbc::ParamArgs pa;
+  int rc = ctrl_args(h, p, p ? p->index : nullptr, &pa);
+  if (!rc) rc = step_host_enqueue(h, kind, n, io, &pa);
+  if (rc || n <= 0) return rc;
   return step_host_wait(h);
 }
 
@@ -1495,12 +1789,6 @@ extern "C" int wbc_plant_set_destroy(wbc_plant_set* s) {
   return WBC_OK;
 }
 
-static bool finite_all(const double* x, size_t n) {
-  for (size_t i = 0; i < n; ++i)
-    if (!std::isfinite(x[i])) return false;
-  return true;
-}
-
 extern "C" int wbc_plant_set_create(wbc_handle* h, int32_t n_variants, const wbc_model* models, const double* mu, wbc_plant_set** out) {
   if (!h) return WBC_ERR_ARG;
   if (!out || !models || n_variants <= 0) return fail_arg(h, "wbc_plant_set_create: models and n_variants > 0 are required");
@@ -1648,8 +1936,8 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
   return WBC_OK;
 }
 
-// Which plant a host entry runs.
-enum class PlantEntry { plain, perturbed, terrain };
+// Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant).
+enum class PlantEntry { plain, perturbed, terrain, params };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -1697,10 +1985,12 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
                          "wbc_plant_step_terrain_host: n >= 0 and dt > 0 are required");
 }
 
-// The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed and wbc_rollout_terrain; pa != nullptr: the plant step runs the
-// variant kernel, or with ta != nullptr the terrain kernel.
+// The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed, wbc_rollout_terrain and wbc_rollout_params; pa != nullptr: the
+// plant step runs the variant kernel, or with ta != nullptr the terrain kernel; cp != nullptr: the controller step runs with
+// these per-robot parameters.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
-                       const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st) {
+                       const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
+                       const wbc::ParamArgs* cp = nullptr) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -1724,7 +2014,7 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
   auto one_step = [&]() -> int {
     int r = wbc_sample_trajectory(h, plan, n, io->plan_index, io->t, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
     if (r) return r;
-    r = wbc_step(h, kind, n, &sio, st);
+    r = device_step(h, kind, n, &sio, st, false, cp);
     if (r) return r;
     if (plant) {
       r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
@@ -1804,9 +2094,27 @@ extern "C" int wbc_rollout(wbc_handle* h, int kind, const wbc_plan* plan, int64_
   return wbc_rollout_ex(h, kind, plan, n, n_steps, dt, io, &o, stream);
 }
 
-// Host buffers of the three rollouts.
+extern "C" int wbc_rollout_params(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                  const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                  const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_params: bad arguments");
+  const bool ground = perturb || terrain;
+  if (ground && !(opts && opts->plant != 0))
+    return fail_arg(h, "wbc_rollout_params: perturbations and terrain act on the ground plant (opts->plant = 1)");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  int rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && ground) rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, ground ? &pa : nullptr, terrain ? &ta : nullptr, (cudaStream_t)stream, &cp);
+}
+
+// Host buffers of the four rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
-                        const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain) {
+                        const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
+                        const wbc_ctrl_params* ctrl = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -1826,9 +2134,13 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (perturb) dp = wbc_plant_perturb{perturb->set, s.in(perturb->variant, N), s.in(perturb->push, N * 8)};
   wbc_plant_terrain dtr{};
   if (terrain) dtr = wbc_plant_terrain{terrain->set, s.in(terrain->index, N)};
+  wbc_ctrl_params dcp{};
+  if (ctrl) dcp = wbc_ctrl_params{ctrl->set, s.in(ctrl->index, N)};
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::terrain ? wbc_rollout_terrain(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+      entry == PlantEntry::params ? wbc_rollout_params(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+                                                       terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, s.st)
+      : entry == PlantEntry::terrain ? wbc_rollout_terrain(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                          terrain ? &dtr : nullptr, s.st)
       : entry == PlantEntry::perturbed ? wbc_rollout_perturbed(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, s.st)
                                        : wbc_rollout_ex(h, kind, plan, n, n_steps, dt, &d, &o, s.st);
@@ -1849,6 +2161,12 @@ extern "C" int wbc_rollout_terrain_host(wbc_handle* h, int kind, const wbc_plan*
                                         const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
                                         const wbc_plant_terrain* terrain) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::terrain, perturb, terrain);
+}
+
+extern "C" int wbc_rollout_params_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                       const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                       const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::params, perturb, terrain, ctrl);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

@@ -1744,4 +1744,37 @@ WBC_DEV void pd_element(const wbc_model& md, const wbc_params& pr, const double*
   tau[inst * WBC_NU + md.act_index[k]] = u;
 }
 
+// ---------------------------------------------------------------- per-robot controller parameters (wbc_step_params)
+// One parameter set: the gains and weights with the constants derived from them on the host (derive_constants), one 16-byte
+// aligned record so that a reduce CTA stages it with the vector loop of the model constants.
+struct alignas(16) ParamRec {
+  wbc_params pr;
+  Derived dv;
+};
+
+// Device inputs of the parameter-aware kernels: K records and the set of each robot (index [N], NULL: set 0).
+struct ParamArgs {
+  const ParamRec* set; const int32_t* index; int n_sets;
+};
+
+// The record robot `inst` is controlled with. An index outside [0, n_sets) sets WBC_ST_BADPARAMS in `status` (the robot's
+// outputs are then zeroed like those of any other failure) and returns record 0, so that every read stays in bounds.
+WBC_DEV const ParamRec& param_record(const ParamArgs& p, long long inst, int& status) {
+  const int k = p.index ? p.index[inst] : 0;
+  const bool bad = !(k >= 0 && k < p.n_sets);
+  if (bad) status |= WBC_ST_BADPARAMS;
+  return p.set[bad ? 0 : k];
+}
+
+// pd_element with the robot's own gains. A bad set index gives tau = 0; thread k = 0 of the robot writes its status word
+// (WBC_ST_BADPARAMS or 0) when `status` is given.
+WBC_DEV void pd_params_element(const wbc_model& md, const ParamArgs& p, const double* q, const double* v, double* tau, int32_t* status,
+                               long long inst, int k) {
+  int st = 0;
+  const ParamRec& r = param_record(p, inst, st);
+  if (st) tau[inst * WBC_NU + md.act_index[k]] = 0.0;
+  else pd_element(md, r.pr, q, v, tau, inst, k);
+  if (status && k == 0) status[inst] = st;
+}
+
 }  // namespace wbc

@@ -15,6 +15,9 @@ a time window, while the controller keeps the handle's nominal model. They run t
 Uneven ground (`terrain_set`, `terrain`; ground plant only): each robot stands on its own terrain - a plane plus an optional
 height field (`Terrain`, defined in include/wbc.h) - while the controller keeps assuming flat ground. It runs through
 `wbc_rollout_terrain` / `wbc_plant_step_terrain`, together with any variants and pushes.
+
+Per-robot controller parameters (`param_set`, `param_index`; either plant): robot i is controlled with its own gains and weights
+(controller.ParamSet). It runs through `wbc_rollout_params`, together with any variants, pushes and terrain.
 """
 from __future__ import annotations
 
@@ -23,8 +26,9 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .capi import (KINDS, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc,
+from .capi import (KINDS, WbcCtrlParams, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc,
                    np_ptr)
+from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
 Q0_MINI_CHEETAH = np.array([1.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.3] + [0.0, -0.8, 1.6] * 4)     # simulate.py:171-176
@@ -132,7 +136,8 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
-            mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None) -> RolloutResult:
+            mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
+            param_index=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -141,9 +146,12 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     push [N,8] = force (world) | point (base frame) | t_on | t_off (None: no pushes); torch tensors on the device with torch
     inputs, arrays otherwise. A robot with an out-of-range variant index is frozen and flagged ST_BADVARIANT.
     Uneven ground (plant=True only): terrain_set (TerrainSet or None: flat ground), terrain [N] int32 (None: terrain 0); an
-    out-of-range terrain index freezes that robot, flagged ST_BADTERRAIN."""
+    out-of-range terrain index freezes that robot, flagged ST_BADTERRAIN.
+    Per-robot controller parameters (either plant): param_set (controller.ParamSet or None: the handle's params), param_index
+    [N] int32 (None: set 0); a robot with an out-of-range index gets zero torques, flagged ST_BADPARAMS."""
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
+    per_robot = param_set is not None or param_index is not None
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
     if _is_torch(q):
         import torch
@@ -155,7 +163,14 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if on_terrain:
+        if per_robot:
+            pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
+            tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
+            check_device_index(param_index, n)
+            cp = WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))
+            ctl._check(ctl.lib.wbc_rollout_params(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                  C.byref(cp), stream), "wbc_rollout_params")
+        elif on_terrain:
             pt, tr = _perturb(plant_set, variant, push, p), _terrain(terrain_set, terrain, p)
             ctl._check(ctl.lib.wbc_rollout_terrain(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
                                                    C.byref(tr), stream), "wbc_rollout_terrain")
@@ -177,7 +192,15 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if on_terrain:
+    if per_robot:
+        vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
+        ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
+        pt = C.byref(_perturb(plant_set, vi, pu, opt)) if perturbed else None
+        tr = C.byref(_terrain(terrain_set, ti, opt)) if on_terrain else None
+        cp = WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))
+        ctl._check(ctl.lib.wbc_rollout_params_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                   C.byref(cp)), "wbc_rollout_params_host")
+    elif on_terrain:
         pt, tr = _perturb(plant_set, *_perturb_arrays(n, variant, push), opt), _terrain(terrain_set, _terrain_index(n, terrain), opt)
         ctl._check(ctl.lib.wbc_rollout_terrain_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), C.byref(pt),
                                                     C.byref(tr)), "wbc_rollout_terrain_host")
