@@ -71,6 +71,7 @@ extern "C" {
 #define WBC_ST_BADVARIANT 512  /* perturbed plant only: variant index out of range; the robot is frozen, zero ground forces */
 #define WBC_ST_BADTERRAIN 1024 /* terrain plant only: terrain index out of range; the robot is frozen, zero ground forces */
 #define WBC_ST_BADPARAMS 2048  /* wbc_step_params only: parameter-set index out of range; zero outputs                  */
+#define WBC_ST_BADLOOP 4096    /* wbc_rollout_loop only: bad loop profile; observed without noise, zero applied torque  */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -498,6 +499,62 @@ int wbc_rollout_params(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
 int wbc_rollout_params_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
                             const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
                             const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl);
+
+/* ---- Imperfect sensing and actuation in the ground-plant loop: each robot's controller reads a noisy state, and its torque
+ * command reaches a motor of its own strength one or more control steps late.
+ *
+ * Loop profile of robot i: noise[i][6] = standard deviations of the base orientation (rad), base position (m), joint angles
+ * (rad), base angular velocity (rad/s), base linear velocity (m/s) and joint velocities (rad/s); delay[i] in [0, 15] control
+ * steps; strength[i] >= 0, a factor on the applied torque; stream[i], a noise stream id (int32 read as uint32). Loop state of
+ * robot i: hist[i][16][12], a ring of the last 16 commanded torques, and tick[i], the number of commands issued so far.
+ *
+ * Noise. Draw j in [0, 18) of step c = tick[i] is Philox4x32-10 (the function of cuRAND's curand_Philox4x32_10, multipliers
+ * 0xD2511F53, 0xCD9E8D57, key increments 0x9E3779B9, 0xBB67AE85) of the counter (j, stream, c_lo, c_hi) under the key
+ * (seed_lo, seed_hi); its words w0..w3 give u_a = (((w1 << 32) | w0) >> 11) 2^-53 + 2^-54 and u_b the same of (w3, w2), both
+ * in (0, 1), and the normals z[2j] = sqrt(-2 ln u_a) cospi(2 u_b), z[2j+1] = sqrt(-2 ln u_a) sinpi(2 u_b). z[0:3] perturb
+ * the orientation, z[3:6] the base position, z[6:18] the joint angles (q order), z[18:21] the angular velocity, z[21:24] the
+ * linear velocity and z[24:36] the joint velocities. A robot's noise depends on (seed, stream, tick) only: not on its row, the
+ * batch size or graph capture.
+ *
+ * Observe (tick unchanged): delta = sigma_rot z[0:3], theta = |delta|, dq = [cos theta/2, sin theta/2 delta / theta] (identity
+ * for theta = 0), observed quaternion normalize(dq (x) q) (a world-frame perturbation, [w x y z]); every other block is
+ * value + sigma z. A block with sigma = 0 is copied, so a zero-noise profile observes the true state bit for bit. Time and the
+ * plan are not perturbed. The controller runs on the observed state (its metrics are what it observed).
+ *
+ * Actuate (after the controller, c = tick[i], d = delay[i]): hist[i][c mod 16] = tau_c; the applied torque is
+ * strength[i] * hist[i][max(c - d, 0) mod 16] (until d commands exist the first one is held); tick[i] = c + 1. With d = 0 and
+ * strength 1 the applied torque is the command bit for bit. The plant applies it to the true state; the controller's status of
+ * step c still decides the plant's freeze in step c; io->tau keeps the last COMMANDED torque.
+ *
+ * Bad profile: a delay outside [0, 15], a sigma or strength that is negative or not finite, or tick < 0. Such a robot is
+ * observed without noise, gets applied torque 0 and WBC_ST_BADLOOP in its controller status of the step (kept by status_or);
+ * its hist and tick are unchanged. The ground plant does not freeze it: it goes limp, as a WBC_ST_BADPARAMS robot does. */
+#define WBC_LOOP_HIST 16
+typedef struct wbc_loop {
+  const double* noise;      /* [N][6] or NULL: no noise                                                                   */
+  const int32_t* delay;     /* [N] or NULL: no delay                                                                      */
+  const double* strength;   /* [N] or NULL: strength 1                                                                    */
+  const int32_t* stream;    /* [N] or NULL: the row index                                                                 */
+  uint64_t seed;
+  double* hist;             /* [N][16][12] and tick [N]: both given (in/out) or both NULL (library scratch from tick 0,   */
+  int64_t* tick;            /* so each call starts a fresh history); only one of them is WBC_ERR_ARG                      */
+} wbc_loop;
+
+/* wbc_rollout_params (opts->plant must be 1) with sample plan -> observe -> controller -> actuate -> ground plant in every
+ * step: two more launches per step, captured into the same graph. loop == NULL gives the bits and the launch count of
+ * wbc_rollout_params. Device pointers (host pointers for _host; hist and tick are copied in and out). */
+int wbc_rollout_loop(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                     const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                     const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop, void* stream);
+int wbc_rollout_loop_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                          const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                          const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop);
+/* The observe kernel alone: q_obs [N][19], v_obs [N][18] as the controller of step tick[i] sees them (tick is read, not
+ * advanced; hist is not used). loop == NULL observes without noise. */
+int wbc_loop_observe(wbc_handle* h, int64_t n, const wbc_loop* loop, const double* q, const double* v, double* q_obs, double* v_obs,
+                     void* stream);
+int wbc_loop_observe_host(wbc_handle* h, int64_t n, const wbc_loop* loop, const double* q, const double* v, double* q_obs,
+                          double* v_obs);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

@@ -24,11 +24,13 @@ ST_NONFINITE = 256
 ST_BADVARIANT = 512
 ST_BADTERRAIN = 1024
 ST_BADPARAMS = 2048
+ST_BADLOOP = 4096
+LOOP_HIST = 16
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
              ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN",
-             ST_BADPARAMS: "BADPARAMS"}
+             ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP"}
 
 
 def status_names(status: int) -> str:
@@ -119,6 +121,12 @@ class WbcPlantTerrain(C.Structure):
 class WbcCtrlParams(C.Structure):
     """ctypes mirror of `wbc_ctrl_params` (parameter set, per-robot set index)."""
     _fields_ = [("set", C.c_void_p), ("index", C.c_void_p)]
+
+
+class WbcLoop(C.Structure):
+    """ctypes mirror of `wbc_loop` (per-robot noise, delay, strength and stream; the seed; the loop state hist / tick)."""
+    _fields_ = [("noise", C.c_void_p), ("delay", C.c_void_p), ("strength", C.c_void_p), ("stream", C.c_void_p), ("seed", C.c_uint64),
+                ("hist", C.c_void_p), ("tick", C.c_void_p)]
 
 
 def np_ptr(a: np.ndarray):
@@ -218,7 +226,13 @@ def load_library() -> C.CDLL:
                                        C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), dp]
     lib.wbc_rollout_params_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
                                             C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams)]
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS:
+    lib.wbc_rollout_loop.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                     C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), C.POINTER(WbcLoop), dp]
+    lib.wbc_rollout_loop_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                          C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), C.POINTER(WbcLoop)]
+    lib.wbc_loop_observe.argtypes = [H, i64, C.POINTER(WbcLoop), dp, dp, dp, dp, dp]
+    lib.wbc_loop_observe_host.argtypes = [H, i64, C.POINTER(WbcLoop), dp, dp, dp, dp]
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -251,7 +265,8 @@ TERRAIN_SYMBOLS = ["wbc_terrain_set_create", "wbc_terrain_set_destroy", "wbc_pla
                    "wbc_rollout_terrain", "wbc_rollout_terrain_host"]
 PARAM_SYMBOLS = ["wbc_param_set_create", "wbc_param_set_destroy", "wbc_step_params", "wbc_step_params_host", "wbc_rollout_params",
                  "wbc_rollout_params_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+LOOP_SYMBOLS = ["wbc_rollout_loop", "wbc_rollout_loop_host", "wbc_loop_observe", "wbc_loop_observe_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

@@ -26,6 +26,7 @@
 #include "wbc_traj.cuh"
 #include "wbc_rollout.cuh"
 #include "wbc_plant.cuh"
+#include "wbc_loop.cuh"
 #include <vector>
 
 namespace {
@@ -620,6 +621,21 @@ struct RolloutScratch {
   }
 };
 
+// Scratch of the loop entries (wbc_rollout_loop, wbc_loop_observe), reserved by them only: the observed state, the applied
+// torque and the loop state of a call that brings none.
+struct LoopScratch {
+  DevArray<double> q_obs, v_obs, applied, hist;
+  DevArray<long long> tick;
+  cudaError_t reserve(int64_t n, bool own_state) {
+    cudaError_t e = q_obs.reserve(n * WBC_NQ);
+    if (e == cudaSuccess) e = v_obs.reserve(n * WBC_NV);
+    if (e == cudaSuccess) e = applied.reserve(n * WBC_NU);
+    if (e == cudaSuccess && own_state) e = hist.reserve(n * WBC_LOOP_HIST * WBC_NU);
+    if (e == cudaSuccess && own_state) e = tick.reserve(n);
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
@@ -642,6 +658,7 @@ struct wbc_handle {
   Event prof_ev[3];                    // wbc_profile_step: before reduce / between / after solve
   Staging stage;
   RolloutScratch ro;
+  LoopScratch loop;
   ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
@@ -1936,8 +1953,9 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
   return WBC_OK;
 }
 
-// Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant).
-enum class PlantEntry { plain, perturbed, terrain, params };
+// Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant; loop: the same with
+// sensing and actuation, on the ground plant).
+enum class PlantEntry { plain, perturbed, terrain, params, loop };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -1985,12 +2003,13 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
                          "wbc_plant_step_terrain_host: n >= 0 and dt > 0 are required");
 }
 
-// The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed, wbc_rollout_terrain and wbc_rollout_params; pa != nullptr: the
-// plant step runs the variant kernel, or with ta != nullptr the terrain kernel; cp != nullptr: the controller step runs with
-// these per-robot parameters.
+// The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed, wbc_rollout_terrain, wbc_rollout_params and wbc_rollout_loop;
+// pa != nullptr: the plant step runs the variant kernel, or with ta != nullptr the terrain kernel; cp != nullptr: the controller
+// step runs with these per-robot parameters; lp != nullptr (ground plant): the controller reads the observed state and the plant
+// applies the actuated torque (wbc_loop.cuh), with the loop state in the handle's scratch when lp->hist is null.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                        const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
-                       const wbc::ParamArgs* cp = nullptr) {
+                       const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -2002,6 +2021,17 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
   const RolloutScratch& ro = h->ro;
   double* tau = io->tau ? io->tau : ro.tau.p;
   double* metrics = io->metrics ? io->metrics : ro.metrics.p;
+  wbcloop::LoopArgs la{};
+  if (lp) {
+    la = *lp;
+    WBC_CUDA(h, h->loop.reserve(n, !la.hist));
+    if (!la.hist) {                                // a fresh history: tick 0 (no slot of hist is read before it is written)
+      la.hist = h->loop.hist.p;
+      la.tick = h->loop.tick.p;
+      WBC_CUDA(h, cudaMemsetAsync(la.tick, 0, n * sizeof(long long), st));
+    }
+  }
+  const unsigned loop_grid = (unsigned)((n + 255) / 256);
   WBC_CUDA(h, cudaMemsetAsync(ro.counter.p, 0, sizeof(int), st));
   if (io->status_or) WBC_CUDA(h, cudaMemsetAsync(io->status_or, 0, n * sizeof(int32_t), st));
   if (io->err_max) WBC_CUDA(h, cudaMemsetAsync(io->err_max, 0, n * sizeof(double), st));
@@ -2010,14 +2040,25 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
     WBC_CUDA(h, cudaMemsetAsync(metrics, 0, n * WBC_NMETRIC * sizeof(double), st));
   }
   // with the ground plant the controller's accelerations are not needed: the step runs without the vd outputs
-  wbc_io sio{io->q, io->v, ro.traj.p, ro.contact.p, tau, metrics, ro.status.p, plant ? nullptr : ro.vd.p, nullptr, nullptr};
+  // with a loop the controller reads the observed state and the plant applies the actuated torque
+  wbc_io sio{lp ? h->loop.q_obs.p : io->q, lp ? h->loop.v_obs.p : io->v, ro.traj.p, ro.contact.p, tau, metrics, ro.status.p,
+             plant ? nullptr : ro.vd.p, nullptr, nullptr};
+  const double* applied = lp ? h->loop.applied.p : tau;
   auto one_step = [&]() -> int {
     int r = wbc_sample_trajectory(h, plan, n, io->plan_index, io->t, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
     if (r) return r;
+    if (lp) {
+      wbcloop::observe_kernel<<<loop_grid, 256, 0, st>>>(la, n, io->q, io->v, h->loop.q_obs.p, h->loop.v_obs.p);
+      h->launches++;
+    }
     r = device_step(h, kind, n, &sio, st, false, cp);
     if (r) return r;
+    if (lp) {
+      wbcloop::actuate_kernel<<<loop_grid, 256, 0, st>>>(la, n, tau, h->loop.applied.p, ro.status.p);
+      h->launches++;
+    }
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, tau, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
+      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, applied, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
     } else {
@@ -2111,10 +2152,77 @@ extern "C" int wbc_rollout_params(wbc_handle* h, int kind, const wbc_plan* plan,
   return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, ground ? &pa : nullptr, terrain ? &ta : nullptr, (cudaStream_t)stream, &cp);
 }
 
-// Host buffers of the four rollouts.
+// ------------------------------------------------------------------------------ sensing and actuation (wbc_loop.cuh)
+// The kernel arguments of a loop whose arrays are already on the device (hist / tick may both be null).
+static int loop_args(wbc_handle* h, const wbc_loop* l, wbcloop::LoopArgs* la) {
+  if (l && !l->hist != !l->tick) return fail_arg(h, "wbc_loop: hist and tick are given together or not at all");
+  *la = l ? wbcloop::LoopArgs{l->noise, l->delay, l->strength, l->stream, (unsigned long long)l->seed, l->hist, (long long*)l->tick}
+          : wbcloop::LoopArgs{};
+  return WBC_OK;
+}
+
+extern "C" int wbc_rollout_loop(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop, void* stream) {
+  if (!loop) return wbc_rollout_params(h, kind, plan, n, n_steps, dt, io, opts, perturb, terrain, ctrl, stream);
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_loop: bad arguments");
+  if (!(opts && opts->plant == 1))
+    return fail_arg(h, "wbc_rollout_loop: sensing and actuation close the loop around the ground plant (opts->plant = 1)");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  wbcloop::LoopArgs la;
+  int rc = loop_args(h, loop, &la);
+  if (!rc) rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && (perturb || terrain))
+    rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, (perturb || terrain) ? &pa : nullptr, terrain ? &ta : nullptr,
+                               (cudaStream_t)stream, &cp, &la);
+}
+
+extern "C" int wbc_loop_observe(wbc_handle* h, int64_t n, const wbc_loop* loop, const double* q, const double* v, double* q_obs,
+                                double* v_obs, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (n < 0 || (n > 0 && (!q || !v || !q_obs || !v_obs))) return fail_arg(h, "wbc_loop_observe: q, v, q_obs and v_obs are required");
+  wbcloop::LoopArgs la;
+  const int rc = loop_args(h, loop, &la);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  wbcloop::observe_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(la, n, q, v, q_obs, v_obs);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Device copies of a host wbc_loop's arrays; hist and tick are copied in and out.
+static wbc_loop loop_to_device(DevScratch& s, const wbc_loop& l, size_t N) {
+  return wbc_loop{s.in(l.noise, N * 6), s.in(l.delay, N), s.in(l.strength, N), s.in(l.stream, N), l.seed,
+                  s.inout(l.hist, N * WBC_LOOP_HIST * WBC_NU), s.inout(l.tick, N)};
+}
+
+extern "C" int wbc_loop_observe_host(wbc_handle* h, int64_t n, const wbc_loop* loop, const double* q, const double* v, double* q_obs,
+                                     double* v_obs) {
+  if (!h) return WBC_ERR_ARG;
+  if (n < 0 || (n > 0 && (!q || !v || !q_obs || !v_obs))) return fail_arg(h, "wbc_loop_observe_host: q, v, q_obs and v_obs are required");
+  if (n == 0) return WBC_OK;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  DevScratch s(h->lane[0]);
+  const size_t N = (size_t)n;
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV);
+  double* dqo = s.out(q_obs, N * WBC_NQ); double* dvo = s.out(v_obs, N * WBC_NV);
+  wbc_loop dl{};
+  if (loop) dl = loop_to_device(s, *loop, N);
+  WBC_SCRATCH_CHECK(h, s);
+  const int rc = wbc_loop_observe(h, n, loop ? &dl : nullptr, dq, dv, dqo, dvo, s.st);
+  return rc ? rc : s.finish(h);
+}
+
+// Host buffers of the five rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                         const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
-                        const wbc_ctrl_params* ctrl = nullptr) {
+                        const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -2136,9 +2244,13 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (terrain) dtr = wbc_plant_terrain{terrain->set, s.in(terrain->index, N)};
   wbc_ctrl_params dcp{};
   if (ctrl) dcp = wbc_ctrl_params{ctrl->set, s.in(ctrl->index, N)};
+  wbc_loop dl{};
+  if (loop) dl = loop_to_device(s, *loop, N);
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::params ? wbc_rollout_params(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+      entry == PlantEntry::loop ? wbc_rollout_loop(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+                                                   terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr, s.st)
+      : entry == PlantEntry::params ? wbc_rollout_params(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                        terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, s.st)
       : entry == PlantEntry::terrain ? wbc_rollout_terrain(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                          terrain ? &dtr : nullptr, s.st)
@@ -2167,6 +2279,12 @@ extern "C" int wbc_rollout_params_host(wbc_handle* h, int kind, const wbc_plan* 
                                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
                                        const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::params, perturb, terrain, ctrl);
+}
+
+extern "C" int wbc_rollout_loop_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                     const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                     const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::loop, perturb, terrain, ctrl, loop);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

@@ -18,6 +18,11 @@ height field (`Terrain`, defined in include/wbc.h) - while the controller keeps 
 
 Per-robot controller parameters (`param_set`, `param_index`; either plant): robot i is controlled with its own gains and weights
 (controller.ParamSet). It runs through `wbc_rollout_params`, together with any variants, pushes and terrain.
+
+Imperfect sensing and actuation (`loop`, a `Loop`; ground plant only): robot i's controller reads its state with Gaussian noise,
+and its torque command reaches the plant `delay` control steps late, scaled by its motor strength (semantics in include/wbc.h,
+wbc_loop). It runs through `wbc_rollout_loop`, together with any variants, pushes, terrain and parameter sets; `observe` runs the
+sensing alone.
 """
 from __future__ import annotations
 
@@ -26,8 +31,8 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .capi import (KINDS, WbcCtrlParams, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc,
-                   np_ptr)
+from .capi import (KINDS, LOOP_HIST, WbcCtrlParams, WbcLoop, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts,
+                   WbcTerrainDesc, np_ptr)
 from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
@@ -123,6 +128,110 @@ def _perturb_arrays(n, variant, push):
     return vi, pu
 
 
+class LoopState:
+    """The persistent loop state of N robots: hist [N,16,12] float64, the ring of the last 16 commanded torques, and tick [N]
+    int64, the number of commands issued so far; both zero. NumPy arrays, or torch tensors on the device of `like`. A rollout
+    given a state continues it and leaves it advanced."""
+
+    def __init__(self, n, like=None):
+        if like is not None and _is_torch(like):
+            import torch
+            self.hist = torch.zeros((n, LOOP_HIST, 12), dtype=torch.float64, device=like.device)
+            self.tick = torch.zeros(n, dtype=torch.int64, device=like.device)
+        else:
+            self.hist, self.tick = np.zeros((n, LOOP_HIST, 12)), np.zeros(n, np.int64)
+
+
+@dataclass
+class Loop:
+    """Per-robot sensing and actuation of the ground-plant loop (include/wbc.h, wbc_loop). noise: standard deviations of base
+    orientation (rad), base position (m), joint angles (rad), angular velocity (rad/s), linear velocity (m/s) and joint
+    velocities (rad/s), shape (6,) for every robot or (N, 6); delay [N] int32 control steps in [0, 15]; strength [N] >= 0;
+    stream [N] int32 noise stream ids (None: the row index); seed, 64 bits; state: a LoopState to continue (None: each call
+    starts a fresh history). None for noise / delay / strength means no noise / no delay / strength 1. With torch inputs, torch
+    values must be contiguous CUDA tensors of the ABI's dtype and shape; other values are broadcast and copied to the device."""
+    noise: object = None
+    delay: object = None
+    strength: object = None
+    stream: object = None
+    seed: int = 0
+    state: LoopState | None = None
+
+
+_LOOP_FIELDS = (("noise", np.float64, 6), ("delay", np.int32, None), ("strength", np.float64, None), ("stream", np.int32, None))
+
+
+def check_device_array(x, shape, dtype, what):
+    """A per-robot array on the device must be a contiguous CUDA tensor of the ABI's dtype and shape: the kernels read it through
+    its device pointer."""
+    import torch
+    dt = {np.float64: torch.float64, np.int32: torch.int32, np.int64: torch.int64}[dtype]
+    if not (_is_torch(x) and x.is_cuda and x.is_contiguous() and x.dtype == dt and tuple(x.shape) == tuple(shape)):
+        raise ValueError(f"{what} on the device must be a contiguous CUDA tensor {np.dtype(dtype).name}{list(shape)}")
+
+
+def _loop_arrays(loop, n, dev=None):
+    """The arrays of a Loop in the layouts of the C ABI (kept alive by the caller for the call): host arrays broadcast to N rows,
+    or with dev != None torch tensors on that device (torch inputs checked, not converted)."""
+    out = {}
+    for name, dtype, width in _LOOP_FIELDS:
+        x = getattr(loop, name)
+        shape = (n,) if width is None else (n, width)
+        if x is None:
+            out[name] = None
+        elif dev is not None and _is_torch(x):
+            check_device_array(x, shape, dtype, f"loop.{name}")
+            out[name] = x
+        else:
+            a = np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype), shape))
+            if dev is not None:
+                import torch
+                a = torch.from_numpy(a.copy()).to(dev)
+            out[name] = a
+    st = loop.state
+    if st is not None:
+        if dev is not None:
+            check_device_array(st.hist, (n, LOOP_HIST, 12), np.float64, "loop.state.hist")
+            check_device_array(st.tick, (n,), np.int64, "loop.state.tick")
+        elif not (isinstance(st.hist, np.ndarray) and st.hist.dtype == np.float64 and st.hist.shape == (n, LOOP_HIST, 12)
+                  and st.hist.flags.c_contiguous and isinstance(st.tick, np.ndarray) and st.tick.dtype == np.int64
+                  and st.tick.shape == (n,) and st.tick.flags.c_contiguous):
+            raise ValueError(f"loop.state must hold contiguous host arrays hist float64[{n}, {LOOP_HIST}, 12] and tick int64[{n}]")
+    return out
+
+
+def _wbc_loop(loop, arrays, ptr):
+    st = loop.state
+    return WbcLoop(*(ptr(arrays[name]) for name, _, _ in _LOOP_FIELDS[:4]), int(loop.seed) & 0xFFFFFFFFFFFFFFFF,
+                   None if st is None else ptr(st.hist), None if st is None else ptr(st.tick))
+
+
+def observe(ctl, q, v, loop):
+    """What the controllers of N robots read at their current ticks (wbc_loop_observe; the ticks are not advanced) -> q_obs [N,19],
+    v_obs [N,18]. Host arrays go through the host entry; torch CUDA tensors stay on the device (torch's current stream)."""
+    if _is_torch(q):
+        import torch
+        n, dev = q.shape[0], q.device
+        check_device_array(q, (n, NQ), np.float64, "q")
+        check_device_array(v, (n, NV), np.float64, "v")
+        arrays = _loop_arrays(loop, n, dev)
+        p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        qo, vo = torch.empty_like(q), torch.empty_like(v)
+        lp = _wbc_loop(loop, arrays, p)
+        ctl._check(ctl.lib.wbc_loop_observe(ctl._h, n, C.byref(lp), p(q), p(v), p(qo), p(vo),
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "wbc_loop_observe")
+        return qo, vo
+    q = np.ascontiguousarray(q, dtype=np.float64).reshape(-1, NQ)
+    n = len(q)
+    v = np.ascontiguousarray(v, dtype=np.float64).reshape(n, NV)
+    arrays = _loop_arrays(loop, n)
+    opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
+    qo, vo = np.empty_like(q), np.empty_like(v)
+    lp = _wbc_loop(loop, arrays, opt)
+    ctl._check(ctl.lib.wbc_loop_observe_host(ctl._h, n, C.byref(lp), np_ptr(q), np_ptr(v), np_ptr(qo), np_ptr(vo)), "wbc_loop_observe_host")
+    return qo, vo
+
+
 class RolloutResult:
     __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact")
 
@@ -137,7 +246,7 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
             mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
-            param_index=None) -> RolloutResult:
+            param_index=None, loop=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -148,7 +257,9 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     Uneven ground (plant=True only): terrain_set (TerrainSet or None: flat ground), terrain [N] int32 (None: terrain 0); an
     out-of-range terrain index freezes that robot, flagged ST_BADTERRAIN.
     Per-robot controller parameters (either plant): param_set (controller.ParamSet or None: the handle's params), param_index
-    [N] int32 (None: set 0); a robot with an out-of-range index gets zero torques, flagged ST_BADPARAMS."""
+    [N] int32 (None: set 0); a robot with an out-of-range index gets zero torques, flagged ST_BADPARAMS.
+    Imperfect sensing and actuation (plant=True only): loop (a Loop) gives each robot's state noise, command delay and motor
+    strength; `tau` is then the last COMMANDED torque. A robot with a bad profile is flagged ST_BADLOOP and gets zero torque."""
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     per_robot = param_set is not None or param_index is not None
@@ -163,7 +274,16 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if per_robot:
+        if loop is not None:
+            arrays = _loop_arrays(loop, n, dev)            # (kept alive for the call)
+            pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
+            tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
+            check_device_index(param_index, n)
+            cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))) if per_robot else None
+            lp = _wbc_loop(loop, arrays, p)
+            ctl._check(ctl.lib.wbc_rollout_loop(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
+                                                C.byref(lp), stream), "wbc_rollout_loop")
+        elif per_robot:
             pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
             tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
             check_device_index(param_index, n)
@@ -192,7 +312,17 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if per_robot:
+    if loop is not None:
+        vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
+        ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
+        arrays = _loop_arrays(loop, n)
+        pt = C.byref(_perturb(plant_set, vi, pu, opt)) if perturbed else None
+        tr = C.byref(_terrain(terrain_set, ti, opt)) if on_terrain else None
+        cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))) if per_robot else None
+        lp = _wbc_loop(loop, arrays, opt)
+        ctl._check(ctl.lib.wbc_rollout_loop_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
+                                                 C.byref(lp)), "wbc_rollout_loop_host")
+    elif per_robot:
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
         ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
         pt = C.byref(_perturb(plant_set, vi, pu, opt)) if perturbed else None
