@@ -556,6 +556,82 @@ int wbc_loop_observe(wbc_handle* h, int64_t n, const wbc_loop* loop, const doubl
 int wbc_loop_observe_host(wbc_handle* h, int64_t n, const wbc_loop* loop, const double* q, const double* v, double* q_obs,
                           double* v_obs);
 
+/* ---- Rollout monitor of the ground-plant loop: per-robot fall detection, time to failure and effort statistics, accumulated on
+ * the device one control step at a time. It only observes: no existing output changes.
+ *
+ * The monitor runs once per control step k, after the plant step. It sees the true post-step state q, v (time t_k + dt); the
+ * plan sample traj, contact that the step's controller tracked (sampled at t_k); the torque the plant applied (the actuated
+ * torque with a loop, else the command); the plant's ground forces f (world axes); and the step's full status word (the
+ * controller status plus the plant's bits). The pose is compared with the sample at t_k, not t_k + dt: this one-step lag is exact
+ * for a standing plan and adds about |pdot_plan| dt to the errors of a moving one.
+ *
+ * Per step, with p = q[4:7], q_hat = q[0:4] / |q[0:4]| and q_ref the quaternion of RollPitchYaw traj[9:12] (qz(yaw) (x) qy(pitch)
+ * (x) qx(roll), Drake's convention):
+ *   e_p     = |p - traj[0:3]|
+ *   e_theta = 2 atan2(|u|, |w|) with (w, u) = conj(q_ref) (x) q_hat: the full rotation angle, accurate near 0 and near pi
+ *   reasons = WBC_MON_POS if !(e_p <= pos_max), | WBC_MON_ANG if !(e_theta <= ang_max), | WBC_MON_STATUS if the status word is
+ *             non-zero. A non-finite error therefore fails; a bound of +inf turns its test off.
+ * Per-robot state (caller-owned, in/out; a zeroed state is a fresh one):
+ *   steps[i]      steps monitored so far (incremented first)
+ *   fail_step[i]  the value of steps at the first step with any reason, 0 while none; written once, never again
+ *   fail_why[i]   the reasons at that step
+ *   stats[i][11]  sums and maxima over every monitored step, before and after a failure; a maximum is m = e > m ? e : m
+ *     SUM_POS2  += e_p^2                      MAX_POS  max e_p
+ *     SUM_ANG2  += e_theta^2                  MAX_ANG  max e_theta
+ *     TAU2_DT   += dt sum_a tau_a^2           WORK_ABS += dt sum_j |tau_{act_index[j]} v[v_index[j]]|
+ *     SAT_MAX   max_j |tau_{act_index[j]}| / effort_j (the handle's model: joint j's effort limit, its actuator's torque)
+ *     F_MAX     max over feet of |f_foot|
+ *     STANCE_UNLOADED += feet planned in stance whose force is exactly 0 (all three components)
+ *     SWING_LOADED    += feet planned in swing whose force is not 0
+ *     DIST_XY   += dt |v[3:5]|
+ *   why[i] (optional)  the reasons at the latest monitored step: the end-state verdict.
+ * WORK_ABS and DIST_XY use the post-step velocities: under the plant's semi-implicit Euler they are exactly tau dtheta and the
+ * step's horizontal base travel. The contact counters are exact tests: the plant's Gauss-Seidel starts from zero impulses and its
+ * freeze writes 0, so an unloaded or frozen foot has a force of exactly 0. */
+#define WBC_MON_NSTAT 11
+#define WBC_MON_POS 1
+#define WBC_MON_ANG 2
+#define WBC_MON_STATUS 4
+#define WBC_MON_SUM_POS2 0
+#define WBC_MON_MAX_POS 1
+#define WBC_MON_SUM_ANG2 2
+#define WBC_MON_MAX_ANG 3
+#define WBC_MON_TAU2_DT 4
+#define WBC_MON_WORK_ABS 5
+#define WBC_MON_SAT_MAX 6
+#define WBC_MON_F_MAX 7
+#define WBC_MON_STANCE_UNLOADED 8
+#define WBC_MON_SWING_LOADED 9
+#define WBC_MON_DIST_XY 10
+typedef struct wbc_monitor {
+  double pos_max, ang_max;  /* failure bounds (m, rad), >= 0 (+inf: off); NaN or negative is WBC_ERR_ARG                    */
+  double* stats;            /* [N][11]  required                                                                         */
+  int64_t* steps;           /* [N]      required                                                                         */
+  int64_t* fail_step;       /* [N]      required                                                                         */
+  int32_t* fail_why;        /* [N]      required                                                                         */
+  int32_t* why;             /* [N] or NULL                                                                               */
+} wbc_monitor;
+
+/* wbc_rollout_loop (opts->plant must be 1; loop, perturb, terrain and ctrl may each be NULL) with the monitor after the plant
+ * in every step: one more launch per step, captured into the same graph. Every existing output (q, v, t, tau, metrics,
+ * status_or, err_max, metrics_log, opts->f_contact) has the bits of the call without a monitor; mon == NULL is wbc_rollout_loop
+ * (its bits and launch count). Device pointers (host pointers for _host; the monitor state is copied in and out). */
+int wbc_rollout_monitor(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                        const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                        const wbc_monitor* mon, void* stream);
+int wbc_rollout_monitor_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                             const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                             const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                             const wbc_monitor* mon);
+/* The monitor alone on one step's records: q [N][19], v [N][18] (post-step), traj [N][54], contact [N][4], tau_applied [N][12],
+ * f_contact [N][12], status [N] (the step's status words, NULL: 0). */
+int wbc_monitor_step(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon, const double* q, const double* v, const double* traj,
+                     const uint8_t* contact, const double* tau_applied, const double* f_contact, const int32_t* status, void* stream);
+int wbc_monitor_step_host(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon, const double* q, const double* v,
+                          const double* traj, const uint8_t* contact, const double* tau_applied, const double* f_contact,
+                          const int32_t* status);
+
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);
 

@@ -26,6 +26,11 @@ ST_BADTERRAIN = 1024
 ST_BADPARAMS = 2048
 ST_BADLOOP = 4096
 LOOP_HIST = 16
+# rollout monitor (include/wbc.h, wbc_monitor): failure reasons and the columns of its per-robot stats
+MON_POS, MON_ANG, MON_STATUS = 1, 2, 4
+MON_NSTAT = 11
+(MON_SUM_POS2, MON_MAX_POS, MON_SUM_ANG2, MON_MAX_ANG, MON_TAU2_DT, MON_WORK_ABS, MON_SAT_MAX, MON_F_MAX, MON_STANCE_UNLOADED,
+ MON_SWING_LOADED, MON_DIST_XY) = range(MON_NSTAT)
 NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
@@ -127,6 +132,12 @@ class WbcLoop(C.Structure):
     """ctypes mirror of `wbc_loop` (per-robot noise, delay, strength and stream; the seed; the loop state hist / tick)."""
     _fields_ = [("noise", C.c_void_p), ("delay", C.c_void_p), ("strength", C.c_void_p), ("stream", C.c_void_p), ("seed", C.c_uint64),
                 ("hist", C.c_void_p), ("tick", C.c_void_p)]
+
+
+class WbcMonitor(C.Structure):
+    """ctypes mirror of `wbc_monitor` (failure bounds; the per-robot state stats / steps / fail_step / fail_why; optional why)."""
+    _fields_ = [("pos_max", C.c_double), ("ang_max", C.c_double), ("stats", C.c_void_p), ("steps", C.c_void_p),
+                ("fail_step", C.c_void_p), ("fail_why", C.c_void_p), ("why", C.c_void_p)]
 
 
 def np_ptr(a: np.ndarray):
@@ -232,7 +243,15 @@ def load_library() -> C.CDLL:
                                           C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), C.POINTER(WbcLoop)]
     lib.wbc_loop_observe.argtypes = [H, i64, C.POINTER(WbcLoop), dp, dp, dp, dp, dp]
     lib.wbc_loop_observe_host.argtypes = [H, i64, C.POINTER(WbcLoop), dp, dp, dp, dp]
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS:
+    lib.wbc_rollout_monitor.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                        C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), C.POINTER(WbcLoop),
+                                        C.POINTER(WbcMonitor), dp]
+    lib.wbc_rollout_monitor_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                             C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                             C.POINTER(WbcLoop), C.POINTER(WbcMonitor)]
+    lib.wbc_monitor_step.argtypes = [H, i64, C.c_double, C.POINTER(WbcMonitor)] + [dp] * 8
+    lib.wbc_monitor_step_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcMonitor)] + [dp] * 7
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -266,7 +285,8 @@ TERRAIN_SYMBOLS = ["wbc_terrain_set_create", "wbc_terrain_set_destroy", "wbc_pla
 PARAM_SYMBOLS = ["wbc_param_set_create", "wbc_param_set_destroy", "wbc_step_params", "wbc_step_params_host", "wbc_rollout_params",
                  "wbc_rollout_params_host"]
 LOOP_SYMBOLS = ["wbc_rollout_loop", "wbc_rollout_loop_host", "wbc_loop_observe", "wbc_loop_observe_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+MONITOR_SYMBOLS = ["wbc_rollout_monitor", "wbc_rollout_monitor_host", "wbc_monitor_step", "wbc_monitor_step_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

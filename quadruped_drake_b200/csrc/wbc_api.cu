@@ -27,6 +27,7 @@
 #include "wbc_rollout.cuh"
 #include "wbc_plant.cuh"
 #include "wbc_loop.cuh"
+#include "wbc_monitor.cuh"
 #include <vector>
 
 namespace {
@@ -636,6 +637,18 @@ struct LoopScratch {
   }
 };
 
+// Scratch of the monitor entries (wbc_rollout_monitor), reserved by them only: the plant's per-step status word, and its ground
+// forces when the caller keeps none.
+struct MonScratch {
+  DevArray<int32_t> word;
+  DevArray<double> f;
+  cudaError_t reserve(int64_t n, bool own_f) {
+    cudaError_t e = word.reserve(n);
+    if (e == cudaSuccess && own_f) e = f.reserve(n * 12);
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
@@ -659,6 +672,7 @@ struct wbc_handle {
   Staging stage;
   RolloutScratch ro;
   LoopScratch loop;
+  MonScratch mon;
   ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
@@ -1954,8 +1968,8 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
 }
 
 // Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant; loop: the same with
-// sensing and actuation, on the ground plant).
-enum class PlantEntry { plain, perturbed, terrain, params, loop };
+// sensing and actuation, on the ground plant; monitor: the loop with the rollout monitor).
+enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -2006,10 +2020,12 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
 // The rollout loop of wbc_rollout_ex, wbc_rollout_perturbed, wbc_rollout_terrain, wbc_rollout_params and wbc_rollout_loop;
 // pa != nullptr: the plant step runs the variant kernel, or with ta != nullptr the terrain kernel; cp != nullptr: the controller
 // step runs with these per-robot parameters; lp != nullptr (ground plant): the controller reads the observed state and the plant
-// applies the actuated torque (wbc_loop.cuh), with the loop state in the handle's scratch when lp->hist is null.
+// applies the actuated torque (wbc_loop.cuh), with the loop state in the handle's scratch when lp->hist is null; mp != nullptr
+// (ground plant): the monitor runs after the plant (wbc_monitor.cuh) on the plant's per-step status word, which it folds into
+// io->status_or.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                        const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
-                       const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr) {
+                       const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr, const wbcmon::MonArgs* mp = nullptr) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -2032,6 +2048,15 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
     }
   }
   const unsigned loop_grid = (unsigned)((n + 255) / 256);
+  // with a monitor the plant ORs each step's status into a word of its own, and writes its forces somewhere in any case
+  int32_t* plant_status_or = io->status_or;
+  double* f_contact = opts ? opts->f_contact : nullptr;
+  if (mp) {
+    WBC_CUDA(h, h->mon.reserve(n, !f_contact));
+    plant_status_or = h->mon.word.p;
+    if (!f_contact) f_contact = h->mon.f.p;
+    WBC_CUDA(h, cudaMemsetAsync(plant_status_or, 0, n * sizeof(int32_t), st));
+  }
   WBC_CUDA(h, cudaMemsetAsync(ro.counter.p, 0, sizeof(int), st));
   if (io->status_or) WBC_CUDA(h, cudaMemsetAsync(io->status_or, 0, n * sizeof(int32_t), st));
   if (io->err_max) WBC_CUDA(h, cudaMemsetAsync(io->err_max, 0, n * sizeof(double), st));
@@ -2058,9 +2083,14 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       h->launches++;
     }
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, applied, io->t, ro.status.p, io->status_or, opts->f_contact, metrics,
+      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, applied, io->t, ro.status.p, plant_status_or, f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
+      if (mp) {
+        wbcmon::monitor_kernel<<<loop_grid, 256, 0, st>>>(*mp, n, io->q, io->v, ro.traj.p, ro.contact.p, applied, f_contact, nullptr,
+                                                          plant_status_or, io->status_or);
+        h->launches++;
+      }
     } else {
       wbcroll::integrate_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, dt, io->q, io->v, ro.vd.p, io->t, ro.status.p, io->status_or,
                                                                            metrics, io->err_max, io->metrics_log, ro.counter.p);
@@ -2219,10 +2249,89 @@ extern "C" int wbc_loop_observe_host(wbc_handle* h, int64_t n, const wbc_loop* l
   return rc ? rc : s.finish(h);
 }
 
-// Host buffers of the five rollouts.
+// ------------------------------------------------------------------------------ rollout monitor (wbc_monitor.cuh)
+// The kernel arguments of a monitor whose arrays are already on the device.
+static int mon_args(wbc_handle* h, const wbc_monitor* m, int64_t n, double dt, wbcmon::MonArgs* ma) {
+  if (!(m->pos_max >= 0.0) || !(m->ang_max >= 0.0)) return fail_arg(h, "wbc_monitor: pos_max and ang_max must be >= 0 (+inf: no bound)");
+  if (n > 0 && (!m->stats || !m->steps || !m->fail_step || !m->fail_why))
+    return fail_arg(h, "wbc_monitor: stats, steps, fail_step and fail_why are required");
+  *ma = wbcmon::MonArgs{m->pos_max, m->ang_max, dt, m->stats, (long long*)m->steps, (long long*)m->fail_step, m->fail_why, m->why, {}, {}, {}};
+  for (int j = 0; j < WBC_NU; ++j) {
+    ma->v_index[j] = h->model.v_index[j];
+    ma->act_index[j] = h->model.act_index[j];
+    ma->effort[j] = h->model.effort[j];
+  }
+  return WBC_OK;
+}
+
+extern "C" int wbc_rollout_monitor(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                   const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                   const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                   const wbc_monitor* mon, void* stream) {
+  if (!mon) return wbc_rollout_loop(h, kind, plan, n, n_steps, dt, io, opts, perturb, terrain, ctrl, loop, stream);
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_monitor: bad arguments");
+  if (!(opts && opts->plant == 1)) return fail_arg(h, "wbc_rollout_monitor: the monitor watches the ground plant (opts->plant = 1)");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  wbcloop::LoopArgs la;
+  wbcmon::MonArgs ma;
+  int rc = mon_args(h, mon, n, dt, &ma);
+  if (!rc && loop) rc = loop_args(h, loop, &la);
+  if (!rc) rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && (perturb || terrain))
+    rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, (perturb || terrain) ? &pa : nullptr, terrain ? &ta : nullptr,
+                               (cudaStream_t)stream, &cp, loop ? &la : nullptr, &ma);
+}
+
+extern "C" int wbc_monitor_step(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon, const double* q, const double* v,
+                                const double* traj, const uint8_t* contact, const double* tau_applied, const double* f_contact,
+                                const int32_t* status, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!mon || n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_monitor_step: mon, n >= 0 and dt > 0 are required");
+  if (n > 0 && (!q || !v || !traj || !contact || !tau_applied || !f_contact))
+    return fail_arg(h, "wbc_monitor_step: q, v, traj, contact, tau_applied and f_contact are required");
+  wbcmon::MonArgs ma;
+  const int rc = mon_args(h, mon, n, dt, &ma);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  wbcmon::monitor_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ma, n, q, v, traj, contact, tau_applied, f_contact,
+                                                                                        status, nullptr, nullptr);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Device copies of a host wbc_monitor's arrays; the state is copied in and out, why out.
+static wbc_monitor monitor_to_device(DevScratch& s, const wbc_monitor& m, size_t N) {
+  return wbc_monitor{m.pos_max, m.ang_max, s.inout(m.stats, N * WBC_MON_NSTAT), s.inout(m.steps, N), s.inout(m.fail_step, N),
+                     s.inout(m.fail_why, N), s.out(m.why, N)};
+}
+
+extern "C" int wbc_monitor_step_host(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon, const double* q, const double* v,
+                                     const double* traj, const uint8_t* contact, const double* tau_applied, const double* f_contact,
+                                     const int32_t* status) {
+  if (!h) return WBC_ERR_ARG;
+  if (!mon || n <= 0) return n == 0 && mon ? WBC_OK : fail_arg(h, "wbc_monitor_step_host: mon and n >= 0 are required");
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  DevScratch s(h->lane[0]);
+  const size_t N = (size_t)n;
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV); const double* dtr = s.in(traj, N * WBC_NTRAJ);
+  const uint8_t* dc = s.in(contact, N * 4); const double* dtau = s.in(tau_applied, N * WBC_NU); const double* df = s.in(f_contact, N * 12);
+  const int32_t* dst = s.in(status, N);
+  const wbc_monitor dm = monitor_to_device(s, *mon, N);
+  WBC_SCRATCH_CHECK(h, s);
+  const int rc = wbc_monitor_step(h, n, dt, &dm, dq, dv, dtr, dc, dtau, df, dst, s.st);
+  return rc ? rc : s.finish(h);
+}
+
+// Host buffers of the six rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                         const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
-                        const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr) {
+                        const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr, const wbc_monitor* mon = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -2246,9 +2355,14 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (ctrl) dcp = wbc_ctrl_params{ctrl->set, s.in(ctrl->index, N)};
   wbc_loop dl{};
   if (loop) dl = loop_to_device(s, *loop, N);
+  wbc_monitor dm{};
+  if (mon) dm = monitor_to_device(s, *mon, N);
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::loop ? wbc_rollout_loop(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+      entry == PlantEntry::monitor ? wbc_rollout_monitor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+                                                         terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr,
+                                                         mon ? &dm : nullptr, s.st)
+      : entry == PlantEntry::loop ? wbc_rollout_loop(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                    terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr, s.st)
       : entry == PlantEntry::params ? wbc_rollout_params(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                        terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, s.st)
@@ -2285,6 +2399,13 @@ extern "C" int wbc_rollout_loop_host(wbc_handle* h, int kind, const wbc_plan* pl
                                      const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
                                      const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::loop, perturb, terrain, ctrl, loop);
+}
+
+extern "C" int wbc_rollout_monitor_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                        const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                        const wbc_monitor* mon) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::monitor, perturb, terrain, ctrl, loop, mon);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

@@ -23,6 +23,11 @@ Imperfect sensing and actuation (`loop`, a `Loop`; ground plant only): robot i's
 and its torque command reaches the plant `delay` control steps late, scaled by its motor strength (semantics in include/wbc.h,
 wbc_loop). It runs through `wbc_rollout_loop`, together with any variants, pushes, terrain and parameter sets; `observe` runs the
 sensing alone.
+
+Rollout monitor (`monitor`, a `Monitor`; ground plant only): after every plant step each robot's true pose is compared with the
+plan sample its controller tracked, the first failing step is kept, and tracking, effort and contact statistics accumulate in a
+`MonitorState` on the device (semantics in include/wbc.h, wbc_monitor). It runs through `wbc_rollout_monitor`, together with
+any loop, variants, pushes, terrain and parameter sets, and changes none of the other outputs.
 """
 from __future__ import annotations
 
@@ -31,8 +36,9 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .capi import (KINDS, LOOP_HIST, WbcCtrlParams, WbcLoop, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts,
-                   WbcTerrainDesc, np_ptr)
+from . import capi
+from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcLoop, WbcMonitor, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain,
+                   WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
 from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
@@ -232,8 +238,77 @@ def observe(ctl, q, v, loop):
     return qo, vo
 
 
+class MonitorState:
+    """The per-robot monitor state of N robots (include/wbc.h, wbc_monitor), zeroed, which is a fresh state: stats [N,11] float64
+    (columns capi.MON_*), steps [N] int64, fail_step [N] int64 (0: not failed yet), fail_why [N] int32 (capi.MON_POS | MON_ANG |
+    MON_STATUS). NumPy arrays, or torch tensors on the device of `like`. A rollout given a state continues it."""
+
+    def __init__(self, n, like=None):
+        if like is not None and _is_torch(like):
+            import torch
+            z = lambda shape, dt_: torch.zeros(shape, dtype=dt_, device=like.device)  # noqa: E731
+            self.stats, self.steps = z((n, MON_NSTAT), torch.float64), z(n, torch.int64)
+            self.fail_step, self.fail_why = z(n, torch.int64), z(n, torch.int32)
+        else:
+            self.stats, self.steps = np.zeros((n, MON_NSTAT)), np.zeros(n, np.int64)
+            self.fail_step, self.fail_why = np.zeros(n, np.int64), np.zeros(n, np.int32)
+
+    @property
+    def failed(self):
+        return self.fail_step > 0
+
+    def fail_time(self, t0=0.0, dt=5e-3):
+        """Time at which each robot was first found failed, t0 + fail_step dt (the end of that step); +inf if it never failed."""
+        if _is_torch(self.fail_step):
+            import torch
+            t = t0 + self.fail_step.to(torch.float64) * dt
+            return torch.where(self.fail_step > 0, t, torch.full_like(t, float("inf")))
+        return np.where(self.fail_step > 0, t0 + self.fail_step * dt, np.inf)
+
+    rms_pos = property(lambda s: (s.stats[:, capi.MON_SUM_POS2] / s.steps) ** 0.5)
+    rms_ang = property(lambda s: (s.stats[:, capi.MON_SUM_ANG2] / s.steps) ** 0.5)
+    max_pos = property(lambda s: s.stats[:, capi.MON_MAX_POS])
+    max_ang = property(lambda s: s.stats[:, capi.MON_MAX_ANG])
+    tau2_dt = property(lambda s: s.stats[:, capi.MON_TAU2_DT])
+    work_abs = property(lambda s: s.stats[:, capi.MON_WORK_ABS])
+    sat_max = property(lambda s: s.stats[:, capi.MON_SAT_MAX])
+    f_max = property(lambda s: s.stats[:, capi.MON_F_MAX])
+    stance_unloaded = property(lambda s: s.stats[:, capi.MON_STANCE_UNLOADED])
+    swing_loaded = property(lambda s: s.stats[:, capi.MON_SWING_LOADED])
+    dist_xy = property(lambda s: s.stats[:, capi.MON_DIST_XY])
+
+
+@dataclass
+class Monitor:
+    """Failure bounds of the rollout monitor: base position error (m) and orientation error (rad) against the plan sample; +inf
+    turns a bound off. state: a MonitorState to continue (None: each call starts a fresh one)."""
+    pos_max: float = 0.05
+    ang_max: float = 0.3
+    state: MonitorState | None = None
+
+
+_MON_FIELDS = (("stats", np.float64, (MON_NSTAT,)), ("steps", np.int64, ()), ("fail_step", np.int64, ()), ("fail_why", np.int32, ()))
+
+
+def _monitor_state(monitor, n, like=None):
+    """The monitor's state, checked (or a fresh one): torch CUDA tensors when `like` is a torch tensor, host arrays otherwise."""
+    st = monitor.state if monitor.state is not None else MonitorState(n, like)
+    for name, dtype, width in _MON_FIELDS:
+        x, shape = getattr(st, name), (n, *width)
+        if like is not None and _is_torch(like):
+            check_device_array(x, shape, dtype, f"monitor.state.{name}")
+        elif not (isinstance(x, np.ndarray) and x.dtype == dtype and x.shape == shape and x.flags.c_contiguous):
+            raise ValueError(f"monitor.state.{name} must be a contiguous host array {np.dtype(dtype).name}{list(shape)}")
+    return st
+
+
+def _wbc_monitor(monitor, st, why, ptr):
+    return WbcMonitor(float(monitor.pos_max), float(monitor.ang_max), ptr(st.stats), ptr(st.steps), ptr(st.fail_step), ptr(st.fail_why),
+                      ptr(why))
+
+
 class RolloutResult:
-    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact")
+    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why")
 
     def __init__(self, **kw):
         for k in self.__slots__:
@@ -246,7 +321,7 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
             mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
-            param_index=None, loop=None) -> RolloutResult:
+            param_index=None, loop=None, monitor=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -259,7 +334,9 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     Per-robot controller parameters (either plant): param_set (controller.ParamSet or None: the handle's params), param_index
     [N] int32 (None: set 0); a robot with an out-of-range index gets zero torques, flagged ST_BADPARAMS.
     Imperfect sensing and actuation (plant=True only): loop (a Loop) gives each robot's state noise, command delay and motor
-    strength; `tau` is then the last COMMANDED torque. A robot with a bad profile is flagged ST_BADLOOP and gets zero torque."""
+    strength; `tau` is then the last COMMANDED torque. A robot with a bad profile is flagged ST_BADLOOP and gets zero torque.
+    Rollout monitor (plant=True only): monitor (a Monitor) accumulates per-robot failure and effort statistics; the result then
+    carries `monitor` (its MonitorState, advanced) and `why` [N] int32, the failure reasons at the last step."""
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     per_robot = param_set is not None or param_index is not None
@@ -274,7 +351,18 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if loop is not None:
+        if monitor is not None:
+            r.monitor, r.why = _monitor_state(monitor, n, q), mk((n,), torch.int32)
+            arrays = None if loop is None else _loop_arrays(loop, n, dev)      # (kept alive for the call)
+            pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
+            tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
+            check_device_index(param_index, n)
+            cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))) if per_robot else None
+            lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, p))
+            mo = _wbc_monitor(monitor, r.monitor, r.why, p)
+            ctl._check(ctl.lib.wbc_rollout_monitor(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
+                                                   lp, C.byref(mo), stream), "wbc_rollout_monitor")
+        elif loop is not None:
             arrays = _loop_arrays(loop, n, dev)            # (kept alive for the call)
             pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
             tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
@@ -312,7 +400,19 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if loop is not None:
+    if monitor is not None:
+        r.monitor, r.why = _monitor_state(monitor, n), np.zeros(n, np.int32)
+        vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
+        ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
+        arrays = None if loop is None else _loop_arrays(loop, n)
+        pt = C.byref(_perturb(plant_set, vi, pu, opt)) if perturbed else None
+        tr = C.byref(_terrain(terrain_set, ti, opt)) if on_terrain else None
+        cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))) if per_robot else None
+        lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, opt))
+        mo = _wbc_monitor(monitor, r.monitor, r.why, opt)
+        ctl._check(ctl.lib.wbc_rollout_monitor_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
+                                                    lp, C.byref(mo)), "wbc_rollout_monitor_host")
+    elif loop is not None:
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
         ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
         arrays = _loop_arrays(loop, n)
