@@ -72,6 +72,7 @@ extern "C" {
 #define WBC_ST_BADTERRAIN 1024 /* terrain plant only: terrain index out of range; the robot is frozen, zero ground forces */
 #define WBC_ST_BADPARAMS 2048  /* wbc_step_params only: parameter-set index out of range; zero outputs                  */
 #define WBC_ST_BADLOOP 4096    /* wbc_rollout_loop only: bad loop profile; observed without noise, zero applied torque  */
+#define WBC_ST_BADMOTOR 8192   /* wbc_rollout_motor / wbc_motor_apply only: motor record index out of range; zero torque */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -631,6 +632,81 @@ int wbc_monitor_step(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon
 int wbc_monitor_step_host(wbc_handle* h, int64_t n, double dt, const wbc_monitor* mon, const double* q, const double* v,
                           const double* traj, const uint8_t* contact, const double* tau_applied, const double* f_contact,
                           const int32_t* status);
+
+/* ---- Actuator model of the ground-plant loop: per-robot torque-speed limits, motor lag and joint friction between the
+ * actuated torque and the plant. Each step is sample plan -> observe -> controller -> actuate -> motor -> ground plant -> monitor.
+ *
+ * A motor set is K records. A record holds seven per-joint arrays [12] in the model's joint order k (the order of
+ * wbc_model.effort): peak torque (N m, >= 0, +inf allowed), speed_knee (rad/s, >= 0, +inf allowed, <= speed_free), speed_free
+ * (rad/s, >= 0, +inf allowed), lag (first-order time constant, s), damping (viscous friction, N m s/rad), coulomb (Coulomb
+ * friction, N m) and coulomb_speed (regularisation speed, rad/s); the last four finite and >= 0, coulomb_speed > 0 where
+ * coulomb > 0. Anything else is WBC_ERR_ARG at creation.
+ *
+ * Per robot i with record r = set[index[i]], for each joint k with actuator a = act_index[k]:
+ *   w   = v[i][v_index[k]], the TRUE joint velocity at the start of the step
+ *   u   = the torque reaching actuator a: the actuated torque with a loop, else the command
+ *   lag: s = u if count[i] == 0 or lag_k == 0 (the first command primes the filter: no start-up transient, as the loop holds
+ *        its first command); else s = m + alpha (u - m) with m = tau_m[i][a], alpha = -expm1(-dt / lag_k)
+ *   envelope: L = peak_k, except in the motoring quadrant (s and w non-zero and of one sign) with |w| > speed_knee_k, where
+ *        L = 0 if |w| >= speed_free_k, else peak_k (speed_free_k - |w|) / (speed_free_k - speed_knee_k) (with speed_free_k = +inf
+ *        its limit, peak_k)
+ *   out = s if |s| <= L, else copysign(L, s): a NaN s stays NaN (the plant's DIVERGED rule then freezes the robot)
+ *   tau_m[i][a] = out: the clamped value is the state, so nothing winds up
+ *   f   = -damping_k w - coulomb_k clamp(w / coulomb_speed_k, -1, 1); a zero coefficient adds nothing (not a signed zero, and
+ *         a NaN w does not pass through it); with both zero the plant input is out itself
+ *   plant input at a = out + f; count[i] += 1
+ * Bad index (< 0 or >= K): motor and plant torque 0 and WBC_ST_BADMOTOR in the step's controller status (kept by status_or);
+ * tau_m and count unchanged. No plant freeze mask holds the bit: the robot goes limp, as with WBC_ST_BADLOOP.
+ * NULL set: one record with peak = the handle's effort and every other field off (knee = free = +inf, lag = damping =
+ * coulomb = 0): saturation at the URDF effort. A record with peak = +inf and every other field off is the ideal motor: the
+ * plant gets u bit for bit.
+ * The monitor sees out (tau_m), the motor's torque, as the applied torque: SAT_MAX, TAU2_DT and WORK_ABS measure motor effort,
+ * not friction (for a robot with a bad index, its unchanged tau_m). io->tau keeps the last COMMANDED torque.
+ *
+ * Explicit friction: friction uses the pre-step w, so damping_k + coulomb_k / coulomb_speed_k acts like the PD law's Kd and is
+ * stable only while (that sum) dt / I < 2 for the joint's effective inertia I (about 1e-3 kg m^2 on the mini_cheetah knee links:
+ * 1.5 N m s/rad diverges at dt = 5e-3). Larger values are legal physics at smaller dt and are not rejected; a robot that runs
+ * away is flagged WBC_ST_DIVERGED by the plant and frozen. */
+typedef struct wbc_motor_desc {
+  double peak[WBC_NU];
+  double speed_knee[WBC_NU];
+  double speed_free[WBC_NU];
+  double lag[WBC_NU];
+  double damping[WBC_NU];
+  double coulomb[WBC_NU];
+  double coulomb_speed[WBC_NU];
+} wbc_motor_desc;
+/* A motor set keeps its device number and may outlive the handle. n_sets >= 1. */
+typedef struct wbc_motor_set wbc_motor_set;
+int wbc_motor_set_create(wbc_handle* h, int32_t n_sets, const wbc_motor_desc* descs, wbc_motor_set** out);
+int wbc_motor_set_destroy(wbc_motor_set* s);
+
+typedef struct wbc_plant_motor {
+  const wbc_motor_set* set;  /* NULL: the one record of the handle's effort limits                                         */
+  const int32_t* index;      /* [N] record of each robot, NULL = record 0                                                    */
+  double* tau_m;             /* [N][12] (actuator order) and count [N]: both given (in/out) or both NULL (library scratch,   */
+  int64_t* count;            /* zeroed at the start of each call); only one of them is WBC_ERR_ARG                           */
+} wbc_plant_motor;
+
+/* wbc_rollout_monitor (opts->plant must be 1; loop, mon, perturb, terrain and ctrl may each be NULL) with the motor between
+ * actuation and the plant in every step: one more launch per step, captured into the same graph. motor == NULL is
+ * wbc_rollout_monitor (its bits and launch count). Device pointers (host pointers for _host; tau_m and count are copied in and
+ * out). */
+int wbc_rollout_motor(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                      const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                      const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop, const wbc_monitor* mon,
+                      const wbc_plant_motor* motor, void* stream);
+int wbc_rollout_motor_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                           const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                           const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                           const wbc_monitor* mon, const wbc_plant_motor* motor);
+/* The motor alone on one step: v [N][18] (the true pre-step velocities), tau_in [N][12] (u, actuator order) -> tau_plant [N][12]
+ * (the plant input); status [N] (or NULL) gets WBC_ST_BADMOTOR ORed in. motor->tau_m and motor->count are required: the motor
+ * torque is motor->tau_m afterwards. */
+int wbc_motor_apply(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* motor, const double* v, const double* tau_in,
+                    double* tau_plant, int32_t* status, void* stream);
+int wbc_motor_apply_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* motor, const double* v, const double* tau_in,
+                         double* tau_plant, int32_t* status);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

@@ -25,6 +25,7 @@ ST_BADVARIANT = 512
 ST_BADTERRAIN = 1024
 ST_BADPARAMS = 2048
 ST_BADLOOP = 4096
+ST_BADMOTOR = 8192
 LOOP_HIST = 16
 # rollout monitor (include/wbc.h, wbc_monitor): failure reasons and the columns of its per-robot stats
 MON_POS, MON_ANG, MON_STATUS = 1, 2, 4
@@ -35,7 +36,7 @@ NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
              ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN",
-             ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP"}
+             ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP", ST_BADMOTOR: "BADMOTOR"}
 
 
 def status_names(status: int) -> str:
@@ -132,6 +133,16 @@ class WbcLoop(C.Structure):
     """ctypes mirror of `wbc_loop` (per-robot noise, delay, strength and stream; the seed; the loop state hist / tick)."""
     _fields_ = [("noise", C.c_void_p), ("delay", C.c_void_p), ("strength", C.c_void_p), ("stream", C.c_void_p), ("seed", C.c_uint64),
                 ("hist", C.c_void_p), ("tick", C.c_void_p)]
+
+
+class WbcMotorDesc(C.Structure):
+    """ctypes mirror of `wbc_motor_desc`: seven per-joint arrays [12] in the model's joint order."""
+    _fields_ = [(name, C.c_double * 12) for name in ("peak", "speed_knee", "speed_free", "lag", "damping", "coulomb", "coulomb_speed")]
+
+
+class WbcPlantMotor(C.Structure):
+    """ctypes mirror of `wbc_plant_motor` (set, index [N]; the state tau_m [N][12] and count [N], both or neither)."""
+    _fields_ = [("set", C.c_void_p), ("index", C.c_void_p), ("tau_m", C.c_void_p), ("count", C.c_void_p)]
 
 
 class WbcMonitor(C.Structure):
@@ -251,7 +262,17 @@ def load_library() -> C.CDLL:
                                              C.POINTER(WbcLoop), C.POINTER(WbcMonitor)]
     lib.wbc_monitor_step.argtypes = [H, i64, C.c_double, C.POINTER(WbcMonitor)] + [dp] * 8
     lib.wbc_monitor_step_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcMonitor)] + [dp] * 7
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS:
+    lib.wbc_motor_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcMotorDesc), C.POINTER(H)]
+    lib.wbc_motor_set_destroy.argtypes = [dp]
+    lib.wbc_rollout_motor.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                      C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams), C.POINTER(WbcLoop),
+                                      C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), dp]
+    lib.wbc_rollout_motor_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                           C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                           C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor)]
+    lib.wbc_motor_apply.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantMotor)] + [dp] * 5
+    lib.wbc_motor_apply_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantMotor)] + [dp] * 4
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -286,7 +307,9 @@ PARAM_SYMBOLS = ["wbc_param_set_create", "wbc_param_set_destroy", "wbc_step_para
                  "wbc_rollout_params_host"]
 LOOP_SYMBOLS = ["wbc_rollout_loop", "wbc_rollout_loop_host", "wbc_loop_observe", "wbc_loop_observe_host"]
 MONITOR_SYMBOLS = ["wbc_rollout_monitor", "wbc_rollout_monitor_host", "wbc_monitor_step", "wbc_monitor_step_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+MOTOR_SYMBOLS = ["wbc_motor_set_create", "wbc_motor_set_destroy", "wbc_rollout_motor", "wbc_rollout_motor_host", "wbc_motor_apply",
+                 "wbc_motor_apply_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

@@ -28,6 +28,7 @@
 #include "wbc_plant.cuh"
 #include "wbc_loop.cuh"
 #include "wbc_monitor.cuh"
+#include "wbc_motor.cuh"
 #include <vector>
 
 namespace {
@@ -649,6 +650,19 @@ struct MonScratch {
   }
 };
 
+// Scratch of the motor entries (wbc_rollout_motor), reserved by them only: the plant input, and the motor state of a call that
+// brings none.
+struct MotorScratch {
+  DevArray<double> plant, tau_m;
+  DevArray<long long> count;
+  cudaError_t reserve(int64_t n, bool own_state) {
+    cudaError_t e = plant.reserve(n * WBC_NU);
+    if (e == cudaSuccess && own_state) e = tau_m.reserve(n * WBC_NU);
+    if (e == cudaSuccess && own_state) e = count.reserve(n);
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
@@ -673,6 +687,7 @@ struct wbc_handle {
   RolloutScratch ro;
   LoopScratch loop;
   MonScratch mon;
+  MotorScratch motor;
   ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
@@ -1968,8 +1983,9 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
 }
 
 // Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant; loop: the same with
-// sensing and actuation, on the ground plant; monitor: the loop with the rollout monitor).
-enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor };
+// sensing and actuation, on the ground plant; monitor: the loop with the rollout monitor; motor: the monitor entry with the
+// actuator model).
+enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor, motor };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -2022,10 +2038,12 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
 // step runs with these per-robot parameters; lp != nullptr (ground plant): the controller reads the observed state and the plant
 // applies the actuated torque (wbc_loop.cuh), with the loop state in the handle's scratch when lp->hist is null; mp != nullptr
 // (ground plant): the monitor runs after the plant (wbc_monitor.cuh) on the plant's per-step status word, which it folds into
-// io->status_or.
+// io->status_or; mt != nullptr (ground plant): the motor (wbc_motor.cuh) turns the applied torque into the plant input, with its
+// state in the handle's scratch when mt->tau_m is null, and the monitor sees the motor torque tau_m.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                        const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
-                       const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr, const wbcmon::MonArgs* mp = nullptr) {
+                       const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr, const wbcmon::MonArgs* mp = nullptr,
+                       const wbcmotor::MotorArgs* mt = nullptr) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -2045,6 +2063,17 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       la.hist = h->loop.hist.p;
       la.tick = h->loop.tick.p;
       WBC_CUDA(h, cudaMemsetAsync(la.tick, 0, n * sizeof(long long), st));
+    }
+  }
+  wbcmotor::MotorArgs ma{};
+  if (mt) {
+    ma = *mt;
+    WBC_CUDA(h, h->motor.reserve(n, !ma.tau_m));
+    if (!ma.tau_m) {                               // a fresh motor state: count 0 (no tau_m is read before it is written)
+      ma.tau_m = h->motor.tau_m.p;
+      ma.count = h->motor.count.p;
+      WBC_CUDA(h, cudaMemsetAsync(ma.tau_m, 0, n * WBC_NU * sizeof(double), st));
+      WBC_CUDA(h, cudaMemsetAsync(ma.count, 0, n * sizeof(long long), st));
     }
   }
   const unsigned loop_grid = (unsigned)((n + 255) / 256);
@@ -2069,6 +2098,8 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
   wbc_io sio{lp ? h->loop.q_obs.p : io->q, lp ? h->loop.v_obs.p : io->v, ro.traj.p, ro.contact.p, tau, metrics, ro.status.p,
              plant ? nullptr : ro.vd.p, nullptr, nullptr};
   const double* applied = lp ? h->loop.applied.p : tau;
+  const double* plant_tau = mt ? h->motor.plant.p : applied;      // with a motor the plant gets its input, the monitor its torque
+  const double* mon_tau = mt ? ma.tau_m : applied;
   auto one_step = [&]() -> int {
     int r = wbc_sample_trajectory(h, plan, n, io->plan_index, io->t, ro.traj.p, ro.contact.p, nullptr, nullptr, nullptr, st);
     if (r) return r;
@@ -2082,12 +2113,17 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       wbcloop::actuate_kernel<<<loop_grid, 256, 0, st>>>(la, n, tau, h->loop.applied.p, ro.status.p);
       h->launches++;
     }
+    if (mt) {
+      wbcmotor::motor_kernel<<<(unsigned)((n + 15) / 16), wbcmotor::MOTOR_BLOCK, 0, st>>>(ma, n, io->v, applied, h->motor.plant.p,
+                                                                                         ro.status.p);
+      h->launches++;
+    }
     if (plant) {
-      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, applied, io->t, ro.status.p, plant_status_or, f_contact, metrics,
+      r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, plant_tau, io->t, ro.status.p, plant_status_or, f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
       if (mp) {
-        wbcmon::monitor_kernel<<<loop_grid, 256, 0, st>>>(*mp, n, io->q, io->v, ro.traj.p, ro.contact.p, applied, f_contact, nullptr,
+        wbcmon::monitor_kernel<<<loop_grid, 256, 0, st>>>(*mp, n, io->q, io->v, ro.traj.p, ro.contact.p, mon_tau, f_contact, nullptr,
                                                           plant_status_or, io->status_or);
         h->launches++;
       }
@@ -2328,10 +2364,117 @@ extern "C" int wbc_monitor_step_host(wbc_handle* h, int64_t n, double dt, const 
   return rc ? rc : s.finish(h);
 }
 
-// Host buffers of the six rollouts.
+// ------------------------------------------------------------------------------ actuator model (wbc_motor.cuh)
+// A set keeps the number of the device its records live on, not its handle: it may be destroyed after the handle.
+struct wbc_motor_set {
+  int device = 0;
+  int32_t n_sets = 0;
+  DevArray<wbc_motor_desc> table;
+  ~wbc_motor_set() { cudaSetDevice(device); }   // the table is freed after this, on the set's device
+};
+
+extern "C" int wbc_motor_set_destroy(wbc_motor_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+extern "C" int wbc_motor_set_create(wbc_handle* h, int32_t n_sets, const wbc_motor_desc* descs, wbc_motor_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !descs || n_sets < 1) return fail_arg(h, "wbc_motor_set_create: descs and n_sets >= 1 are required");
+  *out = nullptr;
+  for (int32_t k = 0; k < n_sets; ++k)
+    if (const char* why = wbcmotor::desc_problem(descs[k])) return fail_arg(h, why);
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_motor_set> ms(new (std::nothrow) wbc_motor_set());
+  if (!ms) return WBC_ERR_NOMEM;
+  ms->device = h->device;
+  ms->n_sets = n_sets;
+  WBC_CUDA(h, ms->table.reserve((size_t)n_sets));
+  WBC_CUDA(h, cudaMemcpy(ms->table.p, descs, (size_t)n_sets * sizeof(wbc_motor_desc), cudaMemcpyHostToDevice));
+  *out = ms.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of a motor whose arrays are already on the device (tau_m / count may both be null).
+static int motor_args(wbc_handle* h, const wbc_plant_motor* m, double dt, wbcmotor::MotorArgs* ma) {
+  if (!m->tau_m != !m->count) return fail_arg(h, "wbc_plant_motor: tau_m and count are given together or not at all");
+  const wbc_motor_set* set = m->set;
+  if (set && set->device != h->device) return fail_arg(h, "wbc_plant_motor: the set lives on another device than the handle");
+  *ma = wbcmotor::MotorArgs{set ? set->table.p : nullptr, m->index, set ? set->n_sets : 1, m->tau_m, (long long*)m->count, dt, {}, {}, {}};
+  for (int j = 0; j < WBC_NU; ++j) {
+    ma->v_index[j] = h->model.v_index[j];
+    ma->act_index[j] = h->model.act_index[j];
+    ma->effort[j] = h->model.effort[j];
+  }
+  return WBC_OK;
+}
+
+extern "C" int wbc_rollout_motor(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                 const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                 const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                 const wbc_monitor* mon, const wbc_plant_motor* motor, void* stream) {
+  if (!motor) return wbc_rollout_monitor(h, kind, plan, n, n_steps, dt, io, opts, perturb, terrain, ctrl, loop, mon, stream);
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_motor: bad arguments");
+  if (!(opts && opts->plant == 1)) return fail_arg(h, "wbc_rollout_motor: the motors drive the ground plant (opts->plant = 1)");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  wbcloop::LoopArgs la;
+  wbcmon::MonArgs ma;
+  wbcmotor::MotorArgs mt;
+  int rc = motor_args(h, motor, dt, &mt);
+  if (!rc && mon) rc = mon_args(h, mon, n, dt, &ma);
+  if (!rc && loop) rc = loop_args(h, loop, &la);
+  if (!rc) rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && (perturb || terrain))
+    rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, (perturb || terrain) ? &pa : nullptr, terrain ? &ta : nullptr,
+                               (cudaStream_t)stream, &cp, loop ? &la : nullptr, mon ? &ma : nullptr, &mt);
+}
+
+extern "C" int wbc_motor_apply(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* motor, const double* v, const double* tau_in,
+                               double* tau_plant, int32_t* status, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!motor || n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_motor_apply: motor, n >= 0 and dt > 0 are required");
+  if (n > 0 && (!v || !tau_in || !tau_plant || !motor->tau_m || !motor->count))
+    return fail_arg(h, "wbc_motor_apply: v, tau_in, tau_plant and the motor state tau_m, count are required");
+  wbcmotor::MotorArgs mt;
+  const int rc = motor_args(h, motor, dt, &mt);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  wbcmotor::motor_kernel<<<(unsigned)((n + 15) / 16), wbcmotor::MOTOR_BLOCK, 0, (cudaStream_t)stream>>>(mt, n, v, tau_in, tau_plant, status);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Device copies of a host wbc_plant_motor's arrays; tau_m and count are copied in and out.
+static wbc_plant_motor motor_to_device(DevScratch& s, const wbc_plant_motor& m, size_t N) {
+  return wbc_plant_motor{m.set, s.in(m.index, N), s.inout(m.tau_m, N * WBC_NU), s.inout(m.count, N)};
+}
+
+extern "C" int wbc_motor_apply_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* motor, const double* v,
+                                    const double* tau_in, double* tau_plant, int32_t* status) {
+  if (!h) return WBC_ERR_ARG;
+  if (!motor || n <= 0) return n == 0 && motor ? WBC_OK : fail_arg(h, "wbc_motor_apply_host: motor and n >= 0 are required");
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  DevScratch s(h->lane[0]);
+  const size_t N = (size_t)n;
+  const double* dv = s.in(v, N * WBC_NV); const double* dti = s.in(tau_in, N * WBC_NU);
+  double* dtp = s.out(tau_plant, N * WBC_NU); int32_t* dst = s.inout(status, N);
+  const wbc_plant_motor dm = motor_to_device(s, *motor, N);
+  WBC_SCRATCH_CHECK(h, s);
+  const int rc = wbc_motor_apply(h, n, dt, &dm, dv, dti, dtp, dst, s.st);
+  return rc ? rc : s.finish(h);
+}
+
+// Host buffers of the seven rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                         const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
-                        const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr, const wbc_monitor* mon = nullptr) {
+                        const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr, const wbc_monitor* mon = nullptr,
+                        const wbc_plant_motor* motor = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -2357,9 +2500,14 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (loop) dl = loop_to_device(s, *loop, N);
   wbc_monitor dm{};
   if (mon) dm = monitor_to_device(s, *mon, N);
+  wbc_plant_motor dmt{};
+  if (motor) dmt = motor_to_device(s, *motor, N);
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::monitor ? wbc_rollout_monitor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+      entry == PlantEntry::motor ? wbc_rollout_motor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+                                                     terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr,
+                                                     mon ? &dm : nullptr, motor ? &dmt : nullptr, s.st)
+      : entry == PlantEntry::monitor ? wbc_rollout_monitor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                          terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr,
                                                          mon ? &dm : nullptr, s.st)
       : entry == PlantEntry::loop ? wbc_rollout_loop(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
@@ -2406,6 +2554,13 @@ extern "C" int wbc_rollout_monitor_host(wbc_handle* h, int kind, const wbc_plan*
                                         const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
                                         const wbc_monitor* mon) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::monitor, perturb, terrain, ctrl, loop, mon);
+}
+
+extern "C" int wbc_rollout_motor_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                      const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                      const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                      const wbc_monitor* mon, const wbc_plant_motor* motor) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::motor, perturb, terrain, ctrl, loop, mon, motor);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

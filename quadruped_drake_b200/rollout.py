@@ -28,6 +28,12 @@ Rollout monitor (`monitor`, a `Monitor`; ground plant only): after every plant s
 plan sample its controller tracked, the first failing step is kept, and tracking, effort and contact statistics accumulate in a
 `MonitorState` on the device (semantics in include/wbc.h, wbc_monitor). It runs through `wbc_rollout_monitor`, together with
 any loop, variants, pushes, terrain and parameter sets, and changes none of the other outputs.
+
+Actuator model (`motor`, a `Motor`; ground plant only): between the actuated torque and the plant each joint's motor follows
+its command through a first-order lag, saturates on a torque-speed envelope, and the joint adds viscous and Coulomb friction
+(semantics in include/wbc.h, wbc_motor_desc). A `MotorSet` holds the records; without one every motor saturates at the URDF
+effort. It runs through `wbc_rollout_motor`, together with any monitor, loop, variants, pushes, terrain and parameter sets;
+`motor_apply` runs the motor alone.
 """
 from __future__ import annotations
 
@@ -37,8 +43,8 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import capi
-from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcLoop, WbcMonitor, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain,
-                   WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
+from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcLoop, WbcMonitor, WbcMotorDesc, WbcPlantMotor, WbcPlantOpts,
+                   WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
 from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
@@ -307,6 +313,116 @@ def _wbc_monitor(monitor, st, why, ptr):
                       ptr(why))
 
 
+def motor_desc(model, peak_scale=1.0, speed_knee=np.inf, speed_free=np.inf, lag=0.0, damping=0.0, coulomb=0.0, coulomb_speed=0.0):
+    """One motor record (WbcMotorDesc) for the joints of `model` (a RobotModel, or a BatchedController's): peak torque
+    peak_scale x the URDF effort; every other field a scalar for all 12 joints or an array in the model's joint order. The
+    defaults are the motor of a NULL set: saturation at the effort and nothing else; peak_scale = inf is the ideal motor."""
+    d = WbcMotorDesc()
+    vals = dict(peak=peak_scale * np.asarray(model.effort, np.float64), speed_knee=speed_knee, speed_free=speed_free, lag=lag,
+                damping=damping, coulomb=coulomb, coulomb_speed=coulomb_speed)
+    for name, x in vals.items():
+        getattr(d, name)[:] = [float(y) for y in np.broadcast_to(np.asarray(x, np.float64), (NU,))]
+    return d
+
+
+class MotorSet:
+    """Device-resident table of K motor records (wbc_motor_set_create); robot i's motors are descs[index[i]]."""
+
+    def __init__(self, ctl, descs):
+        self.ctl, self.lib = ctl, ctl.lib
+        self.n_sets = len(descs)
+        arr = (WbcMotorDesc * self.n_sets)(*descs)
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_motor_set_create(ctl._h, self.n_sets, arr, C.byref(self._p)), "wbc_motor_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_motor_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class MotorState:
+    """The motor state of N robots: tau_m [N,12] float64, each actuator's last motor torque (actuator order), and count [N] int64,
+    the number of motor steps so far; both zero (a fresh state). NumPy arrays, or torch tensors on the device of `like`. A rollout
+    given a state continues it and leaves it advanced."""
+
+    def __init__(self, n, like=None):
+        if like is not None and _is_torch(like):
+            import torch
+            self.tau_m = torch.zeros((n, NU), dtype=torch.float64, device=like.device)
+            self.count = torch.zeros(n, dtype=torch.int64, device=like.device)
+        else:
+            self.tau_m, self.count = np.zeros((n, NU)), np.zeros(n, np.int64)
+
+
+@dataclass
+class Motor:
+    """Per-robot actuator model of the ground-plant loop. set: a MotorSet (None: saturation at the URDF effort); index [N] int32
+    record of each robot (None: record 0); state: a MotorState to continue (None: each call starts a fresh one)."""
+    set: MotorSet | None = None
+    index: object = None
+    state: MotorState | None = None
+
+
+def _motor_arrays(motor, n, dev=None):
+    """(index, state) of a Motor in the layouts of the C ABI, checked: the index broadcast to N rows (a host copy, or on `dev`
+    torch tensors are checked, not converted), the state as given."""
+    idx, st = motor.index, motor.state
+    if dev is not None:
+        check_device_index(idx, n, "motor.index")
+        if st is not None:
+            check_device_array(st.tau_m, (n, NU), np.float64, "motor.state.tau_m")
+            check_device_array(st.count, (n,), np.int64, "motor.state.count")
+        return idx, st
+    if st is not None and not (isinstance(st.tau_m, np.ndarray) and st.tau_m.dtype == np.float64 and st.tau_m.shape == (n, NU)
+                               and st.tau_m.flags.c_contiguous and isinstance(st.count, np.ndarray) and st.count.dtype == np.int64
+                               and st.count.shape == (n,) and st.count.flags.c_contiguous):
+        raise ValueError(f"motor.state must hold contiguous host arrays tau_m float64[{n}, {NU}] and count int64[{n}]")
+    return _terrain_index(n, idx), st
+
+
+def _wbc_motor(motor, idx, st, ptr):
+    return WbcPlantMotor(None if motor.set is None else motor.set._p, ptr(idx), None if st is None else ptr(st.tau_m),
+                         None if st is None else ptr(st.count))
+
+
+def motor_apply(ctl, v, tau, motor, dt=5e-3):
+    """The motor alone on one step (wbc_motor_apply) -> (tau_plant [N,12], status [N] int32: ST_BADMOTOR for a bad index). v [N,18]
+    the true joint velocities, tau [N,12] the torque reaching the motors (actuator order); motor.state is required and advanced
+    (its tau_m is the motor torque). Host arrays go through the host entry; torch CUDA tensors stay on the device (torch's
+    current stream)."""
+    if motor.state is None:
+        raise ValueError("motor_apply: motor.state is required (a MotorState)")
+    if _is_torch(v):
+        import torch
+        n, dev = v.shape[0], v.device
+        check_device_array(v, (n, NV), np.float64, "v")
+        check_device_array(tau, (n, NU), np.float64, "tau")
+        idx, st = _motor_arrays(motor, n, dev)
+        p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        out, status = torch.empty_like(tau), torch.zeros(n, dtype=torch.int32, device=dev)
+        mt = _wbc_motor(motor, idx, st, p)
+        ctl._check(ctl.lib.wbc_motor_apply(ctl._h, n, float(dt), C.byref(mt), p(v), p(tau), p(out), p(status),
+                                           C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "wbc_motor_apply")
+        return out, status
+    v = np.ascontiguousarray(v, dtype=np.float64).reshape(-1, NV)
+    n = len(v)
+    tau = np.ascontiguousarray(tau, dtype=np.float64).reshape(n, NU)
+    idx, st = _motor_arrays(motor, n)
+    opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
+    out, status = np.empty_like(tau), np.zeros(n, np.int32)
+    mt = _wbc_motor(motor, idx, st, opt)
+    ctl._check(ctl.lib.wbc_motor_apply_host(ctl._h, n, float(dt), C.byref(mt), np_ptr(v), np_ptr(tau), np_ptr(out), np_ptr(status)),
+               "wbc_motor_apply_host")
+    return out, status
+
+
 class RolloutResult:
     __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why")
 
@@ -321,7 +437,7 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
             mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
-            param_index=None, loop=None, monitor=None) -> RolloutResult:
+            param_index=None, loop=None, monitor=None, motor=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -336,7 +452,10 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     Imperfect sensing and actuation (plant=True only): loop (a Loop) gives each robot's state noise, command delay and motor
     strength; `tau` is then the last COMMANDED torque. A robot with a bad profile is flagged ST_BADLOOP and gets zero torque.
     Rollout monitor (plant=True only): monitor (a Monitor) accumulates per-robot failure and effort statistics; the result then
-    carries `monitor` (its MonitorState, advanced) and `why` [N] int32, the failure reasons at the last step."""
+    carries `monitor` (its MonitorState, advanced) and `why` [N] int32, the failure reasons at the last step.
+    Actuator model (plant=True only): motor (a Motor) puts each robot's motors between the actuated torque and the plant; `tau`
+    stays the last COMMANDED torque, and a monitor sees the motor torque. A robot with a bad record index is flagged ST_BADMOTOR
+    and gets zero torque."""
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     per_robot = param_set is not None or param_index is not None
@@ -351,17 +470,23 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if monitor is not None:
-            r.monitor, r.why = _monitor_state(monitor, n, q), mk((n,), torch.int32)
+        if monitor is not None or motor is not None:
+            if monitor is not None:
+                r.monitor, r.why = _monitor_state(monitor, n, q), mk((n,), torch.int32)
             arrays = None if loop is None else _loop_arrays(loop, n, dev)      # (kept alive for the call)
             pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
             tr = C.byref(_terrain(terrain_set, terrain, p)) if on_terrain else None
             check_device_index(param_index, n)
             cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))) if per_robot else None
             lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, p))
-            mo = _wbc_monitor(monitor, r.monitor, r.why, p)
-            ctl._check(ctl.lib.wbc_rollout_monitor(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
-                                                   lp, C.byref(mo), stream), "wbc_rollout_monitor")
+            mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, p))
+            if motor is None:
+                ctl._check(ctl.lib.wbc_rollout_monitor(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                       cp, lp, mo, stream), "wbc_rollout_monitor")
+            else:
+                mt = C.byref(_wbc_motor(motor, *_motor_arrays(motor, n, dev), p))
+                ctl._check(ctl.lib.wbc_rollout_motor(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                     cp, lp, mo, mt, stream), "wbc_rollout_motor")
         elif loop is not None:
             arrays = _loop_arrays(loop, n, dev)            # (kept alive for the call)
             pt = C.byref(_perturb(plant_set, variant, push, p)) if perturbed else None
@@ -400,8 +525,9 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if monitor is not None:
-        r.monitor, r.why = _monitor_state(monitor, n), np.zeros(n, np.int32)
+    if monitor is not None or motor is not None:
+        if monitor is not None:
+            r.monitor, r.why = _monitor_state(monitor, n), np.zeros(n, np.int32)
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
         ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
         arrays = None if loop is None else _loop_arrays(loop, n)
@@ -409,9 +535,15 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         tr = C.byref(_terrain(terrain_set, ti, opt)) if on_terrain else None
         cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))) if per_robot else None
         lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, opt))
-        mo = _wbc_monitor(monitor, r.monitor, r.why, opt)
-        ctl._check(ctl.lib.wbc_rollout_monitor_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr, cp,
-                                                    lp, C.byref(mo)), "wbc_rollout_monitor_host")
+        mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, opt))
+        if motor is None:
+            ctl._check(ctl.lib.wbc_rollout_monitor_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                        cp, lp, mo), "wbc_rollout_monitor_host")
+        else:
+            mi, ms = _motor_arrays(motor, n)             # (kept alive for the call)
+            mt = C.byref(_wbc_motor(motor, mi, ms, opt))
+            ctl._check(ctl.lib.wbc_rollout_motor_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
+                                                      cp, lp, mo, mt), "wbc_rollout_motor_host")
     elif loop is not None:
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
         ti, ci = _terrain_index(n, terrain), _terrain_index(n, param_index)
