@@ -73,6 +73,7 @@ extern "C" {
 #define WBC_ST_BADPARAMS 2048  /* wbc_step_params only: parameter-set index out of range; zero outputs                  */
 #define WBC_ST_BADLOOP 4096    /* wbc_rollout_loop only: bad loop profile; observed without noise, zero applied torque  */
 #define WBC_ST_BADMOTOR 8192   /* wbc_rollout_motor / wbc_motor_apply only: motor record index out of range; zero torque */
+#define WBC_ST_BADESTIM 16384  /* wbc_rollout_estimator / wbc_estimator_step only: bad record index or failed filter step   */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -707,6 +708,92 @@ int wbc_motor_apply(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* 
                     double* tau_plant, int32_t* status, void* stream);
 int wbc_motor_apply_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_motor* motor, const double* v, const double* tau_in,
                          double* tau_plant, int32_t* status);
+
+/* ---- State estimation in the ground-plant loop: a per-robot linear Kalman filter fuses a synthesised accelerometer with leg
+ * kinematics, and the controller reads the estimated base position and linear velocity instead of observed ones. Each step is
+ * sample plan -> observe -> estimate -> controller -> actuate -> motor -> ground plant -> monitor.
+ *
+ * Robot i has a filter state x[i][18] = (p, v, foot LF, RF, LH, RH), all world frame, its covariance P[i][18][18], v_prev[i][3]
+ * (the true base linear velocity at its previous step) and count[i] (steps estimated so far), and uses record r = set[index[i]].
+ * At step c = loop tick[i] it reads the loop's observed q_obs, v_obs, the true q, v (for the accelerometer and the statistics
+ * only) and the step's planned contact flags. r_k(q) is foot k relative to the base origin in base axes and J_k(q) thetadot its
+ * velocity from the leg's joint rates, both from the handle's joint_xyz / joint_axis / foot_xyz; R_true, R_obs are the base
+ * rotations of q, q_obs; w_obs = v_obs[0:3] (world frame); g the model's gravity; s_k = 1 for a foot planned in stance and
+ * swing_scale for one planned in swing.
+ *   accelerometer  a_w = (v[3:6] - v_prev) / dt; f_b = R_true' (a_w - g) + sigma_acc z, z the normals of Philox draws 18 (two) and
+ *                  19 (the first) of the loop counter (j, stream, c_lo, c_hi) under the loop seed, so that every draw of the loop
+ *                  keeps its bits; sigma_acc = accel_noise[i] (NULL: 0, and 0 draws nothing); input a = R_obs f_b + g
+ *   prime          (count <= 0) p = q_obs[4:7], v = v_obs[3:6], foot_k = p + R_obs r_k(q_obs); P = diag(p0_pos^2 (3), p0_vel^2 (3),
+ *                  p0_foot^2 (12)); the output is the observed state; v_prev = v[3:6]; count = 1
+ *   predict        v += dt a; p += dt v (the plant's semi-implicit Euler); feet unchanged; P = A P A' + Q with
+ *                  Q = dt diag(q_pos^2 (3), q_vel^2 (3), (q_foot s_k)^2 (3 per foot)). With a perfect IMU and an exact prime,
+ *                  prediction alone reproduces the plant's base position and velocity up to rounding.
+ *   update         28 scalar rows with constant H and diagonal R, leg by leg:
+ *                  y_p,k = R_obs r_k(q_obs), predicted foot_k - p, std r_pos s_k (3 rows)
+ *                  y_v,k = -(w_obs x R_obs r_k + R_obs J_k(q_obs) thetadot_obs,k), predicted v, std r_vel s_k (3 rows: the
+ *                          stance-foot zero-velocity constraint)
+ *                  y_z,k = 0, predicted foot_k,z, std r_height s_k (flat ground, as the controller assumes)
+ *                  A std of +inf drops its row: r_pos = r_vel = r_height = +inf is pure IMU dead reckoning. The batch form is
+ *                  S = H P H' + R, K = P H' S^-1, x += K (y - H x), P = (I - K H) P, then P = (P + P') / 2; the kernel makes
+ *                  the rows as sequential scalar updates, the same filter in exact arithmetic.
+ *   output         the controller reads q_obs with [4:7] = p and v_obs with [3:6] = v, written in place into the loop's observed
+ *                  state; orientation, angular velocity and joints stay observed. With an estimator the loop's base-position and
+ *                  base-linear-velocity noise (blocks 1 and 4 of its profile) therefore no longer reach the controller (they
+ *                  still perturb the prime).
+ *                  v_prev = v[3:6]; count += 1; stats[i] (optional, [N][4]) += |p - p_true|^2, max= |p - p_true|,
+ *                  += |v - v_true|^2, max= |v - v_true| against the true state at the start of the step, after the update
+ *                  (prime steps included)
+ *   failure        a scalar innovation variance not > 0, or x or P not finite after the step: the robot is controlled from the
+ *                  observed state, count = 0 (a fresh prime next step), x, P, v_prev and stats unchanged, WBC_ST_BADESTIM
+ *   bad index      (< 0 or >= K) WBC_ST_BADESTIM, nothing changes
+ * WBC_ST_BADESTIM goes into the word the plant ORs its own status into: io->status_or without a monitor, the monitor's per-step
+ * word with one (the step then fails with WBC_MON_STATUS, and the bit reaches io->status_or through the monitor). It is not a
+ * controller status: no plant freeze mask holds it.
+ *
+ * Record fields are standard deviations: q_pos (m/sqrt(s)), q_vel (m/s/sqrt(s)), q_foot (m/sqrt(s)) of the process; r_pos (m),
+ * r_vel (m/s), r_height (m) of the measurements (+inf allowed); swing_scale >= 1 (finite); p0_pos (m), p0_vel (m/s), p0_foot (m)
+ * of the prime. NaN, a negative value, a non-finite process or initial std, or swing_scale < 1 or +inf is WBC_ERR_ARG at creation. */
+typedef struct wbc_estimator_desc {
+  double q_pos, q_vel, q_foot;
+  double r_pos, r_vel, r_height;
+  double swing_scale;
+  double p0_pos, p0_vel, p0_foot;
+} wbc_estimator_desc;
+/* An estimator set keeps its device number and may outlive the handle. n_sets >= 1. */
+typedef struct wbc_estimator_set wbc_estimator_set;
+int wbc_estimator_set_create(wbc_handle* h, int32_t n_sets, const wbc_estimator_desc* descs, wbc_estimator_set** out);
+int wbc_estimator_set_destroy(wbc_estimator_set* s);
+
+typedef struct wbc_estimator {
+  const wbc_estimator_set* set;  /* required                                                                                  */
+  const int32_t* index;          /* [N] record of each robot, NULL = record 0                                                 */
+  const double* accel_noise;     /* [N] accelerometer noise std (m/s^2), NULL = 0                                             */
+  double* x;                     /* [N][18], P [N][18][18], v_prev [N][3] and count [N]: all given (in/out) or all NULL       */
+  double* P;                     /* (library scratch, count 0: each call starts with a fresh prime); anything between is      */
+  double* v_prev;                /* WBC_ERR_ARG                                                                               */
+  int64_t* count;
+  double* stats;                 /* [N][4] or NULL: sum |p err|^2, max |p err|, sum |v err|^2, max |v err| (accumulated)       */
+} wbc_estimator;
+
+/* wbc_rollout_motor (opts->plant must be 1, loop required; motor, mon, perturb, terrain and ctrl may each be NULL) with the
+ * estimator between observe and the controller in every step: one more launch per step, captured into the same graph.
+ * est == NULL is wbc_rollout_motor (its bits and launch count); an estimator without a loop or without the ground plant is
+ * WBC_ERR_ARG. Device pointers (host pointers for _host; the estimator state and stats are copied in and out). */
+int wbc_rollout_estimator(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                          const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                          const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                          const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est, void* stream);
+int wbc_rollout_estimator_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                               const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                               const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                               const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est);
+/* The estimator alone on one step: true q [N][19], v [N][18]; q_obs [N][19], v_obs [N][18] (in/out); contact [N][4]; the loop
+ * gives seed, stream and tick (NULL tick: 0; the tick is read, not advanced); status_or [N] (or NULL) gets WBC_ST_BADESTIM ORed
+ * in. est->x, P, v_prev and count are required. */
+int wbc_estimator_step(wbc_handle* h, int64_t n, double dt, const wbc_estimator* est, const wbc_loop* loop, const double* q,
+                       const double* v, double* q_obs, double* v_obs, const uint8_t* contact, int32_t* status_or, void* stream);
+int wbc_estimator_step_host(wbc_handle* h, int64_t n, double dt, const wbc_estimator* est, const wbc_loop* loop, const double* q,
+                            const double* v, double* q_obs, double* v_obs, const uint8_t* contact, int32_t* status_or);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

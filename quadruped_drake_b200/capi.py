@@ -26,6 +26,7 @@ ST_BADTERRAIN = 1024
 ST_BADPARAMS = 2048
 ST_BADLOOP = 4096
 ST_BADMOTOR = 8192
+ST_BADESTIM = 16384
 LOOP_HIST = 16
 # rollout monitor (include/wbc.h, wbc_monitor): failure reasons and the columns of its per-robot stats
 MON_POS, MON_ANG, MON_STATUS = 1, 2, 4
@@ -36,7 +37,8 @@ NLAM = 42
 _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RANKDEF", ST_GIMBAL: "GIMBAL", ST_NOTPD: "NOTPD",
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
              ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN",
-             ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP", ST_BADMOTOR: "BADMOTOR"}
+             ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP", ST_BADMOTOR: "BADMOTOR",
+             ST_BADESTIM: "BADESTIM"}
 
 
 def status_names(status: int) -> str:
@@ -143,6 +145,18 @@ class WbcMotorDesc(C.Structure):
 class WbcPlantMotor(C.Structure):
     """ctypes mirror of `wbc_plant_motor` (set, index [N]; the state tau_m [N][12] and count [N], both or neither)."""
     _fields_ = [("set", C.c_void_p), ("index", C.c_void_p), ("tau_m", C.c_void_p), ("count", C.c_void_p)]
+
+
+class WbcEstimatorDesc(C.Structure):
+    """ctypes mirror of `wbc_estimator_desc`: process, measurement and initial standard deviations, and the swing scale."""
+    _fields_ = [(name, C.c_double) for name in ("q_pos", "q_vel", "q_foot", "r_pos", "r_vel", "r_height", "swing_scale", "p0_pos",
+                                                "p0_vel", "p0_foot")]
+
+
+class WbcEstimator(C.Structure):
+    """ctypes mirror of `wbc_estimator` (set, index [N], accel_noise [N]; the state x [N][18], P [N][18][18], v_prev [N][3] and
+    count [N], all or none; stats [N][4] or NULL)."""
+    _fields_ = [(name, C.c_void_p) for name in ("set", "index", "accel_noise", "x", "P", "v_prev", "count", "stats")]
 
 
 class WbcMonitor(C.Structure):
@@ -272,7 +286,17 @@ def load_library() -> C.CDLL:
                                            C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor)]
     lib.wbc_motor_apply.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantMotor)] + [dp] * 5
     lib.wbc_motor_apply_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcPlantMotor)] + [dp] * 4
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS:
+    lib.wbc_estimator_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcEstimatorDesc), C.POINTER(H)]
+    lib.wbc_estimator_set_destroy.argtypes = [dp]
+    lib.wbc_rollout_estimator.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                          C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                          C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), C.POINTER(WbcEstimator), dp]
+    lib.wbc_rollout_estimator_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                               C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                               C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), C.POINTER(WbcEstimator)]
+    lib.wbc_estimator_step.argtypes = [H, i64, C.c_double, C.POINTER(WbcEstimator), C.POINTER(WbcLoop)] + [dp] * 7
+    lib.wbc_estimator_step_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcEstimator), C.POINTER(WbcLoop)] + [dp] * 6
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -309,7 +333,9 @@ LOOP_SYMBOLS = ["wbc_rollout_loop", "wbc_rollout_loop_host", "wbc_loop_observe",
 MONITOR_SYMBOLS = ["wbc_rollout_monitor", "wbc_rollout_monitor_host", "wbc_monitor_step", "wbc_monitor_step_host"]
 MOTOR_SYMBOLS = ["wbc_motor_set_create", "wbc_motor_set_destroy", "wbc_rollout_motor", "wbc_rollout_motor_host", "wbc_motor_apply",
                  "wbc_motor_apply_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+ESTIMATOR_SYMBOLS = ["wbc_estimator_set_create", "wbc_estimator_set_destroy", "wbc_rollout_estimator", "wbc_rollout_estimator_host",
+                     "wbc_estimator_step", "wbc_estimator_step_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

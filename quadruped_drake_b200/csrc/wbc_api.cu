@@ -29,6 +29,7 @@
 #include "wbc_loop.cuh"
 #include "wbc_monitor.cuh"
 #include "wbc_motor.cuh"
+#include "wbc_estimator.cuh"
 #include <vector>
 
 namespace {
@@ -663,6 +664,19 @@ struct MotorScratch {
   }
 };
 
+// Scratch of the estimator entries (wbc_rollout_estimator), reserved by them only: the filter state of a call that brings none.
+struct EstScratch {
+  DevArray<double> x, P, v_prev;
+  DevArray<long long> count;
+  cudaError_t reserve(int64_t n) {
+    cudaError_t e = x.reserve(n * wbcest::NX);
+    if (e == cudaSuccess) e = P.reserve(n * wbcest::NX * wbcest::NX);
+    if (e == cudaSuccess) e = v_prev.reserve(n * 3);
+    if (e == cudaSuccess) e = count.reserve(n);
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
@@ -688,6 +702,7 @@ struct wbc_handle {
   LoopScratch loop;
   MonScratch mon;
   MotorScratch motor;
+  EstScratch est;
   ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
@@ -1985,7 +2000,7 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
 // Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant; loop: the same with
 // sensing and actuation, on the ground plant; monitor: the loop with the rollout monitor; motor: the monitor entry with the
 // actuator model).
-enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor, motor };
+enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor, motor, estimator };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -2039,11 +2054,13 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
 // applies the actuated torque (wbc_loop.cuh), with the loop state in the handle's scratch when lp->hist is null; mp != nullptr
 // (ground plant): the monitor runs after the plant (wbc_monitor.cuh) on the plant's per-step status word, which it folds into
 // io->status_or; mt != nullptr (ground plant): the motor (wbc_motor.cuh) turns the applied torque into the plant input, with its
-// state in the handle's scratch when mt->tau_m is null, and the monitor sees the motor torque tau_m.
+// state in the handle's scratch when mt->tau_m is null, and the monitor sees the motor torque tau_m; ep != nullptr (with a loop):
+// the estimator (wbc_estimator.cuh) replaces the observed base position and linear velocity in place, with its state in the
+// handle's scratch when ep->x is null, and ORs its status bit into the plant's status word.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                        const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
                        const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr, const wbcmon::MonArgs* mp = nullptr,
-                       const wbcmotor::MotorArgs* mt = nullptr) {
+                       const wbcmotor::MotorArgs* mt = nullptr, const wbcest::EstArgs* ep = nullptr) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -2076,6 +2093,16 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       WBC_CUDA(h, cudaMemsetAsync(ma.count, 0, n * sizeof(long long), st));
     }
   }
+  wbcest::EstArgs ea{};
+  if (ep) {
+    ea = *ep;
+    ea.seed = la.seed; ea.stream = la.stream; ea.tick = la.tick;
+    if (!ea.x) {                                   // a fresh filter state: count 0 (the first step primes it)
+      WBC_CUDA(h, h->est.reserve(n));
+      ea.x = h->est.x.p; ea.P = h->est.P.p; ea.v_prev = h->est.v_prev.p; ea.count = h->est.count.p;
+      WBC_CUDA(h, cudaMemsetAsync(ea.count, 0, n * sizeof(long long), st));
+    }
+  }
   const unsigned loop_grid = (unsigned)((n + 255) / 256);
   // with a monitor the plant ORs each step's status into a word of its own, and writes its forces somewhere in any case
   int32_t* plant_status_or = io->status_or;
@@ -2105,6 +2132,11 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
     if (r) return r;
     if (lp) {
       wbcloop::observe_kernel<<<loop_grid, 256, 0, st>>>(la, n, io->q, io->v, h->loop.q_obs.p, h->loop.v_obs.p);
+      h->launches++;
+    }
+    if (ep) {
+      wbcest::estimate_kernel<<<(unsigned)((n + 3) / 4), wbcest::EST_BLOCK, 0, st>>>(ea, n, io->q, io->v, h->loop.q_obs.p, h->loop.v_obs.p,
+                                                                                  ro.contact.p, plant_status_or);
       h->launches++;
     }
     r = device_step(h, kind, n, &sio, st, false, cp);
@@ -2470,11 +2502,138 @@ extern "C" int wbc_motor_apply_host(wbc_handle* h, int64_t n, double dt, const w
   return rc ? rc : s.finish(h);
 }
 
-// Host buffers of the seven rollouts.
+// ------------------------------------------------------------------------------ state estimator (wbc_estimator.cuh)
+// A set keeps the number of the device its records live on, not its handle: it may be destroyed after the handle.
+struct wbc_estimator_set {
+  int device = 0;
+  int32_t n_sets = 0;
+  DevArray<wbc_estimator_desc> table;
+  ~wbc_estimator_set() { cudaSetDevice(device); }   // the table is freed after this, on the set's device
+};
+
+extern "C" int wbc_estimator_set_destroy(wbc_estimator_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+extern "C" int wbc_estimator_set_create(wbc_handle* h, int32_t n_sets, const wbc_estimator_desc* descs, wbc_estimator_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !descs || n_sets < 1) return fail_arg(h, "wbc_estimator_set_create: descs and n_sets >= 1 are required");
+  *out = nullptr;
+  for (int32_t k = 0; k < n_sets; ++k)
+    if (const char* why = wbcest::desc_problem(descs[k])) return fail_arg(h, why);
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_estimator_set> es(new (std::nothrow) wbc_estimator_set());
+  if (!es) return WBC_ERR_NOMEM;
+  es->device = h->device;
+  es->n_sets = n_sets;
+  WBC_CUDA(h, es->table.reserve((size_t)n_sets));
+  WBC_CUDA(h, cudaMemcpy(es->table.p, descs, (size_t)n_sets * sizeof(wbc_estimator_desc), cudaMemcpyHostToDevice));
+  *out = es.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of an estimator whose arrays are already on the device (x / P / v_prev / count may all be null); the
+// loop's seed, stream and tick are filled in by the caller.
+static int est_args(wbc_handle* h, const wbc_estimator* e, double dt, wbcest::EstArgs* ea) {
+  const int given = (e->x != nullptr) + (e->P != nullptr) + (e->v_prev != nullptr) + (e->count != nullptr);
+  if (given != 0 && given != 4) return fail_arg(h, "wbc_estimator: x, P, v_prev and count are given together or not at all");
+  const wbc_estimator_set* set = e->set;
+  if (!set) return fail_arg(h, "wbc_estimator: a set is required");
+  if (set->device != h->device) return fail_arg(h, "wbc_estimator: the set lives on another device than the handle");
+  *ea = wbcest::EstArgs{};
+  ea->set = set->table.p; ea->index = e->index; ea->n_sets = set->n_sets; ea->accel_noise = e->accel_noise;
+  ea->x = e->x; ea->P = e->P; ea->v_prev = e->v_prev; ea->count = (long long*)e->count; ea->stats = e->stats;
+  ea->dt = dt;
+  const wbc_model& m = h->model;
+  for (int c = 0; c < 3; ++c) ea->gravity[c] = m.gravity[c];
+  for (int k = 0; k < WBC_NU; ++k) {
+    ea->v_index[k] = m.v_index[k];
+    for (int c = 0; c < 3; ++c) { ea->joint_xyz[k][c] = m.joint_xyz[k][c]; ea->joint_axis[k][c] = m.joint_axis[k][c]; }
+  }
+  for (int l = 0; l < WBC_NLEG; ++l)
+    for (int c = 0; c < 3; ++c) ea->foot_xyz[l][c] = m.foot_xyz[l][c];
+  return WBC_OK;
+}
+
+extern "C" int wbc_rollout_estimator(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                     const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                     const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                     const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est, void* stream) {
+  if (!est) return wbc_rollout_motor(h, kind, plan, n, n_steps, dt, io, opts, perturb, terrain, ctrl, loop, mon, motor, stream);
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_estimator: bad arguments");
+  if (!(opts && opts->plant == 1)) return fail_arg(h, "wbc_rollout_estimator: the estimator runs in the ground-plant loop (opts->plant = 1)");
+  if (!loop) return fail_arg(h, "wbc_rollout_estimator: the estimator needs a loop (its observed state, seed, streams and ticks)");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  wbcloop::LoopArgs la;
+  wbcmon::MonArgs ma;
+  wbcmotor::MotorArgs mt;
+  wbcest::EstArgs ea;
+  int rc = est_args(h, est, dt, &ea);
+  if (!rc && motor) rc = motor_args(h, motor, dt, &mt);
+  if (!rc && mon) rc = mon_args(h, mon, n, dt, &ma);
+  if (!rc) rc = loop_args(h, loop, &la);
+  if (!rc) rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && (perturb || terrain))
+    rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, (perturb || terrain) ? &pa : nullptr, terrain ? &ta : nullptr,
+                               (cudaStream_t)stream, &cp, &la, mon ? &ma : nullptr, motor ? &mt : nullptr, &ea);
+}
+
+extern "C" int wbc_estimator_step(wbc_handle* h, int64_t n, double dt, const wbc_estimator* est, const wbc_loop* loop, const double* q,
+                                  const double* v, double* q_obs, double* v_obs, const uint8_t* contact, int32_t* status_or, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!est || n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_estimator_step: est, n >= 0 and dt > 0 are required");
+  if (n > 0 && (!q || !v || !q_obs || !v_obs || !contact || !est->x))
+    return fail_arg(h, "wbc_estimator_step: q, v, q_obs, v_obs, contact and the filter state x, P, v_prev, count are required");
+  wbcest::EstArgs ea;
+  int rc = est_args(h, est, dt, &ea);
+  wbcloop::LoopArgs la;
+  if (!rc) rc = loop_args(h, loop, &la);
+  if (rc || n == 0) return rc;
+  ea.seed = la.seed; ea.stream = la.stream; ea.tick = la.tick;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  wbcest::estimate_kernel<<<(unsigned)((n + 3) / 4), wbcest::EST_BLOCK, 0, (cudaStream_t)stream>>>(ea, n, q, v, q_obs, v_obs, contact,
+                                                                                                   status_or);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Device copies of a host wbc_estimator's arrays; the filter state and the statistics are copied in and out.
+static wbc_estimator est_to_device(DevScratch& s, const wbc_estimator& e, size_t N) {
+  return wbc_estimator{e.set, s.in(e.index, N), s.in(e.accel_noise, N), s.inout(e.x, N * wbcest::NX),
+                       s.inout(e.P, N * wbcest::NX * wbcest::NX), s.inout(e.v_prev, N * 3), s.inout(e.count, N), s.inout(e.stats, N * 4)};
+}
+
+extern "C" int wbc_estimator_step_host(wbc_handle* h, int64_t n, double dt, const wbc_estimator* est, const wbc_loop* loop,
+                                       const double* q, const double* v, double* q_obs, double* v_obs, const uint8_t* contact,
+                                       int32_t* status_or) {
+  if (!h) return WBC_ERR_ARG;
+  if (!est || n <= 0) return n == 0 && est ? WBC_OK : fail_arg(h, "wbc_estimator_step_host: est and n >= 0 are required");
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  DevScratch s(h->lane[0]);
+  const size_t N = (size_t)n;
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV);
+  double* dqo = s.inout(q_obs, N * WBC_NQ); double* dvo = s.inout(v_obs, N * WBC_NV);
+  const uint8_t* dc = s.in(contact, N * WBC_NLEG); int32_t* dst = s.inout(status_or, N);
+  const wbc_estimator de = est_to_device(s, *est, N);
+  wbc_loop dl{};
+  if (loop) dl = loop_to_device(s, *loop, N);
+  WBC_SCRATCH_CHECK(h, s);
+  const int rc = wbc_estimator_step(h, n, dt, &de, loop ? &dl : nullptr, dq, dv, dqo, dvo, dc, dst, s.st);
+  return rc ? rc : s.finish(h);
+}
+
+// Host buffers of the eight rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                         const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
                         const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr, const wbc_monitor* mon = nullptr,
-                        const wbc_plant_motor* motor = nullptr) {
+                        const wbc_plant_motor* motor = nullptr, const wbc_estimator* est = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -2502,9 +2661,15 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (mon) dm = monitor_to_device(s, *mon, N);
   wbc_plant_motor dmt{};
   if (motor) dmt = motor_to_device(s, *motor, N);
+  wbc_estimator de{};
+  if (est) de = est_to_device(s, *est, N);
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::motor ? wbc_rollout_motor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
+      entry == PlantEntry::estimator
+          ? wbc_rollout_estimator(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, terrain ? &dtr : nullptr,
+                                  ctrl ? &dcp : nullptr, loop ? &dl : nullptr, mon ? &dm : nullptr, motor ? &dmt : nullptr,
+                                  est ? &de : nullptr, s.st)
+      : entry == PlantEntry::motor ? wbc_rollout_motor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
                                                      terrain ? &dtr : nullptr, ctrl ? &dcp : nullptr, loop ? &dl : nullptr,
                                                      mon ? &dm : nullptr, motor ? &dmt : nullptr, s.st)
       : entry == PlantEntry::monitor ? wbc_rollout_monitor(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr,
@@ -2561,6 +2726,13 @@ extern "C" int wbc_rollout_motor_host(wbc_handle* h, int kind, const wbc_plan* p
                                       const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
                                       const wbc_monitor* mon, const wbc_plant_motor* motor) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::motor, perturb, terrain, ctrl, loop, mon, motor);
+}
+
+extern "C" int wbc_rollout_estimator_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                          const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                          const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                          const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::estimator, perturb, terrain, ctrl, loop, mon, motor, est);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

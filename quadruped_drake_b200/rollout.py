@@ -34,6 +34,12 @@ its command through a first-order lag, saturates on a torque-speed envelope, and
 (semantics in include/wbc.h, wbc_motor_desc). A `MotorSet` holds the records; without one every motor saturates at the URDF
 effort. It runs through `wbc_rollout_motor`, together with any monitor, loop, variants, pushes, terrain and parameter sets;
 `motor_apply` runs the motor alone.
+
+State estimation (`estimator`, an `Estimator`; with a loop only): each robot's controller reads the base position and linear
+velocity of a linear Kalman filter that fuses a synthesised accelerometer with leg kinematics, instead of observed ones
+(semantics in include/wbc.h, wbc_estimator). An `EstimatorSet` holds the records (`estimator_desc`), an `EstimatorState` the
+per-robot filter. It runs through `wbc_rollout_estimator`, together with any motor, monitor, variants, pushes, terrain and
+parameter sets; `estimator_step` runs the filter alone.
 """
 from __future__ import annotations
 
@@ -43,8 +49,8 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import capi
-from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcLoop, WbcMonitor, WbcMotorDesc, WbcPlantMotor, WbcPlantOpts,
-                   WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
+from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcEstimator, WbcEstimatorDesc, WbcLoop, WbcMonitor, WbcMotorDesc,
+                   WbcPlantMotor, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
 from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
@@ -423,8 +429,153 @@ def motor_apply(ctl, v, tau, motor, dt=5e-3):
     return out, status
 
 
+# Defaults in the spirit of the linear Kalman filter of the open-source MIT Cheetah software (oracle/estimator.py); not measured.
+ESTIMATOR_DEFAULTS = dict(q_pos=0.02, q_vel=0.1, q_foot=0.02, r_pos=0.002, r_vel=0.05, r_height=0.005, swing_scale=100.0, p0_pos=0.01,
+                          p0_vel=0.1, p0_foot=0.01)
+
+
+def estimator_desc(**kw):
+    """One estimator record (WbcEstimatorDesc): ESTIMATOR_DEFAULTS with the given fields replaced. Process stds q_pos (m/sqrt(s)),
+    q_vel (m/s/sqrt(s)), q_foot (m/sqrt(s)); measurement stds r_pos (m), r_vel (m/s), r_height (m), +inf drops those rows;
+    swing_scale >= 1 multiplies the stds of a foot planned in swing; p0_pos, p0_vel, p0_foot the stds of the prime."""
+    vals = dict(ESTIMATOR_DEFAULTS)
+    for k, x in kw.items():
+        if k not in vals:
+            raise TypeError(f"estimator_desc: unknown field {k!r}")
+        vals[k] = float(x)
+    return WbcEstimatorDesc(**vals)
+
+
+class EstimatorSet:
+    """Device-resident table of K estimator records (wbc_estimator_set_create); robot i's filter uses descs[index[i]]."""
+
+    def __init__(self, ctl, descs):
+        self.ctl, self.lib = ctl, ctl.lib
+        self.n_sets = len(descs)
+        arr = (WbcEstimatorDesc * self.n_sets)(*descs)
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_estimator_set_create(ctl._h, self.n_sets, arr, C.byref(self._p)), "wbc_estimator_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_estimator_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+_EST_FIELDS = (("x", np.float64, (18,)), ("P", np.float64, (18, 18)), ("v_prev", np.float64, (3,)), ("count", np.int64, ()),
+               ("stats", np.float64, (4,)))
+
+
+class EstimatorState:
+    """The filter state of N robots: x [N,18] (base position, base velocity, feet LF RF LH RH; world), P [N,18,18], v_prev [N,3],
+    count [N] int64 (0: the next step primes the filter) and stats [N,4] (sum |p err|^2, max |p err|, sum |v err|^2, max |v err|);
+    all zero. NumPy arrays, or torch tensors on the device of `like`. A rollout given a state continues it and leaves it advanced."""
+
+    def __init__(self, n, like=None):
+        for name, dtype, width in _EST_FIELDS:
+            if like is not None and _is_torch(like):
+                import torch
+                x = torch.zeros((n, *width), dtype={np.float64: torch.float64, np.int64: torch.int64}[dtype], device=like.device)
+            else:
+                x = np.zeros((n, *width), dtype)
+            setattr(self, name, x)
+
+    rms_pos = property(lambda s: (s.stats[:, 0] / s.count) ** 0.5)
+    max_pos = property(lambda s: s.stats[:, 1])
+    rms_vel = property(lambda s: (s.stats[:, 2] / s.count) ** 0.5)
+    max_vel = property(lambda s: s.stats[:, 3])
+
+
+@dataclass
+class Estimator:
+    """Per-robot state estimation of the ground-plant loop. set: an EstimatorSet (required); index [N] int32 record of each robot
+    (None: record 0); accel_noise [N] accelerometer noise std in m/s^2 (None: none); state: an EstimatorState to continue (None:
+    each call primes a fresh filter in library scratch, and keeps no statistics)."""
+    set: EstimatorSet
+    index: object = None
+    accel_noise: object = None
+    state: EstimatorState | None = None
+
+
+def _estimator_arrays(est, n, dev=None):
+    """(index, accel_noise, state) of an Estimator in the layouts of the C ABI, checked: index and accel_noise broadcast to N rows
+    (host copies, or on `dev` torch tensors checked, not converted), the state as given."""
+    if not isinstance(est.set, EstimatorSet):
+        raise ValueError("estimator.set must be an EstimatorSet")
+    st = est.state
+    if dev is not None:
+        check_device_index(est.index, n, "estimator.index")
+        if est.accel_noise is not None:
+            check_device_array(est.accel_noise, (n,), np.float64, "estimator.accel_noise")
+        if st is not None:
+            for name, dtype, width in _EST_FIELDS:
+                check_device_array(getattr(st, name), (n, *width), dtype, f"estimator.state.{name}")
+        return est.index, est.accel_noise, st
+    if st is not None:
+        for name, dtype, width in _EST_FIELDS:
+            x = getattr(st, name)
+            if not (isinstance(x, np.ndarray) and x.dtype == dtype and x.shape == (n, *width) and x.flags.c_contiguous):
+                raise ValueError(f"estimator.state.{name} must be a contiguous host array {np.dtype(dtype).name}{[n, *width]}")
+    an = None if est.accel_noise is None else np.ascontiguousarray(np.broadcast_to(np.asarray(est.accel_noise, np.float64), (n,)))
+    return _terrain_index(n, est.index), an, st
+
+
+def _wbc_estimator(est, idx, an, st, ptr):
+    s = (None,) * 5 if st is None else tuple(ptr(getattr(st, name)) for name, _, _ in _EST_FIELDS)
+    return WbcEstimator(est.set._p, ptr(idx), ptr(an), *s)
+
+
+def estimator_step(ctl, q, v, q_obs, v_obs, contact, estimator, loop=None, dt=5e-3):
+    """The estimator alone on one step (wbc_estimator_step) -> (q_obs, v_obs, status_or [N] int32: ST_BADESTIM for a bad index or
+    a failed step). q [N,19], v [N,18] the true state at the start of the step; q_obs, v_obs what the loop observed (the returned
+    arrays carry the estimate in [4:7] and [3:6]); contact [N,4] uint8 the planned stance flags; loop gives the seed, streams and
+    ticks (read, not advanced; None: seed 0, row streams, tick 0). estimator.state is required and advanced. Host arrays go
+    through the host entry (q_obs, v_obs copied); torch CUDA tensors stay on the device and q_obs, v_obs are updated in place."""
+    if estimator.state is None:
+        raise ValueError("estimator_step: estimator.state is required (an EstimatorState)")
+    if _is_torch(q):
+        import torch
+        n, dev = q.shape[0], q.device
+        check_device_array(q, (n, NQ), np.float64, "q")
+        check_device_array(v, (n, NV), np.float64, "v")
+        check_device_array(q_obs, (n, NQ), np.float64, "q_obs")
+        check_device_array(v_obs, (n, NV), np.float64, "v_obs")
+        if not (_is_torch(contact) and contact.is_cuda and contact.is_contiguous() and contact.dtype == torch.uint8
+                and tuple(contact.shape) == (n, 4)):
+            raise ValueError("contact on the device must be a contiguous CUDA tensor uint8[N, 4]")
+        idx, an, st = _estimator_arrays(estimator, n, dev)
+        arrays = None if loop is None else _loop_arrays(loop, n, dev)      # (kept alive for the call)
+        p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        status = torch.zeros(n, dtype=torch.int32, device=dev)
+        es = _wbc_estimator(estimator, idx, an, st, p)
+        lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, p))
+        ctl._check(ctl.lib.wbc_estimator_step(ctl._h, n, float(dt), C.byref(es), lp, p(q), p(v), p(q_obs), p(v_obs), p(contact), p(status),
+                                              C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "wbc_estimator_step")
+        return q_obs, v_obs, status
+    q = np.ascontiguousarray(q, dtype=np.float64).reshape(-1, NQ)
+    n = len(q)
+    v = np.ascontiguousarray(v, dtype=np.float64).reshape(n, NV)
+    qo, vo = np.array(q_obs, dtype=np.float64).reshape(n, NQ), np.array(v_obs, dtype=np.float64).reshape(n, NV)
+    ct = np.ascontiguousarray(contact, dtype=np.uint8).reshape(n, 4)
+    idx, an, st = _estimator_arrays(estimator, n)
+    arrays = None if loop is None else _loop_arrays(loop, n)
+    opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
+    status = np.zeros(n, np.int32)
+    es = _wbc_estimator(estimator, idx, an, st, opt)
+    lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, opt))
+    ctl._check(ctl.lib.wbc_estimator_step_host(ctl._h, n, float(dt), C.byref(es), lp, np_ptr(q), np_ptr(v), np_ptr(qo), np_ptr(vo),
+                                               np_ptr(ct), np_ptr(status)), "wbc_estimator_step_host")
+    return qo, vo, status
+
+
 class RolloutResult:
-    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why")
+    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why", "estimator")
 
     def __init__(self, **kw):
         for k in self.__slots__:
@@ -437,7 +588,7 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
             mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
-            param_index=None, loop=None, monitor=None, motor=None) -> RolloutResult:
+            param_index=None, loop=None, monitor=None, motor=None, estimator=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -455,7 +606,12 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     carries `monitor` (its MonitorState, advanced) and `why` [N] int32, the failure reasons at the last step.
     Actuator model (plant=True only): motor (a Motor) puts each robot's motors between the actuated torque and the plant; `tau`
     stays the last COMMANDED torque, and a monitor sees the motor torque. A robot with a bad record index is flagged ST_BADMOTOR
-    and gets zero torque."""
+    and gets zero torque.
+    State estimation (plant=True and a loop only): estimator (an Estimator) gives each robot's controller the filter's base
+    position and linear velocity; the result then carries `estimator` (its EstimatorState, advanced, or None). A robot with a bad
+    record index or a failed filter step is controlled from the observed state and flagged ST_BADESTIM."""
+    if estimator is not None and (loop is None or not plant):
+        raise ValueError("rollout: an estimator needs loop= (its observed state, seed, streams and ticks) and plant=True")
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     per_robot = param_set is not None or param_index is not None
@@ -470,7 +626,8 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if monitor is not None or motor is not None:
+        if monitor is not None or motor is not None or estimator is not None:
+            ea = None if estimator is None else _estimator_arrays(estimator, n, dev)
             if monitor is not None:
                 r.monitor, r.why = _monitor_state(monitor, n, q), mk((n,), torch.int32)
             arrays = None if loop is None else _loop_arrays(loop, n, dev)      # (kept alive for the call)
@@ -480,7 +637,13 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
             cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))) if per_robot else None
             lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, p))
             mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, p))
-            if motor is None:
+            if estimator is not None:
+                mt = None if motor is None else C.byref(_wbc_motor(motor, *_motor_arrays(motor, n, dev), p))
+                es = C.byref(_wbc_estimator(estimator, *ea, p))
+                r.estimator = estimator.state
+                ctl._check(ctl.lib.wbc_rollout_estimator(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt,
+                                                         tr, cp, lp, mo, mt, es, stream), "wbc_rollout_estimator")
+            elif motor is None:
                 ctl._check(ctl.lib.wbc_rollout_monitor(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
                                                        cp, lp, mo, stream), "wbc_rollout_monitor")
             else:
@@ -525,7 +688,8 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if monitor is not None or motor is not None:
+    if monitor is not None or motor is not None or estimator is not None:
+        ea = None if estimator is None else _estimator_arrays(estimator, n)      # (kept alive for the call)
         if monitor is not None:
             r.monitor, r.why = _monitor_state(monitor, n), np.zeros(n, np.int32)
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
@@ -536,7 +700,14 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))) if per_robot else None
         lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, opt))
         mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, opt))
-        if motor is None:
+        if estimator is not None:
+            mi, ms = (None, None) if motor is None else _motor_arrays(motor, n)      # (kept alive for the call)
+            mt = None if motor is None else C.byref(_wbc_motor(motor, mi, ms, opt))
+            es = C.byref(_wbc_estimator(estimator, *ea, opt))
+            r.estimator = estimator.state
+            ctl._check(ctl.lib.wbc_rollout_estimator_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt,
+                                                          tr, cp, lp, mo, mt, es), "wbc_rollout_estimator_host")
+        elif motor is None:
             ctl._check(ctl.lib.wbc_rollout_monitor_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt, tr,
                                                         cp, lp, mo), "wbc_rollout_monitor_host")
         else:
