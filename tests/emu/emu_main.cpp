@@ -10,7 +10,7 @@ thread_local EmuWarp* emu_warp;
 
 namespace {
 struct Job {
-  EmuWarp* warp; int lane; wbc::WarpSmem* sm; wbc::SolveSmemVd* ssm; double* rec; double* vdmap; wbc::PcSmem* pcs; double* Cout; double* Jdout; const wbc_model* md; const wbc_params* pr; wbc::Derived dv;
+  EmuWarp* warp; int lane; wbc::WarpSmem* sm; wbc::SolveSmemVd* ssm; wbc::SolveSmem* ssm0; double* rec; double* vdmap; wbc::PcSmem* pcs; double* Cout; double* Jdout; const wbc_model* md; const wbc_params* pr; wbc::Derived dv;
   wbc::StepArgs args; wbc::DynOut dyn; const double* q; const double* v; long long n; int mode;
   wbcplant::PlantSmem* psm; wbcplant::PlantArgs pargs;
 };
@@ -21,9 +21,17 @@ template <int KIND> void split_step(Job* j, long long i) {
   __syncwarp();
   if (j->lane == 0) memcpy(j->rec, &j->sm->Y[0][0], sizeof(double) * wbc::REC_Y);
   __syncwarp();
-  if (j->lane == 0) memcpy(&j->ssm->Y[0][0], j->rec, sizeof(double) * wbc::REC_Y);
-  __syncwarp();
-  wbc::solve_instance<KIND, wbc::SolveSmemVd>(*j->ssm, *j->md, *j->pr, j->args, i, j->lane, c, vd, j->rec);
+  // the solve kernel variant launch_split picks: with vd, L kept beside R^-1 (SolveSmemVd) and the x recovery from the
+  // record; without, R^-1 overlaid on L (SolveSmem), no acceleration maps and no record read-back
+  if (vd) {
+    if (j->lane == 0) memcpy(&j->ssm->Y[0][0], j->rec, sizeof(double) * wbc::REC_Y);
+    __syncwarp();
+    wbc::solve_instance<KIND, wbc::SolveSmemVd>(*j->ssm, *j->md, *j->pr, j->args, i, j->lane, c, vd, j->rec);
+  } else {
+    if (j->lane == 0) memcpy(&j->ssm0->Y[0][0], j->rec, sizeof(double) * wbc::REC_Y);
+    __syncwarp();
+    wbc::solve_instance<KIND, wbc::SolveSmem>(*j->ssm0, *j->md, *j->pr, j->args, i, j->lane, c);
+  }
   __syncwarp();
 }
 void* lane_main(void* p) {
@@ -55,13 +63,15 @@ int run(Job proto) {
   memset(pcs, 0, sizeof(*pcs));
   wbc::SolveSmemVd* ssm = new wbc::SolveSmemVd();
   memset(ssm, 0, sizeof(*ssm));
+  wbc::SolveSmem* ssm0 = new wbc::SolveSmem();
+  memset(ssm0, 0, sizeof(*ssm0));
   wbcplant::PlantSmem* psm = new wbcplant::PlantSmem();
   memset(psm, 0, sizeof(*psm));
   std::vector<double> rec(wbc::REC_DOUBLES), vdmap(wbc::VDMAP_DOUBLES);
   std::vector<Job> jobs(32, proto);
   std::vector<pthread_t> th(32);
   for (int l = 0; l < 32; ++l) {
-    jobs[l].warp = &warp; jobs[l].lane = l; jobs[l].sm = sm; jobs[l].pcs = pcs; jobs[l].ssm = ssm; jobs[l].psm = psm; jobs[l].rec = rec.data(); jobs[l].vdmap = vdmap.data();
+    jobs[l].warp = &warp; jobs[l].lane = l; jobs[l].sm = sm; jobs[l].pcs = pcs; jobs[l].ssm = ssm; jobs[l].ssm0 = ssm0; jobs[l].psm = psm; jobs[l].rec = rec.data(); jobs[l].vdmap = vdmap.data();
     pthread_create(&th[l], nullptr, lane_main, &jobs[l]);
   }
   for (int l = 0; l < 32; ++l) pthread_join(th[l], nullptr);
@@ -69,6 +79,7 @@ int run(Job proto) {
   delete sm;
   delete pcs;
   delete ssm;
+  delete ssm0;
   delete psm;
   return 0;
 }

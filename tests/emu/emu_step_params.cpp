@@ -11,7 +11,7 @@ thread_local EmuWarp* emu_warp;
 
 namespace {
 struct Lane {
-  EmuWarp* warp; int lane; wbc::WarpSmem* sm; wbc::SolveSmemVd* ssm; wbc::PcSmem* pcs; double* rec; double* vdmap;
+  EmuWarp* warp; int lane; wbc::WarpSmem* sm; wbc::SolveSmemVd* ssm; wbc::SolveSmem* ssm0; wbc::PcSmem* pcs; double* rec; double* vdmap;
   const wbc_model* md; wbc::ParamArgs p; wbc::StepArgs a;
 };
 template <int KIND> void step(Lane* j, long long i) {
@@ -24,12 +24,15 @@ template <int KIND> void step(Lane* j, long long i) {
   __syncwarp();
   if (j->lane == 0) memcpy(j->rec, &j->sm->Y[0][0], sizeof(double) * wbc::REC_Y);
   __syncwarp();
-  if (j->lane == 0) memcpy(&j->ssm->Y[0][0], j->rec, sizeof(double) * wbc::REC_Y);
+  double* const ybuf = vd ? &j->ssm->Y[0][0] : &j->ssm0->Y[0][0];
+  if (j->lane == 0) memcpy(ybuf, j->rec, sizeof(double) * wbc::REC_Y);
   __syncwarp();
   int sstatus = 0;                 // the solve kernel selects the record again from the index
   const wbc::ParamRec& rs = wbc::param_record(j->p, i, sstatus);
   c.status |= sstatus;
-  wbc::solve_instance<KIND, wbc::SolveSmemVd>(*j->ssm, *j->md, rs.pr, j->a, i, j->lane, c, vd, j->rec);
+  // the variant the launch picks: SolveSmemVd (L kept, x recovered from the record) only when vd is requested
+  if (vd) wbc::solve_instance<KIND, wbc::SolveSmemVd>(*j->ssm, *j->md, rs.pr, j->a, i, j->lane, c, vd, j->rec);
+  else wbc::solve_instance<KIND, wbc::SolveSmem>(*j->ssm0, *j->md, rs.pr, j->a, i, j->lane, c);
   __syncwarp();
 }
 void* lane_main(void* p) {
@@ -68,11 +71,13 @@ extern "C" int emu_step_params(const wbc_model* md, const wbc_params* params, in
   memset(pcs, 0, sizeof(*pcs));
   wbc::SolveSmemVd* ssm = new wbc::SolveSmemVd();
   memset(ssm, 0, sizeof(*ssm));
+  wbc::SolveSmem* ssm0 = new wbc::SolveSmem();
+  memset(ssm0, 0, sizeof(*ssm0));
   std::vector<double> rec(wbc::REC_DOUBLES), vdmap(wbc::VDMAP_DOUBLES);
   std::vector<Lane> lanes(32);
   std::vector<pthread_t> th(32);
   for (int l = 0; l < 32; ++l) {
-    lanes[l] = Lane{&warp, l, sm, ssm, pcs, rec.data(), vdmap.data(), md, p, a};
+    lanes[l] = Lane{&warp, l, sm, ssm, ssm0, pcs, rec.data(), vdmap.data(), md, p, a};
     pthread_create(&th[l], nullptr, lane_main, &lanes[l]);
   }
   for (int l = 0; l < 32; ++l) pthread_join(th[l], nullptr);
@@ -80,5 +85,6 @@ extern "C" int emu_step_params(const wbc_model* md, const wbc_params* params, in
   delete sm;
   delete pcs;
   delete ssm;
+  delete ssm0;
   return 0;
 }
