@@ -74,6 +74,7 @@ extern "C" {
 #define WBC_ST_BADLOOP 4096    /* wbc_rollout_loop only: bad loop profile; observed without noise, zero applied torque  */
 #define WBC_ST_BADMOTOR 8192   /* wbc_rollout_motor / wbc_motor_apply only: motor record index out of range; zero torque */
 #define WBC_ST_BADESTIM 16384  /* wbc_rollout_estimator / wbc_estimator_step only: bad record index or failed filter step   */
+#define WBC_ST_BADCONTACT 32768 /* wbc_rollout_contact / wbc_contact_step only: bad record index or non-finite force estimate */
 
 /* controller kinds: reference controllers/__init__.py:1-5 */
 #define WBC_CTRL_ID 0          /* controllers/inverse_dynamics_controller.py */
@@ -794,6 +795,91 @@ int wbc_estimator_step(wbc_handle* h, int64_t n, double dt, const wbc_estimator*
                        const double* v, double* q_obs, double* v_obs, const uint8_t* contact, int32_t* status_or, void* stream);
 int wbc_estimator_step_host(wbc_handle* h, int64_t n, double dt, const wbc_estimator* est, const wbc_loop* loop, const double* q,
                             const double* v, double* q_obs, double* v_obs, const uint8_t* contact, int32_t* status_or);
+
+/* ---- Contact detection in the ground-plant loop: per robot, each foot's ground force is estimated from the joint torques and
+ * the motion they produced, and a hysteresis on its world-z component gives the foot's stance flag. The estimator and the
+ * controller may read the detected flags instead of the planned ones. Each step is
+ * sample plan -> observe -> detect -> estimate -> controller -> actuate -> motor -> ground plant -> record -> monitor.
+ *
+ * Robot i has the state q_prev[i][19], v_prev[i][18] (what the detector read at its previous step), tau_prev[i][12] (the measured
+ * torque of its latest step, actuator order), f_true[i][12] (the plant's ground forces of its latest step, statistics only),
+ * f_hat[i][12] (filtered force, world axes, foot k at 3 k), flag[i][4] and count[i], and uses record r = set[index[i]]. At each step
+ * it reads q, v: the loop's observed state (before the estimator overwrites it) with a loop, the true state without one.
+ *   prime     (count <= 0) flag = the plan's flags, f_hat = 0, q_prev = q, v_prev = v, count = 1
+ *   estimate  M, Cv + tau_g (controller sign) and the foot Jacobians J_k taken at q_prev, v_prev with the handle's model; per leg k
+ *             the three joint rows of  r = M (v - v_prev) - dt (B tau_prev - Cv - tau_g)  give r_k, and  J_k,leg' p_k = r_k
+ *             (J_k,leg the 3 x 3 block of J_k over leg k's joint columns) gives f_raw,k = p_k / dt in world axes.
+ *             The plant's step is v+ = v + dt M^-1 (B tau - Cv - tau_g) + M^-1 (J_c' p + push), with a push on base rows only,
+ *             so with the true state and the torque the plant received, f_raw reproduces the plant's f_contact up to rounding.
+ *   singular  |det J_k,leg| <= 1e-9 |a0| |a1| |a2|, a_j the columns of J_k,leg: f_hat and flag of that foot are held and it adds
+ *             nothing to the statistics of the step
+ *   filter    f_hat = f_raw on the first estimate after a prime (count == 1) or with tau_f = 0, else
+ *             f_hat += alpha (f_raw - f_hat), alpha = -expm1(-dt / tau_f)
+ *   flags     a foot at 0 goes to 1 when f_hat_z >= f_on; a foot at 1 goes to 0 when f_hat_z <= f_off
+ *   stats     (optional, [N][6], accumulated) sum over estimated steps of sum_k |f_raw,k - f_true,k|^2, the maximum over steps and
+ *             feet of |f_raw,k - f_true,k|, then per foot and step the counts of true stance (flag 1, loaded), true swing (0, not
+ *             loaded), false stance (1, not loaded) and false swing (0, loaded); a foot is loaded when any component of its
+ *             f_true is non-zero (the monitor's rule). f_true is the previous step's: the forces of the step that led to q, v.
+ *   then      q_prev = q, v_prev = v, count += 1
+ *   failure   a non-finite f_raw of a foot that is not singular: count = 0, everything else unchanged, WBC_ST_BADCONTACT
+ *   bad index (< 0 or >= K) WBC_ST_BADCONTACT, nothing changes (the record step leaves the robot alone too)
+ * A failed or bad robot outputs the plan's flags for the step. WBC_ST_BADCONTACT goes into the word the plant ORs its own status
+ * into, as WBC_ST_BADESTIM does; no plant freeze mask holds it.
+ * After the plant, the record step copies the measured torque (the motor torque tau_m with a motor - joint friction is not
+ * measured -, else the actuated torque with a loop, else the command: the torque the monitor treats as applied) into tau_prev and
+ * the plant's forces into f_true, so that the state carries everything a later call needs.
+ *
+ * Consumers (feed, a mask): WBC_CONTACT_FEED_ESTIMATOR - the estimator's s_k uses the detected flags instead of the planned ones
+ * (WBC_ERR_ARG without an estimator); WBC_CONTACT_FEED_CONTROLLER - the controller's contact input is plan AND detected, so that a
+ * late touchdown waits and a slipping or unloaded planned-stance foot carries no QP force, while a loaded foot is still released
+ * to swing at lift-off. feed = 0 only observes. The monitor reads the planned flags in every mode.
+ *
+ * Record fields: tau_f (s) finite and >= 0; f_on, f_off (N) not NaN with f_off <= f_on (+-inf allowed: f_off = -inf never
+ * releases a detected foot). Anything else is WBC_ERR_ARG at creation. */
+#define WBC_CONTACT_FEED_ESTIMATOR 1
+#define WBC_CONTACT_FEED_CONTROLLER 2
+typedef struct wbc_contact_desc {
+  double tau_f, f_on, f_off;
+} wbc_contact_desc;
+/* A contact set keeps its device number and may outlive the handle. n_sets >= 1. */
+typedef struct wbc_contact_set wbc_contact_set;
+int wbc_contact_set_create(wbc_handle* h, int32_t n_sets, const wbc_contact_desc* descs, wbc_contact_set** out);
+int wbc_contact_set_destroy(wbc_contact_set* s);
+
+typedef struct wbc_contact {
+  const wbc_contact_set* set;    /* required                                                                                  */
+  const int32_t* index;          /* [N] record of each robot, NULL = record 0                                                 */
+  int32_t feed;                  /* WBC_CONTACT_FEED_* mask                                                                   */
+  double* q_prev;                /* [N][19], v_prev [N][18], tau_prev [N][12], f_true [N][12], f_hat [N][12], flag [N][4] and */
+  double* v_prev;                /* count [N]: all given (in/out) or all NULL (library scratch, count 0: each call starts with */
+  double* tau_prev;              /* a prime); anything between is WBC_ERR_ARG                                                 */
+  double* f_true;
+  double* f_hat;
+  uint8_t* flag;
+  int64_t* count;
+  double* stats;                 /* [N][6] or NULL (accumulated, see above)                                                   */
+} wbc_contact;
+
+/* wbc_rollout_estimator (opts->plant must be 1; loop, est, motor, mon, perturb, terrain and ctrl may each be NULL) with the
+ * detector after observe and the record step after the plant: two more launches per step, captured into the same graph.
+ * det == NULL is wbc_rollout_estimator (its bits and launch count). Without opts->f_contact the plant's forces go to scratch.
+ * Device pointers (host pointers for _host; the detector state and stats are copied in and out). */
+int wbc_rollout_contact(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                        const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                        const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est, const wbc_contact* det,
+                        void* stream);
+int wbc_rollout_contact_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                             const wbc_rollout_io* host_io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                             const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                             const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est, const wbc_contact* det);
+/* The detector alone on one step: q [N][19], v [N][18] (what it reads), contact [N][4] (the plan's flags) -> detected [N][4];
+ * status_or [N] (or NULL) gets WBC_ST_BADCONTACT ORed in. tau_prev and f_true are read from the state, which is required;
+ * det->feed is ignored. */
+int wbc_contact_step(wbc_handle* h, int64_t n, double dt, const wbc_contact* det, const double* q, const double* v,
+                     const uint8_t* contact, uint8_t* detected, int32_t* status_or, void* stream);
+int wbc_contact_step_host(wbc_handle* h, int64_t n, double dt, const wbc_contact* det, const double* q, const double* v,
+                          const uint8_t* contact, uint8_t* detected, int32_t* status_or);
 
 /* Number of kernel launches issued through this handle since creation. */
 int64_t wbc_launch_count(const wbc_handle* h);

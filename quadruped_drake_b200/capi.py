@@ -27,7 +27,11 @@ ST_BADPARAMS = 2048
 ST_BADLOOP = 4096
 ST_BADMOTOR = 8192
 ST_BADESTIM = 16384
+ST_BADCONTACT = 32768
 LOOP_HIST = 16
+# contact detector (include/wbc.h, wbc_contact): consumers of the detected flags, and the columns of its per-robot stats
+CONTACT_FEED_ESTIMATOR, CONTACT_FEED_CONTROLLER = 1, 2
+CONTACT_NSTAT = 6
 # rollout monitor (include/wbc.h, wbc_monitor): failure reasons and the columns of its per-robot stats
 MON_POS, MON_ANG, MON_STATUS = 1, 2, 4
 MON_NSTAT = 11
@@ -38,7 +42,7 @@ _ST_NAMES = {ST_MAXITER: "MAXITER", ST_INFEASIBLE: "INFEASIBLE", ST_RANKDEF: "RA
              ST_BADQUAT: "BADQUAT", ST_UNSUPPORTED: "UNSUPPORTED", ST_DIVERGED: "DIVERGED",
              ST_NONFINITE: "NONFINITE", ST_BADVARIANT: "BADVARIANT", ST_BADTERRAIN: "BADTERRAIN",
              ST_BADPARAMS: "BADPARAMS", ST_BADLOOP: "BADLOOP", ST_BADMOTOR: "BADMOTOR",
-             ST_BADESTIM: "BADESTIM"}
+             ST_BADESTIM: "BADESTIM", ST_BADCONTACT: "BADCONTACT"}
 
 
 def status_names(status: int) -> str:
@@ -151,6 +155,18 @@ class WbcEstimatorDesc(C.Structure):
     """ctypes mirror of `wbc_estimator_desc`: process, measurement and initial standard deviations, and the swing scale."""
     _fields_ = [(name, C.c_double) for name in ("q_pos", "q_vel", "q_foot", "r_pos", "r_vel", "r_height", "swing_scale", "p0_pos",
                                                 "p0_vel", "p0_foot")]
+
+
+class WbcContactDesc(C.Structure):
+    """ctypes mirror of `wbc_contact_desc`: force filter time constant (s) and the stance thresholds f_on >= f_off (N)."""
+    _fields_ = [(name, C.c_double) for name in ("tau_f", "f_on", "f_off")]
+
+
+class WbcContact(C.Structure):
+    """ctypes mirror of `wbc_contact` (set, index [N], feed; the state q_prev [N][19], v_prev [N][18], tau_prev [N][12],
+    f_true [N][12], f_hat [N][12], flag [N][4] and count [N], all or none; stats [N][6] or NULL)."""
+    _fields_ = [("set", C.c_void_p), ("index", C.c_void_p), ("feed", C.c_int32)] + \
+        [(name, C.c_void_p) for name in ("q_prev", "v_prev", "tau_prev", "f_true", "f_hat", "flag", "count", "stats")]
 
 
 class WbcEstimator(C.Structure):
@@ -296,7 +312,20 @@ def load_library() -> C.CDLL:
                                                C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), C.POINTER(WbcEstimator)]
     lib.wbc_estimator_step.argtypes = [H, i64, C.c_double, C.POINTER(WbcEstimator), C.POINTER(WbcLoop)] + [dp] * 7
     lib.wbc_estimator_step_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcEstimator), C.POINTER(WbcLoop)] + [dp] * 6
-    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS:
+    lib.wbc_contact_set_create.argtypes = [H, C.c_int32, C.POINTER(WbcContactDesc), C.POINTER(H)]
+    lib.wbc_contact_set_destroy.argtypes = [dp]
+    lib.wbc_rollout_contact.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                        C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                        C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), C.POINTER(WbcEstimator),
+                                        C.POINTER(WbcContact), dp]
+    lib.wbc_rollout_contact_host.argtypes = [H, i32, dp, i64, C.c_int32, C.c_double, C.POINTER(WbcRolloutIO), C.POINTER(WbcRolloutOpts),
+                                             C.POINTER(WbcPlantPerturb), C.POINTER(WbcPlantTerrain), C.POINTER(WbcCtrlParams),
+                                             C.POINTER(WbcLoop), C.POINTER(WbcMonitor), C.POINTER(WbcPlantMotor), C.POINTER(WbcEstimator),
+                                             C.POINTER(WbcContact)]
+    lib.wbc_contact_step.argtypes = [H, i64, C.c_double, C.POINTER(WbcContact)] + [dp] * 6
+    lib.wbc_contact_step_host.argtypes = [H, i64, C.c_double, C.POINTER(WbcContact)] + [dp] * 5
+    for name in PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS + \
+            CONTACT_SYMBOLS:
         getattr(lib, name).restype = C.c_int
     for name in WIRE_SYMBOLS:
         getattr(lib, name).restype = C.c_int
@@ -335,7 +364,9 @@ MOTOR_SYMBOLS = ["wbc_motor_set_create", "wbc_motor_set_destroy", "wbc_rollout_m
                  "wbc_motor_apply_host"]
 ESTIMATOR_SYMBOLS = ["wbc_estimator_set_create", "wbc_estimator_set_destroy", "wbc_rollout_estimator", "wbc_rollout_estimator_host",
                      "wbc_estimator_step", "wbc_estimator_step_host"]
-TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
+CONTACT_SYMBOLS = ["wbc_contact_set_create", "wbc_contact_set_destroy", "wbc_rollout_contact", "wbc_rollout_contact_host",
+                   "wbc_contact_step", "wbc_contact_step_host"]
+TRAJ_SYMBOLS = ROLLOUT_SYMBOLS + PERTURB_SYMBOLS + TERRAIN_SYMBOLS + PARAM_SYMBOLS + LOOP_SYMBOLS + MONITOR_SYMBOLS + MOTOR_SYMBOLS + ESTIMATOR_SYMBOLS + CONTACT_SYMBOLS + ["wbc_step_plan_host", "wbc_plan_create", "wbc_plan_destroy", "wbc_sample_trajectory", "wbc_sample_trajectory_host"]
 MULTI_SYMBOLS = ["wbc_multi_create", "wbc_multi_destroy", "wbc_multi_last_error", "wbc_multi_device_count", "wbc_multi_launch_count",
                  "wbc_multi_step_host"]
 EXPORTED_SYMBOLS = WIRE_SYMBOLS + TRAJ_SYMBOLS + MULTI_SYMBOLS + ["wbc_default_params", "wbc_create", "wbc_destroy", "wbc_last_error", "wbc_dynamics", "wbc_coriolis",

@@ -30,6 +30,7 @@
 #include "wbc_monitor.cuh"
 #include "wbc_motor.cuh"
 #include "wbc_estimator.cuh"
+#include "wbc_contact.cuh"
 #include <vector>
 
 namespace {
@@ -677,6 +678,29 @@ struct EstScratch {
   }
 };
 
+// Scratch of the contact entries (wbc_rollout_contact), reserved by them only: the detected flags, the controller's flags (plan
+// AND detected), the plant's forces of a call that asks for none, and the detector state of a call that brings none.
+struct ContactScratch {
+  DevArray<uint8_t> detected, ctrl, flag;
+  DevArray<double> f, q_prev, v_prev, tau_prev, f_true, f_hat;
+  DevArray<long long> count;
+  cudaError_t reserve(int64_t n, bool own_f, bool own_state) {
+    cudaError_t e = detected.reserve(n * WBC_NLEG);
+    if (e == cudaSuccess) e = ctrl.reserve(n * WBC_NLEG);
+    if (e == cudaSuccess && own_f) e = f.reserve(n * 12);
+    if (own_state) {
+      if (e == cudaSuccess) e = q_prev.reserve(n * WBC_NQ);
+      if (e == cudaSuccess) e = v_prev.reserve(n * WBC_NV);
+      if (e == cudaSuccess) e = tau_prev.reserve(n * WBC_NU);
+      if (e == cudaSuccess) e = f_true.reserve(n * 12);
+      if (e == cudaSuccess) e = f_hat.reserve(n * 12);
+      if (e == cudaSuccess) e = flag.reserve(n * WBC_NLEG);
+      if (e == cudaSuccess) e = count.reserve(n);
+    }
+    return e;
+  }
+};
+
 }  // namespace
 
 constexpr int WBC_NSLOT = 4;
@@ -703,6 +727,7 @@ struct wbc_handle {
   MonScratch mon;
   MotorScratch motor;
   EstScratch est;
+  ContactScratch contact;
   ~wbc_handle() { cudaSetDevice(device); }   // the members are released after this, on the handle's device
 };
 
@@ -2000,7 +2025,7 @@ extern "C" int wbc_plant_step_terrain(wbc_handle* h, int64_t n, double dt, const
 // Which plant a host entry runs (params: the rollout with per-robot controller parameters, on any plant; loop: the same with
 // sensing and actuation, on the ground plant; monitor: the loop with the rollout monitor; motor: the monitor entry with the
 // actuator model).
-enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor, motor, estimator };
+enum class PlantEntry { plain, perturbed, terrain, params, loop, monitor, motor, estimator, contact };
 
 // Host buffers of the three plant steps.
 static int plant_step_host(wbc_handle* h, int64_t n, double dt, const wbc_plant_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb,
@@ -2056,11 +2081,14 @@ extern "C" int wbc_plant_step_terrain_host(wbc_handle* h, int64_t n, double dt, 
 // io->status_or; mt != nullptr (ground plant): the motor (wbc_motor.cuh) turns the applied torque into the plant input, with its
 // state in the handle's scratch when mt->tau_m is null, and the monitor sees the motor torque tau_m; ep != nullptr (with a loop):
 // the estimator (wbc_estimator.cuh) replaces the observed base position and linear velocity in place, with its state in the
-// handle's scratch when ep->x is null, and ORs its status bit into the plant's status word.
+// handle's scratch when ep->x is null, and ORs its status bit into the plant's status word; cd != nullptr (ground plant): the
+// contact detector (wbc_contact.cuh) runs after observe and its record step after the plant, with its state in the handle's
+// scratch when cd->q_prev is null; `feed` routes the detected flags to the estimator and / or the controller.
 static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                        const wbc_rollout_opts* opts, const wbcplant::PerturbArgs* pa, const wbcplant::TerrainArgs* ta, cudaStream_t st,
                        const wbc::ParamArgs* cp = nullptr, const wbcloop::LoopArgs* lp = nullptr, const wbcmon::MonArgs* mp = nullptr,
-                       const wbcmotor::MotorArgs* mt = nullptr, const wbcest::EstArgs* ep = nullptr) {
+                       const wbcmotor::MotorArgs* mt = nullptr, const wbcest::EstArgs* ep = nullptr,
+                       const wbccontact::ContactArgs* cd = nullptr, int feed = 0) {
   const bool plant = opts && opts->plant != 0;
   const int use_graph = opts ? opts->use_graph : 1;
   if (kind == WBC_CTRL_PD && !plant) return fail_arg(h, "wbc_rollout: the PD law returns no accelerations to integrate (use the ground plant)");
@@ -2113,6 +2141,18 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
     if (!f_contact) f_contact = h->mon.f.p;
     WBC_CUDA(h, cudaMemsetAsync(plant_status_or, 0, n * sizeof(int32_t), st));
   }
+  wbccontact::ContactArgs ca{};
+  if (cd) {                                        // the record step reads the plant's forces: scratch when nobody asked for them
+    ca = *cd;
+    WBC_CUDA(h, h->contact.reserve(n, !f_contact, !ca.q_prev));
+    if (!f_contact) f_contact = h->contact.f.p;
+    if (!ca.q_prev) {                              // a fresh detector state: count 0 (the first step primes it)
+      ca.q_prev = h->contact.q_prev.p; ca.v_prev = h->contact.v_prev.p; ca.tau_prev = h->contact.tau_prev.p;
+      ca.f_true = h->contact.f_true.p; ca.f_hat = h->contact.f_hat.p; ca.flag = h->contact.flag.p; ca.count = h->contact.count.p;
+      WBC_CUDA(h, cudaMemsetAsync(ca.count, 0, n * sizeof(long long), st));
+    }
+  }
+  const uint8_t* est_contact = (cd && (feed & WBC_CONTACT_FEED_ESTIMATOR)) ? h->contact.detected.p : ro.contact.p;
   WBC_CUDA(h, cudaMemsetAsync(ro.counter.p, 0, sizeof(int), st));
   if (io->status_or) WBC_CUDA(h, cudaMemsetAsync(io->status_or, 0, n * sizeof(int32_t), st));
   if (io->err_max) WBC_CUDA(h, cudaMemsetAsync(io->err_max, 0, n * sizeof(double), st));
@@ -2122,8 +2162,10 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
   }
   // with the ground plant the controller's accelerations are not needed: the step runs without the vd outputs
   // with a loop the controller reads the observed state and the plant applies the actuated torque
-  wbc_io sio{lp ? h->loop.q_obs.p : io->q, lp ? h->loop.v_obs.p : io->v, ro.traj.p, ro.contact.p, tau, metrics, ro.status.p,
-             plant ? nullptr : ro.vd.p, nullptr, nullptr};
+  // with the detector feeding the controller the controller reads plan AND detected
+  uint8_t* ctrl_contact = (cd && (feed & WBC_CONTACT_FEED_CONTROLLER)) ? h->contact.ctrl.p : nullptr;
+  wbc_io sio{lp ? h->loop.q_obs.p : io->q, lp ? h->loop.v_obs.p : io->v, ro.traj.p, ctrl_contact ? ctrl_contact : ro.contact.p, tau, metrics,
+             ro.status.p, plant ? nullptr : ro.vd.p, nullptr, nullptr};
   const double* applied = lp ? h->loop.applied.p : tau;
   const double* plant_tau = mt ? h->motor.plant.p : applied;      // with a motor the plant gets its input, the monitor its torque
   const double* mon_tau = mt ? ma.tau_m : applied;
@@ -2134,9 +2176,15 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       wbcloop::observe_kernel<<<loop_grid, 256, 0, st>>>(la, n, io->q, io->v, h->loop.q_obs.p, h->loop.v_obs.p);
       h->launches++;
     }
+    if (cd) {
+      wbccontact::contact_detect_kernel<<<(unsigned)((n + 3) / 4), wbccontact::CONTACT_BLOCK, 0, st>>>(
+          ca, &h->d_const.p->md, n, lp ? h->loop.q_obs.p : io->q, lp ? h->loop.v_obs.p : io->v, ro.contact.p, h->contact.detected.p,
+          ctrl_contact, plant_status_or);
+      h->launches++;
+    }
     if (ep) {
       wbcest::estimate_kernel<<<(unsigned)((n + 3) / 4), wbcest::EST_BLOCK, 0, st>>>(ea, n, io->q, io->v, h->loop.q_obs.p, h->loop.v_obs.p,
-                                                                                  ro.contact.p, plant_status_or);
+                                                                                  est_contact, plant_status_or);
       h->launches++;
     }
     r = device_step(h, kind, n, &sio, st, false, cp);
@@ -2154,6 +2202,10 @@ static int rollout_run(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n,
       r = plant_launch(h, n, dt, &opts->plant_opts, pa, ta, io->q, io->v, plant_tau, io->t, ro.status.p, plant_status_or, f_contact, metrics,
                        io->err_max, io->metrics_log, ro.counter.p, st);
       if (r) return r;
+      if (cd) {
+        wbccontact::contact_record_kernel<<<(unsigned)((n * WBC_NU + 255) / 256), 256, 0, st>>>(ca, n, mon_tau, f_contact);
+        h->launches++;
+      }
       if (mp) {
         wbcmon::monitor_kernel<<<loop_grid, 256, 0, st>>>(*mp, n, io->q, io->v, ro.traj.p, ro.contact.p, mon_tau, f_contact, nullptr,
                                                           plant_status_or, io->status_or);
@@ -2629,11 +2681,130 @@ extern "C" int wbc_estimator_step_host(wbc_handle* h, int64_t n, double dt, cons
   return rc ? rc : s.finish(h);
 }
 
-// Host buffers of the eight rollouts.
+// ------------------------------------------------------------------------------ contact detection (wbc_contact.cuh)
+// A set keeps the number of the device its records live on, not its handle: it may be destroyed after the handle.
+struct wbc_contact_set {
+  int device = 0;
+  int32_t n_sets = 0;
+  DevArray<wbc_contact_desc> table;
+  ~wbc_contact_set() { cudaSetDevice(device); }   // the table is freed after this, on the set's device
+};
+
+extern "C" int wbc_contact_set_destroy(wbc_contact_set* s) {
+  delete s;
+  return WBC_OK;
+}
+
+extern "C" int wbc_contact_set_create(wbc_handle* h, int32_t n_sets, const wbc_contact_desc* descs, wbc_contact_set** out) {
+  if (!h) return WBC_ERR_ARG;
+  if (!out || !descs || n_sets < 1) return fail_arg(h, "wbc_contact_set_create: descs and n_sets >= 1 are required");
+  *out = nullptr;
+  for (int32_t k = 0; k < n_sets; ++k)
+    if (const char* why = wbccontact::desc_problem(descs[k])) return fail_arg(h, why);
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  std::unique_ptr<wbc_contact_set> cs(new (std::nothrow) wbc_contact_set());
+  if (!cs) return WBC_ERR_NOMEM;
+  cs->device = h->device;
+  cs->n_sets = n_sets;
+  WBC_CUDA(h, cs->table.reserve((size_t)n_sets));
+  WBC_CUDA(h, cudaMemcpy(cs->table.p, descs, (size_t)n_sets * sizeof(wbc_contact_desc), cudaMemcpyHostToDevice));
+  *out = cs.release();
+  return WBC_OK;
+}
+
+// The kernel arguments of a detector whose arrays are already on the device (the state may be all null).
+static int contact_args(wbc_handle* h, const wbc_contact* c, double dt, wbccontact::ContactArgs* ca) {
+  const int given = (c->q_prev != nullptr) + (c->v_prev != nullptr) + (c->tau_prev != nullptr) + (c->f_true != nullptr) +
+                    (c->f_hat != nullptr) + (c->flag != nullptr) + (c->count != nullptr);
+  if (given != 0 && given != 7)
+    return fail_arg(h, "wbc_contact: q_prev, v_prev, tau_prev, f_true, f_hat, flag and count are given together or not at all");
+  if (c->feed & ~(WBC_CONTACT_FEED_ESTIMATOR | WBC_CONTACT_FEED_CONTROLLER)) return fail_arg(h, "wbc_contact: unknown feed bits");
+  const wbc_contact_set* set = c->set;
+  if (!set) return fail_arg(h, "wbc_contact: a set is required");
+  if (set->device != h->device) return fail_arg(h, "wbc_contact: the set lives on another device than the handle");
+  *ca = wbccontact::ContactArgs{set->table.p, c->index, set->n_sets, c->q_prev, c->v_prev, c->tau_prev, c->f_true, c->f_hat, c->flag,
+                                (long long*)c->count, c->stats, dt};
+  return WBC_OK;
+}
+
+extern "C" int wbc_rollout_contact(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                   const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                   const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                   const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est, const wbc_contact* det,
+                                   void* stream) {
+  if (!det) return wbc_rollout_estimator(h, kind, plan, n, n_steps, dt, io, opts, perturb, terrain, ctrl, loop, mon, motor, est, stream);
+  if (!h) return WBC_ERR_ARG;
+  if (!plan || !io || n < 0 || n_steps < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_rollout_contact: bad arguments");
+  if (!(opts && opts->plant == 1)) return fail_arg(h, "wbc_rollout_contact: the detector watches the ground plant (opts->plant = 1)");
+  if (est && !loop) return fail_arg(h, "wbc_rollout_contact: the estimator needs a loop (its observed state, seed, streams and ticks)");
+  if ((det->feed & WBC_CONTACT_FEED_ESTIMATOR) && !est) return fail_arg(h, "wbc_rollout_contact: FEED_ESTIMATOR needs an estimator");
+  wbc::ParamArgs cp;
+  wbcplant::PerturbArgs pa;
+  wbcplant::TerrainArgs ta;
+  wbcloop::LoopArgs la;
+  wbcmon::MonArgs ma;
+  wbcmotor::MotorArgs mt;
+  wbcest::EstArgs ea;
+  wbccontact::ContactArgs ca;
+  int rc = contact_args(h, det, dt, &ca);
+  if (!rc && est) rc = est_args(h, est, dt, &ea);
+  if (!rc && motor) rc = motor_args(h, motor, dt, &mt);
+  if (!rc && mon) rc = mon_args(h, mon, n, dt, &ma);
+  if (!rc && loop) rc = loop_args(h, loop, &la);
+  if (!rc) rc = ctrl_args(h, ctrl, ctrl ? ctrl->index : nullptr, &cp);
+  if (!rc && (perturb || terrain))
+    rc = perturb_args(h, perturb, perturb ? perturb->variant : nullptr, perturb ? perturb->push : nullptr, io->t != nullptr, &pa);
+  if (!rc && terrain) rc = terrain_args(h, terrain, &ta);
+  return rc ? rc : rollout_run(h, kind, plan, n, n_steps, dt, io, opts, (perturb || terrain) ? &pa : nullptr, terrain ? &ta : nullptr,
+                               (cudaStream_t)stream, &cp, loop ? &la : nullptr, mon ? &ma : nullptr, motor ? &mt : nullptr,
+                               est ? &ea : nullptr, &ca, det->feed);
+}
+
+extern "C" int wbc_contact_step(wbc_handle* h, int64_t n, double dt, const wbc_contact* det, const double* q, const double* v,
+                                const uint8_t* contact, uint8_t* detected, int32_t* status_or, void* stream) {
+  if (!h) return WBC_ERR_ARG;
+  if (!det || n < 0 || !(dt > 0.0)) return fail_arg(h, "wbc_contact_step: det, n >= 0 and dt > 0 are required");
+  if (n > 0 && (!q || !v || !contact || !detected || !det->q_prev))
+    return fail_arg(h, "wbc_contact_step: q, v, contact, detected and the detector state are required");
+  wbccontact::ContactArgs ca;
+  const int rc = contact_args(h, det, dt, &ca);
+  if (rc || n == 0) return rc;
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  wbccontact::contact_detect_kernel<<<(unsigned)((n + 3) / 4), wbccontact::CONTACT_BLOCK, 0, (cudaStream_t)stream>>>(
+      ca, &h->d_const.p->md, n, q, v, contact, detected, nullptr, status_or);
+  h->launches++;
+  WBC_CUDA(h, cudaGetLastError());
+  return WBC_OK;
+}
+
+// Device copies of a host wbc_contact's arrays; the detector state and the statistics are copied in and out.
+static wbc_contact contact_to_device(DevScratch& s, const wbc_contact& c, size_t N) {
+  return wbc_contact{c.set, s.in(c.index, N), c.feed, s.inout(c.q_prev, N * WBC_NQ), s.inout(c.v_prev, N * WBC_NV),
+                     s.inout(c.tau_prev, N * WBC_NU), s.inout(c.f_true, N * 12), s.inout(c.f_hat, N * 12),
+                     s.inout(c.flag, N * WBC_NLEG), s.inout(c.count, N), s.inout(c.stats, N * wbccontact::NSTAT)};
+}
+
+extern "C" int wbc_contact_step_host(wbc_handle* h, int64_t n, double dt, const wbc_contact* det, const double* q, const double* v,
+                                     const uint8_t* contact, uint8_t* detected, int32_t* status_or) {
+  if (!h) return WBC_ERR_ARG;
+  if (!det || n <= 0) return n == 0 && det ? WBC_OK : fail_arg(h, "wbc_contact_step_host: det and n >= 0 are required");
+  WBC_CUDA(h, cudaSetDevice(h->device));
+  DevScratch s(h->lane[0]);
+  const size_t N = (size_t)n;
+  const double* dq = s.in(q, N * WBC_NQ); const double* dv = s.in(v, N * WBC_NV);
+  const uint8_t* dc = s.in(contact, N * WBC_NLEG); uint8_t* ddet = s.out(detected, N * WBC_NLEG); int32_t* dst = s.inout(status_or, N);
+  const wbc_contact dd = contact_to_device(s, *det, N);
+  WBC_SCRATCH_CHECK(h, s);
+  const int rc = wbc_contact_step(h, n, dt, &dd, dq, dv, dc, ddet, dst, s.st);
+  return rc ? rc : s.finish(h);
+}
+
+// Host buffers of the nine rollouts.
 static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt, const wbc_rollout_io* io,
                         const wbc_rollout_opts* opts, PlantEntry entry, const wbc_plant_perturb* perturb, const wbc_plant_terrain* terrain,
                         const wbc_ctrl_params* ctrl = nullptr, const wbc_loop* loop = nullptr, const wbc_monitor* mon = nullptr,
-                        const wbc_plant_motor* motor = nullptr, const wbc_estimator* est = nullptr) {
+                        const wbc_plant_motor* motor = nullptr, const wbc_estimator* est = nullptr,
+                        const wbc_contact* det = nullptr) {
   if (!h) return WBC_ERR_ARG;
   if (!plan || !io || n < 0 || n_steps < 0) return fail_arg(h, "wbc_rollout_host: bad arguments");
   if (n == 0) return WBC_OK;
@@ -2663,9 +2834,15 @@ static int rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n
   if (motor) dmt = motor_to_device(s, *motor, N);
   wbc_estimator de{};
   if (est) de = est_to_device(s, *est, N);
+  wbc_contact dd{};
+  if (det) dd = contact_to_device(s, *det, N);
   WBC_SCRATCH_CHECK(h, s);
   const int rc =
-      entry == PlantEntry::estimator
+      entry == PlantEntry::contact
+          ? wbc_rollout_contact(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, terrain ? &dtr : nullptr,
+                                ctrl ? &dcp : nullptr, loop ? &dl : nullptr, mon ? &dm : nullptr, motor ? &dmt : nullptr,
+                                est ? &de : nullptr, det ? &dd : nullptr, s.st)
+      : entry == PlantEntry::estimator
           ? wbc_rollout_estimator(h, kind, plan, n, n_steps, dt, &d, opts ? &o : nullptr, perturb ? &dp : nullptr, terrain ? &dtr : nullptr,
                                   ctrl ? &dcp : nullptr, loop ? &dl : nullptr, mon ? &dm : nullptr, motor ? &dmt : nullptr,
                                   est ? &de : nullptr, s.st)
@@ -2733,6 +2910,14 @@ extern "C" int wbc_rollout_estimator_host(wbc_handle* h, int kind, const wbc_pla
                                           const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
                                           const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est) {
   return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::estimator, perturb, terrain, ctrl, loop, mon, motor, est);
+}
+
+extern "C" int wbc_rollout_contact_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,
+                                        const wbc_rollout_io* io, const wbc_rollout_opts* opts, const wbc_plant_perturb* perturb,
+                                        const wbc_plant_terrain* terrain, const wbc_ctrl_params* ctrl, const wbc_loop* loop,
+                                        const wbc_monitor* mon, const wbc_plant_motor* motor, const wbc_estimator* est,
+                                        const wbc_contact* det) {
+  return rollout_host(h, kind, plan, n, n_steps, dt, io, opts, PlantEntry::contact, perturb, terrain, ctrl, loop, mon, motor, est, det);
 }
 
 extern "C" int wbc_rollout_host(wbc_handle* h, int kind, const wbc_plan* plan, int64_t n, int32_t n_steps, double dt,

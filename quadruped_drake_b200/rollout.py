@@ -40,6 +40,13 @@ velocity of a linear Kalman filter that fuses a synthesised accelerometer with l
 (semantics in include/wbc.h, wbc_estimator). An `EstimatorSet` holds the records (`estimator_desc`), an `EstimatorState` the
 per-robot filter. It runs through `wbc_rollout_estimator`, together with any motor, monitor, variants, pushes, terrain and
 parameter sets; `estimator_step` runs the filter alone.
+
+Contact detection (`contact`, a `ContactDetector`; ground plant only): each robot's foot forces are estimated from the joint
+torques and the motion they produced, and a hysteresis on their vertical component gives stance flags (semantics in
+include/wbc.h, wbc_contact). `feed` routes the detected flags to the estimator and / or the controller (plan AND detected);
+feed = 0 only observes. A `ContactSet` holds the records (`contact_desc`), a `ContactState` the per-robot detector and its
+statistics. It runs through `wbc_rollout_contact`, together with any estimator, motor, monitor, loop, variants, pushes, terrain
+and parameter sets; `contact_step` runs the detector alone.
 """
 from __future__ import annotations
 
@@ -49,8 +56,8 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import capi
-from .capi import (KINDS, LOOP_HIST, MON_NSTAT, WbcCtrlParams, WbcEstimator, WbcEstimatorDesc, WbcLoop, WbcMonitor, WbcMotorDesc,
-                   WbcPlantMotor, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
+from .capi import (CONTACT_FEED_ESTIMATOR, CONTACT_NSTAT, KINDS, LOOP_HIST, MON_NSTAT, WbcContact, WbcContactDesc, WbcCtrlParams,
+                   WbcEstimator, WbcEstimatorDesc, WbcLoop, WbcMonitor, WbcMotorDesc, WbcPlantMotor, WbcPlantOpts, WbcPlantPerturb, WbcPlantTerrain, WbcRolloutIO, WbcRolloutOpts, WbcTerrainDesc, np_ptr)
 from .controller import check_device_index
 from .model import NQ, NU, NV, RobotModel, WbcModelStruct
 
@@ -183,7 +190,7 @@ def check_device_array(x, shape, dtype, what):
     """A per-robot array on the device must be a contiguous CUDA tensor of the ABI's dtype and shape: the kernels read it through
     its device pointer."""
     import torch
-    dt = {np.float64: torch.float64, np.int32: torch.int32, np.int64: torch.int64}[dtype]
+    dt = {np.float64: torch.float64, np.int32: torch.int32, np.int64: torch.int64, np.uint8: torch.uint8}[dtype]
     if not (_is_torch(x) and x.is_cuda and x.is_contiguous() and x.dtype == dt and tuple(x.shape) == tuple(shape)):
         raise ValueError(f"{what} on the device must be a contiguous CUDA tensor {np.dtype(dtype).name}{list(shape)}")
 
@@ -574,8 +581,149 @@ def estimator_step(ctl, q, v, q_obs, v_obs, contact, estimator, loop=None, dt=5e
     return qo, vo, status
 
 
+# Untuned: a 10 ms force filter, and thresholds of about a quarter and a tenth of a mini_cheetah foot's standing load (~22 N).
+CONTACT_DEFAULTS = dict(tau_f=0.01, f_on=6.0, f_off=2.0)
+
+
+def contact_desc(**kw):
+    """One detector record (WbcContactDesc): CONTACT_DEFAULTS with the given fields replaced. tau_f (s) the low-pass time constant
+    of the force estimate (0: raw); a foot becomes stance when the filtered vertical force reaches f_on (N) and swing when it falls
+    to f_off <= f_on (N); f_off = -inf never releases a detected foot."""
+    vals = dict(CONTACT_DEFAULTS)
+    for k, x in kw.items():
+        if k not in vals:
+            raise TypeError(f"contact_desc: unknown field {k!r}")
+        vals[k] = float(x)
+    return WbcContactDesc(**vals)
+
+
+class ContactSet:
+    """Device-resident table of K detector records (wbc_contact_set_create); robot i's detector uses descs[index[i]]."""
+
+    def __init__(self, ctl, descs):
+        self.ctl, self.lib = ctl, ctl.lib
+        self.n_sets = len(descs)
+        arr = (WbcContactDesc * self.n_sets)(*descs)
+        self._p = C.c_void_p()
+        self.ctl._check(self.lib.wbc_contact_set_create(ctl._h, self.n_sets, arr, C.byref(self._p)), "wbc_contact_set_create")
+
+    def close(self):
+        if getattr(self, "_p", None):
+            self.lib.wbc_contact_set_destroy(self._p)
+            self._p = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+_CONTACT_FIELDS = (("q_prev", np.float64, (NQ,)), ("v_prev", np.float64, (NV,)), ("tau_prev", np.float64, (NU,)),
+                   ("f_true", np.float64, (12,)), ("f_hat", np.float64, (12,)), ("flag", np.uint8, (4,)), ("count", np.int64, ()),
+                   ("stats", np.float64, (CONTACT_NSTAT,)))
+
+
+class ContactState:
+    """The detector state of N robots: q_prev [N,19], v_prev [N,18] (what it read at the previous step), tau_prev [N,12] (the
+    measured torque of the latest step), f_true [N,12] (the plant's forces of the latest step), f_hat [N,12] (filtered force
+    estimate, world axes, foot k at 3k), flag [N,4] uint8, count [N] int64 (0: the next step primes it) and stats [N,6] (sum
+    |f err|^2, max |f err|, true stance, true swing, false stance, false swing; per foot and step); all zero. NumPy arrays, or
+    torch tensors on the device of `like`. A rollout given a state continues it and leaves it advanced."""
+
+    def __init__(self, n, like=None):
+        for name, dtype, width in _CONTACT_FIELDS:
+            if like is not None and _is_torch(like):
+                import torch
+                tdt = {np.float64: torch.float64, np.int64: torch.int64, np.uint8: torch.uint8}[dtype]
+                x = torch.zeros((n, *width), dtype=tdt, device=like.device)
+            else:
+                x = np.zeros((n, *width), dtype)
+            setattr(self, name, x)
+
+    # per robot: RMS force error over its estimated foot-steps, and the confusion counts (foot-steps)
+    rms_force = property(lambda s: (s.stats[:, 0] / (s.stats[:, 2:6].sum(axis=1))) ** 0.5)
+    max_force = property(lambda s: s.stats[:, 1])
+    true_stance = property(lambda s: s.stats[:, 2])
+    true_swing = property(lambda s: s.stats[:, 3])
+    false_stance = property(lambda s: s.stats[:, 4])
+    false_swing = property(lambda s: s.stats[:, 5])
+
+
+@dataclass
+class ContactDetector:
+    """Per-robot contact detection of the ground-plant loop. set: a ContactSet (required); index [N] int32 record of each robot
+    (None: record 0); feed: a mask of CONTACT_FEED_ESTIMATOR (the estimator's stance legs) and CONTACT_FEED_CONTROLLER (the
+    controller's contacts, plan AND detected), 0: observe only; state: a ContactState to continue (None: each call primes a fresh
+    detector in library scratch, and keeps no statistics)."""
+    set: ContactSet
+    index: object = None
+    feed: int = 0
+    state: ContactState | None = None
+
+
+def _contact_arrays(det, n, dev=None):
+    """(index, state) of a ContactDetector in the layouts of the C ABI, checked: the index broadcast to N rows (a host copy, or on
+    `dev` a torch tensor checked, not converted), the state as given."""
+    if not isinstance(det.set, ContactSet):
+        raise ValueError("contact.set must be a ContactSet")
+    st = det.state
+    if dev is not None:
+        check_device_index(det.index, n, "contact.index")
+        if st is not None:
+            for name, dtype, width in _CONTACT_FIELDS:
+                check_device_array(getattr(st, name), (n, *width), dtype, f"contact.state.{name}")
+        return det.index, st
+    if st is not None:
+        for name, dtype, width in _CONTACT_FIELDS:
+            x = getattr(st, name)
+            if not (isinstance(x, np.ndarray) and x.dtype == dtype and x.shape == (n, *width) and x.flags.c_contiguous):
+                raise ValueError(f"contact.state.{name} must be a contiguous host array {np.dtype(dtype).name}{[n, *width]}")
+    return _terrain_index(n, det.index), st
+
+
+def _wbc_contact(det, idx, st, ptr):
+    s = (None,) * 8 if st is None else tuple(ptr(getattr(st, name)) for name, _, _ in _CONTACT_FIELDS)
+    return WbcContact(det.set._p, ptr(idx), int(det.feed), *s)
+
+
+def contact_step(ctl, q, v, contact, detector, dt=5e-3):
+    """The detector alone on one step (wbc_contact_step) -> (detected [N,4] uint8, status_or [N] int32: ST_BADCONTACT for a bad
+    index or a non-finite estimate). q [N,19], v [N,18] the state it reads; contact [N,4] uint8 the plan's flags. detector.state
+    is required and advanced; its tau_prev and f_true are the torque and forces of the step that led to q, v. Host arrays go
+    through the host entry; torch CUDA tensors stay on the device."""
+    if detector.state is None:
+        raise ValueError("contact_step: detector.state is required (a ContactState)")
+    if _is_torch(q):
+        import torch
+        n, dev = q.shape[0], q.device
+        check_device_array(q, (n, NQ), np.float64, "q")
+        check_device_array(v, (n, NV), np.float64, "v")
+        check_device_array(contact, (n, 4), np.uint8, "contact")
+        idx, st = _contact_arrays(detector, n, dev)
+        p = lambda x: None if x is None else C.c_void_p(x.data_ptr())  # noqa: E731
+        detected = torch.zeros((n, 4), dtype=torch.uint8, device=dev)
+        status = torch.zeros(n, dtype=torch.int32, device=dev)
+        cd = _wbc_contact(detector, idx, st, p)
+        ctl._check(ctl.lib.wbc_contact_step(ctl._h, n, float(dt), C.byref(cd), p(q), p(v), p(contact), p(detected), p(status),
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), "wbc_contact_step")
+        return detected, status
+    q = np.ascontiguousarray(q, dtype=np.float64).reshape(-1, NQ)
+    n = len(q)
+    v = np.ascontiguousarray(v, dtype=np.float64).reshape(n, NV)
+    ct = np.ascontiguousarray(contact, dtype=np.uint8).reshape(n, 4)
+    idx, st = _contact_arrays(detector, n)
+    opt = lambda a: None if a is None else np_ptr(a)  # noqa: E731
+    detected, status = np.zeros((n, 4), np.uint8), np.zeros(n, np.int32)
+    cd = _wbc_contact(detector, idx, st, opt)
+    ctl._check(ctl.lib.wbc_contact_step_host(ctl._h, n, float(dt), C.byref(cd), np_ptr(q), np_ptr(v), np_ptr(ct), np_ptr(detected),
+                                             np_ptr(status)), "wbc_contact_step_host")
+    return detected, status
+
+
 class RolloutResult:
-    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why", "estimator")
+    __slots__ = ("q", "v", "t", "tau", "metrics", "status_or", "err_max", "metrics_log", "f_contact", "monitor", "why", "estimator",
+                 "contact")
 
     def __init__(self, **kw):
         for k in self.__slots__:
@@ -588,7 +736,7 @@ def _opts(use_graph, plant, mu, erp, iters, f_ptr=None):
 
 def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_metrics=False, use_graph=True, plant=False,
             mu=1.0, erp=0.2, iters=30, plant_set=None, variant=None, push=None, terrain_set=None, terrain=None, param_set=None,
-            param_index=None, loop=None, monitor=None, motor=None, estimator=None) -> RolloutResult:
+            param_index=None, loop=None, monitor=None, motor=None, estimator=None, contact=None) -> RolloutResult:
     """Advance N robots by n_steps control periods of length dt (simulate.py:20-21: dt = 5e-3, 6 s = 1200 steps).
     NumPy inputs are copied (host entry); torch CUDA tensors are updated IN PLACE on torch's current stream.
     plant=True: ground-contact simulation driven by the torques (mu: ground friction, simulate.py:44-46); the result then
@@ -609,9 +757,17 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     and gets zero torque.
     State estimation (plant=True and a loop only): estimator (an Estimator) gives each robot's controller the filter's base
     position and linear velocity; the result then carries `estimator` (its EstimatorState, advanced, or None). A robot with a bad
-    record index or a failed filter step is controlled from the observed state and flagged ST_BADESTIM."""
+    record index or a failed filter step is controlled from the observed state and flagged ST_BADESTIM.
+    Contact detection (plant=True only): contact (a ContactDetector) estimates each robot's foot forces and stance flags and feeds
+    them to the estimator and / or the controller as its `feed` asks; the result then carries `contact` (its ContactState,
+    advanced, or None). A robot with a bad record index or a non-finite estimate uses the plan's flags and is flagged
+    ST_BADCONTACT."""
     if estimator is not None and (loop is None or not plant):
         raise ValueError("rollout: an estimator needs loop= (its observed state, seed, streams and ticks) and plant=True")
+    if contact is not None and not plant:
+        raise ValueError("rollout: the contact detector watches the ground plant (plant=True)")
+    if contact is not None and (int(contact.feed) & CONTACT_FEED_ESTIMATOR) and estimator is None:
+        raise ValueError("rollout: contact feed CONTACT_FEED_ESTIMATOR needs an estimator")
     on_terrain = terrain_set is not None or terrain is not None
     perturbed = plant_set is not None or variant is not None or push is not None
     per_robot = param_set is not None or param_index is not None
@@ -626,8 +782,9 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         io = WbcRolloutIO(p(q), p(v), p(t), p(plan_index), p(r.tau), p(r.metrics), p(r.status_or), p(r.err_max), p(r.metrics_log))
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         o = _opts(use_graph, plant, mu, erp, iters, p(r.f_contact))
-        if monitor is not None or motor is not None or estimator is not None:
+        if monitor is not None or motor is not None or estimator is not None or contact is not None:
             ea = None if estimator is None else _estimator_arrays(estimator, n, dev)
+            ca = None if contact is None else _contact_arrays(contact, n, dev)
             if monitor is not None:
                 r.monitor, r.why = _monitor_state(monitor, n, q), mk((n,), torch.int32)
             arrays = None if loop is None else _loop_arrays(loop, n, dev)      # (kept alive for the call)
@@ -637,7 +794,15 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
             cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, p(param_index))) if per_robot else None
             lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, p))
             mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, p))
-            if estimator is not None:
+            if contact is not None:
+                mt = None if motor is None else C.byref(_wbc_motor(motor, *_motor_arrays(motor, n, dev), p))
+                es = None if estimator is None else C.byref(_wbc_estimator(estimator, *ea, p))
+                r.estimator = None if estimator is None else estimator.state
+                cd = C.byref(_wbc_contact(contact, *ca, p))
+                r.contact = contact.state
+                ctl._check(ctl.lib.wbc_rollout_contact(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt,
+                                                       tr, cp, lp, mo, mt, es, cd, stream), "wbc_rollout_contact")
+            elif estimator is not None:
                 mt = None if motor is None else C.byref(_wbc_motor(motor, *_motor_arrays(motor, n, dev), p))
                 es = C.byref(_wbc_estimator(estimator, *ea, p))
                 r.estimator = estimator.state
@@ -688,8 +853,9 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
     io = WbcRolloutIO(np_ptr(q), np_ptr(v), np_ptr(t), opt(pi), np_ptr(r.tau), np_ptr(r.metrics), np_ptr(r.status_or), np_ptr(r.err_max),
                       opt(r.metrics_log))
     o = _opts(use_graph, plant, mu, erp, iters, opt(r.f_contact))
-    if monitor is not None or motor is not None or estimator is not None:
+    if monitor is not None or motor is not None or estimator is not None or contact is not None:
         ea = None if estimator is None else _estimator_arrays(estimator, n)      # (kept alive for the call)
+        ca = None if contact is None else _contact_arrays(contact, n)
         if monitor is not None:
             r.monitor, r.why = _monitor_state(monitor, n), np.zeros(n, np.int32)
         vi, pu = _perturb_arrays(n, variant, push)      # (kept alive for the call)
@@ -700,7 +866,16 @@ def rollout(ctl, sampler, kind, q, v, t, n_steps, dt=5e-3, plan_index=None, log_
         cp = C.byref(WbcCtrlParams(None if param_set is None else param_set._p, opt(ci))) if per_robot else None
         lp = None if loop is None else C.byref(_wbc_loop(loop, arrays, opt))
         mo = None if monitor is None else C.byref(_wbc_monitor(monitor, r.monitor, r.why, opt))
-        if estimator is not None:
+        if contact is not None:
+            mi, ms = (None, None) if motor is None else _motor_arrays(motor, n)      # (kept alive for the call)
+            mt = None if motor is None else C.byref(_wbc_motor(motor, mi, ms, opt))
+            es = None if estimator is None else C.byref(_wbc_estimator(estimator, *ea, opt))
+            r.estimator = None if estimator is None else estimator.state
+            cd = C.byref(_wbc_contact(contact, *ca, opt))
+            r.contact = contact.state
+            ctl._check(ctl.lib.wbc_rollout_contact_host(ctl._h, k, sampler._p, n, int(n_steps), float(dt), C.byref(io), C.byref(o), pt,
+                                                        tr, cp, lp, mo, mt, es, cd), "wbc_rollout_contact_host")
+        elif estimator is not None:
             mi, ms = (None, None) if motor is None else _motor_arrays(motor, n)      # (kept alive for the call)
             mt = None if motor is None else C.byref(_wbc_motor(motor, mi, ms, opt))
             es = C.byref(_wbc_estimator(estimator, *ea, opt))
